@@ -380,8 +380,34 @@ class Rig:
         return total_ms, wall
 
 
-def run_workload(rig, workload, steps, warmup, with_pipelined=True):
-    """One workload on the rig's GPUs: returns the fields of its bench record (rank 0; None elsewhere)."""
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, ds, trackers):
+    """What a caller of the timed path holds after its last step, as float32 .npy files in `out_dir`:
+    downsampled_cloud (N x 7: x, y, z and the r, g, b, a bytes of rgba), result (one pose per tracker) and
+    particles (every tracker's particles, tracker after tracker); poses and particles carry the fields of
+    pcl.PARTICLE in order (x, y, z, one, roll, pitch, yaw, weight)."""
+    from numpy.lib import recfunctions as rfn
+    from pcl_tracking_b200 import pcl
+    pts = ds.to_numpy()
+    argb = np.ascontiguousarray(pts["rgba"]).view(np.uint8).reshape(-1, 4)  # little-endian bytes of a<<24 | r<<16 | g<<8 | b
+    arrays = {
+        "downsampled_cloud": np.column_stack([pts["x"], pts["y"], pts["z"], argb[:, [2, 1, 0, 3]].astype(np.float32)]),
+        "result": rfn.structured_to_unstructured(np.array([t.getResult() for t in trackers], dtype=pcl.PARTICLE)),
+        "particles": rfn.structured_to_unstructured(np.concatenate([t.getParticles() for t in trackers])),
+    }
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
+def run_workload(rig, workload, steps, warmup, with_pipelined=True, dump_dir=None):
+    """One workload on the rig's GPUs: returns the fields of its bench record (rank 0; None elsewhere).  With `dump_dir`,
+    rank 0 writes the outputs of the last timed step there (dump_outputs)."""
     from pcl_tracking_b200 import pcl, synth
     args, ctx, world, rank, dist = rig.args, rig.ctx, rig.world, rig.rank, rig.dist
     sensor = "qhd" if workload == "qhd" else "sd"
@@ -533,6 +559,8 @@ def run_workload(rig, workload, steps, warmup, with_pipelined=True):
     total_ms, wall_s = rig.timed(step_resident, steps, W, sampler)
     evals_timed = eval_count() - evals0
     launches = pcl.kernel_launch_count() - launches0
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, ds, trackers)  # before the e2e passes below track further frames
     ms_per_step = total_ms / steps
     evals_per_step = float(evals_timed) / steps
     value = evals_per_step / (ms_per_step * 1e-3)
@@ -663,8 +691,12 @@ def workload_config(args, workload, M, n_particles, n_pts=217088, scene_mode="re
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=300)
+    ap.add_argument("--steps", type=int, default=300, help="timed steps of the headline workload and of each e2e variant (the --also workloads "
+                                                           "time min(steps, 60), c4 min(steps, 30), at least 3)")
     ap.add_argument("--warmup", type=int, default=10)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of the headline workload, write what its last step computed to DIR/*.npy (float32): "
+                         "downsampled_cloud, result, particles; the inputs are seeded, so runs with the same arguments compare output for output")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="c2", choices=["c1", "c2", "c3", "c4", "c5", "qhd"])
     ap.add_argument("--also", default=None, help="comma-separated extra workloads reported under `workloads` of the same line "
@@ -685,7 +717,11 @@ def main():
                          "with --exchange peer); 'broadcast' = the same with ncclBroadcast (default with --exchange nccl); 'replicate' = "
                          "every rank uploads and downsamples the frame itself")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
         return reference_arm(args)
     if args.workload == "c1":
         print("bench.py: c1 is the CPU configuration (BASELINE configs[0]): use --impl reference --workload c1", file=sys.stderr)
@@ -725,7 +761,7 @@ def main():
         print("bench.py: the %s workload runs on one GPU" % args.workload, file=sys.stderr)
         return 2
 
-    head = run_workload(rig, args.workload, args.steps, args.warmup)
+    head = run_workload(rig, args.workload, args.steps, args.warmup, dump_dir=args.dump_outputs)
     line = None
     if rank == 0:
         line = {"metric": METRIC, "value": head["value"], "unit": UNIT, "n_gpus": world * (len(args.devices.split(",")) if args.devices else 1), "steps": args.steps, "warmup": head["warmup"],

@@ -1,6 +1,7 @@
 """The drop-in claim of the boundary, checked on the reference's own text: `initialize_trackers()` (ref:
 src/auto_tracking.cpp:181-259), the class typedefs it relies on (ref :139-156) and the scene filters
-(ref :536-575) are read from /root/reference AT TEST TIME (nothing of them is committed here) and compiled
+(ref :536-575) are read AT TEST TIME from the checkout of cmaestre/pcl_tracking that PCL_TRACKING_REFERENCE names
+(nothing of them is committed here; without it the test skips) and compiled
 verbatim against include/pft/pcl_shim.hpp, with boost::shared_ptr and Eigen::Affine3f as the reference spells
 them.  Boost and Eigen are not installed in this image: two tiny stand-in headers written by the test provide
 `boost::shared_ptr` (= std::shared_ptr) and an `Eigen::Affine3f` with Identity(), operator()(r, c) and
@@ -11,7 +12,7 @@ import subprocess
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/src/auto_tracking.cpp"
+REF = os.path.join(os.environ.get("PCL_TRACKING_REFERENCE", ""), "src", "auto_tracking.cpp")
 
 STANDIN_BOOST = """#pragma once
 #include <memory>
@@ -39,7 +40,8 @@ def ref_lines(first, last):
     return "".join(lines[first - 1:last])
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="the reference tree is only present in the build container")
+@pytest.mark.skipif(not os.environ.get("PCL_TRACKING_REFERENCE") or not os.path.exists(REF),
+                    reason="needs the reference's src/auto_tracking.cpp: set PCL_TRACKING_REFERENCE to a checkout of cmaestre/pcl_tracking")
 def test_reference_initialize_trackers_and_filters_compile_verbatim(tmp_path):
     inc = tmp_path / "standins"
     (inc / "boost").mkdir(parents=True)
