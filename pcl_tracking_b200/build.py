@@ -38,15 +38,6 @@ def build(force=False, verbose=False):
     return LIB_PATH
 
 
-def build_variant(threads, extra=(), name=None):
-    """Kernel-tuning build: weight kernel with `threads` per CTA (plus extra -D flags)."""
-    os.makedirs(LIB_DIR, exist_ok=True)
-    out = os.path.join(LIB_DIR, name or "libpft_t%d.so" % threads)
-    cmd = [NVCC] + FLAGS + ["-DPFT_WEIGHT_THREADS=%d" % threads] + list(extra) + ["-o", out] + SOURCES + ["-ldl"]
-    subprocess.check_call(cmd, cwd=CSRC)
-    return out
-
-
 if __name__ == "__main__":
     import sys
     print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))

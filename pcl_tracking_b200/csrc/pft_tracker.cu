@@ -23,9 +23,6 @@
 #include <vector>
 
 #include "pft_internal.h"
-#ifndef PFT_WEIGHT_THREADS
-#define PFT_WEIGHT_THREADS 1024
-#endif
 #include "pft_tracker_kernels.cuh"
 
 using namespace pft;
@@ -122,14 +119,12 @@ struct pft_tracker {
   int max_cells = 1 << 20;  // cap of the index grid; a larger crop box gets coarser cells
   int list_mode = 1;             // PFT_CANDIDATE_LISTS
   int list_max_cells = 1 << 19;  // fine cells the candidate lists are sized for (kListK x 2 B each); 0 disables the lists
-  int index_level = -1;     // cell edge of the index = search resolution x 2^level (internal; results do not depend on it);
-                            // -1: chosen per weight() from the nearest-neighbour distances of the previous one
   int cur = 0;          // live particle buffer
   int inj_slots = 0, inj_stride = 0;
   int draw_cap = 0;
   bool timing = false;
   float t_weight_ms = 0.f, t_compute_ms = 0.f;
-  std::vector<cudaEvent_t> ev_w;  // pairs around weight_kernel launches of the last compute
+  std::vector<cudaEvent_t> ev_w;  // pairs around the lookup launches of the last compute
   cudaEvent_t ev_c0 = nullptr, ev_c1 = nullptr;
   int n_ev_used = 0;
   // timing mode: one event after every kernel of the last compute(), for the per-kernel breakdown
@@ -166,8 +161,7 @@ struct pft_tracker {
   bool use_cd = false;
   int cd_interval = 10, cd_filter = 10, change_counter = 0, cd_tests = 0, cd_last_found = -1, cd_node_cap = 0, cd_resets = 0;
   double cd_res = 0.01;
-  int weight_smem = 0;  // dynamic shared memory of the weight kernel (bytes)
-  int lists_smem = 0;   // ... of weight_lists_kernel
+  int lists_smem = 0;   // dynamic shared memory of weight_lists_kernel (bytes)
   int tbl_size = 0;
   int n_slots = 0;
   int chunks = 1, chunk_len = 0;
@@ -250,19 +244,26 @@ double kl_bound(int k, double delta, double eps) {
 
 constexpr long long kMarkCountMaxQueries = 16ll << 20;  // up to this many (particle, model point) pairs cand_mark_kernel counts the queries of every cell
 constexpr int kClusterMinParticles = 4096;  // above this capacity the O(N) replicated stages run as a cluster of kClusterCtas CTAs
-constexpr int kWeightThreads = PFT_WEIGHT_THREADS;  // CTA size of the persistent weight kernel (one CTA per SM), large particle sets
-constexpr int kWeightThreadsSmall = 768;            // small sets (static item split): 85 registers per thread instead of 64 (measured -6 %)
-#ifndef PFT_LIST_THREADS
-#define PFT_LIST_THREADS 640
-#endif
-#ifndef PFT_LIST_THREADS_BIG
-#define PFT_LIST_THREADS_BIG 896
-#endif
 // CTA size of weight_lists_kernel (one CTA per SM): 96 registers per thread, no spills; large query sets (measured on 100 000
 // particles: -4 %) trade 72 registers and a few spilled values for 28 warps per SM
-constexpr int kListThreads = PFT_LIST_THREADS;
-constexpr int kListThreadsBig = PFT_LIST_THREADS_BIG;
+constexpr int kListThreads = 640;
+constexpr int kListThreadsBig = 896;
 constexpr long long kListBigQueries = 48ll << 20;   // (particle, model point) pairs per weight() from which the large variant runs
+constexpr long long kDynItemsPerWarp = 5;           // items per warp from which they are handed out dynamically (measured: 10k-25k particles -7 %)
+// choose_chunks: model chunks per particle for ~kItemsPerWarp items per warp of kChunkWarpsPerSm warps per SM (the
+// chunking fixes the order of the fp64 sums of a weight)
+constexpr int kItemsPerWarp = 6;
+constexpr int kChunkWarpsPerSm = 24;
+constexpr float kIndexDilate = 0.03f;  // margin (m) of the index around the crop box when the lists are on and a compute() has further weight() calls
+constexpr int kListRatio = 2;          // the lists are built when this rank's queries outnumber the fine cells of the crop box by this factor
+
+// The O(N) replicated stages (cdf_kernel, normalize_kernel, update_kernel) run as one CTA, above kClusterMinParticles
+// as one cluster of kClusterCtas CTAs
+template <typename... P, typename... A>
+void launch_replicated(const pft_tracker* t, void (*one)(P...), void (*cluster)(P...), A... args) {
+  if (t->n_cap > kClusterMinParticles) cluster<<<kClusterCtas, 1024, 0, t->run_stream()>>>(args...);
+  else one<<<1, 1024, 0, t->run_stream()>>>(args...);
+}
 
 // Row table of the nearest-neighbour search: the (dy,dz) offsets within kRT cells sorted by the lower bound
 // gap(dy)^2 + gap(dz)^2 of their distance (gap(d) = max(|d|-1, 0)), nearer rows first.
@@ -286,15 +287,6 @@ int upload_row_table(pft_tracker* t) {
   int dev = t->ctx->device, max_optin = 0;
   PFT_CUDA_TRY(cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
   cudaFuncAttributes fa;
-  PFT_CUDA_TRY(cudaFuncGetAttributes(&fa, weight_kernel<true, kWeightThreads, true>));
-  int dyn = max_optin - (int)fa.sharedSizeBytes - 1024;
-  if (dyn < 0) dyn = 0;
-  dyn &= ~15;
-  PFT_CUDA_TRY(cudaFuncSetAttribute(weight_kernel<true, kWeightThreads, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
-  PFT_CUDA_TRY(cudaFuncSetAttribute(weight_kernel<true, kWeightThreadsSmall, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
-  PFT_CUDA_TRY(cudaFuncSetAttribute(weight_kernel<false, kWeightThreads, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
-  PFT_CUDA_TRY(cudaFuncSetAttribute(weight_kernel<false, kWeightThreadsSmall, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
-  t->weight_smem = dyn;
   PFT_CUDA_TRY(cudaFuncGetAttributes(&fa, weight_lists_kernel<true, kListThreads, true>));
   int dyn_l = (max_optin - (int)fa.sharedSizeBytes - 1024) & ~15;
   if (dyn_l < 0) dyn_l = 0;
@@ -421,6 +413,16 @@ int ensure_draw_buffers(pft_tracker* t, int slots, int stride) {
   return PFT_OK;
 }
 
+// Buffers of `count` generated draws (slot 0).
+int reserve_generated_draws(pft_tracker* t, int count) {
+  if (t->draw_cap >= count) return PFT_OK;
+  int rc = ensure_draw_buffers(t, 1, count);
+  if (rc) return rc;
+  t->draw_cap = count;
+  invalidate_graph(t);
+  return PFT_OK;
+}
+
 // Draw arrays of one resample slot: injected (slot-indexed) or generated on the device into slot 0.
 int prepare_draws(pft_tracker* t, int slot, int count, const float** usel, const float** normals, const float** umot) {
   cudaStream_t s = t->run_stream();
@@ -434,12 +436,8 @@ int prepare_draws(pft_tracker* t, int slot, int count, const float** usel, const
     *umot = t->d_umot.as<float>() + (size_t)slot * t->inj_stride;
     return PFT_OK;
   }
-  if (t->draw_cap < count) {
-    int rc = ensure_draw_buffers(t, 1, count);
-    if (rc) return rc;
-    t->draw_cap = count;
-    invalidate_graph(t);
-  }
+  int rc = reserve_generated_draws(t, count);
+  if (rc) return rc;
   draws_kernel<<<blocks_for(count, 256, t->ctx->sm_count * 4), 256, 0, s>>>(t->st.as<TrackerState>(), t->d_usel.as<float>(), t->d_normals.as<float>(),
                                                                         t->d_umot.as<float>(), count, t->seed);
   PFT_LAUNCH_CHECK();
@@ -465,9 +463,8 @@ int ensure_index_buffers(pft_tracker* t) {
 // warp of the persistent grid keeps the tail short; a chunk is a multiple of 32 points (one per lane).
 void choose_chunks(pft_tracker* t) {
   const int n_expected = std::max(1, (t->particle_num > 0 ? t->particle_num : t->n_cap) / t->nranks);
-  const int total_warps = t->ctx->sm_count * (kWeightThreadsSmall / 32);  // (chunking only matters for small sets: the static split)
-  static const int per_warp = [] { const char* e = getenv("PFT_ITEMS_PER_WARP"); const int v = e ? atoi(e) : 0; return v > 0 ? v : 6; }();  // tuning knob
-  const int target_items = total_warps * per_warp;
+  const int total_warps = t->ctx->sm_count * kChunkWarpsPerSm;  // (chunking only matters for small sets: the static split)
+  const int target_items = total_warps * kItemsPerWarp;
   const int max_chunks = std::max(1, (t->M + 63) / 64);
   int chunks = (target_items + n_expected - 1) / n_expected;
   chunks = std::min(std::max(chunks, 1), std::min(max_chunks, 256));
@@ -521,10 +518,8 @@ int stage_resample(pft_tracker* t, int slot) {
   TrackerState* st = t->st.as<TrackerState>();
   const DevParticle* old_parts = t->parts[t->cur].as<DevParticle>();
   DevParticle* new_parts = t->parts[t->cur ^ 1].as<DevParticle>();
-  if (t->n_cap > kClusterMinParticles) cdf_kernel<kClusterCtas><<<kClusterCtas, 1024, 0, s>>>(st, old_parts, t->cdf.as<unsigned long long>(), t->cdf_total.as<unsigned long long>(), t->tbl_rep.as<int>(),
-                                t->tbl_min.as<int>(), t->kld ? t->tbl_size : 0, t->kld ? 0 : t->particle_num, t->input->d_hdr());
-  else cdf_kernel<1><<<1, 1024, 0, s>>>(st, old_parts, t->cdf.as<unsigned long long>(), t->cdf_total.as<unsigned long long>(), t->tbl_rep.as<int>(),
-                                t->tbl_min.as<int>(), t->kld ? t->tbl_size : 0, t->kld ? 0 : t->particle_num, t->input->d_hdr());
+  launch_replicated(t, cdf_kernel<1>, cdf_kernel<kClusterCtas>, st, old_parts, t->cdf.as<unsigned long long>(), t->cdf_total.as<unsigned long long>(),
+                    t->tbl_rep.as<int>(), t->tbl_min.as<int>(), t->kld ? t->tbl_size : 0, t->kld ? 0 : t->particle_num, t->input->d_hdr());
   PFT_LAUNCH_CHECK();
   stage_mark(t, "cdf_kernel");
   if (t->sampler == PFT_SAMPLER_ALIAS_PCL) {  // (buffers sized by prepare_compute: nothing is allocated inside a graph capture)
@@ -610,6 +605,33 @@ int weight_comm_box(pft_tracker* t) {
   return PFT_OK;
 }
 
+// The launch of the nearest-neighbour lookup, bracketed in timing mode by the pair of events pft_tracker_get_timing reads
+template <typename Launch>
+int timed_lookup(pft_tracker* t, const char* name, Launch launch) {
+  cudaStream_t s = t->run_stream();
+  if (t->timing) {
+    while ((int)t->ev_w.size() < 2 * (t->n_ev_used + 1)) { cudaEvent_t e; PFT_CUDA_TRY(cudaEventCreate(&e)); t->ev_w.push_back(e); }
+    PFT_CUDA_TRY(cudaEventRecord(t->ev_w[2 * t->n_ev_used], s));
+  }
+  launch();
+  PFT_LAUNCH_CHECK();
+  stage_mark(t, name);
+  if (t->timing) { PFT_CUDA_TRY(cudaEventRecord(t->ev_w[2 * t->n_ev_used + 1], s)); t->n_ev_used++; }
+  return PFT_OK;
+}
+
+// Per-chunk partials -> this rank's raw weights, when a stage reads them: the phase API (force_raw) and the sharded
+// exchanges.  (Single rank, or peer mode inside compute(): normalize_kernel sums the partials itself.)
+int launch_raw_weights(pft_tracker* t, bool force_raw) {
+  if (!force_raw && (t->nranks == 1 || t->peer_fused)) return PFT_OK;
+  const int local_cap = t->slice_cap();
+  raw_weights_kernel<<<blocks_for(local_cap, 256, t->ctx->sm_count * 4), 256, 0, t->run_stream()>>>(
+      t->st.as<TrackerState>(), t->partial.as<double>(), t->chunks, t->n_cap, t->raw.as<float>(), local_cap, t->nranks, t->rank, t->peers, t->peer_mode ? 1 : 0);
+  PFT_LAUNCH_CHECK();
+  stage_mark(t, "raw_weights_kernel");
+  return PFT_OK;
+}
+
 // Parity mode PFT_NN_PCL_APPROX (see octree_build_kernel): the octree of the cropped cloud and the greedy search
 int weight_eval_pcl_approx(pft_tracker* t, bool force_raw) {
   cudaStream_t s = t->run_stream();
@@ -626,36 +648,21 @@ int weight_eval_pcl_approx(pft_tracker* t, bool force_raw) {
   w.partial = t->partial.as<double>(); w.chunks = t->chunks; w.chunk_len = t->chunk_len; w.n_max = t->n_cap; w.nranks = t->nranks; w.rank_id = t->rank;
   w.co = make_coherence(t);
   w.dbg_k = t->debug_nn; w.dbg_idx = t->dbg_idx.as<int>(); w.dbg_d2 = t->dbg_d2.as<float>();
-  if (t->timing) {
-    while ((int)t->ev_w.size() < 2 * (t->n_ev_used + 1)) { cudaEvent_t e; PFT_CUDA_TRY(cudaEventCreate(&e)); t->ev_w.push_back(e); }
-    PFT_CUDA_TRY(cudaEventRecord(t->ev_w[2 * t->n_ev_used], s));
-  }
-  weight_approx_kernel<<<sm * 8, 256, 0, s>>>(w);
-  PFT_LAUNCH_CHECK();
-  stage_mark(t, "weight_approx_kernel");
-  if (t->timing) { PFT_CUDA_TRY(cudaEventRecord(t->ev_w[2 * t->n_ev_used + 1], s)); t->n_ev_used++; }
-  if (t->nranks > 1 || force_raw) {
-    const int local_cap = t->slice_cap();
-    raw_weights_kernel<<<blocks_for(local_cap, 256, sm * 4), 256, 0, s>>>(st, t->partial.as<double>(), t->chunks, t->n_cap, t->raw.as<float>(), local_cap,
-                                                                         t->nranks, t->rank, t->peers, t->peer_mode ? 1 : 0);
-    PFT_LAUNCH_CHECK();
-    stage_mark(t, "raw_weights_kernel");
-  }
-  return PFT_OK;
+  int rc = timed_lookup(t, "weight_approx_kernel", [&] { weight_approx_kernel<<<sm * 8, 256, 0, s>>>(w); });
+  if (rc) return rc;
+  return launch_raw_weights(t, force_raw);
 }
 
 // crop box -> index header (also what in_crop() reads) + reset of the per-weight() counters
 int launch_index_begin(pft_tracker* t, bool reuse_allowed = false) {
   const int sm = t->ctx->sm_count;
   const float inv_leaf = 1.0f / (float)t->search_res;
-  // one index per frame (see IndexHeader): with the lists on, the crop box is dilated by this margin; the later weight()
+  // one index per frame (see IndexHeader): with the lists on, the crop box is dilated by kIndexDilate; the later weight()
   // calls of a compute() reuse the index when their crop box fits
-  static const float dilate = [] { const char* e = getenv("PFT_INDEX_DILATE"); return e ? (float)atof(e) : 0.03f; }();
-  static const int list_ratio = [] { const char* e = getenv("PFT_LIST_RATIO"); const int v = e ? atoi(e) : 0; return v > 0 ? v : 2; }();  // tuning knob
-  index_begin_kernel<<<sm, 256, 0, t->run_stream()>>>(t->st.as<TrackerState>(), t->idx_hdr.as<IndexHeader>(), t->icount.as<int>(), inv_leaf, t->index_level,
-                                                      t->max_cells, t->list_mode ? t->list_max_cells : 0, t->list_mode == 2 ? 0 : t->M, t->nranks, t->rank,
+  index_begin_kernel<<<sm, 256, 0, t->run_stream()>>>(t->st.as<TrackerState>(), t->idx_hdr.as<IndexHeader>(), t->icount.as<int>(), inv_leaf, t->max_cells,
+                                                      t->list_mode ? t->list_max_cells : 0, t->list_mode == 2 ? 0 : t->M, t->nranks, t->rank,
                                                       t->fneeded.as<unsigned int>(), t->xcount.as<int>(), t->fbuilt_bits.as<unsigned int>(),
-                                                      reuse_allowed ? 1 : 0, t->iteration_num > 1 ? dilate : 0.f, list_ratio, t->idx_hdr_prev.as<IndexHeader>());
+                                                      reuse_allowed ? 1 : 0, t->iteration_num > 1 ? kIndexDilate : 0.f, kListRatio, t->idx_hdr_prev.as<IndexHeader>());
   PFT_LAUNCH_CHECK();
   stage_mark(t, "index_begin_kernel");
   return PFT_OK;
@@ -673,16 +680,12 @@ int weight_phase_eval(pft_tracker* t, bool force_raw = false, bool reuse_allowed
   IndexHeader* hdr = t->idx_hdr.as<IndexHeader>();
   const float inv_leaf = 1.0f / (float)t->search_res;
   const int gscene = blocks_for(ncap_scene, 256, sm * 4);
-  if ((rc = launch_index_begin(t, reuse_allowed && t->list_max_cells > 0 && t->list_mode && t->nn_mode == PFT_NN_EXACT))) return rc;
-  const bool build_lists = t->list_max_cells > 0 && t->list_mode && t->nn_mode == PFT_NN_EXACT;
-  if (build_lists) {
+  // candidate lists for the exact search (the index header may still turn them off for this crop)
+  const bool lists = t->list_max_cells > 0 && t->list_mode && t->nn_mode == PFT_NN_EXACT;
+  if ((rc = launch_index_begin(t, reuse_allowed && lists))) return rc;
+  if (lists) {
     // which fine cells the queries fall into (mark + collect) does not depend on the point index being built (count +
     // scan + scatter): the two chains of small kernels run side by side on two streams and join before the list build
-    if (!t->aux_stream) {
-      PFT_CUDA_TRY(cudaStreamCreateWithFlags(&t->aux_stream, cudaStreamNonBlocking));
-      PFT_CUDA_TRY(cudaEventCreateWithFlags(&t->ev_fork, cudaEventDisableTiming));
-      PFT_CUDA_TRY(cudaEventCreateWithFlags(&t->ev_join, cudaEventDisableTiming));
-    }
     cudaStream_t sa = t->aux_stream;
     PFT_CUDA_TRY(cudaEventRecord(t->ev_fork, s));
     PFT_CUDA_TRY(cudaStreamWaitEvent(sa, t->ev_fork, 0));
@@ -706,7 +709,7 @@ int weight_phase_eval(pft_tracker* t, bool force_raw = false, bool reuse_allowed
                                               t->ihsv.as<unsigned int>(), t->ipts2.as<float4>());
   PFT_LAUNCH_CHECK();
   stage_mark(t, "index_scatter_kernel");
-  if (build_lists) {
+  if (lists) {
     PFT_CUDA_TRY(cudaStreamWaitEvent(s, t->ev_join, 0));
     stage_mark(t, "cand_mark+collect (beside the index)");
     cand_build_kernel<<<sm * 8, 256, 0, s>>>(hdr, t->cell_start.as<int>(), t->ipts.as<float4>(), t->max_dist * t->max_dist, t->flists.as<unsigned int>(),
@@ -727,70 +730,37 @@ int weight_phase_eval(pft_tracker* t, bool force_raw = false, bool reuse_allowed
     PFT_LAUNCH_CHECK();
     stage_mark(t, "cand_octant_kernel");
   }
-  const bool lists_built = t->list_max_cells > 0 && t->list_mode && t->nn_mode == PFT_NN_EXACT;
   if (t->nn_mode == PFT_NN_PCL_APPROX) return weight_eval_pcl_approx(t, force_raw);
   WeightArgs a;
-  const bool fallback_kernel = !lists_built;  // (weight_lists_kernel runs the row-table search itself when the index header says the lists are off)
   a.st = st; a.hdr = hdr; a.pts2 = t->ipts2.as<float4>();
   a.flists = t->flists.as<unsigned int>(); a.pool = t->fpool.as<unsigned int>(); a.xlists = t->xlists.as<unsigned int>();
   a.cell_start = t->cell_start.as<int>(); a.pts = t->ipts.as<float4>();
-  a.hsv = t->ihsv.as<unsigned int>(); a.table = t->row_table.as<RowEntry>(); a.smem_bytes = t->weight_smem;
+  a.hsv = t->ihsv.as<unsigned int>(); a.table = t->row_table.as<RowEntry>(); a.smem_bytes = t->lists_smem;
   a.model = t->model.as<float4>(); a.model_perm = t->model_perm.as<int>(); a.M = t->M;
   a.mats = t->mats.as<float>();
   a.partial = t->partial.as<double>(); a.chunks = t->chunks; a.chunk_len = t->chunk_len; a.n_max = t->n_cap;
   a.nranks = t->nranks; a.rank_id = t->rank;
-  // many items per warp (large particle sets): dynamic hand-out; few: static interleaved split (see weight_items)
-  static const long long dyn_per_warp = [] { const char* e = getenv("PFT_DYN_ITEMS_PER_WARP"); const int v = e ? atoi(e) : 0; return (long long)(v > 0 ? v : 5); }();  // tuning knob (measured: dynamic wins from ~5 items per warp up, 10k-25k particles -7 %)
-  const bool dyn = (long long)std::max(1, (t->particle_num > 0 ? t->particle_num : t->n_cap) / t->nranks) * t->chunks >= dyn_per_warp * sm * (kWeightThreads / 32);
   a.co = make_coherence(t);
   a.dbg_k = t->debug_nn; a.dbg_idx = t->dbg_idx.as<int>(); a.dbg_d2 = t->dbg_d2.as<float>();
-  const int local_cap = t->slice_cap();
   const int wgrid = sm;  // persistent: one CTA per SM
-  if (t->timing) {
-    while ((int)t->ev_w.size() < 2 * (t->n_ev_used + 1)) { cudaEvent_t e; PFT_CUDA_TRY(cudaEventCreate(&e)); t->ev_w.push_back(e); }
-    PFT_CUDA_TRY(cudaEventRecord(t->ev_w[2 * t->n_ev_used], s));
-  }
-  if (lists_built) {
-    // the product path: candidate lists (the same launch runs the row-table search when the index header says they are off for this crop)
-    a.smem_bytes = t->lists_smem;
-    const long long n_local = std::max(1, (t->particle_num > 0 ? t->particle_num : t->n_cap) / t->nranks);
-    const bool dyn_l = n_local * t->chunks >= dyn_per_warp * sm * (kListThreads / 32);
+  // many items per warp (large particle sets): dynamic hand-out; few: static interleaved split (see weight_items)
+  const long long n_local = std::max(1, (t->particle_num > 0 ? t->particle_num : t->n_cap) / t->nranks);
+  const bool dyn = n_local * t->chunks >= kDynItemsPerWarp * sm * (kListThreads / 32);
+  // one launch either way: it runs the row-table search itself when the index header says the lists are off
+  rc = timed_lookup(t, "weight_lists_kernel", [&] {
     if (n_local * t->M >= kListBigQueries) {
       if (t->use_hsv) weight_lists_kernel<true, kListThreadsBig, true><<<wgrid, kListThreadsBig, t->lists_smem, s>>>(a);
       else weight_lists_kernel<false, kListThreadsBig, true><<<wgrid, kListThreadsBig, t->lists_smem, s>>>(a);
     } else if (t->use_hsv) {
-      if (dyn_l) weight_lists_kernel<true, kListThreads, true><<<wgrid, kListThreads, t->lists_smem, s>>>(a);
+      if (dyn) weight_lists_kernel<true, kListThreads, true><<<wgrid, kListThreads, t->lists_smem, s>>>(a);
       else weight_lists_kernel<true, kListThreads, false><<<wgrid, kListThreads, t->lists_smem, s>>>(a);
     } else {
-      if (dyn_l) weight_lists_kernel<false, kListThreads, true><<<wgrid, kListThreads, t->lists_smem, s>>>(a);
+      if (dyn) weight_lists_kernel<false, kListThreads, true><<<wgrid, kListThreads, t->lists_smem, s>>>(a);
       else weight_lists_kernel<false, kListThreads, false><<<wgrid, kListThreads, t->lists_smem, s>>>(a);
     }
-    PFT_LAUNCH_CHECK();
-    stage_mark(t, "weight_lists_kernel");
-    // (timing: the event pair brackets the kernel that evaluates the lists -- the launch below returns at once then)
-    if (t->timing) { PFT_CUDA_TRY(cudaEventRecord(t->ev_w[2 * t->n_ev_used + 1], s)); t->n_ev_used++; }
-    a.smem_bytes = t->weight_smem;
-  }
-  // row-table search over the grid: crops the lists do not cover (returns at once otherwise)
-  if (fallback_kernel) {
-    if (t->use_hsv) {
-      if (dyn) weight_kernel<true, kWeightThreads, true><<<wgrid, kWeightThreads, t->weight_smem, s>>>(a);
-      else weight_kernel<true, kWeightThreadsSmall, false><<<wgrid, kWeightThreadsSmall, t->weight_smem, s>>>(a);
-    } else {
-      if (dyn) weight_kernel<false, kWeightThreads, true><<<wgrid, kWeightThreads, t->weight_smem, s>>>(a);
-      else weight_kernel<false, kWeightThreadsSmall, false><<<wgrid, kWeightThreadsSmall, t->weight_smem, s>>>(a);
-    }
-    PFT_LAUNCH_CHECK();
-    stage_mark(t, "weight_kernel");
-  }
-  if (t->timing && !lists_built) { PFT_CUDA_TRY(cudaEventRecord(t->ev_w[2 * t->n_ev_used + 1], s)); t->n_ev_used++; }
-  if ((t->nranks > 1 || force_raw) && !(t->peer_mode && t->peer_fused && !force_raw)) {  // (single rank, or peer mode inside compute(): normalize_kernel sums the per-chunk partials itself)
-    raw_weights_kernel<<<blocks_for(local_cap, 256, sm * 4), 256, 0, s>>>(st, t->partial.as<double>(), t->chunks, t->n_cap, t->raw.as<float>(), local_cap,
-                                                                         t->nranks, t->rank, t->peers, t->peer_mode ? 1 : 0);
-    PFT_LAUNCH_CHECK();
-    stage_mark(t, "raw_weights_kernel");
-  }
-  return PFT_OK;
+  });
+  if (rc) return rc;
+  return launch_raw_weights(t, force_raw);
 }
 
 // raw weight exchange: every rank ends up with all raw weights
@@ -806,15 +776,11 @@ int weight_comm_raw(pft_tracker* t) {
 int weight_phase_normalize(pft_tracker* t, bool fuse_update = false) {
   int rc = check_weight_ready(t);
   if (rc) return rc;
-  const bool push = t->peer_mode && t->peer_fused && t->nn_mode == PFT_NN_EXACT;  // (the launch pushes this rank's raw weights to the peers itself)
-  if (t->n_cap > kClusterMinParticles) normalize_kernel<kClusterCtas><<<kClusterCtas, 1024, 0, t->run_stream()>>>(t->st.as<TrackerState>(), t->parts[t->cur].as<DevParticle>(), t->raw.as<float>(), t->alpha, t->nranks,
-                                                   t->slice_cap(), t->input->d_hdr(), t->peer_mode ? reinterpret_cast<PeerWindow*>(t->peer_local) : nullptr, t->M,
-                                                   t->nranks == 1 ? t->partial.as<double>() : nullptr, t->chunks, t->n_cap, t->raw.as<float>(), fuse_update ? 1 : 0,
-                                                   t->peers, push ? t->partial.as<double>() : nullptr, t->rank);
-  else normalize_kernel<1><<<1, 1024, 0, t->run_stream()>>>(t->st.as<TrackerState>(), t->parts[t->cur].as<DevParticle>(), t->raw.as<float>(), t->alpha, t->nranks,
-                                                   t->slice_cap(), t->input->d_hdr(), t->peer_mode ? reinterpret_cast<PeerWindow*>(t->peer_local) : nullptr, t->M,
-                                                   t->nranks == 1 ? t->partial.as<double>() : nullptr, t->chunks, t->n_cap, t->raw.as<float>(), fuse_update ? 1 : 0,
-                                                   t->peers, push ? t->partial.as<double>() : nullptr, t->rank);
+  const bool push = t->peer_fused;  // (the launch pushes this rank's raw weights to the peers itself)
+  launch_replicated(t, normalize_kernel<1>, normalize_kernel<kClusterCtas>, t->st.as<TrackerState>(), t->parts[t->cur].as<DevParticle>(), t->raw.as<float>(),
+                    t->alpha, t->nranks, t->slice_cap(), t->input->d_hdr(), t->peer_mode ? reinterpret_cast<PeerWindow*>(t->peer_local) : nullptr, t->M,
+                    t->nranks == 1 ? t->partial.as<double>() : nullptr, t->chunks, t->n_cap, t->raw.as<float>(), fuse_update ? 1 : 0, t->peers,
+                    push ? t->partial.as<double>() : nullptr, t->rank);
   PFT_LAUNCH_CHECK();
   stage_mark(t, "normalize_kernel");
   t->changed = true;  // change detector is off upstream => changed_ = true after every weight()
@@ -854,10 +820,8 @@ int weight_phase_renormalize(pft_tracker* t) {
   weights_to_raw_kernel<<<blocks_for(t->n_cap, 256, t->ctx->sm_count * 4), 256, 0, s>>>(st, parts, t->raw.as<float>(), t->nranks, t->slice_cap());
   PFT_LAUNCH_CHECK();
   stage_mark(t, "weights_to_raw_kernel");
-  if (t->n_cap > kClusterMinParticles) normalize_kernel<kClusterCtas><<<kClusterCtas, 1024, 0, s>>>(st, parts, t->raw.as<float>(), t->alpha, t->nranks, t->slice_cap(), t->input->d_hdr(),
-                                                   nullptr, 0, nullptr, t->chunks, t->n_cap, t->raw.as<float>(), 0, t->peers, nullptr, t->rank);
-  else normalize_kernel<1><<<1, 1024, 0, s>>>(st, parts, t->raw.as<float>(), t->alpha, t->nranks, t->slice_cap(), t->input->d_hdr(),
-                                              nullptr, 0, nullptr, t->chunks, t->n_cap, t->raw.as<float>(), 0, t->peers, nullptr, t->rank);
+  launch_replicated(t, normalize_kernel<1>, normalize_kernel<kClusterCtas>, st, parts, t->raw.as<float>(), t->alpha, t->nranks, t->slice_cap(),
+                    t->input->d_hdr(), nullptr, 0, nullptr, t->chunks, t->n_cap, t->raw.as<float>(), 0, t->peers, nullptr, t->rank);
   PFT_LAUNCH_CHECK();
   stage_mark(t, "normalize_kernel");
   t->changed = false;
@@ -891,8 +855,7 @@ int stage_weight(pft_tracker* t, bool fuse_update = false, bool reuse_allowed = 
 
 int stage_update(pft_tracker* t) {
   if (!t->has_particles || !t->input) { set_last_error("update before weight"); return PFT_ERR_STATE; }
-  if (t->n_cap > kClusterMinParticles) update_kernel<kClusterCtas><<<kClusterCtas, 1024, 0, t->run_stream()>>>(t->st.as<TrackerState>(), t->parts[t->cur].as<DevParticle>(), t->input->d_hdr());
-  else update_kernel<1><<<1, 1024, 0, t->run_stream()>>>(t->st.as<TrackerState>(), t->parts[t->cur].as<DevParticle>(), t->input->d_hdr());
+  launch_replicated(t, update_kernel<1>, update_kernel<kClusterCtas>, t->st.as<TrackerState>(), t->parts[t->cur].as<DevParticle>(), t->input->d_hdr());
   PFT_LAUNCH_CHECK();
   stage_mark(t, "update_kernel");
   return PFT_OK;
@@ -911,11 +874,19 @@ int enqueue_tracking(pft_tracker* t) {
   return PFT_OK;
 }
 
+// Every lazy allocation of the frame path happens here, before any stage is enqueued: nothing may be allocated inside a
+// graph capture, nor between the enqueues of the ranks of the multi-device mode (see compute_multi_device).
 int prepare_compute(pft_tracker* t) {
   int rc = ensure_particle_buffers(t);
   if (rc) return rc;
   if (t->input && (rc = t->input->join_upload())) return rc;  // frame still arriving on the copy stream (pft_cloud_upload_async)
   if ((rc = ensure_index_buffers(t))) return rc;
+  if (t->inj_stride == 0 && (rc = reserve_generated_draws(t, t->n_cap))) return rc;
+  if (!t->aux_stream) {  // the candidate-list chain that runs beside the index build (weight_phase_eval)
+    PFT_CUDA_TRY(cudaStreamCreateWithFlags(&t->aux_stream, cudaStreamNonBlocking));
+    PFT_CUDA_TRY(cudaEventCreateWithFlags(&t->ev_fork, cudaEventDisableTiming));
+    PFT_CUDA_TRY(cudaEventCreateWithFlags(&t->ev_join, cudaEventDisableTiming));
+  }
   choose_chunks(t);
   const size_t need_partial = (size_t)t->chunks * t->n_cap * sizeof(double);
   if (need_partial > t->partial.bytes) {
@@ -996,10 +967,6 @@ int pft_tracker_create(pft_context* ctx, int kld, pft_tracker** out) {
   t->kld = kld != 0;
   const char* ng = getenv("PFT_NO_GRAPH");
   t->graph_enabled = !(ng && ng[0] == '1');
-  const char* il = getenv("PFT_INDEX_LEVEL");  // tuning: cell edge of the index = resolution x 2^level
-  if (il && il[0] >= '0' && il[0] <= '9') t->index_level = il[0] - '0';
-  const char* nl = getenv("PFT_NO_LISTS");  // tuning: row-table search only
-  if (nl && nl[0] == '1') t->list_mode = 0;
   *out = t;
   return PFT_OK;
 }
@@ -1212,11 +1179,6 @@ static int compute_one(pft_tracker* t) {
                        t->graph_scene_hdr[g] == (const void*)t->input->d_hdr();
     if (!valid) {
       if (t->graph_exec[g]) { cudaGraphExecDestroy(t->graph_exec[g]); t->graph_exec[g] = nullptr; }
-      // make sure every lazily sized buffer exists before capture (no allocation inside a capture)
-      if (t->inj_stride == 0) {
-        const int count = t->kld ? t->max_particle_num : t->n_cap;
-        if (t->draw_cap < count) { if ((rc = ensure_draw_buffers(t, 1, count))) return rc; t->draw_cap = count; }
-      }
       const unsigned long long version = t->config_version;
       const int cur0 = t->cur;
       const bool changed0 = t->changed;
@@ -1331,10 +1293,6 @@ static int preload_kernels() {
       (const void*)update_kernel<1>,
       (const void*)update_kernel<kClusterCtas>,
       (const void*)weight_approx_kernel,
-      (const void*)weight_kernel<false, kWeightThreads, true>,
-      (const void*)weight_kernel<false, kWeightThreadsSmall, false>,
-      (const void*)weight_kernel<true, kWeightThreads, true>,
-      (const void*)weight_kernel<true, kWeightThreadsSmall, false>,
       (const void*)weight_lists_kernel<false, kListThreads, false>,
       (const void*)weight_lists_kernel<false, kListThreads, true>,
       (const void*)weight_lists_kernel<false, kListThreadsBig, true>,
@@ -1387,15 +1345,6 @@ static int compute_multi_device(pft_tracker* t) {
       PFT_CUDA_TRY(cudaSetDevice(x->ctx->device));
       if (!x->md_prepared) { if ((rc = preload_kernels())) return rc; }
       if ((rc = prepare_compute(x))) return rc;
-      if (x->inj_stride == 0) {
-        const int count = x->kld ? x->max_particle_num : x->n_cap;
-        if (x->draw_cap < count) { if ((rc = ensure_draw_buffers(x, 1, count))) return rc; x->draw_cap = count; }
-      }
-      if (!x->aux_stream) {
-        PFT_CUDA_TRY(cudaStreamCreateWithFlags(&x->aux_stream, cudaStreamNonBlocking));
-        PFT_CUDA_TRY(cudaEventCreateWithFlags(&x->ev_fork, cudaEventDisableTiming));
-        PFT_CUDA_TRY(cudaEventCreateWithFlags(&x->ev_join, cudaEventDisableTiming));
-      }
       x->md_prepared = true;
     }
   }

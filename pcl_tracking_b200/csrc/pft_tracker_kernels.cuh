@@ -6,7 +6,7 @@
 //   matrices_kernel      ParticleXYZRPY::toEigenMatrix = pcl::getTransformation          (A.6)
 //   aabb_kernel          transformPointCloud per particle + calcBoundingBox               (A.3)
 //   index_*_kernel       cropInputPointCloud + search::Octree::setInputCloud              (A.3, A.5)
-//   weight_kernel        NearestPairPointCloudCoherence::computeCoherence + Distance/HSV  (A.4)
+//   weight_lists_kernel  NearestPairPointCloudCoherence::computeCoherence + Distance/HSV  (A.4)
 //   normalize_kernel     ParticleFilterTracker::normalizeWeight                           (A.6)
 //   update_kernel        ParticleFilterTracker::update                                    (A.6)
 //   cdf/resample/kld_*   (KLDAdaptive)ParticleFilterTracker::resample                     (A.7)
@@ -48,7 +48,6 @@ struct TrackerState {
   unsigned int work_counter;     // next (particle, model chunk) item of the running weight kernel (reset by index_begin_kernel)
   unsigned long long evals;      // likelihood evaluations so far: sum over weight() calls of particles x model points (whole job)
   unsigned int aabb_blocks_done; // blocks of the running aabb_kernel that have added their boxes (peer mode: the last one exchanges the box)
-  int lists_on;                  // the last weight() ran on the candidate lists (read back with the state: the host then stops launching the row-table kernel behind weight_lists_kernel)
 };
 
 // ------------------------------------------------------------------ NVLink peer exchange (one process per GPU)
@@ -452,10 +451,10 @@ __device__ inline void compute_index_header(const float* crop, const float* aabb
 
 // Every block derives the header from the crop box (a pure function of it), block 0 publishes it, and all
 // blocks clear the per-cell counters.
-// base_level < 0: choose the cell edge from the mean nearest-neighbour distance of the previous weight() (a query
-// that is d away from the surface walks ~pi (d/cell + 1)^2 rows and ~(d + cell)^2 candidates: cell ~ d balances them)
-__global__ void index_begin_kernel(TrackerState* st, IndexHeader* hdr, int* cell_count, float inv_leaf, int base_level,
-                                   int max_cells, int list_max_cells, int M, int nranks, int rank, unsigned int* needed_words,
+// The cell edge follows the mean nearest-neighbour distance of the previous weight() (a query that is d away from the
+// surface walks ~pi (d/cell + 1)^2 rows and ~(d + cell)^2 candidates: cell ~ d balances them).
+__global__ void index_begin_kernel(TrackerState* st, IndexHeader* hdr, int* cell_count, float inv_leaf, int max_cells,
+                                   int list_max_cells, int M, int nranks, int rank, unsigned int* needed_words,
                                    int* list_counters /* [0] extended lists handed out, [1] needed blocks, [2] cells queued for the far pass, [3] pool groups handed out, [4] cells queued for the octant pass */,
                                    unsigned int* built_bits /* one bit per fine cell: its lists exist (this frame) */, int reuse_allowed, float dilate,
                                    int list_ratio /* the lists are built when this rank's queries outnumber the fine cells of the crop box by this factor */,
@@ -485,13 +484,11 @@ __global__ void index_begin_kernel(TrackerState* st, IndexHeader* hdr, int* cell
 #pragma unroll
       for (int d = 0; d < 3; ++d) { h.core[d] = fminf(old.core[d], st->aabb[d] + old.dilate); h.core[3 + d] = fmaxf(old.core[3 + d], st->aabb[3 + d] - old.dilate); }
     } else {
-      if (base_level < 0) {
-        base_level = 1;
-        if (st->nn_count > 0) {
-          const float mean_d = (float)((double)st->nn_sum_um / (double)st->nn_count) * 1.0e-6f;
-          const float want = mean_d * 1.15f * inv_leaf;  // cell edge in units of the resolution
-          base_level = want <= 1.5f ? 1 : (want <= 3.0f ? 1 : (want <= 6.0f ? 2 : (want <= 12.0f ? 3 : 4)));
-        }
+      int base_level = 1;
+      if (st->nn_count > 0) {
+        const float mean_d = (float)((double)st->nn_sum_um / (double)st->nn_count) * 1.0e-6f;
+        const float want = mean_d * 1.15f * inv_leaf;  // cell edge in units of the resolution
+        base_level = want <= 1.5f ? 1 : (want <= 3.0f ? 1 : (want <= 6.0f ? 2 : (want <= 12.0f ? 3 : 4)));
       }
       // candidate lists pay off when this rank's queries outnumber the fine cells they are built for
       const int n = st->particle_num;
@@ -601,7 +598,6 @@ __global__ void __launch_bounds__(1024) index_scan_kernel(const IndexHeader* __r
   if (threadIdx.x == 0) {
     st->nn_sum_um = 0ull; st->nn_count = 0ull;  // consumed by index_begin; refilled by the weight kernel
     *hdr_prev = *hdr;  // what the next weight() of the frame tests its crop box against (the point counts are final by now)
-    st->lists_on = (hdr->use_lists && hdr->n_cropped < 65535) ? 1 : 0;  // (= lists_on(*hdr))
   }
   if (hdr->reuse) return;
   const int total = block_exclusive_scan<int>(
@@ -813,10 +809,7 @@ __device__ __forceinline__ float box_maxdist2(const float* lo, const float* hi, 
 // remembers the cells it has flagged in a bitmap of the fine grid in shared memory (f_cells bits, dynamic): every
 // block stores every cell at most once.
 constexpr int kMarkUnroll = 4;
-#ifndef PFT_COARSE_BELOW
-#define PFT_COARSE_BELOW 24
-#endif
-constexpr unsigned int kCoarseBelow = PFT_COARSE_BELOW;  // queries of a cell below which its list is not split into octants
+constexpr unsigned int kCoarseBelow = 24u;               // queries of a cell below which its list is not split into octants
 constexpr unsigned int kLightBelow = 256u;               // ... below which a list that fits one record is not split either
 template <bool COUNT>
 __global__ void __launch_bounds__(256) cand_mark_kernel(const TrackerState* __restrict__ st, const IndexHeader* __restrict__ hdr, const float4* __restrict__ model, int M,
@@ -1847,9 +1840,9 @@ __device__ __forceinline__ void weight_items(const WeightArgs& a, const IndexHea
   }
 }
 
-// Persistent launch: one CTA per SM, each warp works through (particle, model chunk) items.
-// The whole weight() of one CTA through the row-table search (crops the candidate lists do not cover).  h, the two
-// look-up tables and s_table live in the caller's shared memory; the tables are filled here.
+// The whole weight() of one CTA of weight_lists_kernel through the row-table search, when the index header says the
+// lists are off (PFT_CANDIDATE_LISTS = 0, too few queries, or a crop too large for the tables).  h, the two look-up
+// tables and s_table live in the caller's shared memory; the tables are filled here.
 template <bool USE_HSV, bool DYN>
 __device__ __noinline__ void weight_rowtable_body(const WeightArgs a /* by value: a reference would pull the caller's kernel parameters into local memory */,
                                                   const IndexHeader& h, float* lut_h, float* lut_s, RowEntry* s_table) {
@@ -1866,11 +1859,7 @@ __device__ __noinline__ void weight_rowtable_body(const WeightArgs a /* by value
   const long long need_hsv = 4ll * ((n_pts + 3) & ~3);
   const long long need_cs = 2ll * (((long long)h.n_cells + 1 + 7) & ~7ll);
   const bool pts_staged = h.valid && need_pts <= (long long)a.smem_bytes;
-#ifdef PFT_NO_HSV_STAGE
-  const bool hsv_staged = false;
-#else
   const bool hsv_staged = USE_HSV && pts_staged && need_pts + need_hsv <= (long long)a.smem_bytes;
-#endif
   const long long used = need_pts + (hsv_staged ? need_hsv : 0);
   const bool cs_staged = pts_staged && n_pts < 65536 && used + need_cs <= (long long)a.smem_bytes;
   uint4* s_pts = dyn_smem;
@@ -1898,19 +1887,8 @@ __device__ __noinline__ void weight_rowtable_body(const WeightArgs a /* by value
   }
 }
 
-// Persistent launch of the row-table search alone (the host knows that no lists are built: PFT_CANDIDATE_LISTS = 0)
-template <bool USE_HSV, int THREADS, bool DYN>
-__global__ void __launch_bounds__(THREADS, 1) weight_kernel(const WeightArgs a) {
-  __shared__ IndexHeader h;
-  __shared__ float lut_h[256], lut_s[256];
-  __shared__ RowEntry s_table[kRows];
-  if (threadIdx.x == 0) h = *a.hdr;
-  __syncthreads();
-  weight_rowtable_body<USE_HSV, DYN>(a, h, lut_h, lut_s, s_table);
-}
-
 // ------------------------------------------------------------------ K3, list path: weight_lists_kernel
-// The product path of weight() whenever the candidate lists are on.  Persistent, one CTA per SM; the indexed points
+// The exact-search weight() (weight_rowtable_body when the lists are off).  Persistent, one CTA per SM; the indexed points
 // {x, y, z, packed HSV} travel into shared memory as ONE bulk asynchronous copy (cp.async.bulk + mbarrier, issued by
 // one thread while the others set up), each warp takes (particle, model chunk) items, a lane = one model point:
 //   transform -> octant of the fine lattice -> ONE 16-byte load (header + seven slots) -> seven candidates from shared
@@ -1946,9 +1924,6 @@ __device__ __noinline__ SlowNN nn_slow_warp(const unsigned char* __restrict__ sb
   return SlowNN{bd, bs};
 }
 
-#ifndef PFT_LIST_PIPE
-#define PFT_LIST_PIPE 0  // 1: two rounds of a warp in flight (measured: the registers are better spent on more warps)
-#endif
 // one 32-byte record (header + seven entries, or a pool group of eight entries) as ONE 256-bit load
 struct Rec8 { unsigned int w[8]; };
 __device__ __forceinline__ Rec8 load_rec8(const unsigned int* __restrict__ p) {
@@ -1977,7 +1952,7 @@ struct ListQuery { float x, y, z; unsigned int hsv; Rec8 r; };
 
 template <bool USE_HSV, bool DYN>
 __device__ __forceinline__ void weight_list_items(const WeightArgs& a, const IndexHeader& h, const unsigned char* __restrict__ sbase,
-                                                  const float* __restrict__ lut_h, const float* __restrict__ lut_s, bool brute) {
+                                                  const float* __restrict__ lut_h, const float* __restrict__ lut_s) {
   const int n = a.st->particle_num;
   const int n_local = n > a.rank_id ? (n - a.rank_id + a.nranks - 1) / a.nranks : 0;
   const int items = n_local * a.chunks;
@@ -2023,7 +1998,7 @@ __device__ __forceinline__ void weight_list_items(const WeightArgs& a, const Ind
       // (cvt.rmi saturates: a far-away or non-finite query fails the range test)
       const int ix = __float2int_rd(q.x * inv2) - o2x, iy = __float2int_rd(q.y * inv2) - o2y, iz = __float2int_rd(q.z * inv2) - o2z;
       q.r.w[0] = kListOverflow;
-      if (!brute && (unsigned int)ix < d2x && (unsigned int)iy < d2y && (unsigned int)iz < d2z)
+      if ((unsigned int)ix < d2x && (unsigned int)iy < d2y && (unsigned int)iz < d2z)
         q.r = load_rec8(a.flists + (size_t)(((unsigned int)iz * d2y + (unsigned int)iy) * d2x + (unsigned int)ix) * 8);
       return q;
     };
@@ -2110,22 +2085,7 @@ __device__ __forceinline__ void weight_list_items(const WeightArgs& a, const Ind
         val += rcp_f64(den);
       }
     };
-#if PFT_LIST_PIPE
-    // two rounds in flight (ping-pong, so that no query is copied between registers): the record of the next round
-    // is on its way while the current one is evaluated
-    ListQuery qa = fetch(j0), qb;
-    for (int jb = j0; jb < j1; jb += 64) {
-      const bool second = jb + 32 < j1;
-      if (second) qb = fetch(jb + 32);
-      eval(qa, jb);
-      if (second) {
-        if (jb + 64 < j1) qa = fetch(jb + 64);
-        eval(qb, jb + 32);
-      }
-    }
-#else
     for (int jb = j0; jb < j1; jb += 32) eval(fetch(jb), jb);
-#endif
     val = warp_sum(val);
     sum_um64 += sum_um;
     if (lane == 0) a.partial[(size_t)c * a.n_max + i] = val;
@@ -2168,7 +2128,6 @@ __global__ void __launch_bounds__(THREADS, 1) weight_lists_kernel(const WeightAr
     weight_rowtable_body<USE_HSV, DYN>(a, h, lut_h, lut_s, s_table);
     return;
   }
-  const bool brute = false;
   PFT_TRACE_MAX(5);
   const int n_pts = h.n_cropped + 1;  // + the dummy point that pads the lists
   const bool staged = 16ll * n_pts <= (long long)a.smem_bytes;
@@ -2188,10 +2147,10 @@ __global__ void __launch_bounds__(THREADS, 1) weight_lists_kernel(const WeightAr
     // 1000 particles, 13 % lost on 100 000: the extra live register costs more than the ~3 us of overlap)
     mbar_wait(&s_bar, 0);
     PFT_TRACE_MAX(6);
-    weight_list_items<USE_HSV, DYN>(a, h, reinterpret_cast<const unsigned char*>(dyn_smem), lut_h, lut_s, brute);
+    weight_list_items<USE_HSV, DYN>(a, h, reinterpret_cast<const unsigned char*>(dyn_smem), lut_h, lut_s);
     PFT_TRACE_MIN(7); PFT_TRACE_MAX(8);
   } else {
-    weight_list_items<USE_HSV, DYN>(a, h, reinterpret_cast<const unsigned char*>(a.pts2), lut_h, lut_s, brute);
+    weight_list_items<USE_HSV, DYN>(a, h, reinterpret_cast<const unsigned char*>(a.pts2), lut_h, lut_s);
   }
 }
 

@@ -1,5 +1,5 @@
 """Particle sharding plan of the multi-GPU path (SURVEY.md section 8e), host-side mirror of the device code
-(pft_tracker_kernels.cuh: raw_slot, weight_kernel's item loop).
+(pft_tracker_kernels.cuh: raw_slot, the item loop of weight_lists_kernel).
 
 Particle i is weighted by rank i % R.  Every rank owns slice_cap = ceil(n_cap / R) slots of the gathered
 raw-weight buffer [R][slice_cap]; particle i sits at row i % R, column i // R."""

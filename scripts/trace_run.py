@@ -18,12 +18,12 @@ dev = [pcl.PointCloud(f, ctx=ctx) for f in frames]
 lib = _capi.load()
 out = (C.c_ulonglong * 64)()
 init = (C.c_ulonglong * 64)()
-MINS = (0, 3, 7, 9, 11)
+MINS = (0, 3, 7, 11)
 for i in range(64):
     init[i] = 0xFFFFFFFFFFFFFFFF if i in MINS else 0
 names = {0: "index_begin first CTA in", 1: "cand_octant last warp out", 2: "cand_build_far last out", 3: "weight_lists first CTA in", 4: "weight_lists last CTA in",
          5: "weight_lists last header+sync", 6: "weight_lists last staged (mbar)", 7: "weight_lists first warp done", 8: "weight_lists last warp done",
-         9: "weight_kernel(old) first in", 10: "weight_kernel(old) last hdr", 11: "normalize first in"}
+         11: "normalize first in"}
 lib.pft_debug_trace(out, init)
 for k in range(14):
     vg.setInputCloud(dev[bench.frame_order(k, 6)]); vg.filter(ds)

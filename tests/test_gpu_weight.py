@@ -2,6 +2,8 @@
 
 north_star bar: nearest-neighbour indices bit-exact against the exact-search coherence configuration
 (ties to the lower index), particle weights within 1e-5 relative."""
+import functools
+
 import numpy as np
 import pytest
 
@@ -242,3 +244,35 @@ def test_lists_switch_off_and_on_again_on_one_tracker():
         np.testing.assert_allclose(g.rawWeights(), o.raw_weights(), rtol=1e-5)
         np.testing.assert_allclose(g.getParticles()["weight"], o.get_particles()["weight"], rtol=1e-5, atol=1e-12)
     assert seen == [1, 0, 1, 0]
+
+
+@functools.lru_cache(maxsize=None)
+def _tracked_with_timing(lists):
+    """Three timed compute() calls of one fixed-N tracker (two iterations each): the kernel names of every compute(),
+    the index header's list decision, and the final pose and particles as bytes."""
+    scene, model, centre = util.small_case(31, n_scene=6000, n_model=400)
+    t = pcl.ParticleFilterOMPTracker(16)
+    pcl.configure_like_reference(t, particle_num=600, use_hsv=True, iteration_num=2)
+    m = np.eye(4, dtype=np.float32)
+    m[:3, 3] = centre
+    t.setTrans(m); t.seed(5); t.setReferenceCloud(model); t.setCandidateLists(lists); t.enableTiming(True)
+    t.setInputCloud(pcl.PointCloud(scene))
+    names = []
+    for _ in range(3):
+        t.compute()
+        names.append([n for n, _ in t.kernelTimes()])
+    return names, t.indexInfo()["use_lists"], t.getResult().tobytes(), t.getParticles().tobytes()
+
+
+@pytest.mark.parametrize("lists", [0, 1, 2])
+def test_one_lookup_kernel_in_every_list_mode(lists):
+    """Every exact-search weight() is one launch of weight_lists_kernel, with the lists off too (it then runs the row-table
+    search), and the mode of the lists never changes a result: pose and particles equal bit for bit across the modes."""
+    names, use_lists, pose, parts = _tracked_with_timing(lists)
+    assert use_lists == (0 if lists == 0 else 1)
+    for frame in names:
+        assert frame.count("weight_lists_kernel") == 2  # once per iteration
+        assert "weight_kernel" not in frame
+    for other in (0, 1, 2):
+        _, _, pose_o, parts_o = _tracked_with_timing(other)
+        assert pose == pose_o and parts == parts_o
