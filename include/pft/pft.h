@@ -289,7 +289,8 @@ PFT_API int pft_tracker_graph_replays(pft_tracker* t, uint64_t* n);
  * used by the single-GPU emulation tests): phase 0 = transforms + this rank's crop box, 1 = index build +
  * coherence of this rank's particles, 2 = normalizeWeight.  The crop box is read/written between 0 and
  * 1, the raw-weight slices ([nranks][slice], particle i -> rank i % nranks, position i / nranks)
- * between 1 and 2. */
+ * between 1 and 2.  A tracker attached to peer windows (pft_tracker_peer_attach, or pft_tracker_set_devices
+ * after its first compute()) exchanges inside its kernels: it refuses every phase with PFT_ERR_STATE. */
 PFT_API int pft_tracker_weight_phase(pft_tracker* t, int phase);
 PFT_API int pft_tracker_get_crop_box(pft_tracker* t, float* aabb6);
 PFT_API int pft_tracker_set_crop_box(pft_tracker* t, const float* aabb6);
@@ -318,9 +319,9 @@ PFT_API int pft_tracker_comm_destroy(pft_tracker* t);
 
 /* ---------------------------------------------------------------- multi-GPU: NVLink peer exchange */
 /* The exchange steps of weight() fused into the producing kernels: every rank owns a window in its HBM
- * that all peers map with CUDA IPC; aabb -> peer stores of the crop box + flag barrier, and the kernel
- * that finishes the raw weights stores them straight into every rank's window (it IS the all-gather);
- * normalizeWeight waits on the flag.  No NCCL call is made per frame.  Call order on every rank (one
+ * that all peers map with CUDA IPC; aabb -> peer stores of the crop box + flag barrier, and normalizeWeight
+ * sums this rank's raw weights, stores them straight into every rank's window (it IS the all-gather) and
+ * waits on the flag.  No NCCL call is made per frame.  Call order on every rank (one
  * process per GPU, same node): pft_tracker_set_shard (or _comm_init) -> particle numbers ->
  * pft_tracker_peer_export -> the host framework all-gathers the PFT_PEER_HANDLE_BYTES handles in rank
  * order -> pft_tracker_peer_attach -> compute().  Results are bit-identical to the NCCL path and to the

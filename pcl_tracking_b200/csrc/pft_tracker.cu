@@ -10,9 +10,10 @@
 // Everything a frame needs lives on the device (particle set, live particle count, crop box, index
 // header, weights, representative state), so one compute() is a fixed kernel sequence without a host
 // round trip; in steady state the sequence is replayed from a CUDA graph.  Multi-GPU: particle i is
-// weighted by rank i % nranks; the crop box is all-reduced and the raw weights all-gathered over NCCL
-// (loaded with dlopen so that the library itself has no link-time NCCL dependency); resample, normalise
-// and update run replicated on every rank from identical draws.
+// weighted by rank i % nranks; the crop box is all-reduced and the raw weights all-gathered either by
+// aabb_kernel and normalize_kernel themselves through NVLink peer windows, or over NCCL (loaded with
+// dlopen so that the library itself has no link-time NCCL dependency); resample, normalise and update
+// run replicated on every rank from identical draws.
 #include <dlfcn.h>
 #include <math.h>
 #include <stdio.h>
@@ -141,7 +142,6 @@ struct pft_tracker {
   struct Follower { pft_context* ctx = nullptr; pft_tracker* t = nullptr; pft_cloud* scene = nullptr; pft_cloud* model = nullptr; cudaEvent_t scene_ready = nullptr, scene_free = nullptr; bool free_recorded = false; };
   std::vector<Follower> followers;
   bool md_attached = false, md_prepared = false;
-  bool peer_fused = false;  // inside compute(): the box exchange rides on aabb_kernel, the raw-weight push on normalize_kernel (the phase API keeps the separate kernels)
   void* peer_local = nullptr;
   size_t peer_bytes = 0;
   PeerSet peers{};
@@ -576,28 +576,27 @@ int weight_phase_box(pft_tracker* t) {
   stage_mark(t, "matrices_kernel");
   if (t->n_slots <= sm * 32) {
     aabb_kernel<4><<<std::min(t->n_slots, sm * 16), 128, 0, s>>>(st, t->model.as<float4>(), t->M, t->mats.as<float>(), t->slot_aabb.as<float>(), t->n_slots,
-                                                                t->nranks, t->rank, t->peers, t->peer_fused ? 1 : 0);
+                                                                t->nranks, t->rank, t->peers, t->peer_mode ? 1 : 0);
   } else {
     aabb_kernel<1><<<std::min(t->n_slots, sm * 64), 32, 0, s>>>(st, t->model.as<float4>(), t->M, t->mats.as<float>(), t->slot_aabb.as<float>(), t->n_slots,
-                                                               t->nranks, t->rank, t->peers, t->peer_fused ? 1 : 0);
+                                                               t->nranks, t->rank, t->peers, t->peer_mode ? 1 : 0);
   }
   PFT_LAUNCH_CHECK();
   stage_mark(t, "aabb_kernel");
   return PFT_OK;
 }
 
-// crop box exchange: union over ranks
+// Who moves the crop box and the raw weights of a sharded weight() between the ranks: in NVLink peer mode the kernels
+// themselves (aabb_kernel, normalize_kernel); with a communicator NCCL; with manual shards (pft_tracker_set_shard) the
+// caller.  With one rank or in peer mode normalize_kernel sums the raw weights from the partials; otherwise
+// raw_weights_kernel first writes this rank's slice of the gathered buffer.
+bool nccl_exchange(const pft_tracker* t) { return t->comm && !t->peer_mode; }
+bool normalize_sums_partials(const pft_tracker* t) { return t->nranks == 1 || t->peer_mode; }
+
+// crop box exchange over NCCL: union over ranks
 int weight_comm_box(pft_tracker* t) {
   cudaStream_t s = t->run_stream();
   TrackerState* st = t->st.as<TrackerState>();
-  if (t->peer_mode && t->peer_fused) return PFT_OK;  // (exchanged by the last block of aabb_kernel)
-  if (t->peer_mode) {
-    peer_box_exchange_kernel<<<1, 32, 0, s>>>(st, t->peers);
-    PFT_LAUNCH_CHECK();
-    stage_mark(t, "peer_box_exchange_kernel");
-    return PFT_OK;
-  }
-  if (!t->comm) return PFT_OK;
   PFT_NCCL_TRY(g_nccl.GroupStart());
   PFT_NCCL_TRY(g_nccl.AllReduce(st->aabb, st->aabb, 3, kNcclFloat, kNcclMin, t->comm, s));
   PFT_NCCL_TRY(g_nccl.AllReduce(st->aabb + 3, st->aabb + 3, 3, kNcclFloat, kNcclMax, t->comm, s));
@@ -620,20 +619,18 @@ int timed_lookup(pft_tracker* t, const char* name, Launch launch) {
   return PFT_OK;
 }
 
-// Per-chunk partials -> this rank's raw weights, when a stage reads them: the phase API (force_raw) and the sharded
-// exchanges.  (Single rank, or peer mode inside compute(): normalize_kernel sums the partials itself.)
-int launch_raw_weights(pft_tracker* t, bool force_raw) {
-  if (!force_raw && (t->nranks == 1 || t->peer_fused)) return PFT_OK;
+// Per-chunk partials -> this rank's slice of the gathered raw weights
+int launch_raw_weights(pft_tracker* t) {
   const int local_cap = t->slice_cap();
   raw_weights_kernel<<<blocks_for(local_cap, 256, t->ctx->sm_count * 4), 256, 0, t->run_stream()>>>(
-      t->st.as<TrackerState>(), t->partial.as<double>(), t->chunks, t->n_cap, t->raw.as<float>(), local_cap, t->nranks, t->rank, t->peers, t->peer_mode ? 1 : 0);
+      t->st.as<TrackerState>(), t->partial.as<double>(), t->chunks, t->n_cap, t->raw.as<float>(), local_cap, t->nranks, t->rank);
   PFT_LAUNCH_CHECK();
   stage_mark(t, "raw_weights_kernel");
   return PFT_OK;
 }
 
 // Parity mode PFT_NN_PCL_APPROX (see octree_build_kernel): the octree of the cropped cloud and the greedy search
-int weight_eval_pcl_approx(pft_tracker* t, bool force_raw) {
+int weight_eval_pcl_approx(pft_tracker* t) {
   cudaStream_t s = t->run_stream();
   const int sm = t->ctx->sm_count;
   TrackerState* st = t->st.as<TrackerState>();
@@ -648,9 +645,7 @@ int weight_eval_pcl_approx(pft_tracker* t, bool force_raw) {
   w.partial = t->partial.as<double>(); w.chunks = t->chunks; w.chunk_len = t->chunk_len; w.n_max = t->n_cap; w.nranks = t->nranks; w.rank_id = t->rank;
   w.co = make_coherence(t);
   w.dbg_k = t->debug_nn; w.dbg_idx = t->dbg_idx.as<int>(); w.dbg_d2 = t->dbg_d2.as<float>();
-  int rc = timed_lookup(t, "weight_approx_kernel", [&] { weight_approx_kernel<<<sm * 8, 256, 0, s>>>(w); });
-  if (rc) return rc;
-  return launch_raw_weights(t, force_raw);
+  return timed_lookup(t, "weight_approx_kernel", [&] { weight_approx_kernel<<<sm * 8, 256, 0, s>>>(w); });
 }
 
 // crop box -> index header (also what in_crop() reads) + reset of the per-weight() counters
@@ -669,7 +664,7 @@ int launch_index_begin(pft_tracker* t, bool reuse_allowed = false) {
 }
 
 // weight(), part 2: cropInputPointCloud + search index rebuild (K2), coherence of this rank's particles (K3)
-int weight_phase_eval(pft_tracker* t, bool force_raw = false, bool reuse_allowed = false) {
+int weight_phase_eval(pft_tracker* t, bool reuse_allowed = false) {
   int rc = check_weight_ready(t);
   if (rc) return rc;
   cudaStream_t s = t->run_stream();
@@ -730,7 +725,7 @@ int weight_phase_eval(pft_tracker* t, bool force_raw = false, bool reuse_allowed
     PFT_LAUNCH_CHECK();
     stage_mark(t, "cand_octant_kernel");
   }
-  if (t->nn_mode == PFT_NN_PCL_APPROX) return weight_eval_pcl_approx(t, force_raw);
+  if (t->nn_mode == PFT_NN_PCL_APPROX) return weight_eval_pcl_approx(t);
   WeightArgs a;
   a.st = st; a.hdr = hdr; a.pts2 = t->ipts2.as<float4>();
   a.flists = t->flists.as<unsigned int>(); a.pool = t->fpool.as<unsigned int>(); a.xlists = t->xlists.as<unsigned int>();
@@ -747,7 +742,7 @@ int weight_phase_eval(pft_tracker* t, bool force_raw = false, bool reuse_allowed
   const long long n_local = std::max(1, (t->particle_num > 0 ? t->particle_num : t->n_cap) / t->nranks);
   const bool dyn = n_local * t->chunks >= kDynItemsPerWarp * sm * (kListThreads / 32);
   // one launch either way: it runs the row-table search itself when the index header says the lists are off
-  rc = timed_lookup(t, "weight_lists_kernel", [&] {
+  return timed_lookup(t, "weight_lists_kernel", [&] {
     if (n_local * t->M >= kListBigQueries) {
       if (t->use_hsv) weight_lists_kernel<true, kListThreadsBig, true><<<wgrid, kListThreadsBig, t->lists_smem, s>>>(a);
       else weight_lists_kernel<false, kListThreadsBig, true><<<wgrid, kListThreadsBig, t->lists_smem, s>>>(a);
@@ -759,13 +754,10 @@ int weight_phase_eval(pft_tracker* t, bool force_raw = false, bool reuse_allowed
       else weight_lists_kernel<false, kListThreads, false><<<wgrid, kListThreads, t->lists_smem, s>>>(a);
     }
   });
-  if (rc) return rc;
-  return launch_raw_weights(t, force_raw);
 }
 
-// raw weight exchange: every rank ends up with all raw weights
+// raw weight exchange over NCCL: every rank ends up with all raw weights
 int weight_comm_raw(pft_tracker* t) {
-  if (t->peer_mode || !t->comm) return PFT_OK;  // peer mode: raw_weights_kernel has already pushed the values
   const int local_cap = t->slice_cap();
   PFT_NCCL_TRY(g_nccl.AllGather(t->raw.as<float>() + (size_t)t->rank * local_cap, t->raw.as<float>(), (size_t)local_cap, kNcclFloat, t->comm,
                                 t->run_stream()));
@@ -776,11 +768,9 @@ int weight_comm_raw(pft_tracker* t) {
 int weight_phase_normalize(pft_tracker* t, bool fuse_update = false) {
   int rc = check_weight_ready(t);
   if (rc) return rc;
-  const bool push = t->peer_fused;  // (the launch pushes this rank's raw weights to the peers itself)
   launch_replicated(t, normalize_kernel<1>, normalize_kernel<kClusterCtas>, t->st.as<TrackerState>(), t->parts[t->cur].as<DevParticle>(), t->raw.as<float>(),
-                    t->alpha, t->nranks, t->slice_cap(), t->input->d_hdr(), t->peer_mode ? reinterpret_cast<PeerWindow*>(t->peer_local) : nullptr, t->M,
-                    t->nranks == 1 ? t->partial.as<double>() : nullptr, t->chunks, t->n_cap, t->raw.as<float>(), fuse_update ? 1 : 0, t->peers,
-                    push ? t->partial.as<double>() : nullptr, t->rank);
+                    t->alpha, t->nranks, t->slice_cap(), t->input->d_hdr(), t->M, normalize_sums_partials(t) ? t->partial.as<double>() : nullptr,
+                    t->chunks, t->n_cap, fuse_update ? 1 : 0, t->peers);
   PFT_LAUNCH_CHECK();
   stage_mark(t, "normalize_kernel");
   t->changed = true;  // change detector is off upstream => changed_ = true after every weight()
@@ -821,7 +811,7 @@ int weight_phase_renormalize(pft_tracker* t) {
   PFT_LAUNCH_CHECK();
   stage_mark(t, "weights_to_raw_kernel");
   launch_replicated(t, normalize_kernel<1>, normalize_kernel<kClusterCtas>, st, parts, t->raw.as<float>(), t->alpha, t->nranks, t->slice_cap(),
-                    t->input->d_hdr(), nullptr, 0, nullptr, t->chunks, t->n_cap, t->raw.as<float>(), 0, t->peers, nullptr, t->rank);
+                    t->input->d_hdr(), 0, nullptr, t->chunks, t->n_cap, 0, t->peers);
   PFT_LAUNCH_CHECK();
   stage_mark(t, "normalize_kernel");
   t->changed = false;
@@ -830,12 +820,8 @@ int weight_phase_renormalize(pft_tracker* t) {
 
 int stage_weight(pft_tracker* t, bool fuse_update = false, bool reuse_allowed = false) {
   int rc;
-  // NVLink peer mode: weight() as a whole fuses the two exchanges into aabb_kernel / normalize_kernel; the phase API
-  // (pft_tracker_weight_phase: tests that emulate several ranks on one GPU) keeps the separate exchange kernels
-  struct Fused { pft_tracker* t; ~Fused() { t->peer_fused = false; } } fused{t};
-  t->peer_fused = t->peer_mode && t->nn_mode == PFT_NN_EXACT;
   if ((rc = weight_phase_box(t))) return rc;
-  if ((rc = weight_comm_box(t))) return rc;
+  if (nccl_exchange(t) && (rc = weight_comm_box(t))) return rc;
   if (t->use_cd && t->nranks > 1) { set_last_error("the change detector is not supported on a sharded tracker"); return PFT_ERR_STATE; }
   if (t->use_cd) {
     // change_counter_ (upstream weight()): a test every `interval` calls; nothing new => the weights are not recomputed
@@ -848,8 +834,11 @@ int stage_weight(pft_tracker* t, bool fuse_update = false, bool reuse_allowed = 
       --t->change_counter;
     }
   }
-  if ((rc = weight_phase_eval(t, false, reuse_allowed))) return rc;
-  if ((rc = weight_comm_raw(t))) return rc;
+  if ((rc = weight_phase_eval(t, reuse_allowed))) return rc;
+  if (!normalize_sums_partials(t)) {
+    if ((rc = launch_raw_weights(t))) return rc;
+    if (nccl_exchange(t) && (rc = weight_comm_raw(t))) return rc;
+  }
   return weight_phase_normalize(t, fuse_update);
 }
 
@@ -1285,7 +1274,6 @@ static int preload_kernels() {
       (const void*)normalize_kernel<1>,
       (const void*)normalize_kernel<kClusterCtas>,
       (const void*)octree_build_kernel,
-      (const void*)peer_box_exchange_kernel,
       (const void*)raw_weights_kernel,
       (const void*)resample_kernel,
       (const void*)result_box_kernel,
@@ -1757,15 +1745,19 @@ int pft_tracker_get_kernel_times(pft_tracker* t, const char** names, float* ms, 
 
 // weight() in its three parts, with the two exchange points exposed, so that a sharded run can be
 // driven (and tested) without a communicator: 0 = transforms + local crop box, 1 = index + coherence of
-// the local particles, 2 = normalise.
+// the local particles, 2 = normalise.  A peer-attached tracker exchanges inside its kernels: it refuses.
 int pft_tracker_weight_phase(pft_tracker* t, int phase) {
   if (!t) { set_last_error("null tracker"); return PFT_ERR_INVALID; }
+  if (t->peer_mode) { set_last_error("the phase API leaves the exchanges to the caller: not on a tracker attached to peer windows"); return PFT_ERR_STATE; }
   PFT_CUDA_TRY(cudaSetDevice(t->ctx->device));
   int rc = prepare_compute(t);
   if (rc) return rc;
   switch (phase) {
     case 0: return weight_phase_box(t);
-    case 1: if (t->timing) t->n_ev_used = 0; return weight_phase_eval(t, true);  // (raw slices are readable between the phases)
+    case 1:  // (raw slices are readable between the phases)
+      if (t->timing) t->n_ev_used = 0;
+      if ((rc = weight_phase_eval(t))) return rc;
+      return launch_raw_weights(t);
     case 2: return weight_phase_normalize(t);
     default: set_last_error("phase must be 0, 1 or 2"); return PFT_ERR_INVALID;
   }

@@ -42,7 +42,6 @@ struct TrackerState {
   // cell size of the next index build.  Integer sums: independent of the order the atomics land in.
   unsigned long long nn_sum_um, nn_count;
   unsigned int peer_epoch;       // weight() calls so far in peer (NVLink P2P) exchange mode
-  unsigned int peer_blocks_done; // raw_weights_kernel blocks that have pushed their slice this epoch
   unsigned int peer_error;       // a wait on a peer's flag timed out (sticky)
   int resample_n_old;            // particle count the running resample draws FROM (cdf_kernel publishes the new count for fixed-N trackers)
   unsigned int work_counter;     // next (particle, model chunk) item of the running weight kernel (reset by index_begin_kernel)
@@ -53,8 +52,9 @@ struct TrackerState {
 // ------------------------------------------------------------------ NVLink peer exchange (one process per GPU)
 // Every rank owns one PeerWindow in its HBM, mapped into all peers with CUDA IPC.  The two exchange steps of weight()
 // are plain peer stores issued by the producing kernels themselves, followed by a flag barrier:
-//   crop box    every rank stores its six values into slot [rank] of every window, signals, waits, reduces locally;
-//   raw weights raw_weights_kernel stores every value into every window; its last block signals; normalize_kernel waits.
+//   crop box    the last block of aabb_kernel stores this rank's six values into slot [rank] of every window, signals,
+//               waits, reduces locally;
+//   raw weights normalize_kernel sums this rank's raw weights, stores every value into every window, signals, waits.
 // Flags only ever grow (epoch numbered), so nothing has to be reset between frames or graph replays.  The box slots
 // are double-buffered by epoch parity; the raw-weight area needs no second buffer: a rank can only push the weights of
 // epoch e+1 after it has passed the box barrier of e+1, which every rank enters after its normalize of epoch e.
@@ -81,14 +81,13 @@ __device__ __forceinline__ bool peer_wait(volatile unsigned int* flag, unsigned 
   return true;
 }
 
-// crop box all-reduce over NVLink: one warp.  Runs right after aabb_kernel.
 // Crop-box exchange by one warp: every rank stores its six values into slot [rank] of every window, raises every rank's
 // flag, waits for its own to show all ranks of this epoch, reduces locally (an all-reduce(min/max) without a collective).
 __device__ __forceinline__ void peer_box_exchange(TrackerState* st, const PeerSet& ps) {
   const int lane = threadIdx.x & 31;
   PeerWindow* me = ps.win[ps.rank];
   unsigned int e = 0;
-  if (lane == 0) { e = st->peer_epoch + 1u; st->peer_epoch = e; st->peer_blocks_done = 0u; }
+  if (lane == 0) { e = st->peer_epoch + 1u; st->peer_epoch = e; }
   e = __shfl_sync(kFull, e, 0);
   const int cur = e & 1u;
   // lane = (destination rank, component): 8 floats to each of up to 4 ranks per pass
@@ -115,7 +114,6 @@ __device__ __forceinline__ void peer_box_exchange(TrackerState* st, const PeerSe
     st->aabb[lane] = v;
   }
 }
-__global__ void peer_box_exchange_kernel(TrackerState* st, PeerSet ps) { peer_box_exchange(st, ps); }
 
 // ---- scene distribution by peer stores: ONE rank owns the sensor (upload + downsample), its kernel stores the
 // downsampled cloud straight into the cloud of every other rank over NVLink (CUDA IPC mappings) and raises their
@@ -2420,33 +2418,20 @@ __global__ void weights_to_raw_kernel(const TrackerState* st, const DevParticle*
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) raw[raw_slot(i, nranks, slice_cap)] = parts[i].weight;
 }
 
-// raw weight = -(float)sum over chunks (fixed order).  In peer mode the kernel IS the all-gather: every value is
-// stored into every rank's window over NVLink and the last block to finish raises the peers' flags.
-__global__ void raw_weights_kernel(TrackerState* st, const double* __restrict__ partial, int chunks, int n_max,
-                                   float* __restrict__ raw, int slice_cap, int nranks, int rank, PeerSet ps, int peer_mode) {
+// Particle i's raw weight: -(float) of its per-chunk partials summed in the fixed chunk order.  Every path that turns
+// partials into raw weights sums here, which is what keeps sharded and unsharded weights bit-identical.
+__device__ __forceinline__ float raw_weight(const double* __restrict__ partial, int chunks, int n_max, int i) {
+  double v = 0.0;
+  for (int c = 0; c < chunks; ++c) v += partial[(size_t)c * n_max + i];
+  return -(float)v;
+}
+
+// this rank's raw weights into its slice of the gathered buffer [nranks][slice_cap]
+__global__ void raw_weights_kernel(const TrackerState* st, const double* __restrict__ partial, int chunks, int n_max,
+                                   float* __restrict__ raw, int slice_cap, int nranks, int rank) {
   const int n = st->particle_num;
-  for (int l = blockIdx.x * blockDim.x + threadIdx.x; rank + l * nranks < n; l += gridDim.x * blockDim.x) {
-    const int i = rank + l * nranks;
-    double v = 0.0;
-    for (int c = 0; c < chunks; ++c) v += partial[(size_t)c * n_max + i];
-    const float w = -(float)v;
-    if (peer_mode) {
-      for (int r = 0; r < nranks; ++r) ps.win[r]->raw[rank * slice_cap + l] = w;
-    } else {
-      raw[rank * slice_cap + l] = w;
-    }
-  }
-  if (peer_mode) {
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      __threadfence_system();  // one system-scope fence per block, after the barrier (cumulative over the block's stores)
-      const unsigned int done = atomicAdd(&st->peer_blocks_done, 1u) + 1u;
-      if (done == gridDim.x) {  // every block of this rank has pushed its values
-        __threadfence_system();
-        for (int r = 0; r < nranks; ++r) atomicAdd_system(&ps.win[r]->flag_raw, 1u);
-      }
-    }
-  }
+  for (int l = blockIdx.x * blockDim.x + threadIdx.x; rank + l * nranks < n; l += gridDim.x * blockDim.x)
+    raw[rank * slice_cap + l] = raw_weight(partial, chunks, n_max, rank + l * nranks);
 }
 
 // ------------------------------------------------------------------ K4a: normalizeWeight
@@ -2458,17 +2443,48 @@ __global__ void raw_weights_kernel(TrackerState* st, const double* __restrict__ 
 namespace cg = cooperative_groups;
 constexpr int kClusterCtas = 8;
 
+// ParticleFilterTracker::update: rep = the weighted sum of the particles' states, motion = its change.  Every thread
+// sums the particles particle(i) of its slice, then the CTA (block_sum6), then the CTAs of the cluster in their fixed
+// order.  update_kernel and the update fused into normalize_kernel both run this: the same result bit for bit.
+template <int CTAS, typename Particle>
+__device__ __forceinline__ void update_state(TrackerState* st, int n, Particle particle, double* red6 /* shared [192] */,
+                                             double* s_part /* shared [6] */) {
+  cg::cluster_group cluster = cg::this_cluster();
+  const unsigned int crank = cluster.block_rank();
+  double acc[6] = {0, 0, 0, 0, 0, 0};
+  for (int i = crank * blockDim.x + threadIdx.x; i < n; i += CTAS * blockDim.x) {
+    const DevParticle p = particle(i);
+    const double w = (double)p.weight;
+    acc[0] += (double)(float)((double)p.x * w); acc[1] += (double)(float)((double)p.y * w); acc[2] += (double)(float)((double)p.z * w);
+    acc[3] += (double)(float)((double)p.roll * w); acc[4] += (double)(float)((double)p.pitch * w); acc[5] += (double)(float)((double)p.yaw * w);
+  }
+  block_sum6(acc, red6);
+  if (threadIdx.x == 0) {
+#pragma unroll
+    for (int d = 0; d < 6; ++d) s_part[d] = acc[d];
+  }
+  cluster.sync();
+  if (crank == 0 && threadIdx.x == 0) {
+    double tot[6] = {0, 0, 0, 0, 0, 0};
+    for (int r = 0; r < CTAS; ++r) {  // fixed order
+      const double* p = cluster.map_shared_rank(s_part, r);
+      for (int d = 0; d < 6; ++d) tot[d] += p[d];
+    }
+    const DevParticle o = st->rep;
+    DevParticle r{(float)tot[0], (float)tot[1], (float)tot[2], 1.f, (float)tot[3], (float)tot[4], (float)tot[5], 1.0f / (float)n};
+    st->rep = r;
+    st->motion = DevParticle{r.x - o.x, r.y - o.y, r.z - o.z, 1.f, r.roll - o.roll, r.pitch - o.pitch, r.yaw - o.yaw, 0.f};
+  }
+}
+
 template <int CTAS>
 __global__ void __cluster_dims__(CTAS, 1, 1) __launch_bounds__(1024)
-normalize_kernel(TrackerState* st, DevParticle* parts, const float* raw, double alpha, int nranks, int slice_cap,
-                 const CloudHeader* __restrict__ scene_hdr, PeerWindow* peer_window /* non-null: wait for the peers' raw weights */, int M,
-                 const double* __restrict__ partial /* non-null (single rank): the raw weights are summed here from the weight kernel's
-                                                       per-chunk partials instead of by raw_weights_kernel */,
-                 int chunks, int n_max, float* raw_out, int fuse_update /* compute(): update() follows every weight(), do it in the same launch */,
-                 PeerSet ps, const double* __restrict__ push_partial /* non-null (NVLink peer mode): this rank's raw weights are summed from these
-                                                                       per-chunk partials and stored straight into EVERY rank's window first -- this
-                                                                       launch is the all-gather, no raw_weights_kernel in between */,
-                 int rank) {
+normalize_kernel(TrackerState* st, DevParticle* parts, float* raw /* [nranks][slice_cap] gathered raw weights */, double alpha, int nranks,
+                 int slice_cap, const CloudHeader* __restrict__ scene_hdr, int M,
+                 const double* __restrict__ partial /* non-null: this rank's raw weights are summed here from the weight kernel's
+                                                       per-chunk partials; null: `raw` already holds every rank's */,
+                 int chunks, int n_max, int fuse_update /* compute(): update() follows every weight(), do it in the same launch */,
+                 PeerSet ps /* NVLink peer mode (ps.nranks > 1): this launch is the all-gather of the raw weights */) {
   cg::cluster_group cluster = cg::this_cluster();
   const unsigned int crank = cluster.block_rank();
   PFT_TRACE_MIN(11);
@@ -2476,25 +2492,23 @@ normalize_kernel(TrackerState* st, DevParticle* parts, const float* raw, double 
   __shared__ double s_part[3];  // this CTA's partial min, max, sum (read by the other CTAs of the cluster)
   __shared__ double s_upd[6];   // fused update(): this CTA's partial weighted state
   __shared__ double red6[192];
-  if (peer_window && push_partial) {
+  if (partial && ps.nranks > 1) {
+    // this rank's raw weights go straight into EVERY rank's window, then every rank's flag is raised; once the local
+    // flag shows all ranks of this epoch, the local window holds them all
     const int np = st->particle_num;
-    for (int l = crank * blockDim.x + threadIdx.x; rank + l * nranks < np; l += CTAS * blockDim.x) {
-      const int i = rank + l * nranks;
-      double v = 0.0;
-      for (int c = 0; c < chunks; ++c) v += push_partial[(size_t)c * n_max + i];
-      const float w = -(float)v;
-      for (int r = 0; r < nranks; ++r) ps.win[r]->raw[rank * slice_cap + l] = w;
+    for (int l = crank * blockDim.x + threadIdx.x; ps.rank + l * nranks < np; l += CTAS * blockDim.x) {
+      const float w = raw_weight(partial, chunks, n_max, ps.rank + l * nranks);
+      for (int r = 0; r < nranks; ++r) ps.win[r]->raw[ps.rank * slice_cap + l] = w;
     }
     cluster.sync();  // every store of this rank is issued ...
     if (crank == 0 && threadIdx.x == 0) {
       __threadfence_system();  // ... and ordered (cumulatively) before the flags
       for (int r = 0; r < nranks; ++r) atomicAdd_system(&ps.win[r]->flag_raw, 1u);
+      peer_wait(&ps.win[ps.rank]->flag_raw, st->peer_epoch * (unsigned int)nranks, &st->peer_error);
     }
-  }
-  if (peer_window) {
-    if (crank == 0 && threadIdx.x == 0) peer_wait(&peer_window->flag_raw, st->peer_epoch * (unsigned int)nranks, &st->peer_error);
     cluster.sync();
-    raw = peer_window->raw;
+    raw = ps.win[ps.rank]->raw;
+    partial = nullptr;
   }
   if (scene_hdr->n <= 0) return;  // Tracker::initCompute fails on an empty input cloud: compute() is a no-op
   const int n = st->particle_num;
@@ -2504,11 +2518,9 @@ normalize_kernel(TrackerState* st, DevParticle* parts, const float* raw, double 
   for (int i = first; i < n; i += stride) {
     double w;
     if (partial) {
-      // raw weight = -(float)sum over chunks (fixed order), exactly as raw_weights_kernel (nranks == 1: slot i)
-      double v = 0.0;
-      for (int c = 0; c < chunks; ++c) v += partial[(size_t)c * n_max + i];
-      const float wf = -(float)v;
-      raw_out[i] = wf;
+      // one rank: raw slot i (every thread re-reads below only the slots it writes here)
+      const float wf = raw_weight(partial, chunks, n_max, i);
+      raw[i] = wf;
       w = (double)wf;
     } else {
       w = (double)__ldcg(&raw[raw_slot(i, nranks, slice_cap)]);
@@ -2516,7 +2528,6 @@ normalize_kernel(TrackerState* st, DevParticle* parts, const float* raw, double 
     if (wmin > w) wmin = w;
     if (w != 0.0 && wmax < w) wmax = w;
   }
-  if (partial) raw = raw_out;  // (every thread re-reads only the slots it has just written)
   for (int o = 16; o > 0; o >>= 1) { wmin = fmin(wmin, __shfl_xor_sync(kFull, wmin, o)); wmax = fmax(wmax, __shfl_xor_sync(kFull, wmax, o)); }
   if (lane == 0) { red[wid] = wmin; red6[wid] = wmax; }
   __syncthreads();
@@ -2549,37 +2560,15 @@ normalize_kernel(TrackerState* st, DevParticle* parts, const float* raw, double 
   for (int r = 0; r < CTAS; ++r) sum += cluster.map_shared_rank(s_part, r)[2];  // fixed order
   if (crank == 0 && threadIdx.x == 0) { st->fit_ratio = wmin; st->weight_sum = sum; st->evals += (unsigned long long)n * (unsigned long long)M; }
   const float fs = (float)sum;
-  double acc[6] = {0, 0, 0, 0, 0, 0};
-  for (int i = first; i < n; i += stride) {
+  auto normalized = [&](int i) {
     DevParticle p = parts[i];
     if (sum != 0.0) p.weight = p.weight / fs;
     else p.weight = 1.0f / (float)n;
     parts[i].weight = p.weight;
-    if (fuse_update) {  // the same terms, slices and reduction order as update_kernel: bit-identical result
-      const double w = (double)p.weight;
-      acc[0] += (double)(float)((double)p.x * w); acc[1] += (double)(float)((double)p.y * w); acc[2] += (double)(float)((double)p.z * w);
-      acc[3] += (double)(float)((double)p.roll * w); acc[4] += (double)(float)((double)p.pitch * w); acc[5] += (double)(float)((double)p.yaw * w);
-    }
-  }
-  if (fuse_update) {
-    block_sum6(acc, red6);
-    if (threadIdx.x == 0) {
-#pragma unroll
-      for (int d = 0; d < 6; ++d) s_upd[d] = acc[d];
-    }
-    cluster.sync();
-    if (crank == 0 && threadIdx.x == 0) {
-      double tot[6] = {0, 0, 0, 0, 0, 0};
-      for (int r = 0; r < CTAS; ++r) {  // fixed order
-        const double* p = cluster.map_shared_rank(s_upd, r);
-        for (int d = 0; d < 6; ++d) tot[d] += p[d];
-      }
-      const DevParticle o = st->rep;
-      DevParticle r{(float)tot[0], (float)tot[1], (float)tot[2], 1.f, (float)tot[3], (float)tot[4], (float)tot[5], 1.0f / (float)n};
-      st->rep = r;
-      st->motion = DevParticle{r.x - o.x, r.y - o.y, r.z - o.z, 1.f, r.roll - o.roll, r.pitch - o.pitch, r.yaw - o.yaw, 0.f};
-    }
-  }
+    return p;
+  };
+  if (fuse_update) update_state<CTAS>(st, n, normalized, red6, s_upd);
+  else for (int i = first; i < n; i += stride) normalized(i);
   cluster.sync();  // the partials of this CTA stay readable until every CTA of the cluster is done with them
 }
 
@@ -2587,37 +2576,11 @@ normalize_kernel(TrackerState* st, DevParticle* parts, const float* raw, double 
 template <int CTAS>
 __global__ void __cluster_dims__(CTAS, 1, 1) __launch_bounds__(1024)
 update_kernel(TrackerState* st, const DevParticle* __restrict__ parts, const CloudHeader* __restrict__ scene_hdr) {
-  cg::cluster_group cluster = cg::this_cluster();
-  const unsigned int crank = cluster.block_rank();
   __shared__ double red6[192];
   __shared__ double s_part[6];
   if (scene_hdr->n <= 0) return;
-  const int n = st->particle_num;
-  double acc[6] = {0, 0, 0, 0, 0, 0};
-  for (int i = crank * blockDim.x + threadIdx.x; i < n; i += CTAS * blockDim.x) {
-    const DevParticle p = parts[i];
-    const double w = (double)p.weight;
-    acc[0] += (double)(float)((double)p.x * w); acc[1] += (double)(float)((double)p.y * w); acc[2] += (double)(float)((double)p.z * w);
-    acc[3] += (double)(float)((double)p.roll * w); acc[4] += (double)(float)((double)p.pitch * w); acc[5] += (double)(float)((double)p.yaw * w);
-  }
-  block_sum6(acc, red6);
-  if (threadIdx.x == 0) {
-#pragma unroll
-    for (int d = 0; d < 6; ++d) s_part[d] = acc[d];
-  }
-  cluster.sync();
-  if (crank == 0 && threadIdx.x == 0) {
-    double tot[6] = {0, 0, 0, 0, 0, 0};
-    for (int r = 0; r < CTAS; ++r) {  // fixed order
-      const double* p = cluster.map_shared_rank(s_part, r);
-      for (int d = 0; d < 6; ++d) tot[d] += p[d];
-    }
-    const DevParticle o = st->rep;
-    DevParticle r{(float)tot[0], (float)tot[1], (float)tot[2], 1.f, (float)tot[3], (float)tot[4], (float)tot[5], 1.0f / (float)n};
-    st->rep = r;
-    st->motion = DevParticle{r.x - o.x, r.y - o.y, r.z - o.z, 1.f, r.roll - o.roll, r.pitch - o.pitch, r.yaw - o.yaw, 0.f};
-  }
-  cluster.sync();
+  update_state<CTAS>(st, st->particle_num, [&](int i) { return parts[i]; }, red6, s_part);
+  cg::this_cluster().sync();
 }
 
 // ------------------------------------------------------------------ K4b: resample

@@ -16,13 +16,23 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 N_PART, N_MAX, FRAMES = 101, 160, 4
 
 
-def _tracker(kld, shard=None, device=0):
+def _coherence(parity):
+    """The default exact search, or the parity search (upstream's greedy octree descent)."""
+    from pcl_tracking_b200 import pcl
+    if not parity:
+        return pcl.NearestPairPointCloudCoherence()
+    c = pcl.ApproxNearestPairPointCloudCoherence()
+    c.setPclApproximateSearch(True)
+    return c
+
+
+def _tracker(kld, shard=None, device=0, parity=False):
     from pcl_tracking_b200 import pcl
     from tests import util
     ctx = pcl.Context(device)
     scene, model, centre = util.small_case(77, n_scene=4000, n_model=260)
     g = (pcl.KLDAdaptiveParticleFilterOMPTracker if kld else pcl.ParticleFilterOMPTracker)(16, ctx=ctx)
-    pcl.configure_like_reference(g, coherence_cls=pcl.NearestPairPointCloudCoherence, particle_num=N_PART, max_particle_num=N_MAX,
+    pcl.configure_like_reference(g, coherence_cls=lambda: _coherence(parity), particle_num=N_PART, max_particle_num=N_MAX,
                                  use_hsv=True, iteration_num=2)
     if kld:
         g.setEpsilon(0.2)
@@ -243,14 +253,14 @@ def test_exported_cloud_refuses_to_grow():
 
 
 # ---------------------------------------------------------------- single-process multi-device mode (pft_tracker_set_devices)
-def _multi_device_tracker(kld, devices):
+def _multi_device_tracker(kld, devices, parity=False):
     from pcl_tracking_b200 import pcl
     from tests import util
     ctx = pcl.Context(devices[0])
     scene, model, centre = util.small_case(77, n_scene=4000, n_model=260)
     g = (pcl.KLDAdaptiveParticleFilterOMPTracker if kld else pcl.ParticleFilterOMPTracker)(16, ctx=ctx)
     g.setDevices(devices)  # first call on the new tracker: the setters below reach every device
-    pcl.configure_like_reference(g, coherence_cls=pcl.NearestPairPointCloudCoherence, particle_num=N_PART, max_particle_num=N_MAX,
+    pcl.configure_like_reference(g, coherence_cls=lambda: _coherence(parity), particle_num=N_PART, max_particle_num=N_MAX,
                                  use_hsv=True, iteration_num=2)
     if kld:
         g.setEpsilon(0.2)
@@ -265,17 +275,18 @@ def _multi_device_tracker(kld, devices):
     return ctx, g, cloud
 
 
-@pytest.mark.parametrize("kld,n_dev", [(False, 2), (True, 3)])
-def test_one_tracker_object_drives_several_devices(kld, n_dev):
+@pytest.mark.parametrize("kld,n_dev,parity", [(False, 2, False), (True, 3, False), (False, 2, True)], ids=["False-2", "True-3", "parity-False-2"])
+def test_one_tracker_object_drives_several_devices(kld, n_dev, parity):
     """One process, one tracker object, n ranks: bit-identical to the plain single-GPU tracker over several frames (graph
-    replays included).  With fewer GPUs than ranks the ranks share GPU 0 (two contexts of this process on one device)."""
+    replays included), with the exact search and with the parity search.  With fewer GPUs than ranks the ranks share
+    GPU 0 (two contexts of this process on one device)."""
     import torch
     have = torch.cuda.device_count()
     devices = list(range(n_dev)) if have >= n_dev else [0] * n_dev
-    ctx, g, cloud = _multi_device_tracker(kld, devices)
+    ctx, g, cloud = _multi_device_tracker(kld, devices, parity)
     got = _run(g)
     assert g.graphReplays() >= 1
-    ctx1, g1, cloud1 = _tracker(kld)
+    ctx1, g1, cloud1 = _tracker(kld, parity=parity)
     want = _run(g1)
     for f in range(FRAMES):
         for j, name in enumerate(("particles", "raw weights", "result")):
@@ -293,3 +304,13 @@ def test_set_devices_must_come_first():
     g.compute()
     with pytest.raises(pcl.PftError):
         g.setDevices([0, 0])
+
+
+def test_weight_phase_refuses_a_peer_attached_tracker():
+    """The phase API leaves the exchanges to its caller, so a tracker whose kernels exchange through peer windows refuses
+    it: a host check, before anything is launched."""
+    from pcl_tracking_b200 import pcl
+    ctx, g, cloud = _multi_device_tracker(False, [0, 0])
+    g.compute()
+    with pytest.raises(pcl.PftError):
+        g.weightPhase(0)
