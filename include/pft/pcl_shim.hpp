@@ -95,24 +95,51 @@ class Context {
   pft_context* h_ = nullptr;
 };
 
+// a device list "0,1,..." from the environment (empty when unset)
+inline std::vector<int> devicesFromEnv(const char* name) {
+  std::vector<int> v;
+  if (const char* e = std::getenv(name)) {
+    for (const char* p = e; *p;) {
+      char* end = nullptr;
+      const long d = std::strtol(p, &end, 10);
+      if (end == p) break;
+      v.push_back((int)d);
+      p = (*end == ',') ? end + 1 : end;
+    }
+  }
+  return v;
+}
+
 // GPUs driven by every tracker constructed afterwards (single-process multi-device mode, pft_tracker_set_devices)
 inline std::vector<int>& trackerDevices() {
-  static std::vector<int> devs = [] {
-    std::vector<int> v;
-    if (const char* e = std::getenv("PFT_DEVICES")) {
-      for (const char* p = e; *p;) {
-        char* end = nullptr;
-        const long d = std::strtol(p, &end, 10);
-        if (end == p) break;
-        v.push_back((int)d);
-        p = (*end == ',') ? end + 1 : end;
-      }
-    }
-    return v;
-  }();
+  static std::vector<int> devs = devicesFromEnv("PFT_DEVICES");
   return devs;
 }
 inline void setTrackerDevices(const std::vector<int>& devices) { trackerDevices() = devices; }
+
+// One object per GPU: the k-th tracker constructed afterwards lives on devices[k % n], in one context per device (created
+// on first use, apart from the default context).  Clouds and filters stay on the default context, the sensor's; every
+// tracker takes the scene from there (pft_tracker_set_input_cloud with a cloud of another context), so the reference's
+// loop setInputCloud(scene); compute() spreads over the GPUs unchanged.  The list comes from pft::setObjectDevices({0,
+// 1, ...}) or the environment (PFT_OBJECT_DEVICES=0,1,...).  It excludes the multi-device mode of one tracker.
+inline std::vector<int>& objectDevices() {
+  static std::vector<int> devs = devicesFromEnv("PFT_OBJECT_DEVICES");
+  return devs;
+}
+inline void setObjectDevices(const std::vector<int>& devices) { objectDevices() = devices; }
+// the context of the next tracker: the default one without object devices
+inline std::shared_ptr<Context> nextTrackerContext() {
+  const std::vector<int>& devs = objectDevices();
+  if (devs.empty()) return Context::Default();
+  if (trackerDevices().size() > 1) throw Error(PFT_ERR_INVALID, "object devices (PFT_OBJECT_DEVICES) and tracker devices (PFT_DEVICES) exclude each other");
+  static std::vector<std::shared_ptr<Context>> per_device;
+  static size_t constructed = 0;
+  const int dev = devs[constructed++ % devs.size()];
+  if (dev < 0) throw Error(PFT_ERR_INVALID, "negative object device");
+  if (per_device.size() <= (size_t)dev) per_device.resize(dev + 1);
+  if (!per_device[dev]) per_device[dev] = std::make_shared<Context>(dev);
+  return per_device[dev];
+}
 
 }  // namespace pft
 
@@ -483,7 +510,7 @@ class ParticleFilterTracker {
   typedef typename CloudCoherence::Ptr CloudCoherencePtr;
   typedef CloudCoherencePtr CoherencePtr;                                                         // ref :154
   ParticleFilterTracker() : ParticleFilterTracker(0, 0) {}
-  virtual ~ParticleFilterTracker() { pft_tracker_destroy(h_); }
+  virtual ~ParticleFilterTracker() { pft_tracker_destroy(h_); }  // (before ctx_ lets go of the context)
   ParticleFilterTracker(const ParticleFilterTracker&) = delete;
   ParticleFilterTracker& operator=(const ParticleFilterTracker&) = delete;
   // any affine type with operator()(row, col): Eigen::Affine3f (ref :225, :674), pft::Affine3f
@@ -556,8 +583,8 @@ class ParticleFilterTracker {
   pft_tracker* handle() const { return h_; }
 
  protected:
-  ParticleFilterTracker(unsigned int nr_threads, int kld) {
-    pft::check(pft_tracker_create(pft::Context::Default()->get(), kld, &h_));
+  ParticleFilterTracker(unsigned int nr_threads, int kld) : ctx_(pft::nextTrackerContext()) {
+    pft::check(pft_tracker_create(ctx_->get(), kld, &h_));
     // single-process multi-device mode: the reference's constructor call (ref :201, :215) cannot name GPUs, so the
     // list comes from pft::setTrackerDevices({0, 1, ...}) or the environment (PFT_DEVICES=0,1,...); first = device 0
     const std::vector<int>& devs = pft::trackerDevices();
@@ -570,6 +597,7 @@ class ParticleFilterTracker {
     if (v.size() != 6) throw pft::Error(PFT_ERR_INVALID, "expected 6 values");
     pft::check(pft_tracker_set_vec6(h_, k, v.data()));
   }
+  std::shared_ptr<pft::Context> ctx_;
   pft_tracker* h_ = nullptr;
   PointCloudInConstPtr ref_, input_;
   CloudCoherencePtr coherence_;

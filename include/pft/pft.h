@@ -203,16 +203,24 @@ PFT_API int pft_tracker_set_vec6(pft_tracker* t, int key, const double* v6);
 /* setTrans(Eigen::Affine3f): row-major 3x4 [R|t] (ref :225, :674) */
 PFT_API int pft_tracker_set_trans(pft_tracker* t, const float* m12);
 /* setReferenceCloud (ref :673): copied into the tracker */
+/* the cloud may belong to another context, as for pft_tracker_set_input_cloud (read once, through a replica) */
 PFT_API int pft_tracker_set_reference_cloud(pft_tracker* t, const pft_cloud* cloud);
 PFT_API int pft_tracker_set_reference_points(pft_tracker* t, const void* host_points, size_t n, int layout);
-/* setInputCloud (ref :691): the cloud handle is borrowed until the next set_input/compute pair */
+/* setInputCloud (ref :691): the cloud handle is borrowed until the next set_input/compute pair.  The cloud may belong
+ * to another context, on the same device or another one (one object per GPU): the tracker's context then reads a
+ * replica of it, shared by all its trackers and refreshed by one fan-out launch on the cloud's stream when a library
+ * call has written the cloud since.  This call enables peer access from the cloud's device to the tracker's (and its
+ * followers') devices: PFT_ERR_COMM where that is impossible.  A tracker attached to a communicator, a shard
+ * (pft_tracker_set_shard) or peer windows refuses a cloud of another context with PFT_ERR_INVALID. */
 PFT_API int pft_tracker_set_input_cloud(pft_tracker* t, const pft_cloud* cloud);
 
 /* ---------------------------------------------------------------- tracker execution */
 /* Tracker::compute (ref :693): iteration_num x { resample (if changed) ; weight ; update }.
  * Enqueued on the context stream; results are read with the getters below (which synchronise). */
 PFT_API int pft_tracker_compute(pft_tracker* t);
-/* compute() of n independent trackers that share one scene (ref :688-697 loops them serially) */
+/* compute() of n independent trackers that share one scene (ref :688-697 loops them serially).  The trackers may sit
+ * on several contexts: stale scene replicas are refreshed first (one launch per source cloud), then every context's
+ * trackers run concurrently on streams forked from and joined to that context's stream.  The host waits for no device. */
 PFT_API int pft_compute_batch(pft_tracker** trackers, int n);
 /* getResult (ref :309) */
 PFT_API int pft_tracker_get_result(pft_tracker* t, pft_particle* out);

@@ -16,6 +16,7 @@ namespace pft {
 
 static thread_local char g_err[512] = "";
 std::atomic<unsigned long long> g_launch_count{0};
+static std::atomic<unsigned long long> g_cloud_serial{0};
 
 void set_last_error(const char* fmt, ...) {
   va_list ap;
@@ -96,7 +97,7 @@ int end_async_upload(pft_cloud* c, size_t n, cudaStream_t cs) {
   if (rc) return rc;
   PFT_CUDA_TRY(cudaEventRecord(c->ready, cs));
   c->upload_pending = true;
-  c->host_n = (long long)n;
+  c->written((long long)n);
   return PFT_OK;
 }
 
@@ -162,6 +163,7 @@ void pft_context_destroy(pft_context* c) {
   if (!c) return;
   cudaSetDevice(c->device);
   cudaStreamSynchronize(c->stream);
+  release_replicas_in(c);
   pft_context_comm_destroy(c);
   pft::DevBuf* bufs[] = {&c->k1_keys, &c->k1_first, &c->k1_vid, &c->k1_slot_of, &c->k1_acc_xyz, &c->k1_acc_rgbc, &c->k1_blk, &c->staging, &c->tmp_cloud_pts, &c->tmp_hdr, &c->tmp_f,
                          &c->cl_grid, &c->cl_cells, &c->cl_work, &c->cl_sel};
@@ -201,6 +203,7 @@ int pft_cloud_create(pft_context* ctx, pft_cloud** out) {
   PFT_CUDA_TRY(cudaSetDevice(ctx->device));
   pft_cloud* c = new pft_cloud();
   c->ctx = ctx;
+  c->serial = ++g_cloud_serial;
   int rc = c->ensure(0);
   if (rc) { delete c; return rc; }
   rc = launch_set_header(ctx->stream, c->d_hdr(), 0);
@@ -215,6 +218,7 @@ void pft_cloud_destroy(pft_cloud* c) {
   cudaSetDevice(c->ctx->device);
   cudaStreamSynchronize(c->ctx->stream);
   if (c->ready) { cudaEventSynchronize(c->ready); cudaEventDestroy(c->ready); }
+  release_replicas_of(c);
   pft_cloud_peer_detach(c);
   c->pts.release();
   c->hdr.release();
@@ -243,7 +247,7 @@ int pft_cloud_upload(pft_cloud* c, const void* host_points, size_t n, int layout
     }
   }
   if ((rc = launch_set_header(s, c->d_hdr(), (int)n))) return rc;
-  c->host_n = (long long)n;
+  c->written((long long)n);
   return PFT_OK;
 }
 
@@ -266,7 +270,7 @@ int pft_cloud_upload_pointcloud2(pft_cloud* c, const void* data, uint32_t width,
     if ((rc = launch_unpack_pointcloud2(s, ctx->staging.p, c->d_pts(), width, height, point_step, row_step, off_x, off_y, off_z, off_rgb))) return rc;
   }
   if ((rc = launch_set_header(s, c->d_hdr(), (int)n))) return rc;
-  c->host_n = (long long)n;
+  c->written((long long)n);
   return PFT_OK;
 }
 

@@ -331,7 +331,7 @@ int pft_cloud_select_cluster(pft_context* ctx, const pft_cloud* in, int k, pft_c
   const int* dlabels = ctx->cl_work.as<int>() + 4 * ctx->cl_n;
   cl_extract_kernel<<<1, 1024, 0, ctx->stream>>>(in->d_pts(), in->d_hdr(), dlabels, k, out->d_pts(), out->d_hdr());
   PFT_LAUNCH_CHECK();
-  out->host_n = -1;
+  out->written(-1);
   return PFT_OK;
 }
 
@@ -587,8 +587,8 @@ int pft_segment_plane(pft_context* ctx, const pft_cloud* in, double distance_thr
   plane_extract_kernel<<<1, 1024, 0, s>>>(in->d_pts(), in->d_hdr(), distance_threshold, res, plane_out ? plane_out->d_pts() : nullptr,
                                           plane_out ? plane_out->d_hdr() : nullptr, rest_out ? rest_out->d_pts() : nullptr, rest_out ? rest_out->d_hdr() : nullptr);
   PFT_LAUNCH_CHECK();
-  if (plane_out) plane_out->host_n = -1;
-  if (rest_out) rest_out->host_n = -1;
+  if (plane_out) plane_out->written(-1);
+  if (rest_out) rest_out->written(-1);
   PlaneResult h;
   PFT_CUDA_TRY(cudaMemcpyAsync(&h, res, sizeof(h), cudaMemcpyDeviceToHost, s));
   PFT_CUDA_TRY(cudaStreamSynchronize(s));

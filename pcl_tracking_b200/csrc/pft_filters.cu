@@ -308,7 +308,7 @@ int run_passthrough(pft_context* ctx, const pft_cloud* in, pft_cloud* out, int f
   if (rc) return rc;
   passthrough_kernel<<<1, 1024, 0, ctx->stream>>>(in->d_pts(), in->d_hdr(), out->d_pts(), out->d_hdr(), field, lo, hi, drop_zero);
   PFT_LAUNCH_CHECK();
-  out->host_n = -1;
+  out->written(-1);
   return PFT_OK;
 }
 
@@ -356,7 +356,7 @@ int run_voxel_grid(pft_context* ctx, const pft_cloud* in, pft_cloud* out, float 
   if ((rc = ctx->k1_acc_rgbc.reserve(cap * 4 * sizeof(unsigned int)))) return rc;
   const int n_tiles = (int)((cap + kTile - 1) / kTile);
   if ((rc = ctx->k1_blk.reserve((size_t)n_tiles * sizeof(int)))) return rc;
-  out->host_n = -1;
+  out->written(-1);
   (void)kFirstInit;
   // A camera stream downsamples frame after frame between the same buffers: the ten operations are captured once
   // into a CUDA graph and replayed (one launch per frame instead of ten).  Everything the sequence touches is in the key.
@@ -400,7 +400,7 @@ int run_approx_voxel_grid_pcl(pft_context* ctx, const pft_cloud* in, pft_cloud* 
   if (rc) return rc;
   approx_voxel_grid_pcl_kernel<<<1, 32, 0, ctx->stream>>>(in->d_pts(), in->d_hdr(), 1.0f / leaf, field, lo, hi, out->d_pts(), out->d_hdr());
   PFT_LAUNCH_CHECK();
-  out->host_n = -1;
+  out->written(-1);
   return PFT_OK;
 }
 

@@ -55,6 +55,10 @@ struct pft_cloud {
   pft::DevBuf hdr;              // CloudHeader
   size_t capacity = 0;          // host-known upper bound on n
   long long host_n = -1;        // exact n if known on the host, else -1
+  // identity of the contents for the replicas that other contexts read (pft_tracker.cu): `serial` is never reused in the
+  // process, `version` changes with every library call that writes the cloud (written())
+  unsigned long long serial = 0, version = 1;
+  void written(long long n) { host_n = n; ++version; }
   // pft_cloud_upload_async: `ready` fires on the copy stream once the points are in place; the first consumer on the
   // context stream waits for it (join_upload)
   pft::DevBuf raw_staging;      // raw PointCloud2 / 32-byte records of an asynchronous upload
@@ -86,5 +90,9 @@ int run_passthrough(pft_context* ctx, const pft_cloud* in, pft_cloud* out, int f
 int run_voxel_grid(pft_context* ctx, const pft_cloud* in, pft_cloud* out, float leaf, int field, float lo, float hi);
 int run_approx_voxel_grid_pcl(pft_context* ctx, const pft_cloud* in, pft_cloud* out, float leaf, int field, float lo, float hi);
 int run_centre_on_centroid(pft_context* ctx, pft_cloud* cloud, float* d_centroid3);
+
+// ---- scene replicas (pft_tracker.cu): every replica of a cloud goes with it, every replica a context holds goes with it
+void release_replicas_of(const pft_cloud* src);
+void release_replicas_in(const pft_context* dst);
 
 }  // namespace pft

@@ -125,15 +125,21 @@ struct CloudPeerSet {
   unsigned int* sync[kMaxPeers];  // [0] flag = number of the last scene that has fully arrived, [1] blocks done (root only)
   int nranks, rank;
 };
-__global__ void __launch_bounds__(256) cloud_push_kernel(const float4* __restrict__ src, const CloudHeader* __restrict__ src_hdr, CloudPeerSet ps,
-                                                         unsigned int epoch, int capacity, unsigned int* error /* host-mapped */) {
+// Stores the header and the n points of `src` (n read from its header) into every cloud of `ps` but ps.rank's, with
+// 16-byte loads and stores.  n > capacity stores an empty cloud and raises *error (if given).
+__device__ __forceinline__ void push_cloud(const float4* __restrict__ src, const CloudHeader* __restrict__ src_hdr, const CloudPeerSet& ps, int capacity,
+                                           unsigned int* error) {
   int n = src_hdr->n;
-  if (n > capacity) { if (blockIdx.x == 0 && threadIdx.x == 0) *error = 1u; n = 0; }  // (loud on the host at the next call; the peers see an empty scene)
+  if (n > capacity) { if (error && blockIdx.x == 0 && threadIdx.x == 0) *error = 1u; n = 0; }
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const float4 p = src[i];
     for (int r = 0; r < ps.nranks; ++r) if (r != ps.rank) ps.pts[r][i] = p;
   }
   if (blockIdx.x == 0 && threadIdx.x < ps.nranks && (int)threadIdx.x != ps.rank) { CloudHeader h = *src_hdr; h.n = n; *ps.hdr[threadIdx.x] = h; }
+}
+__global__ void __launch_bounds__(256) cloud_push_kernel(const float4* __restrict__ src, const CloudHeader* __restrict__ src_hdr, CloudPeerSet ps,
+                                                         unsigned int epoch, int capacity, unsigned int* error /* host-mapped */) {
+  push_cloud(src, src_hdr, ps, capacity, error);  // (an overflow is loud on the host at the next call; the peers see an empty scene)
   __syncthreads();
   if (threadIdx.x == 0) {
     __threadfence_system();  // one system-scope fence per block, after the barrier (cumulative over the block's stores)
@@ -147,6 +153,12 @@ __global__ void __launch_bounds__(256) cloud_push_kernel(const float4* __restric
 }
 __global__ void cloud_wait_kernel(unsigned int* sync, unsigned int epoch, unsigned int* error /* host-mapped */) {
   peer_wait(&sync[0], epoch, error);
+}
+// The scene replicas of other contexts in one process (pft_tracker.cu): the same stores into every cloud of `ps`
+// (ps.rank = -1), ordered by stream events instead of flags.  The replicas are sized for the source's capacity.
+__global__ void __launch_bounds__(256) cloud_fanout_kernel(const float4* __restrict__ src, const CloudHeader* __restrict__ src_hdr, CloudPeerSet ps,
+                                                           int capacity) {
+  push_cloud(src, src_hdr, ps, capacity, nullptr);
 }
 
 struct NoiseParams {      // host-precomputed square roots (IEEE, identical to the oracle's)

@@ -569,6 +569,8 @@ class ParticleFilterOMPTracker:
             check(capi.load().pft_tracker_set_reference_points(self._h, ptr(a), a.shape[0], layout))
 
     def setInputCloud(self, cloud):
+        """The cloud may belong to another context than the tracker's, also on another GPU: the tracker's context then
+        reads a replica of it, refreshed once per change (one object per GPU; not for sharded trackers)."""
         self._input = cloud  # keep the handle alive: the tracker borrows it
         check(capi.load().pft_tracker_set_input_cloud(self._h, cloud._h if cloud is not None else None))
 
@@ -852,7 +854,8 @@ def savePCDFile(path, cloud, binary=False):
 
 
 def compute_batch(trackers):
-    """compute() of several trackers that share one scene (ref :688-697)."""
+    """compute() of several trackers that share one scene (ref :688-697).  The trackers may sit on other contexts than
+    the scene, and on several (one object per GPU): each context's trackers run concurrently on its own stream."""
     arr = (C.c_void_p * len(trackers))(*[t._h for t in trackers])
     check(capi.load().pft_compute_batch(arr, len(trackers)))
 
