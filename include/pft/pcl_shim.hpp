@@ -201,6 +201,29 @@ class PointCloud {
     width = w; height = h;
     mark_device_written();
   }
+  // Frame ingest from the registered images the points topic is computed from (kinect2_bridge <res>/image_depth_rect
+  // 16UC1 mm, <res>/image_color_rect bgr8, <res>/camera_info), replacing the depth_image_proc/point_cloud_xyzrgb
+  // nodelet behind ref: src/auto_tracking.cpp:775 (pft_cloud_upload_depth_image): the conversion runs on the device;
+  // the host vector stays empty until download().  Steps in bytes (msg.step); fx, fy, cx, cy = K[0], K[4], K[2], K[5].
+  void fromDepthImage(const uint16_t* depth, uint32_t depth_step, const uint8_t* bgr, uint32_t bgr_step, uint32_t w, uint32_t h, double fx,
+                      double fy, double cx, double cy, const std::shared_ptr<pft::Context>& ctx = pft::Context::Default()) {
+    if (!dev_) { ctx_ = ctx; pft::check(pft_cloud_create(ctx_->get(), &dev_)); }
+    pft::check(pft_cloud_upload_depth_image(dev_, depth, depth_step, bgr, bgr_step, w, h, fx, fy, cx, cy));
+    points.clear();
+    width = w; height = h;
+    mark_device_written();
+  }
+  // The same on the context's copy stream (pft_cloud_upload_depth_image_async): returns at once, the copy overlaps the
+  // tracking enqueued after the call, the first consumer of this cloud waits for it on the device.  Both images must be
+  // pinned (pft_host_alloc) and stay untouched until that consumer has finished.  Use two clouds alternately.
+  void fromDepthImageAsync(const uint16_t* depth, uint32_t depth_step, const uint8_t* bgr, uint32_t bgr_step, uint32_t w, uint32_t h, double fx,
+                           double fy, double cx, double cy, const std::shared_ptr<pft::Context>& ctx = pft::Context::Default()) {
+    if (!dev_) { ctx_ = ctx; pft::check(pft_cloud_create(ctx_->get(), &dev_)); }
+    pft::check(pft_cloud_upload_depth_image_async(dev_, depth, depth_step, bgr, bgr_step, w, h, fx, fy, cx, cy));
+    points.clear();
+    width = w; height = h;
+    mark_device_written();
+  }
   // a filter wrote the device mirror: the host vector is stale until download()
   void mark_device_written() { device_only_ = true; host_dirty_ = false; }
   void download() {

@@ -80,7 +80,19 @@ PFT_API int pft_cloud_upload(pft_cloud* cloud, const void* host_points, size_t n
  * row-major, NaN points are kept (the PassThrough that follows drops them, ref :637). */
 PFT_API int pft_cloud_upload_pointcloud2(pft_cloud* cloud, const void* data, uint32_t width, uint32_t height, uint32_t point_step,
                                          uint32_t row_step, int32_t off_x, int32_t off_y, int32_t off_z, int32_t off_rgb, int is_bigendian);
-/* Frame ingest overlapped with the previous frame's compute (SURVEY 8 f-1).  Same arguments as the two uploads above,
+/* frame ingest one step earlier: the registered depth and colour images the points topic is computed from (kinect2_bridge
+ * <res>/image_depth_rect, <res>/image_color_rect, <res>/camera_info), 5 bytes per pixel instead of a 32-byte record.
+ * Replaces the depth_image_proc/point_cloud_xyzrgb nodelet behind the topic of ref: src/auto_tracking.cpp:775, with its
+ * rounding: `depth` holds `height` rows of `depth_step` bytes (even) of uint16 millimetres, `bgr` `height` rows of
+ * `bgr_step` bytes of bgr8 pixels; fx, fy, cx, cy are camera_info.K[0], K[4], K[2], K[5].  Pixel (u, v) with depth d
+ * becomes x = ((u - (float)cx) * d) * (float)(0.001f / fx), y likewise with v, fy, cy, z = d * 0.001f, all in fp32;
+ * d == 0 gives x = y = z = NaN.  rgba = b | g << 8 | r << 16 | 255 << 24 for every pixel.  The cloud is organised,
+ * width * height points in row-major order, as pft_cloud_upload_pointcloud2 leaves it.  Only (height - 1) * step +
+ * width * bytes-per-pixel bytes of each image are read.  PFT_ERR_INVALID: a null image with pixels, a step below
+ * width * bytes-per-pixel or an odd depth step, fx or fy zero or not finite, cx or cy not finite, 2^31 pixels or more. */
+PFT_API int pft_cloud_upload_depth_image(pft_cloud* cloud, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step,
+                                         uint32_t width, uint32_t height, double fx, double fy, double cx, double cy);
+/* Frame ingest overlapped with the previous frame's compute (SURVEY 8 f-1).  Same arguments as the three uploads above,
  * but the copy (and the unpack kernel) run on a copy stream of the context instead of its compute stream: the call
  * returns at once, the copy starts when everything enqueued on the context BEFORE this call has finished (so earlier
  * readers of `cloud` are safe), and it overlaps whatever is enqueued AFTER it.  The first library call that consumes
@@ -91,6 +103,8 @@ PFT_API int pft_cloud_upload_pointcloud2(pft_cloud* cloud, const void* data, uin
 PFT_API int pft_cloud_upload_async(pft_cloud* cloud, const void* host_points, size_t n, int layout);
 PFT_API int pft_cloud_upload_pointcloud2_async(pft_cloud* cloud, const void* data, uint32_t width, uint32_t height, uint32_t point_step,
                                                uint32_t row_step, int32_t off_x, int32_t off_y, int32_t off_z, int32_t off_rgb, int is_bigendian);
+PFT_API int pft_cloud_upload_depth_image_async(pft_cloud* cloud, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step,
+                                               uint32_t width, uint32_t height, double fx, double fy, double cx, double cy);
 PFT_API int pft_cloud_wait_upload(pft_cloud* cloud);
 PFT_API int pft_cloud_size(pft_cloud* cloud, size_t* n);
 PFT_API int pft_cloud_download(pft_cloud* cloud, void* host_points, size_t capacity, int layout, size_t* n);

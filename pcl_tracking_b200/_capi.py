@@ -64,6 +64,8 @@ SIGNATURES = {
     "pft_cloud_upload_pointcloud2": (_i, [_vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _i]),
     "pft_cloud_upload_async": (_i, [_vp, _vp, _sz, _i]),
     "pft_cloud_upload_pointcloud2_async": (_i, [_vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _i]),
+    "pft_cloud_upload_depth_image": (_i, [_vp, _vp, C.c_uint32, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _d, _d, _d, _d]),
+    "pft_cloud_upload_depth_image_async": (_i, [_vp, _vp, C.c_uint32, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _d, _d, _d, _d]),
     "pft_cloud_wait_upload": (_i, [_vp]),
     "pft_cloud_size": (_i, [_vp, _psz]),
     "pft_cloud_download": (_i, [_vp, _vp, _sz, _i, _psz]),

@@ -3,9 +3,11 @@
 // Host-side plumbing only; the kernels live in pft_filters.cu / pft_tracker_kernels.cuh.  Everything
 // here replaces glue the reference does on the CPU around PCL containers:
 //   pft_cloud_upload        pcl::fromPCLPointCloud2 into PointCloud<PointXYZRGBA>  (ref: src/auto_tracking.cpp:619-622)
+//   pft_cloud_upload_depth_image  depth_image_proc/point_cloud_xyzrgb, which computes the points topic of ref :775
 //   pft_passthrough         filterPassThrough                                       (ref: src/auto_tracking.cpp:536-547)
 //   pft_passthrough_voxel_grid  filterPassThrough + gridSampleApprox / gridSample   (ref: src/auto_tracking.cpp:637, :683, :641)
 //   pft_prepare_model       removeZeroPoints + centroid + translate + gridSample    (ref: src/auto_tracking.cpp:656-674)
+#include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
 #include <string.h>
@@ -120,6 +122,53 @@ int check_pointcloud2_layout(size_t n, uint32_t width, uint32_t point_step, uint
     }
   }
   return PFT_OK;
+}
+
+// A depth + colour frame checked and laid out for one staging buffer: the depth rows, then the colour rows from a
+// 16-byte aligned offset.  Only the bytes the images occupy are copied, (height - 1) * step + width * bytes per pixel
+// each, so a caller's view into a larger buffer is never read past its last pixel.
+struct DepthImageFrame {
+  size_t n = 0, depth_bytes = 0, bgr_off = 0, bgr_bytes = 0;
+  float cx = 0.f, cy = 0.f, kx = 0.f, ky = 0.f;
+};
+
+int check_depth_image(const char* fn, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step, uint32_t width, uint32_t height,
+                      double fx, double fy, double cx, double cy, DepthImageFrame* f) {
+  const size_t n = (size_t)width * height;
+  if (n > 0x7fffffffull) { set_last_error("%s: image too large", fn); return PFT_ERR_INVALID; }
+  if (!(fx != 0.0 && fy != 0.0 && isfinite(fx) && isfinite(fy) && isfinite(cx) && isfinite(cy))) {
+    set_last_error("%s: bad intrinsics fx %g fy %g cx %g cy %g (fx, fy finite and non-zero; cx, cy finite)", fn, fx, fy, cx, cy);
+    return PFT_ERR_INVALID;
+  }
+  if (n) {
+    if (!depth || !bgr) { set_last_error("%s: null image", fn); return PFT_ERR_INVALID; }
+    if ((depth_step & 1) || (size_t)depth_step < (size_t)width * 2 || (size_t)bgr_step < (size_t)width * 3) {
+      set_last_error("%s: bad steps: depth %u (even, >= 2 * width), bgr %u (>= 3 * width), width %u", fn, depth_step, bgr_step, width);
+      return PFT_ERR_INVALID;
+    }
+    f->depth_bytes = (size_t)(height - 1) * depth_step + (size_t)width * 2;
+    f->bgr_off = (f->depth_bytes + 15) & ~(size_t)15;
+    f->bgr_bytes = (size_t)(height - 1) * bgr_step + (size_t)width * 3;
+  }
+  f->n = n;
+  // the constants of depth_image_proc::convert<uint16_t>: float centre, float(double(0.001f) / f)
+  f->cx = (float)cx;
+  f->cy = (float)cy;
+  f->kx = (float)((double)0.001f / fx);
+  f->ky = (float)((double)0.001f / fy);
+  return PFT_OK;
+}
+
+// The two copies and the conversion kernel of one frame, on stream `s` through `staging`.
+int enqueue_depth_image(cudaStream_t s, pft::DevBuf& staging, pft_cloud* c, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step,
+                        uint32_t width, uint32_t height, const DepthImageFrame& f) {
+  if (!f.n) return PFT_OK;
+  int rc = staging.reserve(f.bgr_off + f.bgr_bytes);
+  if (rc) return rc;
+  unsigned char* base = staging.as<unsigned char>();
+  PFT_CUDA_TRY(cudaMemcpyAsync(base, depth, f.depth_bytes, cudaMemcpyHostToDevice, s));
+  PFT_CUDA_TRY(cudaMemcpyAsync(base + f.bgr_off, bgr, f.bgr_bytes, cudaMemcpyHostToDevice, s));
+  return launch_depth_image(s, base, f.bgr_off, c->d_pts(), width, height, depth_step, bgr_step, f.cx, f.cy, f.kx, f.ky);
 }
 
 }  // namespace
@@ -309,6 +358,35 @@ int pft_cloud_upload_pointcloud2_async(pft_cloud* c, const void* data, uint32_t 
     if ((rc = launch_unpack_pointcloud2(cs, c->raw_staging.p, c->d_pts(), width, height, point_step, row_step, off_x, off_y, off_z, off_rgb))) return rc;
   }
   return end_async_upload(c, n, cs);
+}
+
+int pft_cloud_upload_depth_image(pft_cloud* c, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step, uint32_t width,
+                                 uint32_t height, double fx, double fy, double cx, double cy) {
+  if (!c) { set_last_error("pft_cloud_upload_depth_image: null cloud"); return PFT_ERR_INVALID; }
+  DepthImageFrame f;
+  int rc = check_depth_image("pft_cloud_upload_depth_image", depth, depth_step, bgr, bgr_step, width, height, fx, fy, cx, cy, &f);
+  if (rc) return rc;
+  pft_context* ctx = c->ctx;
+  PFT_CUDA_TRY(cudaSetDevice(ctx->device));
+  if ((rc = c->join_upload())) return rc;
+  if ((rc = c->ensure(f.n))) return rc;
+  cudaStream_t s = ctx->stream;
+  if ((rc = enqueue_depth_image(s, ctx->staging, c, depth, depth_step, bgr, bgr_step, width, height, f))) return rc;
+  if ((rc = launch_set_header(s, c->d_hdr(), (int)f.n))) return rc;
+  c->written((long long)f.n);
+  return PFT_OK;
+}
+
+int pft_cloud_upload_depth_image_async(pft_cloud* c, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step, uint32_t width,
+                                       uint32_t height, double fx, double fy, double cx, double cy) {
+  if (!c) { set_last_error("pft_cloud_upload_depth_image_async: null cloud"); return PFT_ERR_INVALID; }
+  DepthImageFrame f;
+  int rc = check_depth_image("pft_cloud_upload_depth_image_async", depth, depth_step, bgr, bgr_step, width, height, fx, fy, cx, cy, &f);
+  if (rc) return rc;
+  cudaStream_t cs = nullptr;
+  if ((rc = begin_async_upload(c, f.n, &cs))) return rc;
+  if ((rc = enqueue_depth_image(cs, c->raw_staging, c, depth, depth_step, bgr, bgr_step, width, height, f))) return rc;
+  return end_async_upload(c, f.n, cs);
 }
 
 int pft_cloud_wait_upload(pft_cloud* c) {

@@ -72,6 +72,36 @@ __global__ void unpack_pointcloud2_kernel(const unsigned int* __restrict__ src, 
     dst[i] = make_float4(__uint_as_float(rec[wx]), __uint_as_float(rec[wy]), __uint_as_float(rec[wz]), __uint_as_float(rgba));
   }
 }
+// Registered depth (16UC1, mm) + colour (bgr8) images -> float4 {x,y,z,rgba}: replaces the depth_image_proc
+// point_cloud_xyzrgb nodelet that computes the /kinect2/<res>/points topic the reference subscribes to (ref:
+// src/auto_tracking.cpp:775), i.e. depth_image_proc::convert<uint16_t> + its colour copy.  Every fp32 operation is
+// rounded on its own (-fmad=false), in the nodelet's order: x = ((u - cx) * d) * (0.001f / fx), z = d * 0.001f; d == 0
+// is a quiet-NaN point (colour still written).  `src` holds the depth rows (`depth_step` bytes apart, even), the colour
+// rows start at byte `bgr_off`.  Thread = pixel along a row: the warp's 2-byte depth loads, 1-byte colour loads and
+// 16-byte stores each cover one contiguous span.  Organised row-major output, as unpack_pointcloud2_kernel.
+__global__ void depth_image_kernel(const unsigned char* __restrict__ src, size_t bgr_off, float4* __restrict__ dst, unsigned int width,
+                                   unsigned int height, unsigned int depth_step, unsigned int bgr_step, float cx, float cy, float kx, float ky) {
+  const float nan = __uint_as_float(0x7fc00000u);
+  for (unsigned int v = blockIdx.y; v < height; v += gridDim.y) {
+    const unsigned short* drow = reinterpret_cast<const unsigned short*>(src + (size_t)v * depth_step);
+    const unsigned char* crow = src + bgr_off + (size_t)v * bgr_step;
+    float4* orow = dst + (size_t)v * width;
+    const float fy = (float)v - cy;
+    for (unsigned int u = blockIdx.x * blockDim.x + threadIdx.x; u < width; u += gridDim.x * blockDim.x) {
+      const unsigned int d = drow[u];
+      const unsigned char* c = crow + 3 * (size_t)u;
+      const unsigned int rgba = (unsigned int)c[0] | ((unsigned int)c[1] << 8) | ((unsigned int)c[2] << 16) | 0xff000000u;
+      float4 p = make_float4(nan, nan, nan, __uint_as_float(rgba));
+      if (d != 0) {
+        const float fd = (float)d;
+        p.x = (((float)u - cx) * fd) * kx;
+        p.y = (fy * fd) * ky;
+        p.z = fd * 0.001f;
+      }
+      orow[u] = p;
+    }
+  }
+}
 __global__ void set_header_kernel(CloudHeader* h, int n) { h->n = n; }
 
 // ---- PassThrough (order-preserving compaction), one thread block: flags -> exclusive scan -> scatter.
@@ -288,6 +318,14 @@ int launch_unpack_pointcloud2(cudaStream_t s, const void* src, float4* dst, unsi
   if (n == 0) return PFT_OK;
   unpack_pointcloud2_kernel<<<grid_for(n, 256, 148), 256, 0, s>>>(reinterpret_cast<const unsigned int*>(src), dst, width, height, point_step / 4, row_step / 4,
                                                                  off_x / 4, off_y / 4, off_z / 4, off_rgb >= 0 ? off_rgb / 4 : -1);
+  PFT_LAUNCH_CHECK();
+  return PFT_OK;
+}
+int launch_depth_image(cudaStream_t s, const void* src, size_t bgr_off, float4* dst, unsigned int width, unsigned int height, unsigned int depth_step,
+                       unsigned int bgr_step, float cx, float cy, float kx, float ky) {
+  if ((size_t)width * height == 0) return PFT_OK;
+  const dim3 grid((width + 127) / 128, height < 65535u ? height : 65535u);
+  depth_image_kernel<<<grid, 128, 0, s>>>(reinterpret_cast<const unsigned char*>(src), bgr_off, dst, width, height, depth_step, bgr_step, cx, cy, kx, ky);
   PFT_LAUNCH_CHECK();
   return PFT_OK;
 }

@@ -61,7 +61,7 @@ struct pft_cloud {
   void written(long long n) { host_n = n; ++version; }
   // pft_cloud_upload_async: `ready` fires on the copy stream once the points are in place; the first consumer on the
   // context stream waits for it (join_upload)
-  pft::DevBuf raw_staging;      // raw PointCloud2 / 32-byte records of an asynchronous upload
+  pft::DevBuf raw_staging;      // raw PointCloud2 / 32-byte records / depth + colour images of an asynchronous upload
   cudaEvent_t ready = nullptr;
   mutable bool upload_pending = false;
   int join_upload() const;
@@ -85,6 +85,9 @@ int launch_unpack_pcl32(cudaStream_t s, const void* src32, float4* dst, size_t n
 int launch_pack_pcl32(cudaStream_t s, const float4* src, void* dst32, size_t n);
 int launch_unpack_pointcloud2(cudaStream_t s, const void* src, float4* dst, unsigned int width, unsigned int height, unsigned int point_step,
                               unsigned int row_step, int off_x, int off_y, int off_z, int off_rgb);
+// depth rows at `src`, colour rows at `src + bgr_off`; cx, cy, kx = 0.001f / fx, ky as the fp32 constants of the conversion
+int launch_depth_image(cudaStream_t s, const void* src, size_t bgr_off, float4* dst, unsigned int width, unsigned int height, unsigned int depth_step,
+                       unsigned int bgr_step, float cx, float cy, float kx, float ky);
 int launch_set_header(cudaStream_t s, CloudHeader* hdr, int n);
 int run_passthrough(pft_context* ctx, const pft_cloud* in, pft_cloud* out, int field, float lo, float hi, int drop_zero);
 int run_voxel_grid(pft_context* ctx, const pft_cloud* in, pft_cloud* out, float leaf, int field, float lo, float hi);

@@ -151,6 +151,40 @@ class PointCloud:
                  int(off_z), int(off_rgb), 1 if is_bigendian else 0))
         return self
 
+    def fromDepthImage(self, depth, bgr, fx, fy, cx, cy, asynchronous=False, width=None, height=None, depth_step=None, bgr_step=None):
+        """Registered depth + colour images -> organised device cloud (pft_cloud_upload_depth_image): what the
+        depth_image_proc/point_cloud_xyzrgb nodelet computes for the points topic of ref: src/auto_tracking.cpp:775.
+        `depth`: (H, W) uint16 millimetres, `bgr`: (H, W, 3) uint8 bgr8, each an array (rows may be padded: the row
+        stride is the step) or a raw host pointer (int; pinned for `asynchronous`) with width, height and the steps in
+        bytes (default: packed rows).  fx, fy, cx, cy: camera_info.K[0], K[4], K[2], K[5]."""
+        keep = []
+
+        def image(img, dtype, channels, step):
+            pixel = np.dtype(dtype).itemsize * channels
+            if isinstance(img, int):
+                if width is None or height is None:
+                    raise ValueError("a pointer image needs width and height")
+                return C.c_void_p(img), int(width), int(height), int(width) * pixel if step is None else int(step)
+            a = np.asarray(img)
+            shape = "(H, W)" if channels == 1 else "(H, W, %d)" % channels
+            if a.dtype != dtype or a.ndim != (2 if channels == 1 else 3) or (channels > 1 and a.shape[2] != channels):
+                raise TypeError("image must be a %s array of shape %s, got %s %r" % (np.dtype(dtype), shape, a.dtype, a.shape))
+            # padded rows (a view into a wider buffer) go as they are, with the row stride as the step
+            packed = a.strides[1] == pixel and (channels == 1 or a.strides[2] == a.itemsize)
+            if not packed or a.shape[0] < 2 or a.strides[0] < a.shape[1] * pixel:
+                a = np.ascontiguousarray(a)
+            keep.append(a)
+            return C.c_void_p(a.ctypes.data if a.size else None), a.shape[1], a.shape[0], a.strides[0]
+
+        dp, w, h, dstep = image(depth, np.uint16, 1, depth_step)
+        bp, w2, h2, bstep = image(bgr, np.uint8, 3, bgr_step)
+        if (w, h) != (w2, h2):
+            raise ValueError("depth is %dx%d, colour %dx%d" % (w, h, w2, h2))
+        self._keep = keep
+        fn = capi.load().pft_cloud_upload_depth_image_async if asynchronous else capi.load().pft_cloud_upload_depth_image
+        check(fn(self._h, dp, dstep, bp, bstep, w, h, float(fx), float(fy), float(cx), float(cy)))
+        return self
+
     def broadcast(self, capacity, root=0):
         """NVLink broadcast of this cloud from `root` over the context communicator."""
         check(capi.load().pft_cloud_broadcast(self._h, int(capacity), int(root)))

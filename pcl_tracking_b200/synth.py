@@ -143,6 +143,21 @@ def render(frame=0, objects=None, sensor=KINECT2_SD, seed=0xC0FFEE, noise=True, 
     return pts, oid
 
 
+def depth_images(pts, sensor=KINECT2_SD):
+    """A rendered frame as the registered images kinect2_bridge publishes next to the points topic: returns
+    (depth (H, W) uint16 millimetres, bgr (H, W, 3) uint8, K 3x3 float64 of camera_info).  z is rounded to the
+    millimetre; a pixel without a reading (z NaN, or outside 1..65535 mm) is 0."""
+    W, H, f, cx, cy = sensor["width"], sensor["height"], sensor["f"], sensor["cx"], sensor["cy"]
+    with np.errstate(invalid="ignore"):
+        mm = np.rint(np.asarray(pts["z"], dtype=np.float64) * 1000.0)
+        ok = (mm >= 1) & (mm <= 65535)
+    depth = np.where(ok, mm, 0).astype(np.uint16).reshape(H, W)
+    rgba = np.asarray(pts["rgba"], dtype=np.uint32)
+    bgr = np.stack([rgba & 0xff, (rgba >> 8) & 0xff, (rgba >> 16) & 0xff], axis=-1).astype(np.uint8).reshape(H, W, 3)
+    K = np.array([[f, 0.0, cx], [0.0, f, cy], [0.0, 0.0, 1.0]])
+    return depth, bgr, K
+
+
 def model_points(pts, oid, k):
     """Raw model cloud of object k as create_model would return it (ref: src/create_model.cpp:209-230)."""
     m = (oid == k) & np.isfinite(pts["x"])
