@@ -141,6 +141,26 @@ inline std::shared_ptr<Context> nextTrackerContext() {
   return per_device[dev];
 }
 
+// One calibrated camera of a fused frame (PointCloud::fromDepthImages): the registered images and intrinsics of
+// fromDepthImage, and optionally the pose of its optical frame in the common frame, T_k of
+// pcl::transformPointCloud(cloud_k, T_k) (e.g. tf2 lookupTransform(target, camera_optical_frame) as Eigen::Affine3f).
+struct DepthCamera {
+  const uint16_t* depth = nullptr;
+  uint32_t depth_step = 0;  // bytes (msg.step)
+  const uint8_t* bgr = nullptr;
+  uint32_t bgr_step = 0;
+  uint32_t width = 0, height = 0;
+  double fx = 0, fy = 0, cx = 0, cy = 0;  // camera_info K[0], K[4], K[2], K[5]
+  bool has_pose = false;
+  float pose[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};  // 3x4 row-major
+  // any affine type with operator()(row, col), as setTrans: Eigen::Affine3f, pft::Affine3f
+  template <typename AffineT> void setPose(const AffineT& t) {
+    for (int r = 0; r < 3; ++r) for (int c = 0; c < 4; ++c) pose[r * 4 + c] = t(r, c);
+    has_pose = true;
+  }
+  void clearPose() { has_pose = false; }
+};
+
 }  // namespace pft
 
 #ifndef PFT_SHIM_USE_PCL_TYPES
@@ -224,6 +244,17 @@ class PointCloud {
     width = w; height = h;
     mark_device_written();
   }
+  // Several calibrated cameras fused into one scene (pft_cloud_upload_depth_images): for each camera,
+  // pcl::transformPointCloud(cloud_k, T_k) of the cloud fromDepthImage makes, then scene += cloud_k, in one kernel
+  // launch.  The cloud is unorganised: width = all the cameras' pixels, height = 1.
+  void fromDepthImages(const std::vector<pft::DepthCamera>& cams, const std::shared_ptr<pft::Context>& ctx = pft::Context::Default()) {
+    upload_depth_cameras(cams, ctx, false);
+  }
+  // The same on the context's copy stream (pft_cloud_upload_depth_images_async), with the pinned-buffer rules of
+  // fromDepthImageAsync for every image.
+  void fromDepthImagesAsync(const std::vector<pft::DepthCamera>& cams, const std::shared_ptr<pft::Context>& ctx = pft::Context::Default()) {
+    upload_depth_cameras(cams, ctx, true);
+  }
   // a filter wrote the device mirror: the host vector is stale until download()
   void mark_device_written() { device_only_ = true; host_dirty_ = false; }
   void download() {
@@ -240,6 +271,20 @@ class PointCloud {
   PointCloud& operator=(const PointCloud& o) { points = o.host_points(); width = o.width; height = o.height; host_dirty_ = true; device_only_ = false; return *this; }
 
  private:
+  void upload_depth_cameras(const std::vector<pft::DepthCamera>& cams, const std::shared_ptr<pft::Context>& ctx, bool asynchronous) {
+    if (!dev_) { ctx_ = ctx; pft::check(pft_cloud_create(ctx_->get(), &dev_)); }
+    std::vector<pft_depth_camera> c(cams.size());
+    size_t n = 0;
+    for (size_t k = 0; k < cams.size(); ++k) {
+      const pft::DepthCamera& s = cams[k];
+      c[k] = pft_depth_camera{s.depth, s.depth_step, s.bgr, s.bgr_step, s.width, s.height, s.fx, s.fy, s.cx, s.cy, s.has_pose ? s.pose : nullptr};
+      n += (size_t)s.width * s.height;
+    }
+    pft::check(asynchronous ? pft_cloud_upload_depth_images_async(dev_, c.data(), (int)c.size()) : pft_cloud_upload_depth_images(dev_, c.data(), (int)c.size()));
+    points.clear();
+    width = (uint32_t)n; height = 1;
+    mark_device_written();
+  }
   size_t device_size() const { size_t n = 0; pft::check(pft_cloud_size(dev_, &n)); return n; }
   const std::vector<PointT>& host_points() const { const_cast<PointCloud*>(this)->download(); return points; }
   mutable pft_cloud* dev_ = nullptr;

@@ -92,7 +92,31 @@ PFT_API int pft_cloud_upload_pointcloud2(pft_cloud* cloud, const void* data, uin
  * width * bytes-per-pixel or an odd depth step, fx or fy zero or not finite, cx or cy not finite, 2^31 pixels or more. */
 PFT_API int pft_cloud_upload_depth_image(pft_cloud* cloud, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step,
                                          uint32_t width, uint32_t height, double fx, double fy, double cx, double cy);
-/* Frame ingest overlapped with the previous frame's compute (SURVEY 8 f-1).  Same arguments as the three uploads above,
+/* One calibrated camera of a fused frame: the images and intrinsics of pft_cloud_upload_depth_image, and `m12`, the
+ * fp32 3x4 row-major matrix from the camera's optical frame to the common frame (Eigen::Affine3f rows 0-2, the
+ * convention of pft_tracker_set_trans; e.g. tf2 lookupTransform(target, camera_optical_frame)), or NULL to keep the
+ * camera's own frame. */
+typedef struct {
+  const void* depth;
+  uint32_t depth_step;
+  const void* bgr;
+  uint32_t bgr_step;
+  uint32_t width, height;
+  double fx, fy, cx, cy;
+  const float* m12;
+} pft_depth_camera;
+#define PFT_MAX_DEPTH_CAMERAS 8
+/* Several calibrated cameras fused into one scene cloud: for each camera k, pcl::transformPointCloud(cloud_k, T_k) of
+ * the nodelet's cloud, then scene += cloud_k.  Pixel (u, v) of camera k becomes the point pft_cloud_upload_depth_image
+ * makes of it; with a matrix, each finite point is then transformed as PCL 1.8.0 does, x' = ((m00 x + m01 y) + m02 z)
+ * + m03, every fp32 operation rounded on its own.  Depth-0 (NaN) points are kept as they are, colour included.  The
+ * cloud is unorganised: camera 0's width * height points in row-major order, then camera 1's, and so on.  Cameras
+ * may differ in size; one with no pixels adds nothing.  All images are converted by one kernel launch.  One camera
+ * without a matrix gives exactly the cloud of pft_cloud_upload_depth_image.  PFT_ERR_INVALID: n < 1 or n >
+ * PFT_MAX_DEPTH_CAMERAS, null `cams`, any camera that pft_cloud_upload_depth_image would reject (the message names
+ * its index), a non-finite matrix entry, 2^31 pixels or more in total. */
+PFT_API int pft_cloud_upload_depth_images(pft_cloud* cloud, const pft_depth_camera* cams, int n);
+/* Frame ingest overlapped with the previous frame's compute (SURVEY 8 f-1).  Same arguments as the four uploads above,
  * but the copy (and the unpack kernel) run on a copy stream of the context instead of its compute stream: the call
  * returns at once, the copy starts when everything enqueued on the context BEFORE this call has finished (so earlier
  * readers of `cloud` are safe), and it overlaps whatever is enqueued AFTER it.  The first library call that consumes
@@ -105,6 +129,7 @@ PFT_API int pft_cloud_upload_pointcloud2_async(pft_cloud* cloud, const void* dat
                                                uint32_t row_step, int32_t off_x, int32_t off_y, int32_t off_z, int32_t off_rgb, int is_bigendian);
 PFT_API int pft_cloud_upload_depth_image_async(pft_cloud* cloud, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step,
                                                uint32_t width, uint32_t height, double fx, double fy, double cx, double cy);
+PFT_API int pft_cloud_upload_depth_images_async(pft_cloud* cloud, const pft_depth_camera* cams, int n);
 PFT_API int pft_cloud_wait_upload(pft_cloud* cloud);
 PFT_API int pft_cloud_size(pft_cloud* cloud, size_t* n);
 PFT_API int pft_cloud_download(pft_cloud* cloud, void* host_points, size_t capacity, int layout, size_t* n);

@@ -42,6 +42,16 @@ class PftError(RuntimeError):
         self.code = code
 
 
+MAX_DEPTH_CAMERAS = 8
+
+
+class DepthCamera(C.Structure):
+    """pft_depth_camera: one calibrated camera of pft_cloud_upload_depth_images (m12 NULL: no transform)."""
+    _fields_ = [("depth", C.c_void_p), ("depth_step", C.c_uint32), ("bgr", C.c_void_p), ("bgr_step", C.c_uint32),
+                ("width", C.c_uint32), ("height", C.c_uint32), ("fx", C.c_double), ("fy", C.c_double), ("cx", C.c_double),
+                ("cy", C.c_double), ("m12", C.POINTER(C.c_float))]
+
+
 _vp, _i, _f, _d, _sz, _u64 = C.c_void_p, C.c_int, C.c_float, C.c_double, C.c_size_t, C.c_uint64
 _pp = C.POINTER(C.c_void_p)
 _psz = C.POINTER(C.c_size_t)
@@ -66,6 +76,8 @@ SIGNATURES = {
     "pft_cloud_upload_pointcloud2_async": (_i, [_vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _i]),
     "pft_cloud_upload_depth_image": (_i, [_vp, _vp, C.c_uint32, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _d, _d, _d, _d]),
     "pft_cloud_upload_depth_image_async": (_i, [_vp, _vp, C.c_uint32, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _d, _d, _d, _d]),
+    "pft_cloud_upload_depth_images": (_i, [_vp, C.POINTER(DepthCamera), _i]),
+    "pft_cloud_upload_depth_images_async": (_i, [_vp, C.POINTER(DepthCamera), _i]),
     "pft_cloud_wait_upload": (_i, [_vp]),
     "pft_cloud_size": (_i, [_vp, _psz]),
     "pft_cloud_download": (_i, [_vp, _vp, _sz, _i, _psz]),

@@ -4,6 +4,7 @@
 // here replaces glue the reference does on the CPU around PCL containers:
 //   pft_cloud_upload        pcl::fromPCLPointCloud2 into PointCloud<PointXYZRGBA>  (ref: src/auto_tracking.cpp:619-622)
 //   pft_cloud_upload_depth_image  depth_image_proc/point_cloud_xyzrgb, which computes the points topic of ref :775
+//   pft_cloud_upload_depth_images  the same per calibrated camera + transformPointCloud(cloud_k, T_k), scene += cloud_k
 //   pft_passthrough         filterPassThrough                                       (ref: src/auto_tracking.cpp:536-547)
 //   pft_passthrough_voxel_grid  filterPassThrough + gridSampleApprox / gridSample   (ref: src/auto_tracking.cpp:637, :683, :641)
 //   pft_prepare_model       removeZeroPoints + centroid + translate + gridSample    (ref: src/auto_tracking.cpp:656-674)
@@ -124,51 +125,130 @@ int check_pointcloud2_layout(size_t n, uint32_t width, uint32_t point_step, uint
   return PFT_OK;
 }
 
-// A depth + colour frame checked and laid out for one staging buffer: the depth rows, then the colour rows from a
-// 16-byte aligned offset.  Only the bytes the images occupy are copied, (height - 1) * step + width * bytes per pixel
-// each, so a caller's view into a larger buffer is never read past its last pixel.
+// A depth + colour frame of one or more cameras, checked and laid out for one staging buffer: per camera its depth
+// rows, then its colour rows, each from a 16-byte aligned offset.  Only the bytes an image occupies are copied,
+// (height - 1) * step + width * bytes per pixel, so a caller's view into a larger buffer is never read past its last
+// pixel.  `cams` holds the cameras with pixels, in order, as depth_image_kernel reads them; their points follow
+// each other in the cloud.
 struct DepthImageFrame {
-  size_t n = 0, depth_bytes = 0, bgr_off = 0, bgr_bytes = 0;
-  float cx = 0.f, cy = 0.f, kx = 0.f, ky = 0.f;
+  DepthCameras cams;
+  const void* depth[PFT_MAX_DEPTH_CAMERAS];
+  const void* bgr[PFT_MAX_DEPTH_CAMERAS];
+  size_t depth_bytes[PFT_MAX_DEPTH_CAMERAS], bgr_bytes[PFT_MAX_DEPTH_CAMERAS];
+  int n;               // cameras with pixels
+  size_t points;       // points of the cloud
+  size_t staging;      // bytes of the staging buffer
 };
 
-int check_depth_image(const char* fn, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step, uint32_t width, uint32_t height,
-                      double fx, double fy, double cx, double cy, DepthImageFrame* f) {
-  const size_t n = (size_t)width * height;
-  if (n > 0x7fffffffull) { set_last_error("%s: image too large", fn); return PFT_ERR_INVALID; }
-  if (!(fx != 0.0 && fy != 0.0 && isfinite(fx) && isfinite(fy) && isfinite(cx) && isfinite(cy))) {
-    set_last_error("%s: bad intrinsics fx %g fy %g cx %g cy %g (fx, fy finite and non-zero; cx, cy finite)", fn, fx, fy, cx, cy);
+inline size_t align16(size_t b) { return (b + 15) & ~(size_t)15; }
+
+// Checks camera `cam` and appends it to `f`.  `cam` < 0: the single-image call, whose messages name no camera.
+int check_depth_image(const char* fn, int cam, const pft_depth_camera& c, DepthImageFrame* f) {
+  char who[24] = "";
+  if (cam >= 0) snprintf(who, sizeof(who), ": camera %d", cam);
+  const size_t n = (size_t)c.width * c.height;
+  if (n > 0x7fffffffull) { set_last_error("%s%s: image too large", fn, who); return PFT_ERR_INVALID; }
+  if (!(c.fx != 0.0 && c.fy != 0.0 && isfinite(c.fx) && isfinite(c.fy) && isfinite(c.cx) && isfinite(c.cy))) {
+    set_last_error("%s%s: bad intrinsics fx %g fy %g cx %g cy %g (fx, fy finite and non-zero; cx, cy finite)", fn, who, c.fx, c.fy, c.cx, c.cy);
     return PFT_ERR_INVALID;
   }
-  if (n) {
-    if (!depth || !bgr) { set_last_error("%s: null image", fn); return PFT_ERR_INVALID; }
-    if ((depth_step & 1) || (size_t)depth_step < (size_t)width * 2 || (size_t)bgr_step < (size_t)width * 3) {
-      set_last_error("%s: bad steps: depth %u (even, >= 2 * width), bgr %u (>= 3 * width), width %u", fn, depth_step, bgr_step, width);
-      return PFT_ERR_INVALID;
+  if (c.m12) {
+    for (int i = 0; i < 12; ++i) {
+      if (!isfinite(c.m12[i])) { set_last_error("%s%s: matrix entry %d is %g (must be finite)", fn, who, i, (double)c.m12[i]); return PFT_ERR_INVALID; }
     }
-    f->depth_bytes = (size_t)(height - 1) * depth_step + (size_t)width * 2;
-    f->bgr_off = (f->depth_bytes + 15) & ~(size_t)15;
-    f->bgr_bytes = (size_t)(height - 1) * bgr_step + (size_t)width * 3;
   }
-  f->n = n;
+  if (!n) return PFT_OK;
+  if (!c.depth || !c.bgr) { set_last_error("%s%s: null image", fn, who); return PFT_ERR_INVALID; }
+  if ((c.depth_step & 1) || (size_t)c.depth_step < (size_t)c.width * 2 || (size_t)c.bgr_step < (size_t)c.width * 3) {
+    set_last_error("%s%s: bad steps: depth %u (even, >= 2 * width), bgr %u (>= 3 * width), width %u", fn, who, c.depth_step, c.bgr_step, c.width);
+    return PFT_ERR_INVALID;
+  }
+  if (f->points + n > 0x7fffffffull) { set_last_error("%s: 2^31 pixels or more in total (at camera %d)", fn, cam); return PFT_ERR_INVALID; }
+  const int i = f->n++;
+  DepthCamera& k = f->cams.cam[i];
+  f->depth[i] = c.depth;
+  f->bgr[i] = c.bgr;
+  f->depth_bytes[i] = (size_t)(c.height - 1) * c.depth_step + (size_t)c.width * 2;
+  f->bgr_bytes[i] = (size_t)(c.height - 1) * c.bgr_step + (size_t)c.width * 3;
+  k.depth_off = f->staging;
+  k.bgr_off = align16(k.depth_off + f->depth_bytes[i]);
+  f->staging = align16(k.bgr_off + f->bgr_bytes[i]);
+  k.out_off = f->points;
+  f->points += n;
+  k.width = c.width;
+  k.height = c.height;
+  k.depth_step = c.depth_step;
+  k.bgr_step = c.bgr_step;
   // the constants of depth_image_proc::convert<uint16_t>: float centre, float(double(0.001f) / f)
-  f->cx = (float)cx;
-  f->cy = (float)cy;
-  f->kx = (float)((double)0.001f / fx);
-  f->ky = (float)((double)0.001f / fy);
+  k.cx = (float)c.cx;
+  k.cy = (float)c.cy;
+  k.kx = (float)((double)0.001f / c.fx);
+  k.ky = (float)((double)0.001f / c.fy);
+  k.has_m = c.m12 != nullptr;
+  if (c.m12) memcpy(k.m, c.m12, sizeof(k.m));
   return PFT_OK;
 }
 
-// The two copies and the conversion kernel of one frame, on stream `s` through `staging`.
-int enqueue_depth_image(cudaStream_t s, pft::DevBuf& staging, pft_cloud* c, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step,
-                        uint32_t width, uint32_t height, const DepthImageFrame& f) {
+int check_depth_cameras(const char* fn, const pft_depth_camera* cams, int n, DepthImageFrame* f) {
+  if (!cams) { set_last_error("%s: null cameras", fn); return PFT_ERR_INVALID; }
+  if (n < 1 || n > PFT_MAX_DEPTH_CAMERAS) { set_last_error("%s: %d cameras (1 to %d)", fn, n, PFT_MAX_DEPTH_CAMERAS); return PFT_ERR_INVALID; }
+  for (int k = 0; k < n; ++k) {
+    int rc = check_depth_image(fn, k, cams[k], f);
+    if (rc) return rc;
+  }
+  return PFT_OK;
+}
+
+// The frame's copies (two per camera) and its one conversion launch, on stream `s` through `staging`.
+int enqueue_depth_image(cudaStream_t s, pft::DevBuf& staging, pft_cloud* c, const DepthImageFrame& f) {
   if (!f.n) return PFT_OK;
-  int rc = staging.reserve(f.bgr_off + f.bgr_bytes);
+  int rc = staging.reserve(f.staging);
   if (rc) return rc;
   unsigned char* base = staging.as<unsigned char>();
-  PFT_CUDA_TRY(cudaMemcpyAsync(base, depth, f.depth_bytes, cudaMemcpyHostToDevice, s));
-  PFT_CUDA_TRY(cudaMemcpyAsync(base + f.bgr_off, bgr, f.bgr_bytes, cudaMemcpyHostToDevice, s));
-  return launch_depth_image(s, base, f.bgr_off, c->d_pts(), width, height, depth_step, bgr_step, f.cx, f.cy, f.kx, f.ky);
+  for (int k = 0; k < f.n; ++k) {
+    PFT_CUDA_TRY(cudaMemcpyAsync(base + f.cams.cam[k].depth_off, f.depth[k], f.depth_bytes[k], cudaMemcpyHostToDevice, s));
+    PFT_CUDA_TRY(cudaMemcpyAsync(base + f.cams.cam[k].bgr_off, f.bgr[k], f.bgr_bytes[k], cudaMemcpyHostToDevice, s));
+  }
+  return launch_depth_image(s, base, c->d_pts(), f.cams, f.n);
+}
+
+// A checked frame into `c`: on the context stream through its staging buffer, or (asynchronous) on the copy stream
+// through the cloud's own.
+int upload_depth_frame(pft_cloud* c, const DepthImageFrame& f, bool asynchronous) {
+  int rc;
+  if (asynchronous) {
+    cudaStream_t cs = nullptr;
+    if ((rc = begin_async_upload(c, f.points, &cs))) return rc;
+    if ((rc = enqueue_depth_image(cs, c->raw_staging, c, f))) return rc;
+    return end_async_upload(c, f.points, cs);
+  }
+  pft_context* ctx = c->ctx;
+  PFT_CUDA_TRY(cudaSetDevice(ctx->device));
+  if ((rc = c->join_upload())) return rc;
+  if ((rc = c->ensure(f.points))) return rc;
+  cudaStream_t s = ctx->stream;
+  if ((rc = enqueue_depth_image(s, ctx->staging, c, f))) return rc;
+  if ((rc = launch_set_header(s, c->d_hdr(), (int)f.points))) return rc;
+  c->written((long long)f.points);
+  return PFT_OK;
+}
+
+int upload_depth_image(const char* fn, pft_cloud* c, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step, uint32_t width,
+                       uint32_t height, double fx, double fy, double cx, double cy, bool asynchronous) {
+  if (!c) { set_last_error("%s: null cloud", fn); return PFT_ERR_INVALID; }
+  const pft_depth_camera cam = {depth, depth_step, bgr, bgr_step, width, height, fx, fy, cx, cy, nullptr};
+  DepthImageFrame f{};
+  int rc = check_depth_image(fn, -1, cam, &f);
+  if (rc) return rc;
+  return upload_depth_frame(c, f, asynchronous);
+}
+
+int upload_depth_images(const char* fn, pft_cloud* c, const pft_depth_camera* cams, int n, bool asynchronous) {
+  if (!c) { set_last_error("%s: null cloud", fn); return PFT_ERR_INVALID; }
+  DepthImageFrame f{};
+  int rc = check_depth_cameras(fn, cams, n, &f);
+  if (rc) return rc;
+  return upload_depth_frame(c, f, asynchronous);
 }
 
 }  // namespace
@@ -362,31 +442,20 @@ int pft_cloud_upload_pointcloud2_async(pft_cloud* c, const void* data, uint32_t 
 
 int pft_cloud_upload_depth_image(pft_cloud* c, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step, uint32_t width,
                                  uint32_t height, double fx, double fy, double cx, double cy) {
-  if (!c) { set_last_error("pft_cloud_upload_depth_image: null cloud"); return PFT_ERR_INVALID; }
-  DepthImageFrame f;
-  int rc = check_depth_image("pft_cloud_upload_depth_image", depth, depth_step, bgr, bgr_step, width, height, fx, fy, cx, cy, &f);
-  if (rc) return rc;
-  pft_context* ctx = c->ctx;
-  PFT_CUDA_TRY(cudaSetDevice(ctx->device));
-  if ((rc = c->join_upload())) return rc;
-  if ((rc = c->ensure(f.n))) return rc;
-  cudaStream_t s = ctx->stream;
-  if ((rc = enqueue_depth_image(s, ctx->staging, c, depth, depth_step, bgr, bgr_step, width, height, f))) return rc;
-  if ((rc = launch_set_header(s, c->d_hdr(), (int)f.n))) return rc;
-  c->written((long long)f.n);
-  return PFT_OK;
+  return upload_depth_image("pft_cloud_upload_depth_image", c, depth, depth_step, bgr, bgr_step, width, height, fx, fy, cx, cy, false);
 }
 
 int pft_cloud_upload_depth_image_async(pft_cloud* c, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step, uint32_t width,
                                        uint32_t height, double fx, double fy, double cx, double cy) {
-  if (!c) { set_last_error("pft_cloud_upload_depth_image_async: null cloud"); return PFT_ERR_INVALID; }
-  DepthImageFrame f;
-  int rc = check_depth_image("pft_cloud_upload_depth_image_async", depth, depth_step, bgr, bgr_step, width, height, fx, fy, cx, cy, &f);
-  if (rc) return rc;
-  cudaStream_t cs = nullptr;
-  if ((rc = begin_async_upload(c, f.n, &cs))) return rc;
-  if ((rc = enqueue_depth_image(cs, c->raw_staging, c, depth, depth_step, bgr, bgr_step, width, height, f))) return rc;
-  return end_async_upload(c, f.n, cs);
+  return upload_depth_image("pft_cloud_upload_depth_image_async", c, depth, depth_step, bgr, bgr_step, width, height, fx, fy, cx, cy, true);
+}
+
+int pft_cloud_upload_depth_images(pft_cloud* c, const pft_depth_camera* cams, int n) {
+  return upload_depth_images("pft_cloud_upload_depth_images", c, cams, n, false);
+}
+
+int pft_cloud_upload_depth_images_async(pft_cloud* c, const pft_depth_camera* cams, int n) {
+  return upload_depth_images("pft_cloud_upload_depth_images_async", c, cams, n, true);
 }
 
 int pft_cloud_wait_upload(pft_cloud* c) {

@@ -76,17 +76,22 @@ __global__ void unpack_pointcloud2_kernel(const unsigned int* __restrict__ src, 
 // point_cloud_xyzrgb nodelet that computes the /kinect2/<res>/points topic the reference subscribes to (ref:
 // src/auto_tracking.cpp:775), i.e. depth_image_proc::convert<uint16_t> + its colour copy.  Every fp32 operation is
 // rounded on its own (-fmad=false), in the nodelet's order: x = ((u - cx) * d) * (0.001f / fx), z = d * 0.001f; d == 0
-// is a quiet-NaN point (colour still written).  `src` holds the depth rows (`depth_step` bytes apart, even), the colour
-// rows start at byte `bgr_off`.  Thread = pixel along a row: the warp's 2-byte depth loads, 1-byte colour loads and
-// 16-byte stores each cover one contiguous span.  Organised row-major output, as unpack_pointcloud2_kernel.
-__global__ void depth_image_kernel(const unsigned char* __restrict__ src, size_t bgr_off, float4* __restrict__ dst, unsigned int width,
-                                   unsigned int height, unsigned int depth_step, unsigned int bgr_step, float cx, float cy, float kx, float ky) {
+// is a quiet-NaN point (colour still written).  Camera blockIdx.z of `cams` has its depth rows (`depth_step` bytes
+// apart, even) at byte `depth_off` of `src`, its colour rows at byte `bgr_off`, and its organised row-major points
+// from point `out_off` of `dst`: several calibrated cameras fused into one cloud (`scene += cloud_k`) in one launch.
+// A camera with a matrix (camera -> common frame) then moves each finite point as pcl::transformPointCloud does
+// (PCL 1.8.0, not dense: non-finite points are copied untouched), x' = ((m00 x + m01 y) + m02 z) + m03; the branch is
+// uniform per block.  Thread = pixel along a row: the warp's 2-byte depth loads, 1-byte colour loads and 16-byte
+// stores each cover one contiguous span.  One camera without a matrix is the single-image ingest.
+__global__ void depth_image_kernel(const unsigned char* __restrict__ src, float4* __restrict__ dst, const __grid_constant__ DepthCameras cams) {
+  const DepthCamera& k = cams.cam[blockIdx.z];
   const float nan = __uint_as_float(0x7fc00000u);
+  const unsigned int width = k.width, height = k.height;
   for (unsigned int v = blockIdx.y; v < height; v += gridDim.y) {
-    const unsigned short* drow = reinterpret_cast<const unsigned short*>(src + (size_t)v * depth_step);
-    const unsigned char* crow = src + bgr_off + (size_t)v * bgr_step;
-    float4* orow = dst + (size_t)v * width;
-    const float fy = (float)v - cy;
+    const unsigned short* drow = reinterpret_cast<const unsigned short*>(src + k.depth_off + (size_t)v * k.depth_step);
+    const unsigned char* crow = src + k.bgr_off + (size_t)v * k.bgr_step;
+    float4* orow = dst + k.out_off + (size_t)v * width;
+    const float fy = (float)v - k.cy;
     for (unsigned int u = blockIdx.x * blockDim.x + threadIdx.x; u < width; u += gridDim.x * blockDim.x) {
       const unsigned int d = drow[u];
       const unsigned char* c = crow + 3 * (size_t)u;
@@ -94,9 +99,16 @@ __global__ void depth_image_kernel(const unsigned char* __restrict__ src, size_t
       float4 p = make_float4(nan, nan, nan, __uint_as_float(rgba));
       if (d != 0) {
         const float fd = (float)d;
-        p.x = (((float)u - cx) * fd) * kx;
-        p.y = (fy * fd) * ky;
+        p.x = (((float)u - k.cx) * fd) * k.kx;
+        p.y = (fy * fd) * k.ky;
         p.z = fd * 0.001f;
+        if (k.has_m && finite3(p)) {
+          const float* m = k.m;
+          const float x = p.x, y = p.y, z = p.z;
+          p.x = ((m[0] * x + m[1] * y) + m[2] * z) + m[3];
+          p.y = ((m[4] * x + m[5] * y) + m[6] * z) + m[7];
+          p.z = ((m[8] * x + m[9] * y) + m[10] * z) + m[11];
+        }
       }
       orow[u] = p;
     }
@@ -321,11 +333,16 @@ int launch_unpack_pointcloud2(cudaStream_t s, const void* src, float4* dst, unsi
   PFT_LAUNCH_CHECK();
   return PFT_OK;
 }
-int launch_depth_image(cudaStream_t s, const void* src, size_t bgr_off, float4* dst, unsigned int width, unsigned int height, unsigned int depth_step,
-                       unsigned int bgr_step, float cx, float cy, float kx, float ky) {
-  if ((size_t)width * height == 0) return PFT_OK;
-  const dim3 grid((width + 127) / 128, height < 65535u ? height : 65535u);
-  depth_image_kernel<<<grid, 128, 0, s>>>(reinterpret_cast<const unsigned char*>(src), bgr_off, dst, width, height, depth_step, bgr_step, cx, cy, kx, ky);
+int launch_depth_image(cudaStream_t s, const void* src, float4* dst, const DepthCameras& cams, int n) {
+  if (n < 1) return PFT_OK;
+  // blocks past a smaller camera's width or height find no pixel and return
+  unsigned int width = 0, height = 0;
+  for (int k = 0; k < n; ++k) {
+    width = cams.cam[k].width > width ? cams.cam[k].width : width;
+    height = cams.cam[k].height > height ? cams.cam[k].height : height;
+  }
+  const dim3 grid((width + 127) / 128, height < 65535u ? height : 65535u, (unsigned int)n);
+  depth_image_kernel<<<grid, 128, 0, s>>>(reinterpret_cast<const unsigned char*>(src), dst, cams);
   PFT_LAUNCH_CHECK();
   return PFT_OK;
 }

@@ -85,9 +85,19 @@ int launch_unpack_pcl32(cudaStream_t s, const void* src32, float4* dst, size_t n
 int launch_pack_pcl32(cudaStream_t s, const float4* src, void* dst32, size_t n);
 int launch_unpack_pointcloud2(cudaStream_t s, const void* src, float4* dst, unsigned int width, unsigned int height, unsigned int point_step,
                               unsigned int row_step, int off_x, int off_y, int off_z, int off_rgb);
-// depth rows at `src`, colour rows at `src + bgr_off`; cx, cy, kx = 0.001f / fx, ky as the fp32 constants of the conversion
-int launch_depth_image(cudaStream_t s, const void* src, size_t bgr_off, float4* dst, unsigned int width, unsigned int height, unsigned int depth_step,
-                       unsigned int bgr_step, float cx, float cy, float kx, float ky);
+// One camera of a depth-image ingest, as depth_image_kernel reads it (by value, one launch for every camera): its two
+// images at byte offsets of the staging buffer, its first point in the output cloud, cx, cy, kx = 0.001f / fx, ky as
+// the fp32 constants of the conversion, and the optional camera -> common frame matrix (3x4 row-major).
+struct DepthCamera {
+  size_t depth_off, bgr_off, out_off;
+  unsigned int width, height, depth_step, bgr_step;
+  float cx, cy, kx, ky;
+  int has_m;
+  float m[12];
+};
+struct DepthCameras { DepthCamera cam[PFT_MAX_DEPTH_CAMERAS]; };
+// cameras 0 .. n-1 of `cams`, none of them empty, converted by one launch (blockIdx.z = camera)
+int launch_depth_image(cudaStream_t s, const void* src, float4* dst, const DepthCameras& cams, int n);
 int launch_set_header(cudaStream_t s, CloudHeader* hdr, int n);
 int run_passthrough(pft_context* ctx, const pft_cloud* in, pft_cloud* out, int field, float lo, float hi, int drop_zero);
 int run_voxel_grid(pft_context* ctx, const pft_cloud* in, pft_cloud* out, float leaf, int field, float lo, float hi);

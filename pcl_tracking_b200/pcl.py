@@ -96,6 +96,35 @@ class PinnedBuffer:
             pass
 
 
+def _image_arg(img, dtype, channels, step, width, height, keep):
+    """(pointer, width, height, step in bytes) of one image: an array (rows may be padded: the row stride is the step),
+    appended to `keep`, or a raw host pointer (int) with width, height and the step (default: packed rows)."""
+    pixel = np.dtype(dtype).itemsize * channels
+    if isinstance(img, int):
+        if width is None or height is None:
+            raise ValueError("a pointer image needs width and height")
+        return C.c_void_p(img), int(width), int(height), int(width) * pixel if step is None else int(step)
+    a = np.asarray(img)
+    shape = "(H, W)" if channels == 1 else "(H, W, %d)" % channels
+    if a.dtype != dtype or a.ndim != (2 if channels == 1 else 3) or (channels > 1 and a.shape[2] != channels):
+        raise TypeError("image must be a %s array of shape %s, got %s %r" % (np.dtype(dtype), shape, a.dtype, a.shape))
+    # padded rows (a view into a wider buffer) go as they are, with the row stride as the step
+    packed = a.strides[1] == pixel and (channels == 1 or a.strides[2] == a.itemsize)
+    if not packed or a.shape[0] < 2 or a.strides[0] < a.shape[1] * pixel:
+        a = np.ascontiguousarray(a)
+    keep.append(a)
+    return C.c_void_p(a.ctypes.data if a.size else None), a.shape[1], a.shape[0], a.strides[0]
+
+
+def _depth_frame(depth, bgr, width, height, depth_step, bgr_step, keep):
+    """(depth pointer, depth step, bgr pointer, bgr step, width, height) of a uint16 depth + bgr8 colour image pair."""
+    dp, w, h, dstep = _image_arg(depth, np.uint16, 1, depth_step, width, height, keep)
+    bp, w2, h2, bstep = _image_arg(bgr, np.uint8, 3, bgr_step, width, height, keep)
+    if (w, h) != (w2, h2):
+        raise ValueError("depth is %dx%d, colour %dx%d" % (w, h, w2, h2))
+    return dp, dstep, bp, bstep, w, h
+
+
 class PointCloud:
     """pcl::PointCloud<pcl::PointXYZRGBA> resident in HBM as float4 {x, y, z, rgba}."""
 
@@ -158,31 +187,42 @@ class PointCloud:
         stride is the step) or a raw host pointer (int; pinned for `asynchronous`) with width, height and the steps in
         bytes (default: packed rows).  fx, fy, cx, cy: camera_info.K[0], K[4], K[2], K[5]."""
         keep = []
-
-        def image(img, dtype, channels, step):
-            pixel = np.dtype(dtype).itemsize * channels
-            if isinstance(img, int):
-                if width is None or height is None:
-                    raise ValueError("a pointer image needs width and height")
-                return C.c_void_p(img), int(width), int(height), int(width) * pixel if step is None else int(step)
-            a = np.asarray(img)
-            shape = "(H, W)" if channels == 1 else "(H, W, %d)" % channels
-            if a.dtype != dtype or a.ndim != (2 if channels == 1 else 3) or (channels > 1 and a.shape[2] != channels):
-                raise TypeError("image must be a %s array of shape %s, got %s %r" % (np.dtype(dtype), shape, a.dtype, a.shape))
-            # padded rows (a view into a wider buffer) go as they are, with the row stride as the step
-            packed = a.strides[1] == pixel and (channels == 1 or a.strides[2] == a.itemsize)
-            if not packed or a.shape[0] < 2 or a.strides[0] < a.shape[1] * pixel:
-                a = np.ascontiguousarray(a)
-            keep.append(a)
-            return C.c_void_p(a.ctypes.data if a.size else None), a.shape[1], a.shape[0], a.strides[0]
-
-        dp, w, h, dstep = image(depth, np.uint16, 1, depth_step)
-        bp, w2, h2, bstep = image(bgr, np.uint8, 3, bgr_step)
-        if (w, h) != (w2, h2):
-            raise ValueError("depth is %dx%d, colour %dx%d" % (w, h, w2, h2))
+        dp, dstep, bp, bstep, w, h = _depth_frame(depth, bgr, width, height, depth_step, bgr_step, keep)
         self._keep = keep
         fn = capi.load().pft_cloud_upload_depth_image_async if asynchronous else capi.load().pft_cloud_upload_depth_image
         check(fn(self._h, dp, dstep, bp, bstep, w, h, float(fx), float(fy), float(cx), float(cy)))
+        return self
+
+    def fromDepthImages(self, cameras, asynchronous=False):
+        """Several calibrated cameras fused into one unorganised device cloud (pft_cloud_upload_depth_images): for
+        each camera k the cloud fromDepthImage makes, moved by pcl::transformPointCloud(cloud_k, T_k) into the common
+        frame, then scene += cloud_k, all converted in one kernel launch.  `cameras`: up to 8 mappings, each with
+        `depth` and `bgr` as for fromDepthImage (and `width`, `height`, `depth_step`, `bgr_step` for pointer images),
+        either `K` (3x3 camera_info matrix) or `fx`, `fy`, `cx`, `cy`, and an optional `pose`: the 4x4 or 3x4 matrix
+        from the camera's optical frame to the common frame, cast to float32 (absent or None: the camera's own frame)."""
+        keep = []
+        cams = list(cameras)
+        arr = (capi.DepthCamera * len(cams))()
+        for k, cam in enumerate(cams):
+            dp, dstep, bp, bstep, w, h = _depth_frame(cam["depth"], cam["bgr"], cam.get("width"), cam.get("height"), cam.get("depth_step"),
+                                                      cam.get("bgr_step"), keep)
+            if "K" in cam:
+                K = np.asarray(cam["K"], dtype=np.float64)
+                fx, fy, cx, cy = K[0, 0], K[1, 1], K[0, 2], K[1, 2]
+            else:
+                fx, fy, cx, cy = cam["fx"], cam["fy"], cam["cx"], cam["cy"]
+            m12 = None
+            if cam.get("pose") is not None:
+                pose = np.asarray(cam["pose"], dtype=np.float32)
+                if pose.shape not in ((4, 4), (3, 4)):
+                    raise ValueError("camera %d: pose must be 4x4 or 3x4, got %r" % (k, pose.shape))
+                m = np.ascontiguousarray(pose[:3, :4])
+                keep.append(m)
+                m12 = m.ctypes.data_as(C.POINTER(C.c_float))
+            arr[k] = capi.DepthCamera(dp.value, dstep, bp.value, bstep, w, h, float(fx), float(fy), float(cx), float(cy), m12)
+        self._keep = keep
+        fn = capi.load().pft_cloud_upload_depth_images_async if asynchronous else capi.load().pft_cloud_upload_depth_images
+        check(fn(self._h, arr, len(cams)))
         return self
 
     def broadcast(self, capacity, root=0):

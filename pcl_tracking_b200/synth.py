@@ -67,14 +67,24 @@ def object_pose(obj, frame, period=20):
     return R, c
 
 
-def render(frame=0, objects=None, sensor=KINECT2_SD, seed=0xC0FFEE, noise=True, holes=0.05):
-    """Returns (points[H*W] POINT, obj_id[H*W] int8 (-1 = background/none))."""
+def render(frame=0, objects=None, sensor=KINECT2_SD, seed=0xC0FFEE, noise=True, holes=0.05, camera=None):
+    """Returns (points[H*W] POINT, obj_id[H*W] int8 (-1 = background/none)).
+
+    The scene (table, wall, objects) is defined in the frame of the default camera.  `camera` = (R, t), the pose of
+    another camera in that frame (world-from-camera: p_world = R p_cam + t), ray-casts the same scene from there; the
+    points are then in that camera's optical frame."""
     if objects is None:
         objects = default_objects(1)
     W, H, f, cx, cy = sensor["width"], sensor["height"], sensor["f"], sensor["cx"], sensor["cy"]
     rng = np.random.default_rng(seed + 7919 * frame)
     uu, vv = np.meshgrid(np.arange(W, dtype=np.float64), np.arange(H, dtype=np.float64))
     d = np.stack([(uu - cx) / f, (vv - cy) / f, np.ones_like(uu)], axis=-1).reshape(-1, 3)
+    d_cam = d
+    # rays o + t d: t is the depth along the camera's optical axis (its z component of d is 1 in the camera frame)
+    o = None
+    if camera is not None:
+        Rc, o = np.asarray(camera[0], dtype=np.float64), np.asarray(camera[1], dtype=np.float64)
+        d = d_cam @ Rc.T
     n_px = d.shape[0]
     t_best = np.full(n_px, np.inf)
     colour = np.zeros((n_px, 3), dtype=np.float64)
@@ -89,17 +99,24 @@ def render(frame=0, objects=None, sensor=KINECT2_SD, seed=0xC0FFEE, noise=True, 
         oid[m] = ident
 
     # back wall z = 3.5
-    hit(np.full(n_px, 3.5), (200, 200, 190), -1)
+    if o is None:
+        hit(np.full(n_px, 3.5), (200, 200, 190), -1)
+    else:
+        with np.errstate(divide="ignore", invalid="ignore"):
+            tw = (3.5 - o[2]) / d[:, 2]
+        hit(np.where(np.isfinite(tw), tw, -1.0), (200, 200, 190), -1)
     # table: bounded rectangle in the plane
     u, v, n = table_frame()
     denom = d @ n
     with np.errstate(divide="ignore", invalid="ignore"):
-        t = (_TABLE_P @ n) / denom
-    P = d * t[:, None] - _TABLE_P
+        t = ((_TABLE_P if o is None else _TABLE_P - o) @ n) / denom
+    P = (d * t[:, None] if o is None else o + d * t[:, None]) - _TABLE_P
     inb = (np.abs(P @ u) < 0.85) & (np.abs(P @ v) < 0.60) & np.isfinite(t)
     hit(np.where(np.isfinite(t), t, -1.0), (120, 100, 80), -1, inb)
     for k, ob in enumerate(objects):
         R, c = object_pose(ob, frame)
+        if o is not None:
+            c = c - o  # the ray origin at 0
         if ob["kind"] == "sphere":
             r = ob["size"][0] / 2
             b = d @ c
@@ -128,10 +145,12 @@ def render(frame=0, objects=None, sensor=KINECT2_SD, seed=0xC0FFEE, noise=True, 
             oid[m] = k
     z = t_best.copy()
     if noise:
-        z = z + rng.normal(0.0, 1.0, n_px) * 0.0015 * z * z
+        with np.errstate(invalid="ignore"):  # inf depth (rays of other viewpoints that hit nothing)
+            z = z + rng.normal(0.0, 1.0, n_px) * 0.0015 * z * z
         colour = np.clip(colour + rng.uniform(-10, 10, colour.shape), 0, 255)
     pts = np.zeros(n_px, dtype=POINT)
-    xyz = d * z[:, None]
+    with np.errstate(invalid="ignore"):  # rays that hit nothing (other viewpoints): inf * 0, dropped below
+        xyz = d_cam * z[:, None]
     bad = ~np.isfinite(z)
     if holes > 0:
         bad |= rng.random(n_px) < holes
@@ -141,6 +160,32 @@ def render(frame=0, objects=None, sensor=KINECT2_SD, seed=0xC0FFEE, noise=True, 
     c8 = colour.astype(np.uint32)
     pts["rgba"] = (255 << 24) | (c8[:, 0] << 16) | (c8[:, 1] << 8) | c8[:, 2]
     return pts, oid
+
+
+def look_at(eye, target, up):
+    """World-from-camera pose (R, t) of a camera at `eye` whose optical axis points at `target` (optical frame: x right,
+    y down, z forward) with `up` up in its image."""
+    eye, target, up = (np.asarray(a, dtype=np.float64) for a in (eye, target, up))
+    z = target - eye
+    z /= np.linalg.norm(z)
+    x = np.cross(-up, z)
+    x /= np.linalg.norm(x)
+    y = np.cross(z, x)
+    return np.stack([x, y, z], axis=1), eye
+
+
+def side_camera():
+    """A second viewpoint of the table: 1.3 m to its side along the table's u axis and 0.55 m above it, looking at its
+    centre.  Returns the world-from-camera pose (R, t) that render(camera=...) takes."""
+    u, v, n = table_frame()
+    return look_at(_TABLE_P + 1.3 * u + 0.55 * n, _TABLE_P + 0.1 * n, n)
+
+
+def pose_matrix(camera):
+    """The 4x4 matrix of a world-from-camera pose (R, t): p_world = M @ [p_cam, 1]."""
+    m = np.eye(4)
+    m[:3, :3], m[:3, 3] = camera[0], camera[1]
+    return m
 
 
 def depth_images(pts, sensor=KINECT2_SD):
