@@ -141,16 +141,33 @@ inline std::shared_ptr<Context> nextTrackerContext() {
   return per_device[dev];
 }
 
+// sensor_msgs/Image::encoding of a depth image -> pft_depth_encoding: "16UC1" and "mono16" (the same bytes, uint16
+// millimetres), "32FC1" (float metres).  Anything else throws pft::Error (PFT_ERR_INVALID).
+inline int32_t depthEncoding(const std::string& e) {
+  if (e == "16UC1" || e == "mono16") return PFT_DEPTH_16UC1;
+  if (e == "32FC1") return PFT_DEPTH_32FC1;
+  throw Error(PFT_ERR_INVALID, ("unknown depth encoding \"" + e + "\" (16UC1, mono16 or 32FC1)").c_str());
+}
+// ... of a colour image -> pft_colour_encoding: "bgr8", "rgb8", "bgra8", "rgba8", "mono8", or "none" for depth alone
+// (depth_image_proc/point_cloud_xyz: rgba = 0, the colour pointer is ignored).  Anything else throws pft::Error.
+inline int32_t colourEncoding(const std::string& e) {
+  static const char* const names[] = {"bgr8", "rgb8", "bgra8", "rgba8", "mono8", "none"};  // in pft_colour_encoding order
+  for (int32_t k = 0; k <= PFT_COLOUR_NONE; ++k) if (e == names[k]) return k;
+  throw Error(PFT_ERR_INVALID, ("unknown colour encoding \"" + e + "\" (bgr8, rgb8, bgra8, rgba8, mono8 or none)").c_str());
+}
+
 // One calibrated camera of a fused frame (PointCloud::fromDepthImages): the registered images and intrinsics of
 // fromDepthImage, and optionally the pose of its optical frame in the common frame, T_k of
 // pcl::transformPointCloud(cloud_k, T_k) (e.g. tf2 lookupTransform(target, camera_optical_frame) as Eigen::Affine3f).
 struct DepthCamera {
-  const uint16_t* depth = nullptr;
+  const void* depth = nullptr;
   uint32_t depth_step = 0;  // bytes (msg.step)
-  const uint8_t* bgr = nullptr;
+  const uint8_t* bgr = nullptr;  // the colour image, in colour_encoding
   uint32_t bgr_step = 0;
   uint32_t width = 0, height = 0;
   double fx = 0, fy = 0, cx = 0, cy = 0;  // camera_info K[0], K[4], K[2], K[5]
+  std::string depth_encoding = "16UC1";   // msg.encoding, as depthEncoding / colourEncoding take it
+  std::string colour_encoding = "bgr8";
   bool has_pose = false;
   float pose[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};  // 3x4 row-major
   // any affine type with operator()(row, col), as setTrans: Eigen::Affine3f, pft::Affine3f
@@ -244,6 +261,22 @@ class PointCloud {
     width = w; height = h;
     mark_device_written();
   }
+  // Both of the above for images in any encoding the depth_image_proc nodelets take (pft_cloud_upload_depth_images_enc,
+  // one camera), named as sensor_msgs/Image::encoding spells it, so that a callback passes its messages through:
+  //   cloud->fromDepthImage(d->data.data(), d->step, d->encoding, c->data.data(), c->step, c->encoding, d->width,
+  //                         d->height, K[0], K[4], K[2], K[5]);
+  // Depth "16UC1" / "mono16" / "32FC1"; colour "bgr8", "rgb8", "bgra8", "rgba8", "mono8", or "none" for depth alone
+  // (point_cloud_xyz: rgba = 0, `colour` is ignored).  An unknown encoding throws pft::Error (PFT_ERR_INVALID).
+  void fromDepthImage(const void* depth, uint32_t depth_step, const std::string& depth_encoding, const uint8_t* colour, uint32_t colour_step,
+                      const std::string& colour_encoding, uint32_t w, uint32_t h, double fx, double fy, double cx, double cy,
+                      const std::shared_ptr<pft::Context>& ctx = pft::Context::Default()) {
+    upload_depth_image(depth, depth_step, depth_encoding, colour, colour_step, colour_encoding, w, h, fx, fy, cx, cy, ctx, false);
+  }
+  void fromDepthImageAsync(const void* depth, uint32_t depth_step, const std::string& depth_encoding, const uint8_t* colour, uint32_t colour_step,
+                           const std::string& colour_encoding, uint32_t w, uint32_t h, double fx, double fy, double cx, double cy,
+                           const std::shared_ptr<pft::Context>& ctx = pft::Context::Default()) {
+    upload_depth_image(depth, depth_step, depth_encoding, colour, colour_step, colour_encoding, w, h, fx, fy, cx, cy, ctx, true);
+  }
   // Several calibrated cameras fused into one scene (pft_cloud_upload_depth_images): for each camera,
   // pcl::transformPointCloud(cloud_k, T_k) of the cloud fromDepthImage makes, then scene += cloud_k, in one kernel
   // launch.  The cloud is unorganised: width = all the cameras' pixels, height = 1.
@@ -271,16 +304,29 @@ class PointCloud {
   PointCloud& operator=(const PointCloud& o) { points = o.host_points(); width = o.width; height = o.height; host_dirty_ = true; device_only_ = false; return *this; }
 
  private:
-  void upload_depth_cameras(const std::vector<pft::DepthCamera>& cams, const std::shared_ptr<pft::Context>& ctx, bool asynchronous) {
+  void upload_depth_image(const void* depth, uint32_t depth_step, const std::string& depth_encoding, const uint8_t* colour, uint32_t colour_step,
+                          const std::string& colour_encoding, uint32_t w, uint32_t h, double fx, double fy, double cx, double cy,
+                          const std::shared_ptr<pft::Context>& ctx, bool asynchronous) {
+    const pft_depth_camera_enc c = {{depth, depth_step, colour, colour_step, w, h, fx, fy, cx, cy, nullptr}, pft::depthEncoding(depth_encoding),
+                                    pft::colourEncoding(colour_encoding)};
     if (!dev_) { ctx_ = ctx; pft::check(pft_cloud_create(ctx_->get(), &dev_)); }
-    std::vector<pft_depth_camera> c(cams.size());
+    pft::check(asynchronous ? pft_cloud_upload_depth_images_enc_async(dev_, &c, 1) : pft_cloud_upload_depth_images_enc(dev_, &c, 1));
+    points.clear();
+    width = w; height = h;
+    mark_device_written();
+  }
+  void upload_depth_cameras(const std::vector<pft::DepthCamera>& cams, const std::shared_ptr<pft::Context>& ctx, bool asynchronous) {
+    std::vector<pft_depth_camera_enc> c(cams.size());
     size_t n = 0;
     for (size_t k = 0; k < cams.size(); ++k) {
       const pft::DepthCamera& s = cams[k];
-      c[k] = pft_depth_camera{s.depth, s.depth_step, s.bgr, s.bgr_step, s.width, s.height, s.fx, s.fy, s.cx, s.cy, s.has_pose ? s.pose : nullptr};
+      c[k] = pft_depth_camera_enc{{s.depth, s.depth_step, s.bgr, s.bgr_step, s.width, s.height, s.fx, s.fy, s.cx, s.cy, s.has_pose ? s.pose : nullptr},
+                                  pft::depthEncoding(s.depth_encoding), pft::colourEncoding(s.colour_encoding)};
       n += (size_t)s.width * s.height;
     }
-    pft::check(asynchronous ? pft_cloud_upload_depth_images_async(dev_, c.data(), (int)c.size()) : pft_cloud_upload_depth_images(dev_, c.data(), (int)c.size()));
+    if (!dev_) { ctx_ = ctx; pft::check(pft_cloud_create(ctx_->get(), &dev_)); }
+    pft::check(asynchronous ? pft_cloud_upload_depth_images_enc_async(dev_, c.data(), (int)c.size())
+                            : pft_cloud_upload_depth_images_enc(dev_, c.data(), (int)c.size()));
     points.clear();
     width = (uint32_t)n; height = 1;
     mark_device_written();

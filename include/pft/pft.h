@@ -116,7 +116,38 @@ typedef struct {
  * PFT_MAX_DEPTH_CAMERAS, null `cams`, any camera that pft_cloud_upload_depth_image would reject (the message names
  * its index), a non-finite matrix entry, 2^31 pixels or more in total. */
 PFT_API int pft_cloud_upload_depth_images(pft_cloud* cloud, const pft_depth_camera* cams, int n);
-/* Frame ingest overlapped with the previous frame's compute (SURVEY 8 f-1).  Same arguments as the four uploads above,
+/* The calls above take 16UC1 depth and bgr8 colour.  Every encoding the depth_image_proc nodelets accept
+ * (point_cloud_xyzrgb, and point_cloud_xyz for depth alone) goes through pft_cloud_upload_depth_images_enc: each camera
+ * names its pair, `cam.bgr` / `cam.bgr_step` then hold the colour image in `colour_encoding`, and any mix of pairs is
+ * converted by the same one launch.  Pixel (u, v) becomes depth_image_proc::convert<T>'s point, every fp32 operation
+ * rounded on its own:
+ *   depth encoding    bytes  valid when      x (y likewise with v, cy, fy)                               z
+ *   PFT_DEPTH_16UC1   2      d != 0          ((u - (float)cx) * (float)d) * (float)((double)0.001f / fx)  (float)d * 0.001f
+ *   PFT_DEPTH_32FC1   4      isfinite(d)     ((u - (float)cx) * d) * (float)(1.0 / fx)                   d
+ * (16UC1 is millimetres, 32FC1 metres; 32FC1 keeps 0 and negative depths, as upstream.)  An invalid pixel gives a
+ * quiet-NaN x, y, z; its colour is still written.  rgba = b | g << 8 | r << 16 | 255 << 24, with r, g, b read at these
+ * byte offsets of the colour pixel:
+ *   colour encoding     bytes  r, g, b
+ *   PFT_COLOUR_BGR8     3      2, 1, 0
+ *   PFT_COLOUR_RGB8     3      0, 1, 2
+ *   PFT_COLOUR_BGRA8    4      2, 1, 0   (alpha ignored)
+ *   PFT_COLOUR_RGBA8    4      0, 1, 2   (alpha ignored)
+ *   PFT_COLOUR_MONO8    1      0, 0, 0
+ *   PFT_COLOUR_NONE     0      rgba = 0 (point_cloud_xyz; `bgr` and `bgr_step` are ignored and nothing is copied)
+ * sensor_msgs/Image "mono16" is 16UC1.  Camera k with {16UC1, bgr8} gives exactly the points of
+ * pft_cloud_upload_depth_images; one camera without a matrix those of pft_cloud_upload_depth_image.  PFT_ERR_INVALID,
+ * naming the camera: any rejection of pft_cloud_upload_depth_images, an unknown encoding, a 32FC1 depth step that is
+ * not a multiple of 4 or below 4 * width, a colour step below bytes-per-pixel * width, a null colour image with pixels
+ * (unless PFT_COLOUR_NONE).  Images are little-endian and of equal size. */
+typedef enum { PFT_DEPTH_16UC1 = 0, PFT_DEPTH_32FC1 = 1 } pft_depth_encoding;
+typedef enum { PFT_COLOUR_BGR8 = 0, PFT_COLOUR_RGB8 = 1, PFT_COLOUR_BGRA8 = 2, PFT_COLOUR_RGBA8 = 3, PFT_COLOUR_MONO8 = 4, PFT_COLOUR_NONE = 5 } pft_colour_encoding;
+typedef struct {
+  pft_depth_camera cam;
+  int32_t depth_encoding;   /* pft_depth_encoding */
+  int32_t colour_encoding;  /* pft_colour_encoding */
+} pft_depth_camera_enc;
+PFT_API int pft_cloud_upload_depth_images_enc(pft_cloud* cloud, const pft_depth_camera_enc* cams, int n);
+/* Frame ingest overlapped with the previous frame's compute (SURVEY 8 f-1).  Same arguments as the five uploads above,
  * but the copy (and the unpack kernel) run on a copy stream of the context instead of its compute stream: the call
  * returns at once, the copy starts when everything enqueued on the context BEFORE this call has finished (so earlier
  * readers of `cloud` are safe), and it overlaps whatever is enqueued AFTER it.  The first library call that consumes
@@ -130,6 +161,7 @@ PFT_API int pft_cloud_upload_pointcloud2_async(pft_cloud* cloud, const void* dat
 PFT_API int pft_cloud_upload_depth_image_async(pft_cloud* cloud, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step,
                                                uint32_t width, uint32_t height, double fx, double fy, double cx, double cy);
 PFT_API int pft_cloud_upload_depth_images_async(pft_cloud* cloud, const pft_depth_camera* cams, int n);
+PFT_API int pft_cloud_upload_depth_images_enc_async(pft_cloud* cloud, const pft_depth_camera_enc* cams, int n);
 PFT_API int pft_cloud_wait_upload(pft_cloud* cloud);
 PFT_API int pft_cloud_size(pft_cloud* cloud, size_t* n);
 PFT_API int pft_cloud_download(pft_cloud* cloud, void* host_points, size_t capacity, int layout, size_t* n);

@@ -52,6 +52,16 @@ class DepthCamera(C.Structure):
                 ("cy", C.c_double), ("m12", C.POINTER(C.c_float))]
 
 
+# pft_depth_encoding, pft_colour_encoding
+DEPTH_16UC1, DEPTH_32FC1 = 0, 1
+COLOUR_BGR8, COLOUR_RGB8, COLOUR_BGRA8, COLOUR_RGBA8, COLOUR_MONO8, COLOUR_NONE = range(6)
+
+
+class DepthCameraEnc(C.Structure):
+    """pft_depth_camera_enc: a pft_depth_camera with its depth and colour encodings (pft_cloud_upload_depth_images_enc)."""
+    _fields_ = [("cam", DepthCamera), ("depth_encoding", C.c_int32), ("colour_encoding", C.c_int32)]
+
+
 _vp, _i, _f, _d, _sz, _u64 = C.c_void_p, C.c_int, C.c_float, C.c_double, C.c_size_t, C.c_uint64
 _pp = C.POINTER(C.c_void_p)
 _psz = C.POINTER(C.c_size_t)
@@ -78,6 +88,8 @@ SIGNATURES = {
     "pft_cloud_upload_depth_image_async": (_i, [_vp, _vp, C.c_uint32, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _d, _d, _d, _d]),
     "pft_cloud_upload_depth_images": (_i, [_vp, C.POINTER(DepthCamera), _i]),
     "pft_cloud_upload_depth_images_async": (_i, [_vp, C.POINTER(DepthCamera), _i]),
+    "pft_cloud_upload_depth_images_enc": (_i, [_vp, C.POINTER(DepthCameraEnc), _i]),
+    "pft_cloud_upload_depth_images_enc_async": (_i, [_vp, C.POINTER(DepthCameraEnc), _i]),
     "pft_cloud_wait_upload": (_i, [_vp]),
     "pft_cloud_size": (_i, [_vp, _psz]),
     "pft_cloud_download": (_i, [_vp, _vp, _sz, _i, _psz]),

@@ -5,6 +5,7 @@
 //   pft_cloud_upload        pcl::fromPCLPointCloud2 into PointCloud<PointXYZRGBA>  (ref: src/auto_tracking.cpp:619-622)
 //   pft_cloud_upload_depth_image  depth_image_proc/point_cloud_xyzrgb, which computes the points topic of ref :775
 //   pft_cloud_upload_depth_images  the same per calibrated camera + transformPointCloud(cloud_k, T_k), scene += cloud_k
+//   pft_cloud_upload_depth_images_enc  the same in every encoding of point_cloud_xyzrgb / point_cloud_xyz
 //   pft_passthrough         filterPassThrough                                       (ref: src/auto_tracking.cpp:536-547)
 //   pft_passthrough_voxel_grid  filterPassThrough + gridSampleApprox / gridSample   (ref: src/auto_tracking.cpp:637, :683, :641)
 //   pft_prepare_model       removeZeroPoints + centroid + translate + gridSample    (ref: src/auto_tracking.cpp:656-674)
@@ -126,9 +127,9 @@ int check_pointcloud2_layout(size_t n, uint32_t width, uint32_t point_step, uint
 }
 
 // A depth + colour frame of one or more cameras, checked and laid out for one staging buffer: per camera its depth
-// rows, then its colour rows, each from a 16-byte aligned offset.  Only the bytes an image occupies are copied,
-// (height - 1) * step + width * bytes per pixel, so a caller's view into a larger buffer is never read past its last
-// pixel.  `cams` holds the cameras with pixels, in order, as depth_image_kernel reads them; their points follow
+// rows, then its colour rows (none for depth alone), each from a 16-byte aligned offset.  Only the bytes an image
+// occupies are copied, (height - 1) * step + width * bytes per pixel, so a caller's view into a larger buffer is never
+// read past its last pixel.  `cams` holds the cameras with pixels, in order, as depth_image_kernel reads them; their points follow
 // each other in the cloud.
 struct DepthImageFrame {
   DepthCameras cams;
@@ -142,10 +143,30 @@ struct DepthImageFrame {
 
 inline size_t align16(size_t b) { return (b + 15) & ~(size_t)15; }
 
+// Bytes per pixel of a colour encoding (pft_colour_encoding; 0: no colour image), -1 for an unknown one.
+int colour_bytes(int32_t enc) {
+  switch (enc) {
+    case PFT_COLOUR_BGR8: case PFT_COLOUR_RGB8: return 3;
+    case PFT_COLOUR_BGRA8: case PFT_COLOUR_RGBA8: return 4;
+    case PFT_COLOUR_MONO8: return 1;
+    case PFT_COLOUR_NONE: return 0;
+    default: return -1;
+  }
+}
+
 // Checks camera `cam` and appends it to `f`.  `cam` < 0: the single-image call, whose messages name no camera.
-int check_depth_image(const char* fn, int cam, const pft_depth_camera& c, DepthImageFrame* f) {
+int check_depth_image(const char* fn, int cam, const pft_depth_camera_enc& e, DepthImageFrame* f) {
+  const pft_depth_camera& c = e.cam;
   char who[24] = "";
   if (cam >= 0) snprintf(who, sizeof(who), ": camera %d", cam);
+  if (e.depth_encoding != PFT_DEPTH_16UC1 && e.depth_encoding != PFT_DEPTH_32FC1) {
+    set_last_error("%s%s: unknown depth encoding %d (PFT_DEPTH_16UC1 or PFT_DEPTH_32FC1)", fn, who, (int)e.depth_encoding);
+    return PFT_ERR_INVALID;
+  }
+  const int cbytes = colour_bytes(e.colour_encoding);
+  if (cbytes < 0) { set_last_error("%s%s: unknown colour encoding %d (PFT_COLOUR_BGR8 .. PFT_COLOUR_NONE)", fn, who, (int)e.colour_encoding); return PFT_ERR_INVALID; }
+  const bool metres = e.depth_encoding == PFT_DEPTH_32FC1;
+  const unsigned int dbytes = metres ? 4 : 2;
   const size_t n = (size_t)c.width * c.height;
   if (n > 0x7fffffffull) { set_last_error("%s%s: image too large", fn, who); return PFT_ERR_INVALID; }
   if (!(c.fx != 0.0 && c.fy != 0.0 && isfinite(c.fx) && isfinite(c.fy) && isfinite(c.cx) && isfinite(c.cy))) {
@@ -158,18 +179,19 @@ int check_depth_image(const char* fn, int cam, const pft_depth_camera& c, DepthI
     }
   }
   if (!n) return PFT_OK;
-  if (!c.depth || !c.bgr) { set_last_error("%s%s: null image", fn, who); return PFT_ERR_INVALID; }
-  if ((c.depth_step & 1) || (size_t)c.depth_step < (size_t)c.width * 2 || (size_t)c.bgr_step < (size_t)c.width * 3) {
-    set_last_error("%s%s: bad steps: depth %u (even, >= 2 * width), bgr %u (>= 3 * width), width %u", fn, who, c.depth_step, c.bgr_step, c.width);
+  if (!c.depth || (cbytes && !c.bgr)) { set_last_error("%s%s: null image", fn, who); return PFT_ERR_INVALID; }
+  if (c.depth_step % dbytes || (size_t)c.depth_step < (size_t)c.width * dbytes || (size_t)c.bgr_step < (size_t)c.width * cbytes) {
+    set_last_error("%s%s: bad steps: depth %u (a multiple of %u, >= %u * width), colour %u (>= %d * width), width %u", fn, who, c.depth_step, dbytes,
+                   dbytes, c.bgr_step, cbytes, c.width);
     return PFT_ERR_INVALID;
   }
   if (f->points + n > 0x7fffffffull) { set_last_error("%s: 2^31 pixels or more in total (at camera %d)", fn, cam); return PFT_ERR_INVALID; }
   const int i = f->n++;
   DepthCamera& k = f->cams.cam[i];
   f->depth[i] = c.depth;
-  f->bgr[i] = c.bgr;
-  f->depth_bytes[i] = (size_t)(c.height - 1) * c.depth_step + (size_t)c.width * 2;
-  f->bgr_bytes[i] = (size_t)(c.height - 1) * c.bgr_step + (size_t)c.width * 3;
+  f->bgr[i] = cbytes ? c.bgr : nullptr;
+  f->depth_bytes[i] = (size_t)(c.height - 1) * c.depth_step + (size_t)c.width * dbytes;
+  f->bgr_bytes[i] = cbytes ? (size_t)(c.height - 1) * c.bgr_step + (size_t)c.width * cbytes : 0;
   k.depth_off = f->staging;
   k.bgr_off = align16(k.depth_off + f->depth_bytes[i]);
   f->staging = align16(k.bgr_off + f->bgr_bytes[i]);
@@ -178,18 +200,22 @@ int check_depth_image(const char* fn, int cam, const pft_depth_camera& c, DepthI
   k.width = c.width;
   k.height = c.height;
   k.depth_step = c.depth_step;
-  k.bgr_step = c.bgr_step;
-  // the constants of depth_image_proc::convert<uint16_t>: float centre, float(double(0.001f) / f)
+  k.bgr_step = cbytes ? c.bgr_step : 0;
+  k.depth_enc = e.depth_encoding;
+  k.colour_enc = e.colour_encoding;
+  // the constants of depth_image_proc::convert<T>: float centre, float(unit / f) with the double unit
+  // DepthTraits<T>::toMeters(T(1)), double(0.001f) for uint16_t millimetres and 1 for float metres
+  const double unit = metres ? 1.0 : (double)0.001f;
   k.cx = (float)c.cx;
   k.cy = (float)c.cy;
-  k.kx = (float)((double)0.001f / c.fx);
-  k.ky = (float)((double)0.001f / c.fy);
+  k.kx = (float)(unit / c.fx);
+  k.ky = (float)(unit / c.fy);
   k.has_m = c.m12 != nullptr;
   if (c.m12) memcpy(k.m, c.m12, sizeof(k.m));
   return PFT_OK;
 }
 
-int check_depth_cameras(const char* fn, const pft_depth_camera* cams, int n, DepthImageFrame* f) {
+int check_depth_cameras(const char* fn, const pft_depth_camera_enc* cams, int n, DepthImageFrame* f) {
   if (!cams) { set_last_error("%s: null cameras", fn); return PFT_ERR_INVALID; }
   if (n < 1 || n > PFT_MAX_DEPTH_CAMERAS) { set_last_error("%s: %d cameras (1 to %d)", fn, n, PFT_MAX_DEPTH_CAMERAS); return PFT_ERR_INVALID; }
   for (int k = 0; k < n; ++k) {
@@ -207,7 +233,7 @@ int enqueue_depth_image(cudaStream_t s, pft::DevBuf& staging, pft_cloud* c, cons
   unsigned char* base = staging.as<unsigned char>();
   for (int k = 0; k < f.n; ++k) {
     PFT_CUDA_TRY(cudaMemcpyAsync(base + f.cams.cam[k].depth_off, f.depth[k], f.depth_bytes[k], cudaMemcpyHostToDevice, s));
-    PFT_CUDA_TRY(cudaMemcpyAsync(base + f.cams.cam[k].bgr_off, f.bgr[k], f.bgr_bytes[k], cudaMemcpyHostToDevice, s));
+    if (f.bgr_bytes[k]) PFT_CUDA_TRY(cudaMemcpyAsync(base + f.cams.cam[k].bgr_off, f.bgr[k], f.bgr_bytes[k], cudaMemcpyHostToDevice, s));
   }
   return launch_depth_image(s, base, c->d_pts(), f.cams, f.n);
 }
@@ -236,19 +262,27 @@ int upload_depth_frame(pft_cloud* c, const DepthImageFrame& f, bool asynchronous
 int upload_depth_image(const char* fn, pft_cloud* c, const void* depth, uint32_t depth_step, const void* bgr, uint32_t bgr_step, uint32_t width,
                        uint32_t height, double fx, double fy, double cx, double cy, bool asynchronous) {
   if (!c) { set_last_error("%s: null cloud", fn); return PFT_ERR_INVALID; }
-  const pft_depth_camera cam = {depth, depth_step, bgr, bgr_step, width, height, fx, fy, cx, cy, nullptr};
+  const pft_depth_camera_enc cam = {{depth, depth_step, bgr, bgr_step, width, height, fx, fy, cx, cy, nullptr}, PFT_DEPTH_16UC1, PFT_COLOUR_BGR8};
   DepthImageFrame f{};
   int rc = check_depth_image(fn, -1, cam, &f);
   if (rc) return rc;
   return upload_depth_frame(c, f, asynchronous);
 }
 
-int upload_depth_images(const char* fn, pft_cloud* c, const pft_depth_camera* cams, int n, bool asynchronous) {
+int upload_depth_images(const char* fn, pft_cloud* c, const pft_depth_camera_enc* cams, int n, bool asynchronous) {
   if (!c) { set_last_error("%s: null cloud", fn); return PFT_ERR_INVALID; }
   DepthImageFrame f{};
   int rc = check_depth_cameras(fn, cams, n, &f);
   if (rc) return rc;
   return upload_depth_frame(c, f, asynchronous);
+}
+
+// The cameras of pft_cloud_upload_depth_images(_async): 16UC1 depth, bgr8 colour.
+int upload_depth_images_bgr8(const char* fn, pft_cloud* c, const pft_depth_camera* cams, int n, bool asynchronous) {
+  pft_depth_camera_enc enc[PFT_MAX_DEPTH_CAMERAS];
+  const bool valid = cams && n >= 1 && n <= PFT_MAX_DEPTH_CAMERAS;  // otherwise check_depth_cameras rejects the call
+  for (int k = 0; valid && k < n; ++k) enc[k] = {cams[k], PFT_DEPTH_16UC1, PFT_COLOUR_BGR8};
+  return upload_depth_images(fn, c, cams ? enc : nullptr, n, asynchronous);
 }
 
 }  // namespace
@@ -451,11 +485,19 @@ int pft_cloud_upload_depth_image_async(pft_cloud* c, const void* depth, uint32_t
 }
 
 int pft_cloud_upload_depth_images(pft_cloud* c, const pft_depth_camera* cams, int n) {
-  return upload_depth_images("pft_cloud_upload_depth_images", c, cams, n, false);
+  return upload_depth_images_bgr8("pft_cloud_upload_depth_images", c, cams, n, false);
 }
 
 int pft_cloud_upload_depth_images_async(pft_cloud* c, const pft_depth_camera* cams, int n) {
-  return upload_depth_images("pft_cloud_upload_depth_images_async", c, cams, n, true);
+  return upload_depth_images_bgr8("pft_cloud_upload_depth_images_async", c, cams, n, true);
+}
+
+int pft_cloud_upload_depth_images_enc(pft_cloud* c, const pft_depth_camera_enc* cams, int n) {
+  return upload_depth_images("pft_cloud_upload_depth_images_enc", c, cams, n, false);
+}
+
+int pft_cloud_upload_depth_images_enc_async(pft_cloud* c, const pft_depth_camera_enc* cams, int n) {
+  return upload_depth_images("pft_cloud_upload_depth_images_enc_async", c, cams, n, true);
 }
 
 int pft_cloud_wait_upload(pft_cloud* c) {

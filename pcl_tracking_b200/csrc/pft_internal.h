@@ -86,11 +86,13 @@ int launch_pack_pcl32(cudaStream_t s, const float4* src, void* dst32, size_t n);
 int launch_unpack_pointcloud2(cudaStream_t s, const void* src, float4* dst, unsigned int width, unsigned int height, unsigned int point_step,
                               unsigned int row_step, int off_x, int off_y, int off_z, int off_rgb);
 // One camera of a depth-image ingest, as depth_image_kernel reads it (by value, one launch for every camera): its two
-// images at byte offsets of the staging buffer, its first point in the output cloud, cx, cy, kx = 0.001f / fx, ky as
-// the fp32 constants of the conversion, and the optional camera -> common frame matrix (3x4 row-major).
+// images at byte offsets of the staging buffer, their encodings (pft_depth_encoding, pft_colour_encoding), its first
+// point in the output cloud, cx, cy, kx = unit / fx, ky as the fp32 constants of the conversion (unit = 0.001f for
+// 16UC1, 1 for 32FC1), and the optional camera -> common frame matrix (3x4 row-major).
 struct DepthCamera {
   size_t depth_off, bgr_off, out_off;
   unsigned int width, height, depth_step, bgr_step;
+  int depth_enc, colour_enc;
   float cx, cy, kx, ky;
   int has_m;
   float m[12];

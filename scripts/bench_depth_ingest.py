@@ -12,7 +12,9 @@ tracker, synchronously and double-buffered (frame k + 1 uploaded on the copy str
 clouds); the poses of the two ingests must be identical at every step.  L2 is flushed (256 MiB write) before every
 step, outside the timed span.  Workloads as bench.py: c2 (sd, 512x424, 1000 particles) and qhd (960x540, the
 reference's KLD tracker of 400 / at most 500 particles).  The conversion kernel is also timed alone (torch.profiler,
-device time of depth_image_kernel per launch) and the synchronous image upload as a whole (CUDA events).
+device time of depth_image_kernel per launch) and the synchronous image upload as a whole (CUDA events), for each of
+the encoding pairs in ENCODINGS: 16UC1 + bgr8 (5 bytes per pixel over PCIe), 32FC1 + rgb8 (7), 32FC1 + bgra8 (8) and
+16UC1 depth alone (2).
 
 Needs a CUDA device; prints the card's name and power limit with the numbers, one JSON line per workload.
 """
@@ -29,6 +31,27 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 from bench import ITERATIONS, LEAF, N_FRAMES, frame_order  # noqa: E402
+
+# the depth + colour encodings the conversion is timed in: the Kinect2 pair, the Gazebo Kinect plugin's depth with an
+# rgb8 and a bgra8 camera, and depth alone
+ENCODINGS = [("16UC1", "bgr8"), ("32FC1", "rgb8"), ("32FC1", "bgra8"), ("16UC1", "none")]
+BYTES_PER_PIXEL = {"16UC1": 2, "32FC1": 4, "bgr8": 3, "rgb8": 3, "bgra8": 4, "none": 0}
+
+
+def encode_depth(depth_mm, encoding):
+    """A uint16 millimetre image in `encoding`: as it is, or float32 metres with NaN for no return."""
+    if encoding == "16UC1":
+        return depth_mm
+    return np.where(depth_mm == 0, np.float32(np.nan), depth_mm.astype(np.float32) * np.float32(0.001)).astype(np.float32)
+
+
+def encode_colour(bgr, encoding):
+    """A bgr8 image in `encoding`."""
+    if encoding == "bgr8":
+        return bgr
+    if encoding == "rgb8":
+        return np.ascontiguousarray(bgr[..., ::-1])
+    return np.concatenate([bgr, np.full(bgr.shape[:2] + (1,), 255, np.uint8)], axis=2)  # bgra8
 
 
 def card():
@@ -150,29 +173,40 @@ def main():
             print(json.dumps(rec), flush=True)
 
         # the conversion kernel alone (device time per launch, torch.profiler) and the synchronous image upload as a
-        # whole (two H2D copies + kernel + header, CUDA events), L2 flushed before each
+        # whole (H2D copies + kernel + header, CUDA events), L2 flushed before each, for each pair of encodings: the
+        # frames' images re-encoded as a camera of that pair would publish them (32FC1: metres, NaN where 16UC1 has 0)
         from torch.profiler import ProfilerActivity, profile
         cloud = pcl.PointCloud(ctx=ctx)
         reps = 100
-        up_ms = 0.0
-        with profile(activities=[ProfilerActivity.CUDA]) as prof:
-            for k in range(reps):
-                with torch.cuda.stream(stream):
-                    flush_buf.fill_(1)
-                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                e0.record(stream)
-                upload("images", cloud, k, False)
-                e1.record(stream)
-                e1.synchronize()
-                up_ms += e0.elapsed_time(e1)
-        kern = [e for e in prof.key_averages() if "depth_image_kernel" in e.key]
-        kernel_us = (getattr(kern[0], "device_time_total", None) or kern[0].cuda_time_total) / kern[0].count if kern else None
-        rec = {"what": "kernel", "workload": workload, "width": w, "height": h, "launches": kern[0].count if kern else 0,
-               "depth_image_kernel_us": kernel_us,
-               "kernel_bytes": 21 * w * h, "kernel_gb_per_s": (21 * w * h / (kernel_us * 1e-6) / 1e9) if kernel_us else None,
-               "image_upload_us": up_ms / reps * 1e3}
-        lines.append(rec)
-        print(json.dumps(rec), flush=True)
+        for denc, cenc in ENCODINGS:
+            pins = [(pcl.PinnedBuffer.of(encode_depth(d, denc)), pcl.PinnedBuffer.of(encode_colour(c, cenc)) if cenc != "none" else None)
+                    for d, c, _ in images]
+            up_ms = 0.0
+            with profile(activities=[ProfilerActivity.CUDA]) as prof:
+                for k in range(reps):
+                    with torch.cuda.stream(stream):
+                        flush_buf.fill_(1)
+                    f = frame_order(k, N_FRAMES)
+                    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                    e0.record(stream)
+                    cloud.fromDepthImage(pins[f][0].ptr, pins[f][1].ptr if pins[f][1] else None, fx, fy, cx, cy, width=w, height=h,
+                                         depth_encoding=denc, colour_encoding=cenc)
+                    e1.record(stream)
+                    e1.synchronize()
+                    up_ms += e0.elapsed_time(e1)
+            kern = [e for e in prof.key_averages() if "depth_image_kernel" in e.key]
+            kernel_us = (getattr(kern[0], "device_time_total", None) or kern[0].cuda_time_total) / kern[0].count if kern else None
+            pixel = BYTES_PER_PIXEL[denc] + BYTES_PER_PIXEL[cenc]
+            rec = {"what": "kernel", "workload": workload, "width": w, "height": h, "depth_encoding": denc, "colour_encoding": cenc,
+                   "h2d_bytes_per_frame": pixel * w * h, "launches": kern[0].count if kern else 0, "depth_image_kernel_us": kernel_us,
+                   "kernel_bytes": (pixel + 16) * w * h, "kernel_gb_per_s": ((pixel + 16) * w * h / (kernel_us * 1e-6) / 1e9) if kernel_us else None,
+                   "image_upload_us": up_ms / reps * 1e3}
+            lines.append(rec)
+            print(json.dumps(rec), flush=True)
+            for d, c in pins:
+                d.free()
+                if c:
+                    c.free()
         for b in pin32:
             b.free()
         for d, c in pin_img:
