@@ -176,6 +176,23 @@ struct DepthCamera {
     has_pose = true;
   }
   void clearPose() { has_pose = false; }
+  // Registration (depth_image_proc/register, on the device): set when `depth` is the image of a separate depth camera,
+  // not yet registered to the colour camera.  `depth` / `depth_step` / `depth_encoding` are then the depth camera's
+  // image, depth_width x depth_height; width, height, fx .. cy and the colour image stay the colour camera's, and the
+  // cloud is organised in its geometry.  Intrinsics are camera_info P[0], P[5], P[2], P[6], Tx = P[3], Ty = P[7].
+  bool has_registration = false;
+  double depth_to_colour[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};  // 3x4 row-major, depth optical -> colour optical
+  uint32_t depth_width = 0, depth_height = 0;
+  double depth_fx = 0, depth_fy = 0, depth_cx = 0, depth_cy = 0, depth_tx = 0, depth_ty = 0;
+  double colour_tx = 0, colour_ty = 0;
+  bool fill_upsampling = false;
+  // any affine type with operator()(row, col), as setPose, with double entries: Eigen::Affine3d of tf2
+  // lookupTransform(colour_frame, depth_frame)
+  template <typename AffineT> void setDepthToColour(const AffineT& t) {
+    for (int r = 0; r < 3; ++r) for (int c = 0; c < 4; ++c) depth_to_colour[r * 4 + c] = (double)t(r, c);
+    has_registration = true;
+  }
+  void clearDepthToColour() { has_registration = false; }
 };
 
 }  // namespace pft
@@ -279,7 +296,8 @@ class PointCloud {
   }
   // Several calibrated cameras fused into one scene (pft_cloud_upload_depth_images): for each camera,
   // pcl::transformPointCloud(cloud_k, T_k) of the cloud fromDepthImage makes, then scene += cloud_k, in one kernel
-  // launch.  The cloud is unorganised: width = all the cameras' pixels, height = 1.
+  // launch.  The cloud is unorganised: width = all the cameras' pixels, height = 1.  Cameras with setDepthToColour are
+  // registered into their colour camera on the device first (pft_cloud_upload_depth_images_reg).
   void fromDepthImages(const std::vector<pft::DepthCamera>& cams, const std::shared_ptr<pft::Context>& ctx = pft::Context::Default()) {
     upload_depth_cameras(cams, ctx, false);
   }
@@ -318,15 +336,28 @@ class PointCloud {
   void upload_depth_cameras(const std::vector<pft::DepthCamera>& cams, const std::shared_ptr<pft::Context>& ctx, bool asynchronous) {
     std::vector<pft_depth_camera_enc> c(cams.size());
     size_t n = 0;
+    bool registration = false;
     for (size_t k = 0; k < cams.size(); ++k) {
       const pft::DepthCamera& s = cams[k];
       c[k] = pft_depth_camera_enc{{s.depth, s.depth_step, s.bgr, s.bgr_step, s.width, s.height, s.fx, s.fy, s.cx, s.cy, s.has_pose ? s.pose : nullptr},
                                   pft::depthEncoding(s.depth_encoding), pft::colourEncoding(s.colour_encoding)};
       n += (size_t)s.width * s.height;
+      registration = registration || s.has_registration;
     }
     if (!dev_) { ctx_ = ctx; pft::check(pft_cloud_create(ctx_->get(), &dev_)); }
-    pft::check(asynchronous ? pft_cloud_upload_depth_images_enc_async(dev_, c.data(), (int)c.size())
-                            : pft_cloud_upload_depth_images_enc(dev_, c.data(), (int)c.size()));
+    if (registration) {  // pft_cloud_upload_depth_images_reg(_async): register on the device, then convert
+      std::vector<pft_depth_camera_reg> r(cams.size());
+      for (size_t k = 0; k < cams.size(); ++k) {
+        const pft::DepthCamera& s = cams[k];
+        r[k] = pft_depth_camera_reg{c[k], s.has_registration ? s.depth_to_colour : nullptr, s.depth_width, s.depth_height, s.depth_fx, s.depth_fy,
+                                    s.depth_cx, s.depth_cy, s.depth_tx, s.depth_ty, s.colour_tx, s.colour_ty, s.fill_upsampling ? 1 : 0};
+      }
+      pft::check(asynchronous ? pft_cloud_upload_depth_images_reg_async(dev_, r.data(), (int)r.size())
+                              : pft_cloud_upload_depth_images_reg(dev_, r.data(), (int)r.size()));
+    } else {
+      pft::check(asynchronous ? pft_cloud_upload_depth_images_enc_async(dev_, c.data(), (int)c.size())
+                              : pft_cloud_upload_depth_images_enc(dev_, c.data(), (int)c.size()));
+    }
     points.clear();
     width = (uint32_t)n; height = 1;
     mark_device_written();

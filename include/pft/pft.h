@@ -162,6 +162,52 @@ PFT_API int pft_cloud_upload_depth_image_async(pft_cloud* cloud, const void* dep
                                                uint32_t width, uint32_t height, double fx, double fy, double cx, double cy);
 PFT_API int pft_cloud_upload_depth_images_async(pft_cloud* cloud, const pft_depth_camera* cams, int n);
 PFT_API int pft_cloud_upload_depth_images_enc_async(pft_cloud* cloud, const pft_depth_camera_enc* cams, int n);
+/* Depth images that are NOT registered to the colour camera: the depth_image_proc/register nodelet
+ * (RegisterNodelet::convert<T>) on the device, followed by the conversion of pft_cloud_upload_depth_images_enc, i.e.
+ * the register -> point_cloud_xyzrgb nodelet chain.  A camera with `depth_to_colour` set has its depth image
+ * (`cam.depth`, `cam.depth_step`, `cam.depth_encoding`) in the depth camera's geometry, depth_width x depth_height;
+ * `cam.width`, `cam.height`, `cam.fx` .. `cam.cy`, the colour image and `cam.m12` are the colour camera's, as for
+ * pft_cloud_upload_depth_images_enc, and so is the cloud: width * height points, organised in the colour camera's
+ * geometry.  Intrinsics are image_geometry::PinholeCameraModel's, P[0], P[5], P[2], P[6], and Tx = P[3], Ty = P[7] (a
+ * monocular camera: K's, Tx = Ty = 0); full resolution (no binning, no ROI).  depth_to_colour: double 3x4 row-major,
+ * Eigen::Affine3d rows 0-2 of tf2 lookupTransform(colour_frame, depth_frame).  Every operation is in double unless
+ * stated, each rounded on its own:
+ *   1. the registered image starts all invalid: 0 (16UC1), quiet NaN (32FC1);
+ *   2. depth pixels (u, v) in raster order; an invalid raw depth (16UC1 0, 32FC1 non-finite) is skipped, otherwise
+ *      depth = (double)toMeters(d), toMeters = the float d * 0.001f (16UC1) or d (32FC1);
+ *   3. without fill_upsampling: X = ((u - cx_d) * depth - Tx_d) * (1.0 / fx_d), Y likewise with v, cy_d, Ty_d, fy_d,
+ *      Z = depth; p = M (X, Y, Z, 1), each row ((m0 X + m1 Y) + m2 Z) + m3; u' = (int)(((fx_c p.x + Tx_c) * (1.0 / p.z)
+ *      + cx_c) + 0.5), v' likewise (truncation toward zero: (-1, 0) lands on column 0); skipped unless 0 <= u' < width
+ *      and 0 <= v' < height; candidate fromMeters((float)p.z): (uint16_t)((float)p.z * 1000.0f + 0.5f) in float for
+ *      16UC1, (float)p.z for 32FC1;
+ *   4. with fill_upsampling: the same for the corners (u - 0.5f, v - 0.5f) and (u + 0.5f, v + 0.5f) (float sums), giving
+ *      (u1, v1) and (u2, v2) and z1, z2; skipped if u1 < 0 || u2 >= width || v1 < 0 || v2 >= height; otherwise every
+ *      pixel of [u1, u2] x [v1, v2] (possibly empty) gets the candidate fromMeters((float)(0.5 * (z1 + z2)));
+ *   5. z-buffer at the target: if (!valid(reg) || reg > new) reg = new.
+ * So a pixel holds the smallest valid candidate after its last reset (a 16UC1 0 or 32FC1 -inf candidate, which
+ * replaces anything), the earliest of equal ones (+0 before -0 if it came first); else +inf, if a +inf candidate came
+ * after that reset; else the reset value; else the initial one.  Where upstream is undefined C++ the candidate is
+ * dropped: a double -> int cast of NaN or of a value whose truncation does not fit an int, a 16UC1 fromMeters whose
+ * z * 1000.0f + 0.5f is NaN or truncates outside 0 .. 65535.  A 32FC1 candidate that is NaN (only a corner at +inf and
+ * one at -inf make one) is dropped as well.  The registered image is then converted exactly as
+ * pft_cloud_upload_depth_images_enc converts a registered one.  A registered camera without depth pixels gives width *
+ * height NaN points with their colour.  depth_to_colour NULL: the camera is exactly the pft_depth_camera_enc `cam`, and
+ * the other fields are ignored; registered and already-registered cameras mix in one call.  Kernel launches per frame:
+ * 2 (conversion and header) when no camera is registered, 5 when any is (reset scatter, z-buffer scatter, finalise),
+ * whatever the number of cameras.  PFT_ERR_INVALID, naming the camera: any rejection of
+ * pft_cloud_upload_depth_images_enc for the colour side, a non-finite matrix entry, depth fx or fy zero or not finite,
+ * a non-finite cx, cy, Tx or Ty on either camera, fill_upsampling not 0 or 1, a depth step that is not a multiple of the
+ * depth pixel or below depth_width pixels, a null depth image with pixels, 2^31 depth pixels or more. */
+typedef struct {
+  pft_depth_camera_enc cam;
+  const double* depth_to_colour;  /* 3x4 row-major; NULL: the depth is already registered */
+  uint32_t depth_width, depth_height;
+  double depth_fx, depth_fy, depth_cx, depth_cy, depth_tx, depth_ty;
+  double colour_tx, colour_ty;
+  int32_t fill_upsampling;        /* 0 or 1 */
+} pft_depth_camera_reg;
+PFT_API int pft_cloud_upload_depth_images_reg(pft_cloud* cloud, const pft_depth_camera_reg* cams, int n);
+PFT_API int pft_cloud_upload_depth_images_reg_async(pft_cloud* cloud, const pft_depth_camera_reg* cams, int n);
 PFT_API int pft_cloud_wait_upload(pft_cloud* cloud);
 PFT_API int pft_cloud_size(pft_cloud* cloud, size_t* n);
 PFT_API int pft_cloud_download(pft_cloud* cloud, void* host_points, size_t capacity, int layout, size_t* n);

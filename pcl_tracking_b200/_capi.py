@@ -62,6 +62,14 @@ class DepthCameraEnc(C.Structure):
     _fields_ = [("cam", DepthCamera), ("depth_encoding", C.c_int32), ("colour_encoding", C.c_int32)]
 
 
+class DepthCameraReg(C.Structure):
+    """pft_depth_camera_reg: a pft_depth_camera_enc whose depth image is in a separate depth camera's geometry, registered
+    into the colour camera on the device (depth_to_colour NULL: already registered)."""
+    _fields_ = [("cam", DepthCameraEnc), ("depth_to_colour", C.POINTER(C.c_double)), ("depth_width", C.c_uint32), ("depth_height", C.c_uint32),
+                ("depth_fx", C.c_double), ("depth_fy", C.c_double), ("depth_cx", C.c_double), ("depth_cy", C.c_double), ("depth_tx", C.c_double),
+                ("depth_ty", C.c_double), ("colour_tx", C.c_double), ("colour_ty", C.c_double), ("fill_upsampling", C.c_int32)]
+
+
 _vp, _i, _f, _d, _sz, _u64 = C.c_void_p, C.c_int, C.c_float, C.c_double, C.c_size_t, C.c_uint64
 _pp = C.POINTER(C.c_void_p)
 _psz = C.POINTER(C.c_size_t)
@@ -90,6 +98,8 @@ SIGNATURES = {
     "pft_cloud_upload_depth_images_async": (_i, [_vp, C.POINTER(DepthCamera), _i]),
     "pft_cloud_upload_depth_images_enc": (_i, [_vp, C.POINTER(DepthCameraEnc), _i]),
     "pft_cloud_upload_depth_images_enc_async": (_i, [_vp, C.POINTER(DepthCameraEnc), _i]),
+    "pft_cloud_upload_depth_images_reg": (_i, [_vp, C.POINTER(DepthCameraReg), _i]),
+    "pft_cloud_upload_depth_images_reg_async": (_i, [_vp, C.POINTER(DepthCameraReg), _i]),
     "pft_cloud_wait_upload": (_i, [_vp]),
     "pft_cloud_size": (_i, [_vp, _psz]),
     "pft_cloud_download": (_i, [_vp, _vp, _sz, _i, _psz]),

@@ -6,6 +6,7 @@
 //   pft_cloud_upload_depth_image  depth_image_proc/point_cloud_xyzrgb, which computes the points topic of ref :775
 //   pft_cloud_upload_depth_images  the same per calibrated camera + transformPointCloud(cloud_k, T_k), scene += cloud_k
 //   pft_cloud_upload_depth_images_enc  the same in every encoding of point_cloud_xyzrgb / point_cloud_xyz
+//   pft_cloud_upload_depth_images_reg  the same behind depth_image_proc/register, for unregistered depth images
 //   pft_passthrough         filterPassThrough                                       (ref: src/auto_tracking.cpp:536-547)
 //   pft_passthrough_voxel_grid  filterPassThrough + gridSampleApprox / gridSample   (ref: src/auto_tracking.cpp:637, :683, :641)
 //   pft_prepare_model       removeZeroPoints + centroid + translate + gridSample    (ref: src/auto_tracking.cpp:656-674)
@@ -131,14 +132,22 @@ int check_pointcloud2_layout(size_t n, uint32_t width, uint32_t point_step, uint
 // occupies are copied, (height - 1) * step + width * bytes per pixel, so a caller's view into a larger buffer is never
 // read past its last pixel.  `cams` holds the cameras with pixels, in order, as depth_image_kernel reads them; their points follow
 // each other in the cloud.
+// A registered camera (pft_cloud_upload_depth_images_reg) copies its raw depth image to its own slot instead, and the
+// register kernels write the registered image to its depth slot; the z-buffers of all registered cameras follow the
+// images, in one span that one memset clears.
 struct DepthImageFrame {
   DepthCameras cams;
-  const void* depth[PFT_MAX_DEPTH_CAMERAS];
+  const void* depth[PFT_MAX_DEPTH_CAMERAS];  // NULL: a registered camera, nothing is copied
   const void* bgr[PFT_MAX_DEPTH_CAMERAS];
   size_t depth_bytes[PFT_MAX_DEPTH_CAMERAS], bgr_bytes[PFT_MAX_DEPTH_CAMERAS];
   int n;               // cameras with pixels
   size_t points;       // points of the cloud
   size_t staging;      // bytes of the staging buffer
+  RegCameras reg;      // cameras 0 .. n-1, `registered` set for those with a depth_to_colour matrix
+  const void* raw[PFT_MAX_DEPTH_CAMERAS];
+  size_t raw_bytes[PFT_MAX_DEPTH_CAMERAS];
+  int n_reg;           // registered cameras
+  size_t zbuf_off, zbuf_bytes;
 };
 
 inline size_t align16(size_t b) { return (b + 15) & ~(size_t)15; }
@@ -215,6 +224,77 @@ int check_depth_image(const char* fn, int cam, const pft_depth_camera_enc& e, De
   return PFT_OK;
 }
 
+// Checks camera `cam` of a pft_cloud_upload_depth_images_reg call and appends it to `f`: check_depth_image for the
+// colour side and the output, as if the registered image were its depth image, then the registration fields.
+int check_registration(const char* fn, int cam, const pft_depth_camera_reg& r, DepthImageFrame* f) {
+  if (!r.depth_to_colour) return check_depth_image(fn, cam, r.cam, f);
+  pft_depth_camera_enc e = r.cam;
+  const unsigned int dbytes = e.depth_encoding == PFT_DEPTH_32FC1 ? 4 : 2;
+  e.cam.depth = f;  // the registered image: written on the device, never null, packed rows
+  e.cam.depth_step = e.cam.width * dbytes;
+  const int before = f->n;
+  int rc = check_depth_image(fn, cam, e, f);
+  if (rc) return rc;
+  for (int i = 0; i < 12; ++i) {
+    if (!isfinite(r.depth_to_colour[i])) { set_last_error("%s: camera %d: depth_to_colour entry %d is %g (must be finite)", fn, cam, i, r.depth_to_colour[i]); return PFT_ERR_INVALID; }
+  }
+  if (!(r.depth_fx != 0.0 && r.depth_fy != 0.0 && isfinite(r.depth_fx) && isfinite(r.depth_fy) && isfinite(r.depth_cx) && isfinite(r.depth_cy) &&
+        isfinite(r.depth_tx) && isfinite(r.depth_ty) && isfinite(r.colour_tx) && isfinite(r.colour_ty))) {
+    set_last_error("%s: camera %d: bad registration intrinsics: depth fx %g fy %g cx %g cy %g Tx %g Ty %g, colour Tx %g Ty %g (depth fx, fy finite and "
+                   "non-zero; the rest finite)", fn, cam, r.depth_fx, r.depth_fy, r.depth_cx, r.depth_cy, r.depth_tx, r.depth_ty, r.colour_tx, r.colour_ty);
+    return PFT_ERR_INVALID;
+  }
+  if (r.fill_upsampling != 0 && r.fill_upsampling != 1) { set_last_error("%s: camera %d: fill_upsampling %d (0 or 1)", fn, cam, (int)r.fill_upsampling); return PFT_ERR_INVALID; }
+  const size_t dn = (size_t)r.depth_width * r.depth_height;
+  if (dn > 0x7fffffffull) { set_last_error("%s: camera %d: depth image too large", fn, cam); return PFT_ERR_INVALID; }
+  if (dn && !r.cam.cam.depth) { set_last_error("%s: camera %d: null depth image", fn, cam); return PFT_ERR_INVALID; }
+  if (dn && (r.cam.cam.depth_step % dbytes || (size_t)r.cam.cam.depth_step < (size_t)r.depth_width * dbytes)) {
+    set_last_error("%s: camera %d: bad depth step %u (a multiple of %u, >= %u * depth_width %u)", fn, cam, r.cam.cam.depth_step, dbytes, dbytes, r.depth_width);
+    return PFT_ERR_INVALID;
+  }
+  if (f->n == before) return PFT_OK;  // no colour pixels: the camera adds nothing
+  const int i = f->n - 1;
+  f->depth[i] = nullptr;
+  f->raw[i] = r.cam.cam.depth;
+  f->raw_bytes[i] = dn ? (size_t)(r.depth_height - 1) * r.cam.cam.depth_step + (size_t)r.depth_width * dbytes : 0;
+  RegCamera& k = f->reg.cam[i];
+  k.raw_off = f->staging;
+  f->staging = align16(k.raw_off + f->raw_bytes[i]);
+  k.reg_off = f->cams.cam[i].depth_off;
+  k.depth_width = dn ? r.depth_width : 0;
+  k.depth_height = dn ? r.depth_height : 0;
+  k.depth_step = r.cam.cam.depth_step;
+  k.width = e.cam.width;
+  k.height = e.cam.height;
+  k.registered = 1;
+  k.depth_enc = e.depth_encoding;
+  k.fill = r.fill_upsampling;
+  k.inv_fx = 1.0 / r.depth_fx;
+  k.inv_fy = 1.0 / r.depth_fy;
+  k.cx = r.depth_cx; k.cy = r.depth_cy; k.tx = r.depth_tx; k.ty = r.depth_ty;
+  k.rgb_fx = e.cam.fx; k.rgb_fy = e.cam.fy; k.rgb_cx = e.cam.cx; k.rgb_cy = e.cam.cy; k.rgb_tx = r.colour_tx; k.rgb_ty = r.colour_ty;
+  memcpy(k.m, r.depth_to_colour, sizeof(k.m));
+  ++f->n_reg;
+  return PFT_OK;
+}
+
+// The z-buffers of the registered cameras, after every image of the frame: per camera a uint64 key and a uint32 reset
+// per colour pixel.
+void place_zbuffers(DepthImageFrame* f) {
+  f->zbuf_off = align16(f->staging);
+  size_t off = f->zbuf_off;
+  for (int i = 0; i < f->n; ++i) {
+    RegCamera& k = f->reg.cam[i];
+    if (!k.registered) continue;
+    const size_t px = (size_t)k.width * k.height;
+    k.key_off = off;
+    k.reset_off = off + px * sizeof(unsigned long long);
+    off = align16(k.reset_off + px * sizeof(unsigned int));
+  }
+  f->zbuf_bytes = off - f->zbuf_off;
+  f->staging = off;
+}
+
 int check_depth_cameras(const char* fn, const pft_depth_camera_enc* cams, int n, DepthImageFrame* f) {
   if (!cams) { set_last_error("%s: null cameras", fn); return PFT_ERR_INVALID; }
   if (n < 1 || n > PFT_MAX_DEPTH_CAMERAS) { set_last_error("%s: %d cameras (1 to %d)", fn, n, PFT_MAX_DEPTH_CAMERAS); return PFT_ERR_INVALID; }
@@ -232,8 +312,13 @@ int enqueue_depth_image(cudaStream_t s, pft::DevBuf& staging, pft_cloud* c, cons
   if (rc) return rc;
   unsigned char* base = staging.as<unsigned char>();
   for (int k = 0; k < f.n; ++k) {
-    PFT_CUDA_TRY(cudaMemcpyAsync(base + f.cams.cam[k].depth_off, f.depth[k], f.depth_bytes[k], cudaMemcpyHostToDevice, s));
+    if (f.depth[k]) PFT_CUDA_TRY(cudaMemcpyAsync(base + f.cams.cam[k].depth_off, f.depth[k], f.depth_bytes[k], cudaMemcpyHostToDevice, s));
+    if (f.raw_bytes[k]) PFT_CUDA_TRY(cudaMemcpyAsync(base + f.reg.cam[k].raw_off, f.raw[k], f.raw_bytes[k], cudaMemcpyHostToDevice, s));
     if (f.bgr_bytes[k]) PFT_CUDA_TRY(cudaMemcpyAsync(base + f.cams.cam[k].bgr_off, f.bgr[k], f.bgr_bytes[k], cudaMemcpyHostToDevice, s));
+  }
+  if (f.n_reg) {
+    PFT_CUDA_TRY(cudaMemsetAsync(base + f.zbuf_off, 0, f.zbuf_bytes, s));
+    if ((rc = launch_register_depth(s, base, f.reg, f.n))) return rc;
   }
   return launch_depth_image(s, base, c->d_pts(), f.cams, f.n);
 }
@@ -274,6 +359,19 @@ int upload_depth_images(const char* fn, pft_cloud* c, const pft_depth_camera_enc
   DepthImageFrame f{};
   int rc = check_depth_cameras(fn, cams, n, &f);
   if (rc) return rc;
+  return upload_depth_frame(c, f, asynchronous);
+}
+
+int upload_depth_images_reg(const char* fn, pft_cloud* c, const pft_depth_camera_reg* cams, int n, bool asynchronous) {
+  if (!c) { set_last_error("%s: null cloud", fn); return PFT_ERR_INVALID; }
+  if (!cams) { set_last_error("%s: null cameras", fn); return PFT_ERR_INVALID; }
+  if (n < 1 || n > PFT_MAX_DEPTH_CAMERAS) { set_last_error("%s: %d cameras (1 to %d)", fn, n, PFT_MAX_DEPTH_CAMERAS); return PFT_ERR_INVALID; }
+  DepthImageFrame f{};
+  for (int k = 0; k < n; ++k) {
+    int rc = check_registration(fn, k, cams[k], &f);
+    if (rc) return rc;
+  }
+  place_zbuffers(&f);
   return upload_depth_frame(c, f, asynchronous);
 }
 
@@ -498,6 +596,14 @@ int pft_cloud_upload_depth_images_enc(pft_cloud* c, const pft_depth_camera_enc* 
 
 int pft_cloud_upload_depth_images_enc_async(pft_cloud* c, const pft_depth_camera_enc* cams, int n) {
   return upload_depth_images("pft_cloud_upload_depth_images_enc_async", c, cams, n, true);
+}
+
+int pft_cloud_upload_depth_images_reg(pft_cloud* c, const pft_depth_camera_reg* cams, int n) {
+  return upload_depth_images_reg("pft_cloud_upload_depth_images_reg", c, cams, n, false);
+}
+
+int pft_cloud_upload_depth_images_reg_async(pft_cloud* c, const pft_depth_camera_reg* cams, int n) {
+  return upload_depth_images_reg("pft_cloud_upload_depth_images_reg_async", c, cams, n, true);
 }
 
 int pft_cloud_wait_upload(pft_cloud* c) {

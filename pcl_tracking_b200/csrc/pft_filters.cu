@@ -172,6 +172,132 @@ DepthImageKernel depth_image_instance(int pair, std::integer_sequence<int, Pair.
   static constexpr DepthImageKernel instances[] = {&depth_image_kernel<Pair>...};
   return instances[pair];
 }
+
+// Depth image of a depth camera -> depth image registered into its colour camera: replaces the depth_image_proc/register
+// nodelet (RegisterNodelet::convert<T>) in front of point_cloud_xyzrgb.  Depth pixel (u, v), visited in raster order
+// upstream, back-projects in double (fill_upsampling: its two corners (u -/+ 0.5f, v -/+ 0.5f)), moves by the 3x4
+// depth -> colour matrix, projects to colour pixel (int)(((fx x + Tx) / z + cx) + 0.5) (a rectangle between the two
+// corners' pixels) and offers its z there as a T: the z-buffer keeps it `if (!valid(reg) || reg > new)`.  A candidate
+// that is itself invalid (16UC1 0, 32FC1 -inf: a reset) replaces anything, so the result depends on the order of the
+// candidates through the resets alone; at each colour pixel it is the smallest valid (or +inf) candidate after the last
+// reset, the earliest of equal ones, else the reset value, else the initial one.  The GPU scatters twice: the reset
+// kernel keeps each pixel's last reset (atomicMax of raster index + 1), the z-buffer kernel the least key (value in
+// order-preserving bits, raster index, sign of a zero) of the later candidates, as atomicMax of its complement so that
+// a zero-filled z-buffer is empty.  The finalise kernel writes the T image.  Thread = depth (colour) pixel along a row.
+// Where upstream is undefined (a double -> int cast of NaN or outside int, a 16UC1 fromMeters outside 0 .. 65535), or
+// a 32FC1 candidate is NaN, the candidate is dropped.
+__device__ __forceinline__ bool to_int(double x, int& i) {
+  if (!(x > -2147483649.0 && x < 2147483648.0)) return false;
+  i = (int)x;  // truncation toward zero: (-1, 0) -> 0, as upstream
+  return true;
+}
+__device__ __forceinline__ bool reg_project(const RegCamera& r, double pu, double pv, double depth, int& cu, int& cv, double& z) {
+  const double X = ((pu - r.cx) * depth - r.tx) * r.inv_fx;
+  const double Y = ((pv - r.cy) * depth - r.ty) * r.inv_fy;
+  const double* m = r.m;
+  const double x = ((m[0] * X + m[1] * Y) + m[2] * depth) + m[3];
+  const double y = ((m[4] * X + m[5] * Y) + m[6] * depth) + m[7];
+  z = ((m[8] * X + m[9] * Y) + m[10] * depth) + m[11];
+  const double inv_z = __drcp_rn(z);  // = 1.0 / z, correctly rounded
+  return to_int(((r.rgb_fx * x + r.rgb_tx) * inv_z + r.rgb_cx) + 0.5, cu) && to_int(((r.rgb_fy * y + r.rgb_ty) * inv_z + r.rgb_cy) + 0.5, cv);
+}
+// z-buffer key of a valid candidate (16UC1: the uint16, 32FC1: the float's bits): the value in order-preserving bits
+// (+0 and -0 alike, +inf above every finite value), then the raster index, then the sign bit that tells -0 from +0
+__device__ __forceinline__ unsigned long long reg_key(bool metres, unsigned int b, unsigned int idx) {
+  const unsigned int o = !metres ? b : (b << 1) == 0 ? 0x80000000u : (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+  return ((unsigned long long)o << 32) | (idx << 1) | (metres ? b >> 31 : 0u);
+}
+__device__ __forceinline__ void reg_value(unsigned long long k, unsigned short& d) { d = (unsigned short)(k >> 32); }
+__device__ __forceinline__ void reg_value(unsigned long long k, float& d) {
+  const unsigned int o = (unsigned int)(k >> 32);
+  d = __uint_as_float(o == 0x80000000u ? (unsigned int)(k & 1u) << 31 : (o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
+}
+
+// The candidate of depth pixel (u, v): the colour rectangle [u1, u2] x [v1, v2] and the value's bits (16UC1: the
+// uint16, 32FC1: the float).  Both encodings and both modes share one projection (one call site of the reciprocal's
+// slow path, so nothing is spilled around it).
+__device__ __forceinline__ bool reg_candidate(const RegCamera& r, const unsigned char* drow, unsigned int u, unsigned int v, int& u1, int& v1, int& u2,
+                                              int& v2, unsigned int& val) {
+  const bool metres = r.depth_enc == PFT_DEPTH_32FC1;
+  const unsigned int d = metres ? reinterpret_cast<const unsigned int*>(drow)[u] : reinterpret_cast<const unsigned short*>(drow)[u];
+  if (metres ? !isfinite(__uint_as_float(d)) : d == 0) return false;
+  const double depth = metres ? (double)__uint_as_float(d) : (double)((float)d * 0.001f);  // DepthTraits<T>::toMeters
+  double z1 = 0.0, z2 = 0.0;
+  // fill_upsampling: corner (u - 0.5f, v - 0.5f), then (u + 0.5f, v + 0.5f), each a float sum upstream; else (u, v)
+#pragma unroll 1
+  for (int c = r.fill ? 0 : 1; c < 2; ++c) {
+    const float off = c ? 0.5f : -0.5f;
+    u1 = u2; v1 = v2; z1 = z2;
+    if (!reg_project(r, r.fill ? (double)((float)u + off) : (double)u, r.fill ? (double)((float)v + off) : (double)v, depth, u2, v2, z2)) return false;
+  }
+  if (!r.fill) { u1 = u2; v1 = v2; }
+  if (u1 < 0 || u2 >= (int)r.width || v1 < 0 || v2 >= (int)r.height) return false;
+  const float m = r.fill ? (float)(0.5 * (z1 + z2)) : (float)z2;
+  if (metres) {  // DepthTraits<float>::fromMeters
+    val = __float_as_uint(m);
+    return !isnan(m);
+  }
+  const float t = m * 1000.0f + 0.5f;  // DepthTraits<uint16_t>::fromMeters, undefined outside 0 .. 65535
+  val = (unsigned int)(int)t;
+  return t > -1.0f && t < 65536.0f;
+}
+// Pass 0: resets, pass 1: the other candidates after the last reset of their pixel.
+template <int Pass>
+__device__ __forceinline__ void register_camera(unsigned char* base, const RegCamera& r) {
+  unsigned int* reset = reinterpret_cast<unsigned int*>(base + r.reset_off);
+  unsigned long long* key = reinterpret_cast<unsigned long long*>(base + r.key_off);
+  const bool metres = r.depth_enc == PFT_DEPTH_32FC1;
+  for (unsigned int v = blockIdx.y; v < r.depth_height; v += gridDim.y) {
+    const unsigned char* drow = base + r.raw_off + (size_t)v * r.depth_step;
+    for (unsigned int u = blockIdx.x * blockDim.x + threadIdx.x; u < r.depth_width; u += gridDim.x * blockDim.x) {
+      int u1 = 0, v1 = 0, u2 = 0, v2 = 0;
+      unsigned int val;
+      if (!reg_candidate(r, drow, u, v, u1, v1, u2, v2, val)) continue;
+      if ((val == (metres ? 0xff800000u : 0u)) != (Pass == 0)) continue;  // 16UC1 0, 32FC1 -inf: a reset
+      const unsigned int idx = v * r.depth_width + u;
+      const unsigned long long k = ~reg_key(metres, val, idx);
+      for (int cv = v1; cv <= v2; ++cv) {
+        for (int cu = u1; cu <= u2; ++cu) {
+          const size_t t = (size_t)cv * r.width + cu;
+          if (Pass == 0) atomicMax(&reset[t], idx + 1);
+          else if (idx >= reset[t]) atomicMax(&key[t], k);
+        }
+      }
+    }
+  }
+}
+template <typename D>
+__device__ __forceinline__ void register_finalise_camera(unsigned char* base, const RegCamera& r) {
+  const unsigned int* reset = reinterpret_cast<const unsigned int*>(base + r.reset_off);
+  const unsigned long long* key = reinterpret_cast<const unsigned long long*>(base + r.key_off);
+  D* reg = reinterpret_cast<D*>(base + r.reg_off);
+  D initial = 0, reset_value = 0;  // 16UC1: 0 and 0
+  if constexpr (sizeof(D) == 4) { initial = __uint_as_float(0x7fc00000u); reset_value = -INFINITY; }
+  for (unsigned int v = blockIdx.y; v < r.height; v += gridDim.y) {
+    for (unsigned int u = blockIdx.x * blockDim.x + threadIdx.x; u < r.width; u += gridDim.x * blockDim.x) {
+      const size_t t = (size_t)v * r.width + u;
+      const unsigned long long k = key[t];
+      D d = reset[t] ? reset_value : initial;
+      if (k) reg_value(~k, d);
+      reg[t] = d;
+    }
+  }
+}
+// The reciprocal's slow path is a subroutine call, and ptxas spills a few bytes around it unless bounded: these bounds
+// give 48 and 40 registers, no stack and no spills (-Xptxas -v).
+__global__ void __launch_bounds__(128, 10) register_reset_kernel(unsigned char* base, const __grid_constant__ RegCameras cams) {
+  register_camera<0>(base, cams.cam[blockIdx.z]);
+}
+__global__ void __launch_bounds__(128, 12) register_zbuffer_kernel(unsigned char* base, const __grid_constant__ RegCameras cams) {
+  register_camera<1>(base, cams.cam[blockIdx.z]);
+}
+__global__ void __launch_bounds__(128) register_finalise_kernel(unsigned char* base, const __grid_constant__ RegCameras cams) {
+  const RegCamera& r = cams.cam[blockIdx.z];
+  if (!r.registered) return;
+  if (r.depth_enc == PFT_DEPTH_32FC1) register_finalise_camera<float>(base, r);
+  else register_finalise_camera<unsigned short>(base, r);
+}
+
 __global__ void set_header_kernel(CloudHeader* h, int n) { h->n = n; }
 
 // ---- PassThrough (order-preserving compaction), one thread block: flags -> exclusive scan -> scatter.
@@ -404,6 +530,27 @@ int launch_depth_image(cudaStream_t s, const void* src, float4* dst, const Depth
   const dim3 grid((width + 127) / 128, height < 65535u ? height : 65535u, (unsigned int)n);
   const DepthImageKernel kernel = depth_image_instance(pair, std::make_integer_sequence<int, kMixedPairs + 1>());
   kernel<<<grid, 128, 0, s>>>(reinterpret_cast<const unsigned char*>(src), dst, cams);
+  PFT_LAUNCH_CHECK();
+  return PFT_OK;
+}
+int launch_register_depth(cudaStream_t s, void* staging, const RegCameras& cams, int n) {
+  // three launches whatever the cameras: a grid without a pixel to visit still runs
+  unsigned int dw = 1, dh = 1, w = 1, h = 1;
+  for (int k = 0; k < n; ++k) {
+    const RegCamera& r = cams.cam[k];
+    if (!r.registered) continue;
+    dw = r.depth_width > dw ? r.depth_width : dw;
+    dh = r.depth_height > dh ? r.depth_height : dh;
+    w = r.width > w ? r.width : w;
+    h = r.height > h ? r.height : h;
+  }
+  unsigned char* base = reinterpret_cast<unsigned char*>(staging);
+  const dim3 scatter((dw + 127) / 128, dh < 65535u ? dh : 65535u, (unsigned int)n), finalise((w + 127) / 128, h < 65535u ? h : 65535u, (unsigned int)n);
+  register_reset_kernel<<<scatter, 128, 0, s>>>(base, cams);
+  PFT_LAUNCH_CHECK();
+  register_zbuffer_kernel<<<scatter, 128, 0, s>>>(base, cams);
+  PFT_LAUNCH_CHECK();
+  register_finalise_kernel<<<finalise, 128, 0, s>>>(base, cams);
   PFT_LAUNCH_CHECK();
   return PFT_OK;
 }

@@ -100,6 +100,23 @@ struct DepthCamera {
 struct DepthCameras { DepthCamera cam[PFT_MAX_DEPTH_CAMERAS]; };
 // cameras 0 .. n-1 of `cams`, none of them empty, converted by one launch (blockIdx.z = camera)
 int launch_depth_image(cudaStream_t s, const void* src, float4* dst, const DepthCameras& cams, int n);
+// The registration of camera k of a depth-image ingest (depth_image_proc::RegisterNodelet::convert<T>), as the three
+// register kernels read it: its raw depth image (depth_width x depth_height, rows depth_step bytes apart) and its
+// z-buffer (reset: uint32, key: uint64 per colour pixel) at byte offsets of the staging buffer, and the registered
+// image (width x height colour pixels, packed rows of pft_depth_encoding `depth_enc`) they write at `reg_off`, where
+// depth_image_kernel reads the camera's depth.  The camera intrinsics are pinhole P entries; m = depth -> colour.
+struct RegCamera {
+  size_t raw_off, reg_off, key_off, reset_off;
+  unsigned int depth_width, depth_height, depth_step, width, height;
+  int registered, depth_enc, fill;
+  double inv_fx, inv_fy, cx, cy, tx, ty;              // depth camera (1 / fx, 1 / fy as upstream computes them)
+  double rgb_fx, rgb_fy, rgb_cx, rgb_cy, rgb_tx, rgb_ty;
+  double m[12];
+};
+struct RegCameras { RegCamera cam[PFT_MAX_DEPTH_CAMERAS]; };
+// The cameras of `cams` with `registered` set, of cameras 0 .. n-1, registered by three launches (blockIdx.z = camera)
+// into `staging`; their z-buffers must be zero.
+int launch_register_depth(cudaStream_t s, void* staging, const RegCameras& cams, int n);
 int launch_set_header(cudaStream_t s, CloudHeader* hdr, int n);
 int run_passthrough(pft_context* ctx, const pft_cloud* in, pft_cloud* out, int field, float lo, float hi, int drop_zero);
 int run_voxel_grid(pft_context* ctx, const pft_cloud* in, pft_cloud* out, float leaf, int field, float lo, float hi);

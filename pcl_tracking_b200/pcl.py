@@ -141,6 +141,67 @@ def _depth_camera(depth, bgr, width, height, depth_step, bgr_step, depth_encodin
     return capi.DepthCameraEnc(cam, denc, cenc)
 
 
+def _intrinsics(cam):
+    """fx, fy, cx, cy of a camera mapping: from `K` (3x3 camera_info matrix) or its own keys."""
+    if "K" in cam:
+        K = np.asarray(cam["K"], dtype=np.float64)
+        return K[0, 0], K[1, 1], K[0, 2], K[1, 2]
+    return cam["fx"], cam["fy"], cam["cx"], cam["cy"]
+
+
+def _pose_m12(cam, k, keep):
+    """The float32 3x4 pointer of a camera mapping's optional `pose`, or None."""
+    if cam.get("pose") is None:
+        return None
+    pose = np.asarray(cam["pose"], dtype=np.float32)
+    if pose.shape not in ((4, 4), (3, 4)):
+        raise ValueError("camera %d: pose must be 4x4 or 3x4, got %r" % (k, pose.shape))
+    m = np.ascontiguousarray(pose[:3, :4])
+    keep.append(m)
+    return m.ctypes.data_as(C.POINTER(C.c_float))
+
+
+def _registration(cam, reg, m12, keep, k):
+    """pft_depth_camera_reg of camera mapping `cam` (its depth image in the depth camera's geometry) and its
+    `registration` mapping `reg` (see PointCloud.fromDepthImages)."""
+    depth_encoding, colour_encoding = cam.get("depth_encoding", "16UC1"), cam.get("colour_encoding", "bgr8")
+    if depth_encoding not in DEPTH_ENCODINGS:
+        raise ValueError("unknown depth encoding %r (one of %s)" % (depth_encoding, ", ".join(DEPTH_ENCODINGS)))
+    if colour_encoding not in COLOUR_ENCODINGS:
+        raise ValueError("unknown colour encoding %r (one of %s)" % (colour_encoding, ", ".join(COLOUR_ENCODINGS)))
+    denc, dtype = DEPTH_ENCODINGS[depth_encoding]
+    cenc, channels = COLOUR_ENCODINGS[colour_encoding]
+    dw, dh = reg.get("depth_width"), reg.get("depth_height")
+    dp, w_d, h_d, dstep = _image_arg(cam["depth"], dtype, 1, cam.get("depth_step"), dw, dh, keep)
+    if (dw is not None and int(dw) != w_d) or (dh is not None and int(dh) != h_d):
+        raise ValueError("camera %d: the depth image is %dx%d, the registration says %sx%s" % (k, w_d, h_d, dw, dh))
+    bp, bstep = C.c_void_p(None), 0
+    if channels:
+        bp, w, h, bstep = _image_arg(cam.get("bgr"), np.uint8, channels, cam.get("bgr_step"), cam.get("width"), cam.get("height"), keep)
+    elif cam.get("width") is None or cam.get("height") is None:
+        raise ValueError("camera %d: without a colour image the colour camera's width and height are needed" % k)
+    else:
+        w, h = int(cam["width"]), int(cam["height"])
+    fx, fy, cx, cy = _intrinsics(cam)
+    if "depth_K" in reg:
+        K = np.asarray(reg["depth_K"], dtype=np.float64)
+        dfx, dfy, dcx, dcy = K[0, 0], K[1, 1], K[0, 2], K[1, 2]
+    else:
+        dfx, dfy, dcx, dcy = reg["depth_fx"], reg["depth_fy"], reg["depth_cx"], reg["depth_cy"]
+    t = np.asarray(reg["depth_to_colour"], dtype=np.float64)
+    if t.shape not in ((4, 4), (3, 4)):
+        raise ValueError("camera %d: depth_to_colour must be 4x4 or 3x4, got %r" % (k, t.shape))
+    t = np.ascontiguousarray(t[:3, :4])
+    keep.append(t)
+    fill = reg.get("fill_upsampling", False)
+    if fill not in (0, 1):
+        raise ValueError("camera %d: fill_upsampling must be a bool, got %r" % (k, fill))
+    cam_enc = capi.DepthCameraEnc(capi.DepthCamera(dp.value, dstep, bp.value, bstep, w, h, float(fx), float(fy), float(cx), float(cy), m12), denc, cenc)
+    return capi.DepthCameraReg(cam_enc, t.ctypes.data_as(C.POINTER(C.c_double)), w_d, h_d, float(dfx), float(dfy), float(dcx), float(dcy),
+                               float(reg.get("depth_Tx", 0.0)), float(reg.get("depth_Ty", 0.0)), float(reg.get("colour_Tx", 0.0)),
+                               float(reg.get("colour_Ty", 0.0)), int(fill))
+
+
 class PointCloud:
     """pcl::PointCloud<pcl::PointXYZRGBA> resident in HBM as float4 {x, y, z, rgba}."""
 
@@ -222,28 +283,45 @@ class PointCloud:
         optionally `depth_encoding` and `colour_encoding` (defaults "16UC1" and "bgr8"; with "none", `bgr` may be
         absent), either `K` (3x3 camera_info matrix) or `fx`, `fy`, `cx`, `cy`, and an optional `pose`: the 4x4 or 3x4
         matrix from the camera's optical frame to the common frame, cast to float32 (absent or None: the camera's own
-        frame).  Cameras may mix encodings."""
+        frame).  Cameras may mix encodings.
+
+        A camera whose depth image is not registered to its colour camera carries a `registration` mapping: its `depth`
+        image is then in the depth camera's geometry and is registered into the colour camera on the device, as the
+        depth_image_proc/register nodelet does, before the conversion (pft_cloud_upload_depth_images_reg).  The mapping
+        holds the depth camera's `depth_K` (3x3) or `depth_fx`, `depth_fy`, `depth_cx`, `depth_cy`, optionally
+        `depth_Tx`, `depth_Ty`, `colour_Tx`, `colour_Ty` (P[3], P[7] of each camera_info; default 0),
+        `depth_to_colour`, the 4x4 or 3x4 matrix from the depth optical frame to the colour optical frame in float64,
+        `fill_upsampling` (default False), and `depth_width`, `depth_height` (needed for a pointer depth image; checked
+        against a depth array).  `K` / `fx` .. `cy`, the colour image, `width`, `height` (needed without a colour image)
+        and `pose` are the colour camera's, and the camera's points are organised in its geometry.  Cameras with and
+        without a registration may be mixed."""
         keep = []
         cams = list(cameras)
+        if any(cam.get("registration") is not None for cam in cams):
+            return self._from_registered(cams, keep, asynchronous)
         arr = (capi.DepthCameraEnc * len(cams))()
         for k, cam in enumerate(cams):
-            if "K" in cam:
-                K = np.asarray(cam["K"], dtype=np.float64)
-                fx, fy, cx, cy = K[0, 0], K[1, 1], K[0, 2], K[1, 2]
-            else:
-                fx, fy, cx, cy = cam["fx"], cam["fy"], cam["cx"], cam["cy"]
-            m12 = None
-            if cam.get("pose") is not None:
-                pose = np.asarray(cam["pose"], dtype=np.float32)
-                if pose.shape not in ((4, 4), (3, 4)):
-                    raise ValueError("camera %d: pose must be 4x4 or 3x4, got %r" % (k, pose.shape))
-                m = np.ascontiguousarray(pose[:3, :4])
-                keep.append(m)
-                m12 = m.ctypes.data_as(C.POINTER(C.c_float))
+            fx, fy, cx, cy = _intrinsics(cam)
+            m12 = _pose_m12(cam, k, keep)
             arr[k] = _depth_camera(cam["depth"], cam.get("bgr"), cam.get("width"), cam.get("height"), cam.get("depth_step"), cam.get("bgr_step"),
                                    cam.get("depth_encoding", "16UC1"), cam.get("colour_encoding", "bgr8"), fx, fy, cx, cy, m12, keep)
         self._keep = keep
         fn = capi.load().pft_cloud_upload_depth_images_enc_async if asynchronous else capi.load().pft_cloud_upload_depth_images_enc
+        check(fn(self._h, arr, len(cams)))
+        return self
+
+    def _from_registered(self, cams, keep, asynchronous):
+        arr = (capi.DepthCameraReg * len(cams))()
+        for k, cam in enumerate(cams):
+            m12 = _pose_m12(cam, k, keep)
+            if cam.get("registration") is not None:
+                arr[k] = _registration(cam, cam["registration"], m12, keep, k)
+                continue
+            fx, fy, cx, cy = _intrinsics(cam)
+            arr[k].cam = _depth_camera(cam["depth"], cam.get("bgr"), cam.get("width"), cam.get("height"), cam.get("depth_step"), cam.get("bgr_step"),
+                                       cam.get("depth_encoding", "16UC1"), cam.get("colour_encoding", "bgr8"), fx, fy, cx, cy, m12, keep)
+        self._keep = keep
+        fn = capi.load().pft_cloud_upload_depth_images_reg_async if asynchronous else capi.load().pft_cloud_upload_depth_images_reg
         check(fn(self._h, arr, len(cams)))
         return self
 

@@ -16,6 +16,13 @@ device time of depth_image_kernel per launch) and the synchronous image upload a
 the encoding pairs in ENCODINGS: 16UC1 + bgr8 (5 bytes per pixel over PCIe), 32FC1 + rgb8 (7), 32FC1 + bgra8 (8) and
 16UC1 depth alone (2).
 
+Workload `registered`: a Kinect2 whose depth is not registered to its colour camera, sd 16UC1 depth (512x424) from
+the depth sensor and qhd bgr8 colour (960x540) from a camera 52 mm away, registered on the device
+(pft_cloud_upload_depth_images_reg, fill_upsampling on) and converted, against the already-registered qhd 16UC1 depth +
+bgr8 colour of the same scene.  It reports the H2D bytes per frame, the three register kernels' device time per frame
+(torch.profiler) and the frames/s end to end with tracking (the qhd tracker), synchronous and double-buffered.  The
+two arms see different clouds, so their poses are not compared.
+
 Needs a CUDA device; prints the card's name and power limit with the numbers, one JSON line per workload.
 """
 import argparse
@@ -69,7 +76,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--steps", type=int, default=200, help="timed steps per ingest and mode")
     ap.add_argument("--warmup", type=int, default=5)
-    ap.add_argument("--workloads", default="c2,qhd")
+    ap.add_argument("--workloads", default="c2,qhd,registered")
     ap.add_argument("--out", default=None, help="also write the JSON lines to this file")
     args = ap.parse_args()
 
@@ -86,6 +93,9 @@ def main():
     print(json.dumps(lines[0]), flush=True)
 
     for workload in args.workloads.split(","):
+        if workload == "registered":
+            lines += registered_workload(args, ctx, stream, flush_buf)
+            continue
         sensor = synth.KINECT2_QHD if workload == "qhd" else synth.KINECT2_SD
         w, h = sensor["width"], sensor["height"]
         objs = synth.default_objects(1)
@@ -217,6 +227,117 @@ def main():
         with open(args.out, "w") as f:
             for line in lines:
                 f.write(json.dumps(line) + "\n")
+
+
+def registered_workload(args, ctx, stream, flush_buf):
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+
+    from pcl_tracking_b200 import pcl, synth
+    sd, qhd = synth.KINECT2_SD, synth.KINECT2_QHD
+    w, h = qhd["width"], qhd["height"]
+    offset = np.array([0.052, 0.0, 0.0])  # the colour camera in the depth camera's frame
+    colour_pose = (np.eye(3), offset)
+    M = np.eye(4)[:3].copy()
+    M[:, 3] = -offset
+    objs = synth.default_objects(1)
+    frames = []
+    for f in range(N_FRAMES):
+        depth_sd, _, Kd = synth.depth_images(synth.render(f, objs, sensor=sd)[0], sd)
+        pts, oid = synth.render(f, objs, sensor=qhd, camera=colour_pose)
+        depth_qhd, bgr, Kc = synth.depth_images(pts, qhd)
+        frames.append((pcl.PinnedBuffer.of(depth_sd), pcl.PinnedBuffer.of(bgr), pcl.PinnedBuffer.of(depth_qhd), oid if f == 0 else None))
+    fx, fy, cx, cy = Kc[0, 0], Kc[1, 1], Kc[0, 2], Kc[1, 2]
+    reg = dict(depth_K=Kd, depth_to_colour=M, fill_upsampling=True, depth_width=sd["width"], depth_height=sd["height"])
+
+    def upload(ingest, cloud, k, asynchronous):
+        d_sd, bgr, d_qhd, _ = frames[frame_order(k, N_FRAMES)]
+        cam = dict(bgr=bgr.ptr, width=w, height=h, fx=fx, fy=fy, cx=cx, cy=cy)
+        if ingest == "register":
+            cam.update(depth=d_sd.ptr, registration=reg)
+        else:
+            cam.update(depth=d_qhd.ptr)
+        cloud.fromDepthImages([cam], asynchronous=asynchronous)
+
+    raw = pcl.PointCloud(ctx=ctx)
+    upload("registered", raw, 0, False)
+    model, centre = pcl.prepare_model(pcl.PointCloud(synth.model_points(raw.to_numpy(), frames[0][3], 0), ctx=ctx), LEAF, ctx=ctx)
+
+    def tracker():
+        t = pcl.KLDAdaptiveParticleFilterOMPTracker(16, ctx=ctx)
+        pcl.configure_like_reference(t, particle_num=400, max_particle_num=500, use_hsv=True, iteration_num=ITERATIONS)
+        m = np.eye(4, dtype=np.float32)
+        m[:3, 3] = centre
+        t.setTrans(m)
+        t.seed(1234)
+        t.setReferenceCloud(model)
+        return t
+
+    lines = []
+    bytes_per_frame = {"register": 2 * sd["width"] * sd["height"] + 3 * w * h, "registered": 5 * w * h}
+    for pipelined in (False, True):
+        rec = {"what": "e2e", "workload": "registered", "width": w, "height": h, "mode": "pipelined" if pipelined else "sync", "steps": args.steps}
+        for ingest in ("register", "registered"):
+            t, vg, ds = tracker(), pcl.ApproximateVoxelGrid(ctx=ctx), pcl.PointCloud(ctx=ctx)
+            vg.setLeafSize(LEAF, LEAF, LEAF)
+            vg.setPassThrough("z", 0.0, 10.0)
+            clouds = [pcl.PointCloud(ctx=ctx), pcl.PointCloud(ctx=ctx)]
+            if pipelined:
+                upload(ingest, clouds[0], 0, True)
+            ms = 0.0
+            for k in range(args.warmup + args.steps):
+                with torch.cuda.stream(stream):
+                    flush_buf.fill_(1)
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record(stream)
+                if pipelined:
+                    upload(ingest, clouds[(k + 1) % 2], k + 1, True)
+                else:
+                    upload(ingest, clouds[k % 2], k, False)
+                vg.setInputCloud(clouds[k % 2])
+                vg.filter(ds)
+                t.setInputCloud(ds)
+                t.compute()
+                t.getResult()  # D2H of the pose: synchronises
+                e1.record(stream)
+                e1.synchronize()
+                if k >= args.warmup:
+                    ms += e0.elapsed_time(e1)
+            ms /= args.steps
+            rec[ingest] = {"h2d_bytes_per_step": bytes_per_frame[ingest], "ms_per_step": ms, "frames_per_s": 1e3 / ms}
+        lines.append(rec)
+        print(json.dumps(rec), flush=True)
+
+    # the register kernels alone (device time per frame) and the synchronous upload as a whole, L2 flushed before each
+    cloud = pcl.PointCloud(ctx=ctx)
+    reps = 100
+    for ingest in ("register", "registered"):
+        up_ms = 0.0
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            for k in range(reps):
+                with torch.cuda.stream(stream):
+                    flush_buf.fill_(1)
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record(stream)
+                upload(ingest, cloud, k, False)
+                e1.record(stream)
+                e1.synchronize()
+                up_ms += e0.elapsed_time(e1)
+        kernels = {}
+        for e in prof.key_averages():
+            for name in ("register_reset_kernel", "register_zbuffer_kernel", "register_finalise_kernel", "depth_image_kernel"):
+                if name in e.key:
+                    kernels[name] = (getattr(e, "device_time_total", None) or e.cuda_time_total) / reps
+        rec = {"what": "kernel", "workload": "registered", "ingest": ingest, "h2d_bytes_per_frame": bytes_per_frame[ingest],
+               "kernel_us_per_frame": kernels, "register_us_per_frame": sum(v for k, v in kernels.items() if k.startswith("register")),
+               "image_upload_us": up_ms / reps * 1e3}
+        lines.append(rec)
+        print(json.dumps(rec), flush=True)
+    for d_sd, bgr, d_qhd, _ in frames:
+        d_sd.free()
+        bgr.free()
+        d_qhd.free()
+    return lines
 
 
 if __name__ == "__main__":
