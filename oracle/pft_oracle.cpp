@@ -1146,13 +1146,26 @@ int orc_voxel_grid_exact(const orc_point* in, int n, float leaf, int field, floa
 // inside [min_size, max_size] are kept with their indices sorted, then ordered by size descending (upstream:
 // std::sort over reverse iterators, ties unspecified; here the lower seed index first).  The radius search is
 // served by a uniform grid instead of a kd-tree (same result set).  labels[i] = cluster rank or -1.
+// Grid keys are floor(((double)x - min) / cell), each operation rounded once in fp64, with cell >= tolerance * 1.0001
+// and at most 2^30 cells along an axis, so a key fits a long long for any finite cloud (an fp32 x / cell for points at
+// 3e38 does not).  A pair that passes the fp32 test is less than (1 - 0.98e-4) cells apart and the keys err by less
+// than 2^-21 cells, so the pair lands in adjacent cells (the argument in pft_cluster.cu, cl_cell_of).
 int orc_euclidean_clusters(const orc_point* pts, int n, double tolerance, int min_size, int max_size, int* labels, int* sizes, int sizes_cap) {
   const float tol2 = (float)(tolerance * tolerance);
-  const float cell = (float)tolerance * 1.0001f;
+  double lo[3] = {HUGE_VAL, HUGE_VAL, HUGE_VAL}, hi[3] = {-HUGE_VAL, -HUGE_VAL, -HUGE_VAL};
+  for (int i = 0; i < n; ++i) {
+    if (!finite3(pts[i])) continue;
+    const double c[3] = {pts[i].x, pts[i].y, pts[i].z};
+    for (int d = 0; d < 3; ++d) { lo[d] = std::min(lo[d], c[d]); hi[d] = std::max(hi[d], c[d]); }
+  }
+  double cell = tolerance * 1.0001;
+  for (int d = 0; d < 3; ++d) if (lo[d] <= hi[d]) cell = std::max(cell, (hi[d] - lo[d]) / 1073741824.0);
   struct Key { long long x, y, z; bool operator==(const Key& o) const { return x == o.x && y == o.y && z == o.z; } };
   struct KeyHash { size_t operator()(const Key& k) const { return (size_t)(k.x * 73856093ll ^ k.y * 19349663ll ^ k.z * 83492791ll); } };
   std::unordered_map<Key, std::vector<int>, KeyHash> grid;
-  auto key_of = [&](const Pt& p) { return Key{(long long)std::floor(p.x / cell), (long long)std::floor(p.y / cell), (long long)std::floor(p.z / cell)}; };
+  auto key_of = [&](const Pt& p) {
+    return Key{(long long)std::floor(((double)p.x - lo[0]) / cell), (long long)std::floor(((double)p.y - lo[1]) / cell), (long long)std::floor(((double)p.z - lo[2]) / cell)};
+  };
   for (int i = 0; i < n; ++i) { labels[i] = -1; if (finite3(pts[i])) grid[key_of(pts[i])].push_back(i); }
   std::vector<char> processed(n, 0);
   std::vector<std::vector<int>> clusters;

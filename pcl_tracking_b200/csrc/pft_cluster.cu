@@ -21,11 +21,10 @@ namespace pft {
 namespace {
 
 struct ClusterGrid {
-  float origin[3];
-  float inv_cell;
+  double origin[3];  // the bounding box's minimum (fp32 values)
+  double cell;
   int dim[3];
   int n_cells;
-  int valid;
 };
 
 constexpr int kMaxClusterCells = 1 << 22;
@@ -33,8 +32,15 @@ constexpr int kMaxClusters = 4096;  // clusters that can pass the size filter (e
 
 __device__ __forceinline__ bool finite3(const float4& p) { return isfinite(p.x) && isfinite(p.y) && isfinite(p.z); }
 
-// bounding box of the finite points -> grid header (one block)
-__global__ void __launch_bounds__(1024) cl_grid_kernel(const float4* __restrict__ pts, const CloudHeader* __restrict__ hdr, float cell, ClusterGrid* g) {
+// bounding box of the finite points -> grid header (one block).
+// Sizing, in fp64: with extents L_d and cell c, each dim is floor(L_d / c) + 1 <= L_d / c + 1, and
+//   prod_d (L_d / c + 1) = 1 + S1 / c + S2 / c^2 + S3 / c^3      (S1 = sum L_d, S2 = sum of the pairwise products, S3 = prod L_d)
+// is at most 1 + 3 q = kMaxClusterCells when each of the three terms is at most q = (kMaxClusterCells - 1) / 3.  So the cell is
+// the larger of min_cell and the three roots that bound the terms; the factor 1 + 2^-20 covers the roundings of the
+// roots and of the quotients L_d / c (each a few 2^-53).  Every dim is then <= 2^22 and every cell index fits an int.  The
+// extents of finite fp32 points are below 2^129, their products finite in fp64: the sizing holds for any cloud and any
+// tolerance (a cell of +inf puts every point in cell 0).
+__global__ void __launch_bounds__(1024) cl_grid_kernel(const float4* __restrict__ pts, const CloudHeader* __restrict__ hdr, double min_cell, ClusterGrid* g) {
   __shared__ float s_mn[32][3], s_mx[32][3];
   const int n = hdr->n;
   float mn[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, mx[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
@@ -50,30 +56,44 @@ __global__ void __launch_bounds__(1024) cl_grid_kernel(const float4* __restrict_
   __syncthreads();
   if (threadIdx.x == 0) {
     for (int w = 1; w < (int)(blockDim.x >> 5); ++w) for (int d = 0; d < 3; ++d) { mn[d] = fminf(mn[d], s_mn[w][d]); mx[d] = fmaxf(mx[d], s_mx[w][d]); }
+    const bool any = mn[0] <= mx[0];
+    double L[3];
+    for (int d = 0; d < 3; ++d) L[d] = any ? (double)mx[d] - (double)mn[d] : 0.0;
+    const double q = (double)((kMaxClusterCells - 1) / 3);
+    double c = min_cell;
+    c = fmax(c, (L[0] + L[1] + L[2]) / q);
+    c = fmax(c, sqrt((L[0] * L[1] + L[0] * L[2] + L[1] * L[2]) / q));
+    c = fmax(c, cbrt(L[0] * L[1] * L[2] / q));
+    c *= 1.0 + 0x1p-20;
     ClusterGrid h;
-    h.valid = mn[0] <= mx[0] ? 1 : 0;
-    // cell edge: the tolerance, doubled until the grid fits (a larger cell only means more candidates per neighbourhood)
-    float c = cell;
-    for (int it = 0; it < 40; ++it) {
-      long long cells = 1;
-      for (int d = 0; d < 3; ++d) {
-        h.dim[d] = h.valid ? (int)fminf(floorf((mx[d] - mn[d]) / c), 2.0e9f) + 1 : 1;
-        cells *= (long long)h.dim[d];
-        if (cells > (1ll << 40)) cells = 1ll << 40;
-      }
-      if (cells <= (long long)kMaxClusterCells) { h.n_cells = (int)cells; break; }
-      c *= 2.0f;
+    h.cell = c;
+    h.n_cells = 1;
+    for (int d = 0; d < 3; ++d) {
+      h.origin[d] = any ? (double)mn[d] : 0.0;
+      h.dim[d] = (int)floor(L[d] / c) + 1;
+      h.n_cells *= h.dim[d];
     }
-    for (int d = 0; d < 3; ++d) h.origin[d] = h.valid ? mn[d] : 0.f;
-    h.inv_cell = 1.0f / c;
     *g = h;
   }
 }
 
+// Cell coordinates in fp64: s = ((double)x - origin) / cell, each operation rounded once.  Any pair the union kernel
+// joins lands in adjacent cells on every axis:
+//  - fp32 d2 < T = (float)(tol^2) implies fl(dx*dx) < T (the sums add non-negative terms, rounding is monotone), so
+//    fl(dx*dx) <= pred(T) and dx*dx <= (pred(T) + T) / 2 <= (double)(tol^2) <= tol^2 (1 + 2^-53), subnormals included;
+//    dx = fl32(a - b) gives |a - b| <= |dx| / (1 - 2^-24), so |a - b| < tol (1 + 2^-23);
+//  - cell >= (double)tol * 1.0001 >= tol (1 + 0.9999e-4), so |a - b| / cell < 1 - 0.98e-4;
+//  - each s is (x - origin) / cell with a relative error below 2^-51 and is at most dim <= 2^22, an absolute error below
+//    2^-29 (plus 2^-1074 if the quotient is subnormal);
+// so |s_a - s_b| < 1 and floor(s_a), floor(s_b) differ by at most 1.  Clamping to [0, dim - 1] keeps that.  (The former
+// fp32 (x - origin) * inv_cell erred by up to an ulp of the product: at about 4000 cells that exceeds the 1e-4 slack.)
+__device__ __forceinline__ int cl_axis_cell(double x, double origin, double cell, int dim) {
+  return (int)fmin(fmax(floor((x - origin) / cell), 0.0), (double)(dim - 1));
+}
 __device__ __forceinline__ void cl_cell_of(const ClusterGrid& g, const float4& p, int& cx, int& cy, int& cz) {
-  cx = min(max((int)floorf((p.x - g.origin[0]) * g.inv_cell), 0), g.dim[0] - 1);
-  cy = min(max((int)floorf((p.y - g.origin[1]) * g.inv_cell), 0), g.dim[1] - 1);
-  cz = min(max((int)floorf((p.z - g.origin[2]) * g.inv_cell), 0), g.dim[2] - 1);
+  cx = cl_axis_cell(p.x, g.origin[0], g.cell, g.dim[0]);
+  cy = cl_axis_cell(p.y, g.origin[1], g.cell, g.dim[1]);
+  cz = cl_axis_cell(p.z, g.origin[2], g.cell, g.dim[2]);
 }
 
 __global__ void cl_count_kernel(const float4* __restrict__ pts, const CloudHeader* __restrict__ hdr, const ClusterGrid* __restrict__ gp, int* cell_count,
@@ -283,7 +303,7 @@ int pft_euclidean_clusters(pft_context* ctx, const pft_cloud* in, double toleran
   ClusterGrid* g = ctx->cl_grid.as<ClusterGrid>();
   const float tol2 = (float)(tolerance * tolerance);  // KdTreeFLANN::radiusSearch passes (float)(radius * radius)
   const int grid = cl_grid_for(n, ctx->sm_count);
-  cl_grid_kernel<<<1, 1024, 0, s>>>(in->d_pts(), in->d_hdr(), (float)tolerance * 1.0001f, g);
+  cl_grid_kernel<<<1, 1024, 0, s>>>(in->d_pts(), in->d_hdr(), tolerance * 1.0001, g);
   PFT_LAUNCH_CHECK();
   PFT_CUDA_TRY(cudaMemsetAsync(cell_count, 0, ((size_t)kMaxClusterCells + 16) * sizeof(int), s));
   cl_count_kernel<<<grid, 256, 0, s>>>(in->d_pts(), in->d_hdr(), g, cell_count, parent, comp_size);
