@@ -561,6 +561,50 @@ class EuclideanClusterExtraction {
   int min_ = 1, max_ = 2147483647;
 };
 
+// pcl::transformPointCloud (PCL 1.8.0, pft_transform_cloud): the model builder's moves into the robot base frame and
+// back (ref: src/create_model.cpp:107-123, :184-204, through pcl_ros with the tf matrix rounded to float) and viz_cb's
+// (ref: src/auto_tracking.cpp:309-316).  On the device, in order, colours kept; a point with a non-finite coordinate is
+// copied as it is.  `out` may be `in` itself.  copy_all_fields is accepted and ignored: x, y, z and rgba are all a
+// PointXYZRGBA holds.
+namespace detail {
+template <typename PointT>
+void transform_point_cloud(const PointCloud<PointT>& in, PointCloud<PointT>& out, const float* m12) {
+  auto& ctx = pft::Context::Default();
+  pft_cloud* src = in.device(ctx);
+  pft::check(pft_transform_cloud(ctx->get(), src, &in == &out ? src : out.device(ctx), m12));
+  out.mark_device_written();
+}
+// the 3x4 row-major [R|t] of any affine type with operator()(row, col)
+template <typename AffineT> void affine_m12(const AffineT& t, float* m12) {
+  for (int r = 0; r < 3; ++r) for (int c = 0; c < 4; ++c) m12[r * 4 + c] = t(r, c);
+}
+}  // namespace detail
+template <typename PointT>
+void transformPointCloud(const PointCloud<PointT>& in, PointCloud<PointT>& out, const pft::Affine3f& transform, bool copy_all_fields = true) {
+  (void)copy_all_fields;
+  float m12[12];
+  detail::affine_m12(transform, m12);
+  detail::transform_point_cloud(in, out, m12);
+}
+#ifdef PFT_SHIM_USE_EIGEN
+template <typename PointT>
+void transformPointCloud(const PointCloud<PointT>& in, PointCloud<PointT>& out, const Eigen::Affine3f& transform, bool copy_all_fields = true) {
+  (void)copy_all_fields;
+  float m12[12];
+  detail::affine_m12(transform, m12);
+  detail::transform_point_cloud(in, out, m12);
+}
+// Eigen::Matrix4f: column-major storage (Eigen's default); row 3 is ignored, as upstream's affine product does
+template <typename PointT>
+void transformPointCloud(const PointCloud<PointT>& in, PointCloud<PointT>& out, const Eigen::Matrix4f& transform, bool copy_all_fields = true) {
+  (void)copy_all_fields;
+  const float* d = transform.data();
+  float m12[12];
+  for (int r = 0; r < 3; ++r) for (int c = 0; c < 4; ++c) m12[r * 4 + c] = d[c * 4 + r];
+  detail::transform_point_cloud(in, out, m12);
+}
+#endif
+
 // pcl::getTime (pcl/common/time.h; ref: src/auto_tracking.cpp:552, :559): seconds, wall clock
 inline double getTime() {
   struct timespec ts;
@@ -722,6 +766,14 @@ class ParticleFilterTracker {
     pft_result_box b;
     pft::check(pft_tracker_get_result_box(h_, z_offset, &b));
     return b;
+  }
+  // the cloud that box is measured on (ref :309-316): the reference cloud moved by toEigenMatrix(getResult()) with
+  // translation z + z_offset, the tracked object's points (device-resident until read)
+  PointCloudInPtr getResultCloud(float z_offset = -0.005f) const {
+    PointCloudInPtr out = pft::sp::make_shared<PointCloud<PointT>>();
+    pft::check(pft_tracker_get_result_cloud(h_, z_offset, out->device(ctx_)));
+    out->mark_device_written();
+    return out;
   }
   void resetTracking() { pft::check(pft_tracker_reset(h_)); }
   double getFitRatio() const { double v = 0; pft::check(pft_tracker_get_fit_ratio(h_, &v)); return v; }

@@ -232,6 +232,22 @@ PFT_API int pft_approx_voxel_grid_pcl(pft_context* ctx, const pft_cloud* in, pft
  * preparation of ref: src/auto_tracking.cpp:656-674.  centroid3 receives the translation that the
  * caller passes to pft_tracker_set_trans. */
 PFT_API int pft_prepare_model(pft_context* ctx, const pft_cloud* raw, pft_cloud* out, float leaf, float* centroid3);
+/* pcl::transformPointCloud (PCL 1.8.0, common/impl/transforms.hpp) as the model builder moves a frame into the robot base
+ * frame and its clusters back to the camera (ref: src/create_model.cpp:107-123, :184-204 through pcl_ros).  `m12` is
+ * the fp32 3x4 row-major [R|t], the convention of pft_tracker_set_trans and pft_depth_camera.m12 (pcl_ros rounds each
+ * entry of the double tf matrix to float: do the same).  `out` receives every point of `in` in the same order, rgba
+ * copied.  A point whose x, y and z are finite becomes x' = ((m00 x + m01 y) + m02 z) + m03 (y', z' likewise), every
+ * fp32 operation rounded on its own; a point with a non-finite coordinate is copied unchanged.  That is PCL's non-dense
+ * branch; for a cloud of finite points it equals the dense one, so the result differs from PCL only for a cloud flagged
+ * is_dense that nevertheless holds non-finite points (PCL then transforms them too).  in == out is allowed (in place);
+ * both clouds belong to `ctx`.  The point count is read from `in`'s device header: the call never waits for the host
+ * and may follow a filter whose count has not been read back.  One kernel launch.  PFT_ERR_INVALID: a null argument,
+ * a non-finite matrix entry, a cloud of another context. */
+PFT_API int pft_transform_cloud(pft_context* ctx, const pft_cloud* in, pft_cloud* out, const float* m12);
+/* removeZeroPoints of the model builder (ref: src/create_model.cpp:59-77) and of pft_prepare_model (ref:
+ * src/auto_tracking.cpp:577-595): drops a point if any coordinate is not finite, or if |x|, |y| and |z| are all < 0.01
+ * (compared in double); order preserving.  in != out.  The same kernel as the first step of pft_prepare_model. */
+PFT_API int pft_remove_zero_points(pft_context* ctx, const pft_cloud* in, pft_cloud* out);
 
 /* ---------------------------------------------------------------- model acquisition */
 /* pcl::EuclideanClusterExtraction::extract as the model builder runs it (ref: src/create_model.cpp:169-179:
@@ -361,6 +377,12 @@ typedef struct {
   int32_t n;          /* model points */
 } pft_result_box;
 PFT_API int pft_tracker_get_result_box(pft_tracker* t, float z_offset, pft_result_box* out);
+/* The cloud pft_tracker_get_result_box measures (ref: src/auto_tracking.cpp:309-316): the reference cloud, in the order
+ * and with the colours it was given, moved by toEigenMatrix(getResult()) with translation.z += z_offset -- the tracked
+ * object's points, e.g. for a grasp planner.  Bit for bit pft_transform_cloud(reference, M) with M =
+ * pft_particle_to_matrix(result) and M[11] += z_offset in fp32.  `out` belongs to the tracker's context; asynchronous,
+ * one kernel launch, outside compute().  PFT_ERR_STATE before a reference cloud and a compute(). */
+PFT_API int pft_tracker_get_result_cloud(pft_tracker* t, float z_offset, pft_cloud* out);
 /* resetTracking */
 PFT_API int pft_tracker_reset(pft_tracker* t);
 /* likelihood evaluations so far (sum over weight() calls of live particles x model points; counted on the device,

@@ -107,6 +107,8 @@ SIGNATURES = {
     "pft_passthrough_voxel_grid": (_i, [_vp, _vp, _vp, _f, _i, _f, _f]),
     "pft_approx_voxel_grid_pcl": (_i, [_vp, _vp, _vp, _f, _i, _f, _f]),
     "pft_prepare_model": (_i, [_vp, _vp, _vp, _f, _vp]),
+    "pft_transform_cloud": (_i, [_vp, _vp, _vp, _vp]),
+    "pft_remove_zero_points": (_i, [_vp, _vp, _vp]),
     "pft_euclidean_clusters": (_i, [_vp, _vp, _d, _i, _i, _vp, _sz, _vp, _sz, _psz]),
     "pft_cloud_select_cluster": (_i, [_vp, _vp, _i, _vp]),
     "pft_segment_plane": (_i, [_vp, _vp, _d, _i, _d, _vp, _i, _u64, _i, _vp, C.POINTER(C.c_int32), _vp, _vp, _psz]),
@@ -125,6 +127,7 @@ SIGNATURES = {
     "pft_tracker_get_particles": (_i, [_vp, _vp, _sz, _psz]),
     "pft_particle_to_matrix": (_i, [_vp, _vp, _vp]),
     "pft_tracker_get_result_box": (_i, [_vp, _f, _vp]),
+    "pft_tracker_get_result_cloud": (_i, [_vp, _f, _vp]),
     "pft_tracker_reset": (_i, [_vp]),
     "pft_tracker_get_eval_count": (_i, [_vp, C.POINTER(C.c_uint64)]),
     "pft_tracker_get_fit_ratio": (_i, [_vp, C.POINTER(C.c_double)]),

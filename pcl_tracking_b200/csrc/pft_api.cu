@@ -10,6 +10,8 @@
 //   pft_passthrough         filterPassThrough                                       (ref: src/auto_tracking.cpp:536-547)
 //   pft_passthrough_voxel_grid  filterPassThrough + gridSampleApprox / gridSample   (ref: src/auto_tracking.cpp:637, :683, :641)
 //   pft_prepare_model       removeZeroPoints + centroid + translate + gridSample    (ref: src/auto_tracking.cpp:656-674)
+//   pft_transform_cloud     pcl(_ros)::transformPointCloud into / out of the base frame (ref: src/create_model.cpp:107-123, :184-204)
+//   pft_remove_zero_points  removeZeroPoints                                        (ref: src/create_model.cpp:59-77)
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
@@ -651,9 +653,9 @@ int pft_cloud_download(pft_cloud* c, void* host_points, size_t capacity, int lay
 }
 
 // ------------------------------------------------------------------ filters
-static int check_filter_args(pft_context* ctx, const pft_cloud* in, pft_cloud* out, const char* who) {
+static int check_filter_args(pft_context* ctx, const pft_cloud* in, pft_cloud* out, const char* who, bool in_place_ok = false) {
   if (!ctx || !in || !out) { set_last_error("%s: null argument", who); return PFT_ERR_INVALID; }
-  if (in == out) { set_last_error("%s: in-place filtering is not supported", who); return PFT_ERR_INVALID; }
+  if (in == out && !in_place_ok) { set_last_error("%s: in-place filtering is not supported", who); return PFT_ERR_INVALID; }
   if (in->ctx != ctx || out->ctx != ctx) { set_last_error("%s: clouds belong to another context", who); return PFT_ERR_INVALID; }
   PFT_CUDA_TRY(cudaSetDevice(ctx->device));
   int rc = in->join_upload();  // an asynchronous upload into the input / output must land before the filter touches it
@@ -680,6 +682,21 @@ int pft_approx_voxel_grid_pcl(pft_context* ctx, const pft_cloud* in, pft_cloud* 
   if (rc) return rc;
   if (field > 2) { set_last_error("pft_approx_voxel_grid_pcl: field must be <0 (off), 0, 1 or 2"); return PFT_ERR_INVALID; }
   return run_approx_voxel_grid_pcl(ctx, in, out, leaf, field, lo, hi);
+}
+
+int pft_transform_cloud(pft_context* ctx, const pft_cloud* in, pft_cloud* out, const float* m12) {
+  if (!m12) { set_last_error("pft_transform_cloud: null matrix"); return PFT_ERR_INVALID; }
+  for (int k = 0; k < 12; ++k)
+    if (!isfinite(m12[k])) { set_last_error("pft_transform_cloud: matrix entry %d (row %d, column %d) is not finite", k, k / 4, k % 4); return PFT_ERR_INVALID; }
+  int rc = check_filter_args(ctx, in, out, "pft_transform_cloud", true);
+  if (rc) return rc;
+  return run_transform_cloud(ctx, in, out, m12);
+}
+
+int pft_remove_zero_points(pft_context* ctx, const pft_cloud* in, pft_cloud* out) {
+  int rc = check_filter_args(ctx, in, out, "pft_remove_zero_points");
+  if (rc) return rc;
+  return run_passthrough(ctx, in, out, -1, 0.f, 0.f, 1);
 }
 
 int pft_prepare_model(pft_context* ctx, const pft_cloud* raw, pft_cloud* out, float leaf, float* centroid3) {

@@ -113,6 +113,20 @@ __device__ __forceinline__ int warp_sum(int v) {
   return v;
 }
 
+// ------------------------------------------------------------------ pcl::transformPointCloud (PCL 1.8.0, common/impl/transforms.hpp)
+// m = 3x4 row-major [R|t].  Dense branch: x' = ((m00 x + m01 y) + m02 z) + m03, y' and z' likewise, every fp32
+// operation rounded on its own (-fmad=false).
+__device__ __forceinline__ void xform(const float* m, float x, float y, float z, float& ox, float& oy, float& oz) {
+  ox = ((m[0] * x + m[1] * y) + m[2] * z) + m[3];
+  oy = ((m[4] * x + m[5] * y) + m[6] * z) + m[7];
+  oz = ((m[8] * x + m[9] * y) + m[10] * z) + m[11];
+}
+// Non-dense branch: a point with a non-finite coordinate is copied as it is; the fourth word (rgba) is kept.
+__device__ __forceinline__ float4 transform_point(const float* m, float4 p) {
+  if (isfinite(p.x) && isfinite(p.y) && isfinite(p.z)) xform(m, p.x, p.y, p.z, p.x, p.y, p.z);
+  return p;
+}
+
 // ------------------------------------------------------------------ bulk async copy (TMA, 1-D) + mbarrier
 // One thread arms the barrier with the byte count and issues the copies; every consumer waits on the phase bit.
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }

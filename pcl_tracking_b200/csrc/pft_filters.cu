@@ -123,13 +123,7 @@ __device__ __forceinline__ void depth_image_camera(const unsigned char* __restri
         p.x = (((float)u - k.cx) * fd) * k.kx;
         p.y = (fy * fd) * k.ky;
         p.z = metres ? fd : fd * 0.001f;
-        if (k.has_m && finite3(p)) {
-          const float* m = k.m;
-          const float x = p.x, y = p.y, z = p.z;
-          p.x = ((m[0] * x + m[1] * y) + m[2] * z) + m[3];
-          p.y = ((m[4] * x + m[5] * y) + m[6] * z) + m[7];
-          p.z = ((m[8] * x + m[9] * y) + m[10] * z) + m[11];
-        }
+        if (k.has_m && finite3(p)) xform(k.m, p.x, p.y, p.z, p.x, p.y, p.z);  // pcl::transformPointCloud, not dense
       }
       orow[u] = p;
     }
@@ -299,6 +293,17 @@ __global__ void __launch_bounds__(128) register_finalise_kernel(unsigned char* b
 }
 
 __global__ void set_header_kernel(CloudHeader* h, int n) { h->n = n; }
+
+// ---- pcl::transformPointCloud (PCL 1.8.0, not dense): every point in input order, finite ones moved by the 3x4
+// matrix, the others copied as they are, rgba kept.  The count is read from the input's header (no host round trip
+// after a filter).  In place (in == out, out_hdr NULL) each thread reads its point before it writes it back.
+struct Matrix12 { float m[12]; };
+__global__ void __launch_bounds__(256) transform_cloud_kernel(const float4* in, const CloudHeader* __restrict__ in_hdr, float4* out,
+                                                              CloudHeader* out_hdr, const Matrix12 m) {
+  const int n = in_hdr->n;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) out[i] = transform_point(m.m, in[i]);
+  if (out_hdr && blockIdx.x == 0 && threadIdx.x == 0) out_hdr->n = n;
+}
 
 // ---- PassThrough (order-preserving compaction), one thread block: flags -> exclusive scan -> scatter.
 __global__ void __launch_bounds__(1024) passthrough_kernel(const float4* __restrict__ in, const CloudHeader* __restrict__ in_hdr,
@@ -572,6 +577,21 @@ int run_passthrough(pft_context* ctx, const pft_cloud* in, pft_cloud* out, int f
   passthrough_kernel<<<1, 1024, 0, ctx->stream>>>(in->d_pts(), in->d_hdr(), out->d_pts(), out->d_hdr(), field, lo, hi, drop_zero);
   PFT_LAUNCH_CHECK();
   out->written(-1);
+  return PFT_OK;
+}
+
+int run_transform_cloud(pft_context* ctx, const pft_cloud* in, pft_cloud* out, const float* m12) {
+  const bool in_place = in == out;
+  if (!in_place) {
+    int rc = out->ensure(in->capacity);
+    if (rc) return rc;
+  }
+  Matrix12 m;
+  memcpy(m.m, m12, sizeof(m.m));
+  transform_cloud_kernel<<<grid_for(in->capacity, 256, ctx->sm_count), 256, 0, ctx->stream>>>(in->d_pts(), in->d_hdr(), out->d_pts(),
+                                                                                           in_place ? nullptr : out->d_hdr(), m);
+  PFT_LAUNCH_CHECK();
+  out->written(in->host_n);
   return PFT_OK;
 }
 

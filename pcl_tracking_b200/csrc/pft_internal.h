@@ -122,6 +122,8 @@ int run_passthrough(pft_context* ctx, const pft_cloud* in, pft_cloud* out, int f
 int run_voxel_grid(pft_context* ctx, const pft_cloud* in, pft_cloud* out, float leaf, int field, float lo, float hi);
 int run_approx_voxel_grid_pcl(pft_context* ctx, const pft_cloud* in, pft_cloud* out, float leaf, int field, float lo, float hi);
 int run_centre_on_centroid(pft_context* ctx, pft_cloud* cloud, float* d_centroid3);
+// pcl::transformPointCloud by the 3x4 row-major `m12` (host); in == out allowed; one launch
+int run_transform_cloud(pft_context* ctx, const pft_cloud* in, pft_cloud* out, const float* m12);
 
 // ---- scene replicas (pft_tracker.cu): every replica of a cloud goes with it, every replica a context holds goes with it
 void release_replicas_of(const pft_cloud* src);

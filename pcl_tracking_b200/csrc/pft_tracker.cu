@@ -160,7 +160,7 @@ struct pft_tracker {
   int graph_nodes[2] = {0, 0};
   // device buffers
   DevBuf st, parts[2], mats, slot_aabb, model, model_perm, model_tmp, sort_keys, sort_idx, bbox, raw, partial, cdf, cdf_total, ancestors, bin_keys, tbl_rep,
-      tbl_min, slot_of, klb, d_usel, d_normals, d_umot, idx_hdr, idx_hdr_prev, fbuilt_bits, cell_start, ipts, ipts2, ihsv, icount, dbg_idx, dbg_d2, d_trans, row_table, flists, fpool, fcell_items, fl1_slots, fneeded, fneeded_list, ffar_list, xlists, xcount, result_box, alias_a, alias_q, alias_hl, oct_hdr, oct_nodes, oct_next, cd_hdr, cd_nodes, cd_out;
+      tbl_min, slot_of, klb, d_usel, d_normals, d_umot, idx_hdr, idx_hdr_prev, fbuilt_bits, cell_start, ipts, ipts2, ihsv, icount, dbg_idx, dbg_d2, d_trans, row_table, flists, fpool, fcell_items, fl1_slots, fneeded, fneeded_list, ffar_list, xlists, xcount, result_box, ref_pts, alias_a, alias_q, alias_hl, oct_hdr, oct_nodes, oct_next, cd_hdr, cd_nodes, cd_out;
   int oct_node_cap = 0;
   // change detector (SURVEY 8 f-4; PCL ctor defaults, off in the reference): host-driven, one read-back per test
   bool use_cd = false;
@@ -203,7 +203,7 @@ void release_all(pft_tracker* t) {
   DevBuf* bufs[] = {&t->st, &t->parts[0], &t->parts[1], &t->mats, &t->slot_aabb, &t->model, &t->model_perm, &t->model_tmp, &t->sort_keys, &t->sort_idx,
                     &t->bbox, &t->raw, &t->partial, &t->cdf, &t->cdf_total, &t->ancestors, &t->bin_keys, &t->tbl_rep, &t->tbl_min, &t->slot_of, &t->klb,
                     &t->d_usel, &t->d_normals, &t->d_umot, &t->idx_hdr, &t->idx_hdr_prev, &t->fbuilt_bits, &t->cell_start, &t->ipts, &t->ipts2, &t->ihsv, &t->icount, &t->dbg_idx,
-                    &t->dbg_d2, &t->d_trans, &t->row_table, &t->flists, &t->fpool, &t->fcell_items, &t->fl1_slots, &t->fneeded, &t->fneeded_list, &t->ffar_list, &t->xlists, &t->xcount, &t->result_box, &t->alias_a, &t->alias_q, &t->alias_hl, &t->oct_hdr, &t->oct_nodes, &t->oct_next, &t->cd_hdr, &t->cd_nodes, &t->cd_out};
+                    &t->dbg_d2, &t->d_trans, &t->row_table, &t->flists, &t->fpool, &t->fcell_items, &t->fl1_slots, &t->fneeded, &t->fneeded_list, &t->ffar_list, &t->xlists, &t->xcount, &t->result_box, &t->ref_pts, &t->alias_a, &t->alias_q, &t->alias_hl, &t->oct_hdr, &t->oct_nodes, &t->oct_next, &t->cd_hdr, &t->cd_nodes, &t->cd_out};
   for (auto* b : bufs) b->release();
 }
 
@@ -1261,6 +1261,9 @@ static int set_reference_device(pft_tracker* t, const float4* d_pts, int n) {
   if ((rc = t->sort_keys.reserve((size_t)n_pad * sizeof(unsigned int)))) return rc;
   if ((rc = t->sort_idx.reserve((size_t)n_pad * sizeof(int)))) return rc;
   if ((rc = t->bbox.reserve(6 * sizeof(float)))) return rc;
+  // the reference cloud as given (order, rgba), for pft_tracker_get_result_cloud: `model` is reordered and holds HSV
+  if ((rc = t->ref_pts.reserve((size_t)n * sizeof(float4)))) return rc;
+  PFT_CUDA_TRY(cudaMemcpyAsync(t->ref_pts.p, d_pts, (size_t)n * sizeof(float4), cudaMemcpyDeviceToDevice, s));
   model_bbox_kernel<<<1, 1024, 0, s>>>(d_pts, n, t->bbox.as<float>());
   PFT_LAUNCH_CHECK();
   model_keys_kernel<<<blocks_for(n_pad, 256, 1024), 256, 0, s>>>(d_pts, n, t->sort_keys.as<unsigned int>(), t->sort_idx.as<int>(), n_pad, t->bbox.as<float>());
@@ -1660,6 +1663,22 @@ int pft_tracker_get_result_box(pft_tracker* t, float z_offset, pft_result_box* o
   PFT_CUDA_TRY(cudaMemcpyAsync(t->ctx->pinned, t->result_box.p, sizeof(ResultBox), cudaMemcpyDeviceToHost, s));
   PFT_CUDA_TRY(cudaStreamSynchronize(s));
   memcpy(out, t->ctx->pinned, sizeof(ResultBox));
+  return PFT_OK;
+}
+
+int pft_tracker_get_result_cloud(pft_tracker* t, float z_offset, pft_cloud* out) {
+  if (!t || !out) { set_last_error("pft_tracker_get_result_cloud: null argument"); return PFT_ERR_INVALID; }
+  if (out->ctx != t->ctx) { set_last_error("pft_tracker_get_result_cloud: the cloud belongs to another context than the tracker"); return PFT_ERR_INVALID; }
+  if (!t->st.p || t->M <= 0) { set_last_error("no result yet: setReferenceCloud and compute() first"); return PFT_ERR_STATE; }
+  PFT_CUDA_TRY(cudaSetDevice(t->ctx->device));
+  int rc = out->join_upload();  // an asynchronous upload into the cloud must land before the kernel overwrites it
+  if (rc) return rc;
+  if ((rc = out->ensure((size_t)t->M))) return rc;
+  cudaStream_t s = t->ctx->stream;  // the cloud's stream (a batch has joined it by now)
+  result_cloud_kernel<<<blocks_for(t->M, 256, 8 * t->ctx->sm_count), 256, 0, s>>>(t->st.as<TrackerState>(), t->ref_pts.as<float4>(), t->M, z_offset,
+                                                                                out->d_pts(), out->d_hdr());
+  PFT_LAUNCH_CHECK();
+  out->written(t->M);
   return PFT_OK;
 }
 

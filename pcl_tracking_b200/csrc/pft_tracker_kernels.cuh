@@ -177,7 +177,8 @@ struct CoherenceParams {
 };
 
 
-// ------------------------------------------------------------------ small math (arithmetic contract)
+// ------------------------------------------------------------------ small math (arithmetic contract; xform and
+// transform_point, pcl::transformPointCloud, are in pft_common.cuh)
 __device__ __forceinline__ void sincos_c(float a, float& s, float& c) {
   double ds, dc;
   sincos((double)a, &ds, &dc);
@@ -198,13 +199,6 @@ __device__ __forceinline__ void matrix_to_rpy(const float* m, float& roll, float
   pitch = (float)asin((double)(-m[8]));
   yaw = (float)atan2((double)m[4], (double)m[0]);
 }
-// pcl::transformPointCloud, dense branch
-__device__ __forceinline__ void xform(const float* m, float x, float y, float z, float& ox, float& oy, float& oz) {
-  ox = ((m[0] * x + m[1] * y) + m[2] * z) + m[3];
-  oy = ((m[4] * x + m[5] * y) + m[6] * z) + m[7];
-  oz = ((m[8] * x + m[9] * y) + m[10] * z) + m[11];
-}
-
 struct Quat { float w, x, y, z; };
 // Eigen::Quaternionf(Matrix3f)
 __device__ inline Quat quat_from_matrix(const float* m) {
@@ -3037,6 +3031,25 @@ __global__ void __launch_bounds__(1024) result_box_kernel(const TrackerState* __
     out->quat[0] = q.w; out->quat[1] = q.x; out->quat[2] = q.y; out->quat[3] = q.z;
     out->n = M;
   }
+}
+
+// The cloud of viz_cb (ref: src/auto_tracking.cpp:309-316): the reference cloud as given, moved by toEigenMatrix of the
+// result with translation.z += z_offset -- the matrix of result_box_kernel -- through pcl::transformPointCloud's
+// routine, so that it equals pft_transform_cloud(reference, that matrix) bit for bit.  Order and rgba are kept.
+__global__ void __launch_bounds__(256) result_cloud_kernel(const TrackerState* __restrict__ st, const float4* __restrict__ ref, int M, float z_offset,
+                                                           float4* __restrict__ out, CloudHeader* __restrict__ out_hdr) {
+  __shared__ float s_m[12];
+  if (threadIdx.x == 0) {
+    const DevParticle rep = st->rep;
+    particle_to_matrix(rep.x, rep.y, rep.z, rep.roll, rep.pitch, rep.yaw, s_m);
+    s_m[11] += z_offset;
+    if (blockIdx.x == 0) out_hdr->n = M;
+  }
+  __syncthreads();
+  float m[12];
+#pragma unroll
+  for (int k = 0; k < 12; ++k) m[k] = s_m[k];
+  for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < M; j += gridDim.x * blockDim.x) out[j] = transform_point(m, ref[j]);
 }
 
 }  // namespace pft

@@ -551,6 +551,27 @@ def prepare_model(raw_cloud, leaf=0.01, ctx=None):
     return out, c
 
 
+def transformPointCloud(cloud, m, out=None):
+    """pcl::transformPointCloud(cloud, out, m) (PCL 1.8.0): every point moved by the affine `m` (4x4 or 3x4, cast to
+    float32 entry by entry, as pcl_ros does with a tf matrix), in order, colours kept; a point with a non-finite
+    coordinate is copied as it is.  `out` may be `cloud` itself (in place).  Returns the output cloud."""
+    a = np.asarray(m)
+    if a.shape not in ((4, 4), (3, 4)):
+        raise ValueError("m must be 4x4 or 3x4, got %r" % (a.shape,))
+    m12 = np.ascontiguousarray(a[:3, :4], dtype=np.float32)
+    out = PointCloud(ctx=cloud.ctx) if out is None else out
+    check(capi.load().pft_transform_cloud(cloud.ctx._h, cloud._h, out._h, ptr(m12)))
+    return out
+
+
+def removeZeroPoints(cloud, out=None):
+    """removeZeroPoints of the model builder (ref: src/create_model.cpp:59-77): drops the points with a non-finite
+    coordinate and those with |x|, |y| and |z| all below 0.01, order preserving.  Returns the output cloud."""
+    out = PointCloud(ctx=cloud.ctx) if out is None else out
+    check(capi.load().pft_remove_zero_points(cloud.ctx._h, cloud._h, out._h))
+    return out
+
+
 # ------------------------------------------------------------------ coherence configuration objects
 class DistanceCoherence:
     """pcl::tracking::DistanceCoherence (ref :240-242)."""
@@ -761,6 +782,13 @@ class ParticleFilterOMPTracker:
         out = np.zeros(1, dtype=capi.RESULT_BOX)
         check(capi.load().pft_tracker_get_result_box(self._h, float(z_offset), ptr(out)))
         return out[0]
+
+    def getResultCloud(self, z_offset=-0.005, out=None):
+        """The reference cloud moved to the result pose, translation z + z_offset (viz_cb, ref: src/auto_tracking.cpp:
+        309-316): the tracked object's points, as a device cloud of the tracker's context."""
+        out = PointCloud(ctx=self.ctx) if out is None else out
+        check(capi.load().pft_tracker_get_result_cloud(self._h, float(z_offset), out._h))
+        return out
 
     def getParticles(self):
         n = C.c_size_t()
