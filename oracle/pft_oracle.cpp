@@ -299,6 +299,13 @@ inline uint32_t pack_rgb_trunc(float r, float g, float b) {
   return ((uint32_t)(int)r << 16) | ((uint32_t)(int)g << 8) | (uint32_t)(int)b;
 }
 
+// Lattice index floor(v * inv), the product rounded to float, saturated to the int range (the GPU's conversion; a plain
+// cast of a float outside the int range is undefined).
+static int voxel_index(float v, float inv) {
+  const float f = std::floor(v * inv);
+  return f >= 2147483648.0f ? INT_MAX : (f < -2147483648.0f ? INT_MIN : (int)f);
+}
+
 // ApproximateVoxelGrid<PointXYZRGBA>::applyFilter [filters/impl/approximate_voxel_grid.hpp],
 // SURVEY A.1; ref: src/auto_tracking.cpp:563-575.  Output capacity: n.
 int approx_voxel_grid_pcl(const Pt* in, int n, float leaf, Pt* out) {
@@ -317,8 +324,9 @@ int approx_voxel_grid_pcl(const Pt* in, int n, float leaf, Pt* out) {
   };
   for (int i = 0; i < n; ++i) {
     const Pt& p = in[i];
-    int ix = (int)std::floor(p.x * inv), iy = (int)std::floor(p.y * inv), iz = (int)std::floor(p.z * inv);
-    unsigned hash = (unsigned)((ix * 7171 + iy * 3079 + iz * 4231) & (histsize - 1));
+    int ix = voxel_index(p.x, inv), iy = voxel_index(p.y, inv), iz = voxel_index(p.z, inv);
+    // upstream's int hash in unsigned arithmetic: the same bits, without signed overflow
+    unsigned hash = ((unsigned)ix * 7171u + (unsigned)iy * 3079u + (unsigned)iz * 4231u) & (unsigned)(histsize - 1);
     He& h = hist[hash];
     if (h.count && (ix != h.ix || iy != h.iy || iz != h.iz)) {
       flush(h);
@@ -388,10 +396,12 @@ int voxel_grid_pcl(const Pt* in, int n, float leaf, Pt* out) {
 
 // Exact one-centroid-per-voxel downsample with the PassThrough predicate folded in: the
 // specification of the CUDA K1 kernel (SURVEY A.1 "New build").  Same lattice as upstream
-// (floor(coord * (1/leaf)), anchored at the origin); voxels are emitted in order of first
-// appearance in the input; coordinate sums are held in double (exact for sensor-range
-// values, hence order independent) and the centroid is the double quotient rounded to
-// float; colour means follow upstream: (int)(float_sum / float_count), alpha = 0.
+// (floor(coord * (1/leaf)), anchored at the origin, saturated to the int range); voxels are
+// emitted in order of first appearance in the input; coordinate sums are held in double and
+// added in input order (exact, hence equal to the GPU's in any order, except in voxels on a
+// coordinate plane that mix coordinates far below the leaf with leaf-sized ones) and the
+// centroid is the double quotient rounded to float; colour means follow upstream:
+// (int)(float_sum / float_count), alpha = 0.
 int voxel_grid_exact(const Pt* in, int n, float leaf, int field, float lo, float hi, Pt* out) {
   const float inv = 1.0f / leaf;
   struct Acc { double sx = 0, sy = 0, sz = 0; uint32_t r = 0, g = 0, b = 0, cnt = 0; };
@@ -407,7 +417,7 @@ int voxel_grid_exact(const Pt* in, int n, float leaf, int field, float lo, float
     if (!finite3(p)) continue;
     float v = field == 0 ? p.x : (field == 1 ? p.y : p.z);
     if (field >= 0 && (v < lo || v > hi)) continue;
-    Key k{(int)std::floor(p.x * inv), (int)std::floor(p.y * inv), (int)std::floor(p.z * inv)};
+    Key k{voxel_index(p.x, inv), voxel_index(p.y, inv), voxel_index(p.z, inv)};
     auto it = map.find(k);
     int id;
     if (it == map.end()) { id = (int)acc.size(); map.emplace(k, id); acc.emplace_back(); } else id = it->second;

@@ -6,9 +6,10 @@
 //
 // Data layout: clouds are float4 {x,y,z,rgba} arrays in HBM with a 16-byte device header holding the
 // point count (no host round trip between stages).  The voxel hash is an open-addressing table of
-// 64-bit packed lattice keys (21 bits per axis); per-voxel sums are kept in double (coordinates) and
-// uint32 (colour bytes), which makes the centroid independent of the order the atomics land in:
-// sums of fp32 sensor-range values are exact in fp64.  Output order = order of first appearance.
+// 16-byte slots holding the voxel's three int32 lattice indices (exact: no two voxels share a key);
+// per-voxel sums are kept in double (coordinates) and uint32 (colour bytes), which makes the centroid
+// independent of the order the atomics land in wherever the fp64 sums are exact (k1_accum_kernel).
+// Output order = order of first appearance.
 #include <stdlib.h>
 #include <string.h>
 
@@ -21,7 +22,6 @@ namespace pft {
 
 namespace {
 
-constexpr unsigned long long kEmptyKey = ~0ull;
 constexpr int kFirstInit = 0x7f7f7f7f;
 
 __device__ __forceinline__ bool finite3(const float4& p) { return isfinite(p.x) && isfinite(p.y) && isfinite(p.z); }
@@ -33,15 +33,12 @@ __device__ __forceinline__ bool passes(const float4& p, int field, float lo, flo
   return !(v < lo || v > hi);
 }
 
-__device__ __forceinline__ unsigned long long voxel_key(const float4& p, float inv) {
-  // lattice of upstream (Approximate)VoxelGrid: floor(coord * inverse_leaf_size)
-  const int ix = (int)floorf(p.x * inv), iy = (int)floorf(p.y * inv), iz = (int)floorf(p.z * inv);
-  const unsigned long long bx = (unsigned long long)((ix + (1 << 20)) & 0x1fffff);
-  const unsigned long long by = (unsigned long long)((iy + (1 << 20)) & 0x1fffff);
-  const unsigned long long bz = (unsigned long long)((iz + (1 << 20)) & 0x1fffff);
-  return (bx << 42) | (by << 21) | bz;
-}
-__device__ __forceinline__ unsigned int hash_key(unsigned long long k) {
+// Lattice index of upstream (Approximate)VoxelGrid: floor(coord * inverse_leaf_size), the product rounded to fp32.
+// Outside the int32 range it saturates (cvt.rmi.s32.f32): |coord * inv| >= 2^31 is index INT_MAX or INT_MIN.
+__device__ __forceinline__ int voxel_index(float v, float inv) { return __float2int_rd(v * inv); }
+// Hash of a voxel's three indices (all 96 bits feed the 64-bit finaliser of MurmurHash3).
+__device__ __forceinline__ unsigned int voxel_hash(int ix, int iy, int iz) {
+  unsigned long long k = (((unsigned long long)(unsigned int)ix << 32) | (unsigned int)iy) ^ ((unsigned long long)(unsigned int)iz * 0x9e3779b97f4a7c15ull);
   k ^= k >> 33; k *= 0xff51afd7ed558ccdull; k ^= k >> 33; k *= 0xc4ceb9fe1a85ec53ull; k ^= k >> 33;
   return (unsigned int)k;
 }
@@ -324,18 +321,19 @@ __global__ void __launch_bounds__(1024) passthrough_kernel(const float4* __restr
 }
 
 // ---- K1a: insert every surviving point's voxel key; remember the lowest point index per voxel.
-__global__ void k1_insert_kernel(const float4* __restrict__ in, const CloudHeader* __restrict__ in_hdr, unsigned long long* keys,
-                                 int* first, int* __restrict__ slot_of, unsigned int mask, float inv, int field, float lo, float hi) {
+// A slot is {ix, iy, iz, 1} once claimed, all zero while empty; one 16-byte compare-and-swap claims it or returns its key.
+__global__ void k1_insert_kernel(const float4* __restrict__ in, const CloudHeader* __restrict__ in_hdr, int4* keys, int* first,
+                                 int* __restrict__ slot_of, unsigned int mask, float inv, int field, float lo, float hi) {
   const int n = in_hdr->n;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const float4 p = in[i];
     int slot = -1;
     if (passes(p, field, lo, hi)) {
-      const unsigned long long key = voxel_key(p, inv);
-      unsigned int s = hash_key(key) & mask;
+      const int4 key = make_int4(voxel_index(p.x, inv), voxel_index(p.y, inv), voxel_index(p.z, inv), 1);
+      unsigned int s = voxel_hash(key.x, key.y, key.z) & mask;
       while (true) {
-        const unsigned long long prev = atomicCAS(&keys[s], kEmptyKey, key);
-        if (prev == kEmptyKey || prev == key) break;
+        const int4 prev = atomicCAS(&keys[s], make_int4(0, 0, 0, 0), key);
+        if (prev.w == 0 || (prev.x == key.x && prev.y == key.y && prev.z == key.z)) break;
         s = (s + 1) & mask;
       }
       slot = (int)s;
@@ -408,7 +406,12 @@ __global__ void __launch_bounds__(1024) k1_tile_assign_kernel(const CloudHeader*
     }
   }
 }
-// ---- K1c: accumulate.  fp64 sums of fp32 sensor coordinates are exact => order independent.
+// ---- K1c: accumulate in fp64.  Every fp32 coordinate is a multiple of its own ulp, so a voxel's sums are exact, and
+// the centroid does not depend on the order the atomics land in, while they stay below 2^53 times the smallest ulp among
+// the voxel's coordinates.  That holds in every voxel whose index is neither 0 nor -1 on an axis: its coordinates on
+// that axis are within a factor of about 2 of each other (2^25 ulps), so up to 2^28 points sum exactly.  A voxel on a
+// coordinate plane can also hold coordinates far below the leaf size; next to leaf-sized ones (below about 2^-36 m
+// with centimetre-scale ones at a 1 cm leaf) the sum rounds, and its last bit can depend on the order.
 __global__ void k1_accum_kernel(const float4* __restrict__ in, const CloudHeader* __restrict__ in_hdr, const int* __restrict__ slot_of,
                                 const int* __restrict__ vid, double* acc_xyz, unsigned int* acc_rgbc) {
   const int n = in_hdr->n;
@@ -464,8 +467,9 @@ __global__ void approx_voxel_grid_pcl_kernel(const float4* __restrict__ in, cons
   for (int i = 0; i < n; ++i) {
     const float4 p = in[i];
     if (!passes(p, field, lo, hi)) continue;  // the PassThrough that precedes the grid (ref :637), order preserving
-    const int ix = (int)floorf(p.x * inv), iy = (int)floorf(p.y * inv), iz = (int)floorf(p.z * inv);
-    const int k = (int)((unsigned int)(ix * 7171 + iy * 3079 + iz * 4231) & (unsigned int)(kHist - 1));
+    const int ix = voxel_index(p.x, inv), iy = voxel_index(p.y, inv), iz = voxel_index(p.z, inv);
+    // upstream's int hash in unsigned arithmetic: the same bits, without signed overflow
+    const int k = (int)(((unsigned int)ix * 7171u + (unsigned int)iy * 3079u + (unsigned int)iz * 4231u) & (unsigned int)(kHist - 1));
     if (s_key[k][3] && (ix != s_key[k][0] || iy != s_key[k][1] || iz != s_key[k][2])) {
       flush(k);
       s_key[k][3] = 0;
@@ -599,13 +603,13 @@ int run_transform_cloud(pft_context* ctx, const pft_cloud* in, pft_cloud* out, c
 static int enqueue_voxel_grid(pft_context* ctx, const pft_cloud* in, pft_cloud* out, float leaf, int field, float lo, float hi, size_t cap, size_t H,
                               int n_tiles) {
   cudaStream_t s = ctx->stream;
-  PFT_CUDA_TRY(cudaMemsetAsync(ctx->k1_keys.p, 0xff, H * sizeof(unsigned long long), s));
+  PFT_CUDA_TRY(cudaMemsetAsync(ctx->k1_keys.p, 0, H * sizeof(int4), s));
   PFT_CUDA_TRY(cudaMemsetAsync(ctx->k1_first.p, 0x7f, H * sizeof(int), s));
   PFT_CUDA_TRY(cudaMemsetAsync(ctx->k1_acc_xyz.p, 0, cap * 3 * sizeof(double), s));
   PFT_CUDA_TRY(cudaMemsetAsync(ctx->k1_acc_rgbc.p, 0, cap * 4 * sizeof(unsigned int), s));
   const float inv = 1.0f / leaf;
   const int grid = grid_for(cap, 256, ctx->sm_count);
-  k1_insert_kernel<<<grid, 256, 0, s>>>(in->d_pts(), in->d_hdr(), ctx->k1_keys.as<unsigned long long>(), ctx->k1_first.as<int>(),
+  k1_insert_kernel<<<grid, 256, 0, s>>>(in->d_pts(), in->d_hdr(), ctx->k1_keys.as<int4>(), ctx->k1_first.as<int>(),
                                         ctx->k1_slot_of.as<int>(), (unsigned int)(H - 1), inv, field, lo, hi);
   PFT_LAUNCH_CHECK();
   k1_tile_count_kernel<<<n_tiles, 1024, 0, s>>>(in->d_hdr(), ctx->k1_slot_of.as<int>(), ctx->k1_first.as<int>(), ctx->k1_blk.as<int>());
@@ -631,7 +635,7 @@ int run_voxel_grid(pft_context* ctx, const pft_cloud* in, pft_cloud* out, float 
   if (cap == 0) return launch_set_header(ctx->stream, out->d_hdr(), 0);
   size_t H = 1024;
   while (H < 2 * cap) H <<= 1;
-  if ((rc = ctx->k1_keys.reserve(H * sizeof(unsigned long long)))) return rc;
+  if ((rc = ctx->k1_keys.reserve(H * sizeof(int4)))) return rc;
   if ((rc = ctx->k1_first.reserve(H * sizeof(int)))) return rc;
   if ((rc = ctx->k1_vid.reserve(H * sizeof(int)))) return rc;
   if ((rc = ctx->k1_slot_of.reserve(cap * sizeof(int)))) return rc;
