@@ -99,6 +99,36 @@ inline int blocks_for(long long n, int block, int cap) {
 
 }  // namespace
 
+// The device storage of the candidate lists (format: CandLists), sized for a table of up to `cells` fine cells
+struct CandListStore {
+  DevBuf records, pool, xlists, cell_items, l1_slots, needed, needed_list, far_list, built_bits, counters;
+
+  // sizes beyond the table: one spare fine cell of records and slots, kSpare entries in the queues and bitmaps, and
+  // blocks of 2x2x2 fine cells, at most ceil(d/2)^3 <= (d+1)^3/8, bounded generously by cells/2 + kBlockSlack
+  static constexpr size_t kSpare = 16, kBlockSlack = 4096;
+  int reserve(int cells) {
+    const size_t n = (size_t)cells;
+    int rc;
+    if ((rc = records.reserve((n + 1) * kCellWords * sizeof(unsigned int)))) return rc;
+    if ((rc = pool.reserve((size_t)kPoolGroups * kRecordWords * sizeof(unsigned int)))) return rc;
+    if ((rc = xlists.reserve((size_t)kListXCells * kListKX * sizeof(unsigned int)))) return rc;
+    if ((rc = cell_items.reserve((n + kSpare) * sizeof(int2)))) return rc;
+    if ((rc = l1_slots.reserve((n + 1) * kL1Cap * sizeof(unsigned short)))) return rc;
+    if ((rc = needed.reserve((n + kSpare) * sizeof(unsigned int)))) return rc;
+    if ((rc = needed_list.reserve((n / 2 + kBlockSlack) * sizeof(int)))) return rc;
+    if ((rc = far_list.reserve((n + kSpare) * sizeof(int)))) return rc;
+    if ((rc = built_bits.reserve((n / 32 + kSpare) * sizeof(unsigned int)))) return rc;
+    return counters.reserve(sizeof(ListCounters));
+  }
+  CandLists view() const {
+    return CandLists{records.as<unsigned int>(), pool.as<unsigned int>(), xlists.as<unsigned int>(), cell_items.as<int2>(), l1_slots.as<unsigned short>(),
+                     needed.as<unsigned int>(), needed_list.as<int>(), far_list.as<int>(), built_bits.as<unsigned int>(), counters.as<ListCounters>()};
+  }
+  void release() {
+    for (DevBuf* b : {&records, &pool, &xlists, &cell_items, &l1_slots, &needed, &needed_list, &far_list, &built_bits, &counters}) b->release();
+  }
+};
+
 // ------------------------------------------------------------------ the tracker object
 struct SceneReplica;
 struct pft_tracker {
@@ -124,7 +154,7 @@ struct pft_tracker {
   size_t scene_cap = 0; // allocated index capacity (scene points)
   int max_cells = 1 << 20;  // cap of the index grid; a larger crop box gets coarser cells
   int list_mode = 1;             // PFT_CANDIDATE_LISTS
-  int list_max_cells = 1 << 19;  // fine cells the candidate lists are sized for (kListK x 2 B each); 0 disables the lists
+  int list_max_cells = kListMaxCells;  // fine cells the candidate lists are sized for; 0 disables the lists
   int cur = 0;          // live particle buffer
   int inj_slots = 0, inj_stride = 0;
   int draw_cap = 0;
@@ -160,7 +190,8 @@ struct pft_tracker {
   int graph_nodes[2] = {0, 0};
   // device buffers
   DevBuf st, parts[2], mats, slot_aabb, model, model_perm, model_tmp, sort_keys, sort_idx, bbox, raw, partial, cdf, cdf_total, ancestors, bin_keys, tbl_rep,
-      tbl_min, slot_of, klb, d_usel, d_normals, d_umot, idx_hdr, idx_hdr_prev, fbuilt_bits, cell_start, ipts, ipts2, ihsv, icount, dbg_idx, dbg_d2, d_trans, row_table, flists, fpool, fcell_items, fl1_slots, fneeded, fneeded_list, ffar_list, xlists, xcount, result_box, ref_pts, alias_a, alias_q, alias_hl, oct_hdr, oct_nodes, oct_next, cd_hdr, cd_nodes, cd_out;
+      tbl_min, slot_of, klb, d_usel, d_normals, d_umot, idx_hdr, idx_hdr_prev, cell_start, ipts, ipts2, ihsv, icount, dbg_idx, dbg_d2, d_trans, row_table, result_box, ref_pts, alias_a, alias_q, alias_hl, oct_hdr, oct_nodes, oct_next, cd_hdr, cd_nodes, cd_out;
+  CandListStore lists;
   int oct_node_cap = 0;
   // change detector (SURVEY 8 f-4; PCL ctor defaults, off in the reference): host-driven, one read-back per test
   bool use_cd = false;
@@ -202,9 +233,10 @@ void stage_mark(pft_tracker* t, const char* name) {
 void release_all(pft_tracker* t) {
   DevBuf* bufs[] = {&t->st, &t->parts[0], &t->parts[1], &t->mats, &t->slot_aabb, &t->model, &t->model_perm, &t->model_tmp, &t->sort_keys, &t->sort_idx,
                     &t->bbox, &t->raw, &t->partial, &t->cdf, &t->cdf_total, &t->ancestors, &t->bin_keys, &t->tbl_rep, &t->tbl_min, &t->slot_of, &t->klb,
-                    &t->d_usel, &t->d_normals, &t->d_umot, &t->idx_hdr, &t->idx_hdr_prev, &t->fbuilt_bits, &t->cell_start, &t->ipts, &t->ipts2, &t->ihsv, &t->icount, &t->dbg_idx,
-                    &t->dbg_d2, &t->d_trans, &t->row_table, &t->flists, &t->fpool, &t->fcell_items, &t->fl1_slots, &t->fneeded, &t->fneeded_list, &t->ffar_list, &t->xlists, &t->xcount, &t->result_box, &t->ref_pts, &t->alias_a, &t->alias_q, &t->alias_hl, &t->oct_hdr, &t->oct_nodes, &t->oct_next, &t->cd_hdr, &t->cd_nodes, &t->cd_out};
+                    &t->d_usel, &t->d_normals, &t->d_umot, &t->idx_hdr, &t->idx_hdr_prev, &t->cell_start, &t->ipts, &t->ipts2, &t->ihsv, &t->icount, &t->dbg_idx,
+                    &t->dbg_d2, &t->d_trans, &t->row_table, &t->result_box, &t->ref_pts, &t->alias_a, &t->alias_q, &t->alias_hl, &t->oct_hdr, &t->oct_nodes, &t->oct_next, &t->cd_hdr, &t->cd_nodes, &t->cd_out};
   for (auto* b : bufs) b->release();
+  t->lists.release();
 }
 
 NoiseParams make_noise(const pft_tracker* t, const double* mean, const double* cov) {
@@ -335,19 +367,7 @@ int ensure_particle_buffers(pft_tracker* t) {
     if ((rc = t->cell_start.reserve(((size_t)t->max_cells + 16) * sizeof(int)))) return rc;
     if ((rc = t->icount.reserve(((size_t)t->max_cells + 16) * sizeof(int)))) return rc;
     if ((rc = upload_row_table(t))) return rc;
-    if (t->list_max_cells > 0) {
-      if ((rc = t->flists.reserve(((size_t)t->list_max_cells + 1) * 8 * 8 * sizeof(unsigned int)))) return rc;  // 8 octant records of 8 words per fine cell
-      if ((rc = t->fpool.reserve((size_t)kPoolGroups * 8 * sizeof(unsigned int)))) return rc;
-      if ((rc = t->fcell_items.reserve(((size_t)t->list_max_cells + 16) * sizeof(int2)))) return rc;
-      if ((rc = t->fl1_slots.reserve(((size_t)t->list_max_cells + 1) * kL1Cap * sizeof(unsigned short)))) return rc;
-      if ((rc = t->fneeded.reserve(((size_t)t->list_max_cells + 16) * sizeof(unsigned int)))) return rc;
-      if ((rc = t->fbuilt_bits.reserve(((size_t)t->list_max_cells / 32 + 16) * sizeof(unsigned int)))) return rc;
-      // blocks of 2x2x2 fine cells: at most ceil(d/2)^3 <= (d+1)^3/8, bounded generously by cells/2 + 4096
-      if ((rc = t->fneeded_list.reserve(((size_t)t->list_max_cells / 2 + 4096) * sizeof(int)))) return rc;
-      if ((rc = t->ffar_list.reserve(((size_t)t->list_max_cells + 16) * sizeof(int)))) return rc;
-      if ((rc = t->xlists.reserve((size_t)kListXCells * kListKX * sizeof(unsigned int)))) return rc;
-      if ((rc = t->xcount.reserve(64))) return rc;
-    }
+    if (t->list_max_cells > 0 && (rc = t->lists.reserve(t->list_max_cells))) return rc;
   }
   if (cap == t->n_cap) return PFT_OK;
   if (t->peer_local) {
@@ -660,8 +680,7 @@ int launch_index_begin(pft_tracker* t, bool reuse_allowed = false) {
   // one index per frame (see IndexHeader): with the lists on, the crop box is dilated by kIndexDilate; the later weight()
   // calls of a compute() reuse the index when their crop box fits
   index_begin_kernel<<<sm, 256, 0, t->run_stream()>>>(t->st.as<TrackerState>(), t->idx_hdr.as<IndexHeader>(), t->icount.as<int>(), inv_leaf, t->max_cells,
-                                                      t->list_mode ? t->list_max_cells : 0, t->list_mode == 2 ? 0 : t->M, t->nranks, t->rank,
-                                                      t->fneeded.as<unsigned int>(), t->xcount.as<int>(), t->fbuilt_bits.as<unsigned int>(),
+                                                      t->list_mode ? t->list_max_cells : 0, t->M, t->nranks, t->rank, t->lists.view(), t->list_mode == 2 ? 1 : 0,
                                                       reuse_allowed ? 1 : 0, t->iteration_num > 1 ? kIndexDilate : 0.f, kListRatio, t->idx_hdr_prev.as<IndexHeader>());
   PFT_LAUNCH_CHECK();
   stage_mark(t, "index_begin_kernel");
@@ -682,6 +701,7 @@ int weight_phase_eval(pft_tracker* t, bool reuse_allowed = false) {
   const int gscene = blocks_for(ncap_scene, 256, sm * 4);
   // candidate lists for the exact search (the index header may still turn them off for this crop)
   const bool lists = t->list_max_cells > 0 && t->list_mode && t->nn_mode == PFT_NN_EXACT;
+  const CandLists L = t->lists.view();
   if ((rc = launch_index_begin(t, reuse_allowed && lists))) return rc;
   if (lists) {
     // which fine cells the queries fall into (mark + collect) does not depend on the point index being built (count +
@@ -692,10 +712,10 @@ int weight_phase_eval(pft_tracker* t, bool reuse_allowed = false) {
     // small query sets: exact query counts per cell (cells with few queries get one list instead of eight octant lists)
     const long long n_queries = (long long)std::max(1, (t->particle_num > 0 ? t->particle_num : t->n_cap) / t->nranks) * t->M;
     const size_t mark_smem = (size_t)(t->list_max_cells / 8 + 64);
-    if (n_queries <= kMarkCountMaxQueries) cand_mark_kernel<true><<<sm * 3, 256, mark_smem, sa>>>(st, hdr, t->model.as<float4>(), t->M, t->mats.as<float>(), t->fneeded.as<unsigned int>(), t->nranks, t->rank, t->fbuilt_bits.as<unsigned int>());
-    else cand_mark_kernel<false><<<sm * 3, 256, mark_smem, sa>>>(st, hdr, t->model.as<float4>(), t->M, t->mats.as<float>(), t->fneeded.as<unsigned int>(), t->nranks, t->rank, t->fbuilt_bits.as<unsigned int>());
+    if (n_queries <= kMarkCountMaxQueries) cand_mark_kernel<true><<<sm * 3, 256, mark_smem, sa>>>(st, hdr, t->model.as<float4>(), t->M, t->mats.as<float>(), L, t->nranks, t->rank);
+    else cand_mark_kernel<false><<<sm * 3, 256, mark_smem, sa>>>(st, hdr, t->model.as<float4>(), t->M, t->mats.as<float>(), L, t->nranks, t->rank);
     PFT_LAUNCH_CHECK();
-    cand_collect_kernel<<<sm * 2, 256, 0, sa>>>(hdr, t->fneeded.as<unsigned int>(), t->fneeded_list.as<int>(), t->xcount.as<int>());
+    cand_collect_kernel<<<sm * 2, 256, 0, sa>>>(hdr, L);
     PFT_LAUNCH_CHECK();
     PFT_CUDA_TRY(cudaEventRecord(t->ev_join, sa));
   }
@@ -712,28 +732,23 @@ int weight_phase_eval(pft_tracker* t, bool reuse_allowed = false) {
   if (lists) {
     PFT_CUDA_TRY(cudaStreamWaitEvent(s, t->ev_join, 0));
     stage_mark(t, "cand_mark+collect (beside the index)");
-    cand_build_kernel<<<sm * 8, 256, 0, s>>>(hdr, t->cell_start.as<int>(), t->ipts.as<float4>(), t->max_dist * t->max_dist, t->flists.as<unsigned int>(),
-                                            t->fneeded.as<unsigned int>(), t->fneeded_list.as<int>(), t->xcount.as<int>(), t->ffar_list.as<int>(),
-                                            t->fcell_items.as<int2>(), t->fl1_slots.as<unsigned short>(), t->fbuilt_bits.as<unsigned int>());
+    cand_build_kernel<<<sm * 8, 256, 0, s>>>(hdr, t->cell_start.as<int>(), t->ipts.as<float4>(), t->max_dist * t->max_dist, L);
     PFT_LAUNCH_CHECK();
     stage_mark(t, "cand_build_kernel");
     // cells far from the surface (long lists): pairwise pruning, one thread block each; most of them join the octant pass
     // (measured and dropped: the far pass on a second stream beside the octant pass of the other cells -- it then takes
     // longer than the octant pass it competes with, and the frame does not get shorter)
-    cand_build_far_kernel<<<sm * 4, 256, 0, s>>>(hdr, t->cell_start.as<int>(), t->ipts.as<float4>(), t->max_dist * t->max_dist,
-                                                t->flists.as<unsigned int>(), t->xlists.as<unsigned int>(), t->xcount.as<int>(), t->ffar_list.as<int>(),
-                                                t->fneeded.as<unsigned int>(), t->fcell_items.as<int2>(), t->fl1_slots.as<unsigned short>(), t->fbuilt_bits.as<unsigned int>());
+    cand_build_far_kernel<<<sm * 4, 256, 0, s>>>(hdr, t->cell_start.as<int>(), t->ipts.as<float4>(), t->max_dist * t->max_dist, L);
     PFT_LAUNCH_CHECK();
     stage_mark(t, "cand_build_far_kernel");
-    cand_octant_kernel<<<sm * 8, 256, 0, s>>>(hdr, t->ipts.as<float4>(), t->max_dist * t->max_dist, t->flists.as<unsigned int>(), t->fpool.as<unsigned int>(),
-                                             t->xcount.as<int>(), t->fcell_items.as<int2>(), t->fl1_slots.as<unsigned short>());
+    cand_octant_kernel<<<sm * 8, 256, 0, s>>>(hdr, t->ipts.as<float4>(), t->max_dist * t->max_dist, L);
     PFT_LAUNCH_CHECK();
     stage_mark(t, "cand_octant_kernel");
   }
   if (t->nn_mode == PFT_NN_PCL_APPROX) return weight_eval_pcl_approx(t);
   WeightArgs a;
   a.st = st; a.hdr = hdr; a.pts2 = t->ipts2.as<float4>();
-  a.flists = t->flists.as<unsigned int>(); a.pool = t->fpool.as<unsigned int>(); a.xlists = t->xlists.as<unsigned int>();
+  a.records = L.records; a.pool = L.pool; a.xlists = L.xlists;
   a.cell_start = t->cell_start.as<int>(); a.pts = t->ipts.as<float4>();
   a.hsv = t->ihsv.as<unsigned int>(); a.table = t->row_table.as<RowEntry>(); a.smem_bytes = t->lists_smem;
   a.model = t->model.as<float4>(); a.model_perm = t->model_perm.as<int>(); a.M = t->M;

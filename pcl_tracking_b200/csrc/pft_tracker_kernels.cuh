@@ -49,6 +49,9 @@ struct TrackerState {
   unsigned int aabb_blocks_done; // blocks of the running aabb_kernel that have added their boxes (peer mode: the last one exchanges the box)
 };
 
+// how many of the n live particles this rank evaluates (particle i belongs to rank i % nranks)
+__device__ __forceinline__ int rank_share(int n, int rank, int nranks) { return n > rank ? (n - rank + nranks - 1) / nranks : 0; }
+
 // ------------------------------------------------------------------ NVLink peer exchange (one process per GPU)
 // Every rank owns one PeerWindow in its HBM, mapped into all peers with CUDA IPC.  The two exchange steps of weight()
 // are plain peer stores issued by the producing kernels themselves, followed by a flag barrier:
@@ -453,22 +456,130 @@ __device__ inline void compute_index_header(const float* crop, const float* aabb
   }
 }
 
+// ---- candidate-list storage, written by the build passes (cand_*_kernel) and read by the lookup (weight_lists_kernel)
+// Octant record = 8 words of 32 bits (one 32-byte sector, read by ONE 256-bit load):
+//   word 0      header: 0..7 = entry count | count (8..71) + (g << 8) = entries beyond the seventh are in pool groups
+//               g, g+1, .. (eight entries each) | kListExtended = word 1 holds the index of an extended list (cells far
+//               from the surface whose list pairwise pruning cannot shorten: up to kListKX entries in input-index order),
+//               word 2 its length | kListOverflow = no list (the query is answered by brute force)
+//   words 1..7  entries as BYTE offsets of the points in the staged array (slot << 4), padded with the dummy slot
+constexpr int kRecordWords = 8;                    // an octant record; also a pool group of eight entries
+constexpr int kCellWords = 8 * kRecordWords;       // the eight octant records of a fine cell
+constexpr int kListMaxCells = 1 << 19;             // fine cells the storage is sized for, at most
+static_assert((long long)kCellWords * (kListMaxCells + 1) < (1ll << 32), "record and word indices of the octant lattice are 32-bit");
+constexpr int kL1Cap = 64;                         // a cell's own list is split into octants up to this length; longer ones become extended lists
+constexpr int kListKX = 1024;                      // entries of an extended list (cells far from the surface)
+constexpr int kListXCells = 8192;                  // extended lists available per build
+constexpr int kPoolGroups = 1 << 18;               // groups of eight entries for octant lists longer than seven
+constexpr unsigned int kListOverflow = 0xffffffffu;  // no list
+constexpr unsigned int kListExtended = 0xfffffffeu;  // extended list
+constexpr int kMaxListSlots = 65535;               // the build passes carry 16-bit slots: larger crops use the row-table search only
+constexpr unsigned int kCoarseBelow = 24u;         // queries of a cell below which its list is not split into octants
+constexpr unsigned int kLightBelow = 256u;         // ... below which a list that fits one record is not split either
+
+// work counters of one build (index_begin_kernel clears them; a weight() that reuses the index of the frame keeps
+// handing out extended lists and pool groups where the earlier ones stopped)
+struct ListCounters {
+  int ext_lists;      // extended lists handed out
+  int needed_blocks;  // blocks of 2x2x2 fine cells queued by cand_collect_kernel
+  int far_cells;      // cells queued for cand_build_far_kernel
+  int pool_groups;    // pool groups handed out
+  int octant_cells;   // cells queued for cand_octant_kernel
+};
+
+// the list storage as the kernels see it (one fine cell = one cell of the fine lattice, edge = resolution).  Kernels take
+// it as a const __grid_constant__ parameter (the pointers are read from the parameter bank, as separate parameters would
+// be) and read the buffers they never write through __ldg (what const __restrict__ parameters would allow)
+struct CandLists {
+  unsigned int* records;      // kCellWords per fine cell: the octant records, one dense lattice (octant_record)
+  unsigned int* pool;         // kPoolGroups groups of eight entries
+  unsigned int* xlists;       // kListXCells extended lists of kListKX entries (byte offsets, ascending input index, padded to a multiple of four)
+  int2* cell_items;           // cells queued for cand_octant_kernel (cell_item_pack)
+  unsigned short* l1_slots;   // kL1Cap slots per fine cell: its own list, handed from the build passes to the octant pass
+  unsigned int* needed;       // per fine cell: queries of this rank in it, or a flag (cand_mark_kernel)
+  int* needed_list;           // blocks of 2x2x2 fine cells that hold a needed cell
+  int* far_list;              // fine cells queued for cand_build_far_kernel
+  unsigned int* built_bits;   // one bit per fine cell: its lists exist (this frame)
+  ListCounters* counters;
+};
+
+__device__ __forceinline__ bool lists_on(const IndexHeader& h) { return h.use_lists && h.n_cropped < kMaxListSlots; }
+
+// index (in records) of octant (ix, iy, iz) of the octant lattice (edge resolution / 2 over the fine cells, x fastest;
+// d2x, d2y = 2 x the fine dimensions), what a query computes from floor(q * 2 / resolution); and of octant o (x | y << 1
+// | z << 2) of fine cell (fx, fy, fz)
+template <typename T>
+__device__ __forceinline__ T octant_record(T ix, T iy, T iz, T d2x, T d2y) { return (iz * d2y + iy) * d2x + ix; }
+template <typename T>
+__device__ __forceinline__ T octant_record(int fx, int fy, int fz, int o, T d2x, T d2y) {
+  return octant_record<T>((T)(2 * fx + (o & 1)), (T)(2 * fy + ((o >> 1) & 1)), (T)(2 * fz + (o >> 2)), d2x, d2y);
+}
+
+// x-fastest lattice index -> coordinates (fine cells, or blocks of 2x2x2 of them)
+__device__ __forceinline__ void lattice_xyz(int c, int dx, int dy, int& x, int& y, int& z) { z = c / (dx * dy); const int r = c - z * dx * dy; y = r / dx; x = r - y * dx; }
+
+// a cell queued for the octant pass: x = cell | list length << 24 | (few queries: one list for the whole cell) << 31,
+// y = fx | fy << 10 | fz << 20 | (not many queries) << 30, or -1 when a coordinate needs more than 10 bits
+__device__ __forceinline__ int2 cell_item_pack(int cell, int n, int fx, int fy, int fz, unsigned int queries) {
+  return make_int2(cell | (n << 24) | (queries < kCoarseBelow ? (int)0x80000000 : 0),
+                   (fx < 1024 && fy < 1024 && fz < 1024) ? (fx | (fy << 10) | (fz << 20) | (queries < kLightBelow ? (1 << 30) : 0)) : -1);
+}
+struct CellItem { int cell, n, fx, fy, fz; bool coarse, light; };
+__device__ __forceinline__ CellItem cell_item_unpack(int2 item, int fdx, int fdy) {
+  CellItem c;
+  c.cell = item.x & 0xffffff;
+  c.n = (item.x >> 24) & 0x7f;
+  c.coarse = item.x < 0;
+  c.light = item.y >= 0 && ((item.y >> 30) & 1);
+  if (item.y >= 0) { c.fx = item.y & 1023; c.fy = (item.y >> 10) & 1023; c.fz = (item.y >> 20) & 1023; }
+  else lattice_xyz(c.cell, fdx, fdy, c.fx, c.fy, c.fz);
+  return c;
+}
+
+// The build passes widen every cell box by this margin (metric), which covers the fp32 rounding of q * inv_leaf near its
+// faces, and cut the lists at this reach (maximum_distance_, rounded up).  The lists are exact only because every pass
+// uses the same two values.
+__device__ __forceinline__ float list_margin(const IndexHeader& h) {
+  const float leaf = 1.0f / h.inv_leaf;
+  return 1.0e-5f + 4.0e-6f * leaf * (float)(abs(h.f_origin[0]) + abs(h.f_origin[1]) + abs(h.f_origin[2]) + h.f_dim[0] + h.f_dim[1] + h.f_dim[2]);
+}
+__device__ __forceinline__ float list_reach(double max_d2) { return max_d2 >= 1.0e30 ? 1.0e15f : (float)sqrt(max_d2) * 1.00001f; }
+
+// coarse cells [a, b] of axis d overlapping the box lo..hi dilated by r.  floor((p * inv_leaf) * 2^-level) is monotone
+// in p, so every point with lo - r <= p <= hi + r lies in them: no padding is needed.
+__device__ __forceinline__ void coarse_range(const IndexHeader& h, const float* lo, const float* hi, int d, float r, int& a, int& b) {
+  a = max((int)floorf(((lo[d] - r) * h.inv_leaf) * h.level_scale) - h.origin[d], 0);
+  b = min((int)floorf(((hi[d] + r) * h.inv_leaf) * h.level_scale) - h.origin[d], h.dim[d] - 1);
+}
+
+// p (offset x, y, z from the centre of a cube of half extent ch) against a competitor c (offset cx, cy, cz): min over
+// the cube of |q-p|^2 - |q-c|^2 = (|p|^2 - |c|^2) - 2 ch (|px-cx| + |py-cy| + |pz-cz|) beyond the rounding slack means
+// c is nearer everywhere in the cube (beaten); otherwise p can win for SOME query of the cube.  (can_win: a box.)
+struct CubeRace {
+  float fmin, slack;
+  __device__ __forceinline__ bool beaten() const { return fmin > slack; }
+  __device__ __forceinline__ bool can_win() const { return fmin <= slack; }
+};
+__device__ __forceinline__ CubeRace cube_race(float x, float y, float z, float cx, float cy, float cz, float ch) {
+  const float pn = (x * x + y * y) + z * z, cn = (cx * cx + cy * cy) + cz * cz;
+  return CubeRace{(pn - cn) - 2.0f * (ch * ((fabsf(x - cx) + fabsf(y - cy)) + fabsf(z - cz))), 1.0e-6f * (pn + cn) + 1.0e-9f};
+}
+
 // Every block derives the header from the crop box (a pure function of it), block 0 publishes it, and all
 // blocks clear the per-cell counters.
 // The cell edge follows the mean nearest-neighbour distance of the previous weight() (a query that is d away from the
 // surface walks ~pi (d/cell + 1)^2 rows and ~(d + cell)^2 candidates: cell ~ d balances them).
 __global__ void index_begin_kernel(TrackerState* st, IndexHeader* hdr, int* cell_count, float inv_leaf, int max_cells,
-                                   int list_max_cells, int M, int nranks, int rank, unsigned int* needed_words,
-                                   int* list_counters /* [0] extended lists handed out, [1] needed blocks, [2] cells queued for the far pass, [3] pool groups handed out, [4] cells queued for the octant pass */,
-                                   unsigned int* built_bits /* one bit per fine cell: its lists exist (this frame) */, int reuse_allowed, float dilate,
-                                   int list_ratio /* the lists are built when this rank's queries outnumber the fine cells of the crop box by this factor */,
+                                   int list_max_cells, int M, int nranks, int rank, const __grid_constant__ CandLists L, int lists_forced /* PFT_CANDIDATE_LISTS = 2 */,
+                                   int reuse_allowed, float dilate,
+                                   int list_ratio /* otherwise the lists are built when this rank's queries outnumber the fine cells of the crop box by this factor */,
                                    const IndexHeader* __restrict__ hdr_prev /* header of the previous weight() (snapshot taken by index_scan_kernel:
                                                                                nothing writes it while this kernel runs, so every block derives the same header) */) {
   __shared__ IndexHeader h;
   PFT_TRACE_MIN(0);
   if (threadIdx.x == 0) {
     const IndexHeader old = *hdr_prev;
-    bool reuse = reuse_allowed && old.valid && old.use_lists && old.n_cropped < 65535;
+    bool reuse = reuse_allowed && old.valid && lists_on(old);
     if (reuse) {
       // the new crop box must lie inside the box the index was built from (an empty crop box reuses nothing)
       reuse = st->aabb[0] <= st->aabb[3] && st->aabb[1] <= st->aabb[4] && st->aabb[2] <= st->aabb[5];
@@ -496,13 +607,12 @@ __global__ void index_begin_kernel(TrackerState* st, IndexHeader* hdr, int* cell
       }
       // candidate lists pay off when this rank's queries outnumber the fine cells they are built for
       const int n = st->particle_num;
-      const long long n_local = n > rank ? (n - rank + nranks - 1) / nranks : 0;
+      const long long n_local = rank_share(n, rank, nranks);
       float box[6];
 #pragma unroll
       for (int d = 0; d < 6; ++d) box[d] = st->aabb[d];
       compute_index_header(st->aabb, box, inv_leaf, base_level, max_cells, h);
-      // (M == 0: the caller forces the lists on)
-      bool lists = h.valid && h.f_cells > 0 && h.f_cells <= list_max_cells && (M == 0 || n_local * (long long)M >= (long long)list_ratio * h.f_cells);
+      bool lists = h.valid && h.f_cells > 0 && h.f_cells <= list_max_cells && (lists_forced || n_local * (long long)M >= (long long)list_ratio * h.f_cells);
       if (lists && dilate > 0.f) {
         // lists on: index the dilated box, so that the next weight() of the frame can reuse the index (when the dilated
         // box does not fit the list tables, the plain crop box is indexed and the next weight() rebuilds)
@@ -528,16 +638,15 @@ __global__ void index_begin_kernel(TrackerState* st, IndexHeader* hdr, int* cell
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < nc; i += gridDim.x * blockDim.x) cell_count[i] = 0;
   }
   if (h.use_lists) {
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < h.f_cells; i += gridDim.x * blockDim.x) needed_words[i] = 0u;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < h.f_cells; i += gridDim.x * blockDim.x) L.needed[i] = 0u;
     if (!h.reuse) {
       const int words = (h.f_cells + 31) >> 5;
-      for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < words; i += gridDim.x * blockDim.x) built_bits[i] = 0u;
+      for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < words; i += gridDim.x * blockDim.x) L.built_bits[i] = 0u;
     }
   }
   if (blockIdx.x == 0 && threadIdx.x == 0) {
-    // (a reusing weight() keeps handing out extended lists and pool groups where the earlier ones stopped)
-    if (!h.reuse) { list_counters[0] = 0; list_counters[3] = 0; }
-    list_counters[1] = 0; list_counters[2] = 0; list_counters[4] = 0;
+    if (!h.reuse) { L.counters->ext_lists = 0; L.counters->pool_groups = 0; }
+    L.counters->needed_blocks = 0; L.counters->far_cells = 0; L.counters->octant_cells = 0;
     st->work_counter = 0u;
   }
 }
@@ -774,21 +883,7 @@ __device__ __forceinline__ NNResult nn_search(const CS* __restrict__ cs, const f
 // some other candidate beats everywhere in the octant can never win) and what remains beyond seven goes to groups of
 // eight taken from a pool.  Every sub-list is in ascending order of the input index, so that the lookup
 // resolves distance ties by position (strict <: the first of equals wins = the lower index, the parity contract).
-//
-// Octant record = 8 words of 32 bits (one 32-byte sector, read by ONE 256-bit load):
-//   word 0      header: 0..7 = entry count | count (8..71) + (g << 8) = entries beyond the seventh are in pool groups
-//               g, g+1, .. (eight entries each) | kListExtended = word 1 holds the index of an extended list (cells far
-//               from the surface whose list pairwise pruning cannot shorten: up to kListKX entries in input-index order),
-//               word 2 its length | kListOverflow = no list (the query is answered by brute force)
-//   words 1..7  entries as BYTE offsets of the points in the staged array (slot << 4), padded with the dummy slot
-constexpr int kL1Cap = 64;                         // a cell's own list is split into octants up to this length; longer ones become extended lists
-constexpr int kListKX = 1024;                      // entries of an extended list (cells far from the surface)
-constexpr int kListXCells = 8192;                  // extended lists available per build
-constexpr int kPoolGroups = 1 << 18;               // groups of eight entries for octant lists longer than seven
-constexpr unsigned int kListOverflow = 0xffffffffu;  // no list
-constexpr unsigned int kListExtended = 0xfffffffeu;  // extended list
-// the build passes carry 16-bit slots: larger crops use the row-table search only
-__device__ __forceinline__ bool lists_on(const IndexHeader& h) { return h.use_lists && h.n_cropped < 65535; }
+// (storage format: see CandLists)
 
 __device__ __forceinline__ float box_mindist2(const float* lo, const float* hi, const float4& p) {
   const float dx = fmaxf(fmaxf(lo[0] - p.x, p.x - hi[0]), 0.f), dy = fmaxf(fmaxf(lo[1] - p.y, p.y - hi[1]), 0.f),
@@ -813,12 +908,9 @@ __device__ __forceinline__ float box_maxdist2(const float* lo, const float* hi, 
 // remembers the cells it has flagged in a bitmap of the fine grid in shared memory (f_cells bits, dynamic): every
 // block stores every cell at most once.
 constexpr int kMarkUnroll = 4;
-constexpr unsigned int kCoarseBelow = 24u;               // queries of a cell below which its list is not split into octants
-constexpr unsigned int kLightBelow = 256u;               // ... below which a list that fits one record is not split either
 template <bool COUNT>
 __global__ void __launch_bounds__(256) cand_mark_kernel(const TrackerState* __restrict__ st, const IndexHeader* __restrict__ hdr, const float4* __restrict__ model, int M,
-                                                        const float* __restrict__ mats, unsigned int* __restrict__ needed, int nranks, int rank,
-                                                        const unsigned int* __restrict__ built_bits) {
+                                                        const float* __restrict__ mats, const __grid_constant__ CandLists L, int nranks, int rank) {
   extern __shared__ unsigned int s_bits[];  // (f_cells + 31) / 32 words
   __shared__ IndexHeader h;
   if (threadIdx.x == 0) h = *hdr;
@@ -829,11 +921,10 @@ __global__ void __launch_bounds__(256) cand_mark_kernel(const TrackerState* __re
   const bool use_bits = !COUNT || h.reuse;
   if (use_bits) {
     const int words = (h.f_cells + 31) >> 5;
-    for (int i = threadIdx.x; i < words; i += blockDim.x) s_bits[i] = h.reuse ? built_bits[i] : 0u;
+    for (int i = threadIdx.x; i < words; i += blockDim.x) s_bits[i] = h.reuse ? L.built_bits[i] : 0u;
     __syncthreads();
   }
-  const int n = st->particle_num;
-  const int n_local = n > rank ? (n - rank + nranks - 1) / nranks : 0;
+  const int n_local = rank_share(st->particle_num, rank, nranks);
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, wpb = blockDim.x >> 5;
   const int groups = (M + 32 * kMarkUnroll - 1) / (32 * kMarkUnroll);
   const int per_group = max(1, (int)gridDim.x / groups);  // blocks that share one group of model points
@@ -862,11 +953,11 @@ __global__ void __launch_bounds__(256) cand_mark_kernel(const TrackerState* __re
           if ((unsigned)ix < (unsigned)fdx && (unsigned)iy < (unsigned)fdy && (unsigned)iz < (unsigned)fdz) {
             const int c = (iz * fdy + iy) * fdx + ix;
             if (COUNT) {
-              if (!use_bits || !((s_bits[c >> 5] >> (c & 31)) & 1u)) atomicAdd(&needed[c], 1u);  // (no return value: a reduction at the L2, nothing comes back)
+              if (!use_bits || !((s_bits[c >> 5] >> (c & 31)) & 1u)) atomicAdd(&L.needed[c], 1u);  // (no return value: a reduction at the L2, nothing comes back)
             } else {
               const unsigned int bit = 1u << (c & 31);
               if (!(s_bits[c >> 5] & bit)) {  // (cheap pre-test; the atomic decides)
-                if (!(atomicOr(&s_bits[c >> 5], bit) & bit)) needed[c] = 0x40000000u;  // (a flag: a busy cell)
+                if (!(atomicOr(&s_bits[c >> 5], bit) & bit)) L.needed[c] = 0x40000000u;  // (a flag: a busy cell)
               }
             }
           }
@@ -878,8 +969,7 @@ __global__ void __launch_bounds__(256) cand_mark_kernel(const TrackerState* __re
 }
 
 // queues every block of 2x2x2 fine cells that holds a marked cell (one thread per block, warp-aggregated append)
-__global__ void __launch_bounds__(256) cand_collect_kernel(const IndexHeader* __restrict__ hdr, const unsigned int* __restrict__ needed,
-                                                           int* __restrict__ needed_list, int* __restrict__ list_counters) {
+__global__ void __launch_bounds__(256) cand_collect_kernel(const IndexHeader* __restrict__ hdr, const __grid_constant__ CandLists L) {
   __shared__ IndexHeader h;
   if (threadIdx.x == 0) h = *hdr;
   __syncthreads();
@@ -892,15 +982,16 @@ __global__ void __launch_bounds__(256) cand_collect_kernel(const IndexHeader* __
     const int blk = b0 + lane;
     bool any = false;
     if (blk < nb) {
-      const int bz = blk / (bdx * bdy), br = blk - bz * bdx * bdy, by = br / bdx, bx = br - by * bdx;
+      int bx, by, bz;
+      lattice_xyz(blk, bdx, bdy, bx, by, bz);
 #pragma unroll
       for (int sub = 0; sub < 8; ++sub) {
         const int fx = 2 * bx + (sub & 1), fy = 2 * by + ((sub >> 1) & 1), fz = 2 * bz + (sub >> 2);
         if (fx < fdx && fy < fdy && fz < fdz) {
           const int c = (fz * fdy + fy) * fdx + fx;
-          if (needed[c] != 0u) any = true;
+          if (__ldg(&L.needed[c]) != 0u) any = true;
 #ifdef PFT_STATS
-          { const unsigned int q = needed[c]; if (q) { const int b = min(31 - __clz(q), 9); PFT_STAT(16 + b, 1); PFT_STAT(26 + b, q); } }
+          { const unsigned int q = __ldg(&L.needed[c]); if (q) { const int b = min(31 - __clz(q), 9); PFT_STAT(16 + b, 1); PFT_STAT(26 + b, q); } }
 #endif
         }
       }
@@ -909,9 +1000,9 @@ __global__ void __launch_bounds__(256) cand_collect_kernel(const IndexHeader* __
     PFT_STAT(36, any ? 1 : 0);
     if (bal) {
       int base = 0;
-      if (lane == 0) base = atomicAdd(&list_counters[1], __popc(bal));
+      if (lane == 0) base = atomicAdd(&L.counters->needed_blocks, __popc(bal));
       base = __shfl_sync(kFull, base, 0);
-      if (any) needed_list[base + __popc(bal & ((1u << lane) - 1u))] = blk;
+      if (any) L.needed_list[base + __popc(bal & ((1u << lane) - 1u))] = blk;
     }
   }
 }
@@ -961,19 +1052,13 @@ __device__ __forceinline__ bool can_win(const float4& p, const float4& p0, const
   return fmin <= 1.0e-6f * (pn + p0n) + 1.0e-9f;
 }
 
-// index (in records of 8 words) of octant (ox, oy, oz) of fine cell (fx, fy, fz): the octants form one dense lattice of
-// edge resolution / 2 over the crop box, x fastest -- what a query computes directly from floor(q * 2 / resolution)
-__device__ __forceinline__ size_t octant_record(const IndexHeader& h, int fx, int fy, int fz, int o) {
-  return ((size_t)(2 * fz + (o >> 2)) * (size_t)(2 * h.f_dim[1]) + (size_t)(2 * fy + ((o >> 1) & 1))) * (size_t)(2 * h.f_dim[0]) + (size_t)(2 * fx + (o & 1));
-}
-
 // All eight octant records of a cell get the same code (lanes 0..7 of the calling warp):
 // kListOverflow / 0 (empty list) / kListExtended with the index and length of the extended list.
-__device__ __forceinline__ void write_octant_codes(const IndexHeader& h, unsigned int* __restrict__ flists, int fx, int fy, int fz, unsigned int code, int xi, int n) {
+__device__ __forceinline__ void write_octant_codes(const IndexHeader& h, unsigned int* __restrict__ records, int fx, int fy, int fz, unsigned int code, int xi, int n) {
   const int lane = threadIdx.x & 31;
   if (lane < 8) {
     const unsigned int dd = (unsigned int)h.n_cropped << 4;
-    uint4* r = reinterpret_cast<uint4*>(flists + octant_record(h, fx, fy, fz, lane) * 8);
+    uint4* r = reinterpret_cast<uint4*>(records + octant_record<size_t>(fx, fy, fz, lane, (size_t)(2 * h.f_dim[0]), (size_t)(2 * h.f_dim[1])) * kRecordWords);
     r[0] = make_uint4(code, code == kListExtended ? (unsigned int)xi : dd, code == kListExtended ? (unsigned int)n : dd, dd);
     r[1] = make_uint4(dd, dd, dd, dd);
   }
@@ -1030,29 +1115,21 @@ __device__ __forceinline__ void block_bitonic_sort(unsigned long long* keys, int
 // cells of blocks whose superset does not fit, i.e. far from the surface, where lists are long (extended lists up to
 // kListKX) and a single warp would walk ~1000 points on its own while the rest of the GPU waits.
 __device__ __forceinline__ void build_cell_direct(const IndexHeader& h, const int* __restrict__ cs, const float4* __restrict__ pts, int cell,
-                                                  float leaf, float margin, float r_max,
-                                                  unsigned int* __restrict__ flists, unsigned int* __restrict__ xlists,
-                                                  int* __restrict__ list_counters, int* pref, int* start, int* s_cnt, float* s_m2, int* s_ms, int* s_xi,
+                                                  float leaf, float margin, float r_max, const CandLists& L,
+                                                  int* pref, int* start, int* s_cnt, float* s_m2, int* s_ms, int* s_xi,
                                                   unsigned short* s_list /* [kListKX] shared */, float4* s_pt4 /* [kListKX] shared */,
-                                                  unsigned long long* s_key /* [kListKX] shared */, unsigned long long* s_key2 /* [kListKX] shared */,
-                                                  const unsigned int* __restrict__ needed,
-                                                  int2* __restrict__ cell_items, unsigned short* __restrict__ l1_slots, unsigned int* __restrict__ built_bits) {
+                                                  unsigned long long* s_key /* [kListKX] shared */, unsigned long long* s_key2 /* [kListKX] shared */) {
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = blockDim.x >> 5;
   const int fdx = h.f_dim[0], fdy = h.f_dim[1];
   const float cell_m = h.cell;
   const int dimx = h.dim[0], dimy = h.dim[1];
-  const int fz = cell / (fdx * fdy), r2 = cell - fz * fdx * fdy, fy = r2 / fdx, fx = r2 - fy * fdx;
+  int fx, fy, fz;
+  lattice_xyz(cell, fdx, fdy, fx, fy, fz);
   // the cell in metric space, widened by the rounding of q * inv_leaf near its faces
   float lo[3], hi[3];
   lo[0] = (float)(h.f_origin[0] + fx) * leaf - margin; hi[0] = (float)(h.f_origin[0] + fx + 1) * leaf + margin;
   lo[1] = (float)(h.f_origin[1] + fy) * leaf - margin; hi[1] = (float)(h.f_origin[1] + fy + 1) * leaf + margin;
   lo[2] = (float)(h.f_origin[2] + fz) * leaf - margin; hi[2] = (float)(h.f_origin[2] + fz + 1) * leaf + margin;
-  // coarse cells overlapping the box dilated by r.  floor((p * inv_leaf) * 2^-level) is monotone in p, so every point
-  // with lo - r <= p <= hi + r (per axis) lies in cells [c0, c1]: no padding is needed.
-  auto coarse_range = [&](int d, float r, int& a, int& b) {
-    a = max((int)floorf(((lo[d] - r) * h.inv_leaf) * h.level_scale) - h.origin[d], 0);
-    b = min((int)floorf(((hi[d] + r) * h.inv_leaf) * h.level_scale) - h.origin[d], h.dim[d] - 1);
-  };
   // (one index per frame: see cand_build_kernel) far from the faces of the crop box the list is built from all points
   // and serves every weight() of the frame; near them it is built from the cropped points, for this weight() only
   const bool dilated = h.dilate > 0.f;
@@ -1065,7 +1142,7 @@ retry:
   float pr = fmaxf(2.0f * leaf, 0.5f * cell_m);
   for (int round = 0; round < 8; ++round, pr *= 2.0f) {
     int x0, x1, y0, y1, z0, z1;
-    coarse_range(0, pr, x0, x1); coarse_range(1, pr, y0, y1); coarse_range(2, pr, z0, z1);
+    coarse_range(h, lo, hi, 0, pr, x0, x1); coarse_range(h, lo, hi, 1, pr, y0, y1); coarse_range(h, lo, hi, 2, pr, z0, z1);
     float m2 = 3.0e38f;
     int ms = -1;
     if (x0 <= x1 && y0 <= y1 && z0 <= z1) {
@@ -1092,8 +1169,8 @@ retry:
   if (U2 >= 3.0e38f) {
     // provably no point within maximum_distance_ of any query of the cell (empty lists), or the probe gave up (the
     // queries of this cell are answered by brute force)
-    if (threadIdx.x < 32) write_octant_codes(h, flists, fx, fy, fz, no_match ? 0u : kListOverflow, 0, 0);
-    if (!crop_only && threadIdx.x == 0) atomicOr(&built_bits[cell >> 5], 1u << (cell & 31));  // (found among all points: holds for every crop box)
+    if (threadIdx.x < 32) write_octant_codes(h, L.records, fx, fy, fz, no_match ? 0u : kListOverflow, 0, 0);
+    if (!crop_only && threadIdx.x == 0) atomicOr(&L.built_bits[cell >> 5], 1u << (cell & 31));  // (found among all points: holds for every crop box)
     return;
   }
   U2 = fminf(U2, r_max * r_max);
@@ -1112,7 +1189,7 @@ retry:
   const float4 p0 = pts[p0_slot];
   // ---- (2) gather: rows of coarse cells that intersect the ball-dilated box
   int c0[3], c1[3];
-  coarse_range(1, reach, c0[1], c1[1]); coarse_range(2, reach, c0[2], c1[2]);
+  coarse_range(h, lo, hi, 1, reach, c0[1], c1[1]); coarse_range(h, lo, hi, 2, reach, c0[2], c1[2]);
   const int ny = c1[1] - c0[1] + 1, nrows = max(ny, 0) * max(c1[2] - c0[2] + 1, 0);
   // one gather into shared memory (up to the capacity of an extended list), then the list goes where its length says
   if (threadIdx.x == 0) *s_cnt = 0;
@@ -1148,7 +1225,7 @@ retry:
                     // this barrier a warp that is scheduled late -- other kernels share the SM when several trackers
                     // run side by side -- read 0 and left the block's barriers out of step: an intermittent fault of
                     // the multi-object batch)
-  if (n > kListKX) { if (threadIdx.x < 32) write_octant_codes(h, flists, fx, fy, fz, kListOverflow, 0, 0); return; }
+  if (n > kListKX) { if (threadIdx.x < 32) write_octant_codes(h, L.records, fx, fy, fz, kListOverflow, 0, 0); return; }
   // ---- (3) pairwise pruning.  Far from the surface the two tests above keep hundreds of points (they only compare
   // with ONE competitor, p0); nearly all of them are beaten everywhere in the cell by some other candidate (a point
   // of the same face that lies nearer to the cell).  Every thread scans the competitors of its candidate and stops at
@@ -1191,14 +1268,10 @@ retry:
     if (r < n) {
       const int t = (int)(s_sorted[r] & 0xffffffffull);
       const float4 p = s_pt4[t];
-      const float pn = (p.x * p.x + p.y * p.y) + p.z * p.z;
       bool alive = true;
       for (int k = 0; k < r; ++k) {
         const float4 c = s_pt4[(int)(s_sorted[k] & 0xffffffffull)];
-        const float cn = (c.x * c.x + c.y * c.y) + c.z * c.z;
-        // min over the cube of |q-p|^2 - |q-c|^2: positive (beyond the rounding slack) = c is nearer everywhere
-        const float fmin = (pn - cn) - 2.0f * (ch * ((fabsf(p.x - c.x) + fabsf(p.y - c.y)) + fabsf(p.z - c.z)));
-        if (fmin > 1.0e-6f * (pn + cn) + 1.0e-9f) { alive = false; break; }
+        if (cube_race(p.x, p.y, p.z, c.x, c.y, c.z, ch).beaten()) { alive = false; break; }  // c is nearer everywhere in the cell
       }
       // key = input index (upper half: the order of the extended list) | position in s_list
       if (alive) s_out[atomicAdd(s_cnt, 1)] = ((unsigned long long)(unsigned int)__float_as_int(p.w) << 32) | (unsigned long long)t;
@@ -1207,15 +1280,11 @@ retry:
   __syncthreads();
   const int m = *s_cnt;
   PFT_STAT(11, threadIdx.x == 0 ? 1 : 0);
-  if (indep && threadIdx.x == 0) atomicOr(&built_bits[cell >> 5], 1u << (cell & 31));  // (the next weight() of the frame need not build it again)
+  if (indep && threadIdx.x == 0) atomicOr(&L.built_bits[cell >> 5], 1u << (cell & 31));  // (the next weight() of the frame need not build it again)
   if (m <= kL1Cap) {
     // a normal cell after all: its list goes to cand_octant_kernel like those of cand_build_kernel
-    if ((int)threadIdx.x < m) l1_slots[(size_t)cell * kL1Cap + threadIdx.x] = s_list[(int)(s_out[threadIdx.x] & 0xffffffffull)];
-    if (threadIdx.x == 0) {
-      const int item = cell | (m << 24) | (needed[cell] < kCoarseBelow ? (int)0x80000000 : 0);
-      const int xyz = (fx < 1024 && fy < 1024 && fz < 1024) ? (fx | (fy << 10) | (fz << 20) | (needed[cell] < kLightBelow ? (1 << 30) : 0)) : -1;
-      cell_items[atomicAdd(&list_counters[4], 1)] = make_int2(item, xyz);
-    }
+    if ((int)threadIdx.x < m) L.l1_slots[(size_t)cell * kL1Cap + threadIdx.x] = s_list[(int)(s_out[threadIdx.x] & 0xffffffffull)];
+    if (threadIdx.x == 0) L.cell_items[atomicAdd(&L.counters->octant_cells, 1)] = cell_item_pack(cell, m, fx, fy, fz, __ldg(&L.needed[cell]));
     return;
   }
   // still long: an extended list in ascending order of the input index, scanned entry by entry by the queries of the cell
@@ -1225,15 +1294,15 @@ retry:
   __syncthreads();
   block_bitonic_sort(s_out, m2);
   s_key = s_out;
-  if (threadIdx.x == 0) *s_xi = atomicAdd(&list_counters[0], 1);
+  if (threadIdx.x == 0) *s_xi = atomicAdd(&L.counters->ext_lists, 1);
   __syncthreads();
   const int xi = *s_xi;
-  if (xi >= kListXCells) { if (threadIdx.x < 32) write_octant_codes(h, flists, fx, fy, fz, kListOverflow, 0, 0); return; }
-  unsigned int* dst = xlists + (size_t)xi * kListKX;
+  if (xi >= kListXCells) { if (threadIdx.x < 32) write_octant_codes(h, L.records, fx, fy, fz, kListOverflow, 0, 0); return; }
+  unsigned int* dst = L.xlists + (size_t)xi * kListKX;
   const unsigned int dummy = (unsigned int)h.n_cropped << 4;
   const int m4 = (m + 3) & ~3;  // the lookup reads four entries at a time
   for (int t = threadIdx.x; t < m4; t += blockDim.x) dst[t] = t < m ? ((unsigned int)s_list[(int)(s_key[t] & 0xffffffffull)] << 4) : dummy;
-  if (threadIdx.x < 32) write_octant_codes(h, flists, fx, fy, fz, kListExtended, xi, m);
+  if (threadIdx.x < 32) write_octant_codes(h, L.records, fx, fy, fz, kListExtended, xi, m);
   PFT_STAT(15, threadIdx.x == 0 ? 1 : 0);
 }
 
@@ -1241,12 +1310,7 @@ retry:
 // query of the BLOCK are gathered once into shared memory (a superset of every cell's list), then each needed cell
 // of the block filters that superset with its own bound and bisector test.
 __global__ void __launch_bounds__(256) cand_build_kernel(const IndexHeader* __restrict__ hdr, const int* __restrict__ cs,
-                                                         const float4* __restrict__ pts, double max_d2,
-                                                         unsigned int* __restrict__ flists,
-                                                         const unsigned int* __restrict__ needed, const int* __restrict__ needed_list,
-                                                         int* __restrict__ list_counters,
-                                                         int* __restrict__ far_list, int2* __restrict__ cell_items,
-                                                         unsigned short* __restrict__ l1_slots, unsigned int* __restrict__ built_bits) {
+                                                         const float4* __restrict__ pts, double max_d2, const __grid_constant__ CandLists L) {
   __shared__ IndexHeader h;
   __shared__ int s_cnt[8];
   __shared__ int s_pref[8][33], s_start[8][32];
@@ -1255,10 +1319,10 @@ __global__ void __launch_bounds__(256) cand_build_kernel(const IndexHeader* __re
   if (threadIdx.x == 0) h = *hdr;
   __syncthreads();
   if (!h.valid || !lists_on(h)) return;
-  const int n_needed = list_counters[1];
+  const int n_needed = L.counters->needed_blocks;
   const float leaf = 1.0f / h.inv_leaf;
-  const float margin = 1.0e-5f + 4.0e-6f * leaf * (float)(abs(h.f_origin[0]) + abs(h.f_origin[1]) + abs(h.f_origin[2]) + h.f_dim[0] + h.f_dim[1] + h.f_dim[2]);
-  const float r_max = max_d2 >= 1.0e30 ? 1.0e15f : (float)sqrt(max_d2) * 1.00001f;
+  const float margin = list_margin(h);
+  const float r_max = list_reach(max_d2);
   const int fdx = h.f_dim[0], fdy = h.f_dim[1], fdz = h.f_dim[2];
   const int bdx = (fdx + 1) >> 1, bdy = (fdy + 1) >> 1;
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -1271,8 +1335,8 @@ __global__ void __launch_bounds__(256) cand_build_kernel(const IndexHeader* __re
   unsigned short* sslot = s_slot[wib];
   if (lane == 0) pref[32] = 0x7fffffff;  // sentinel for the binary search
   for (int idx = warp; idx < n_needed; idx += nwarps) {
-    const int blk = needed_list[idx];
-    const int bz = blk / (bdx * bdy), br = blk - bz * bdx * bdy, by = br / bdx, bx = br - by * bdx;
+    int bx, by, bz;
+    lattice_xyz(__ldg(&L.needed_list[idx]), bdx, bdy, bx, by, bz);
     // the block (2x2x2 fine cells) in metric space, widened by the rounding of q * inv_leaf near its faces
     float lo[3], hi[3];
     lo[0] = (float)(h.f_origin[0] + 2 * bx) * leaf - margin; hi[0] = (float)(h.f_origin[0] + 2 * bx + 2) * leaf + margin;
@@ -1285,18 +1349,12 @@ __global__ void __launch_bounds__(256) cand_build_kernel(const IndexHeader* __re
         if (fx < fdx && fy < fdy && fz < fdz) {
           const int c = (fz * fdy + fy) * fdx + fx;
           // every octant: header + dummy slots (value 0 = empty list: nothing within maximum_distance_)
-          if (needed[c]) {
-            write_octant_codes(h, flists, fx, fy, fz, value, 0, 0);
-            if (reusable && lane == 0) atomicOr(&built_bits[c >> 5], 1u << (c & 31));
+          if (__ldg(&L.needed[c])) {
+            write_octant_codes(h, L.records, fx, fy, fz, value, 0, 0);
+            if (reusable && lane == 0) atomicOr(&L.built_bits[c >> 5], 1u << (c & 31));
           }
         }
       }
-    };
-    // coarse cells overlapping the box dilated by r.  floor((p * inv_leaf) * 2^-level) is monotone in p, so every point
-    // with lo - r <= p <= hi + r (per axis) lies in cells [c0, c1]: no padding is needed.
-    auto coarse_range = [&](int d, float r, int& a, int& b) {
-      a = max((int)floorf(((lo[d] - r) * h.inv_leaf) * h.level_scale) - h.origin[d], 0);
-      b = min((int)floorf(((hi[d] + r) * h.inv_leaf) * h.level_scale) - h.origin[d], h.dim[d] - 1);
     };
     // One index per frame (IndexHeader::built): when the index holds more than the crop box, a block whose lists cannot
     // depend on where the faces of the crop box are -- every point that matters lies well inside it -- is built from all
@@ -1312,7 +1370,7 @@ __global__ void __launch_bounds__(256) cand_build_kernel(const IndexHeader* __re
     float pr = fmaxf(2.0f * leaf, 0.5f * cell_m);
     for (int round = 0; round < 8; ++round, pr *= 2.0f) {
       int x0, x1, y0, y1, z0, z1;
-      coarse_range(0, pr, x0, x1); coarse_range(1, pr, y0, y1); coarse_range(2, pr, z0, z1);
+      coarse_range(h, lo, hi, 0, pr, x0, x1); coarse_range(h, lo, hi, 1, pr, y0, y1); coarse_range(h, lo, hi, 2, pr, z0, z1);
       float m2 = 3.0e38f;
       int ms = -1;
       if (x0 <= x1 && y0 <= y1 && z0 <= z1) {
@@ -1353,7 +1411,7 @@ __global__ void __launch_bounds__(256) cand_build_kernel(const IndexHeader* __re
     const float4 p0 = pts[p0_slot];
     // ---- (2) superset of the block: { p : mindist(block, p) <= U_B and p can beat p0 somewhere in the block }
     int c0[3], c1[3];
-    coarse_range(1, reach, c0[1], c1[1]); coarse_range(2, reach, c0[2], c1[2]);
+    coarse_range(h, lo, hi, 1, reach, c0[1], c1[1]); coarse_range(h, lo, hi, 2, reach, c0[2], c1[2]);
     const int ny = c1[1] - c0[1] + 1, nrows = max(ny, 0) * max(c1[2] - c0[2] + 1, 0);
     if (lane == 0) s_cnt[wib] = 0;
     __syncwarp();
@@ -1393,7 +1451,7 @@ __global__ void __launch_bounds__(256) cand_build_kernel(const IndexHeader* __re
         const int fx = 2 * bx + (lane & 1), fy = 2 * by + ((lane >> 1) & 1), fz = 2 * bz + (lane >> 2);
         if (fx < fdx && fy < fdy && fz < fdz) {
           const int c = (fz * fdy + fy) * fdx + fx;
-          if (needed[c]) { far_list[atomicAdd(&list_counters[2], 1)] = c; PFT_STAT(10, 1); }
+          if (__ldg(&L.needed[c])) { L.far_list[atomicAdd(&L.counters->far_cells, 1)] = c; PFT_STAT(10, 1); }
         }
       }
       continue;
@@ -1404,11 +1462,11 @@ __global__ void __launch_bounds__(256) cand_build_kernel(const IndexHeader* __re
       bool mine = false;
       if (lane < 8) {
         const int fx = 2 * bx + (lane & 1), fy = 2 * by + ((lane >> 1) & 1), fz = 2 * bz + (lane >> 2);
-        mine = fx < fdx && fy < fdy && fz < fdz && needed[(fz * fdy + fy) * fdx + fx] != 0u;
+        mine = fx < fdx && fy < fdy && fz < fdz && __ldg(&L.needed[(fz * fdy + fy) * fdx + fx]) != 0u;
       }
       sub_mask = __ballot_sync(kFull, mine);
     }
-    int my_item = 0, my_xyz = 0;  // lane `sub` remembers the cell it has to queue
+    int2 my_item = make_int2(0, 0);  // lane `sub` remembers the cell it has to queue
     bool my_valid = false;
     for (int sub = 0; sub < 8; ++sub) {
       if (!((sub_mask >> sub) & 1u)) continue;
@@ -1448,12 +1506,12 @@ __global__ void __launch_bounds__(256) cand_build_kernel(const IndexHeader* __re
       }
       if (n > kL1Cap) {
         // long list (far from the surface): the far pass prunes it pairwise
-        if (lane == 0) { far_list[atomicAdd(&list_counters[2], 1)] = cell; PFT_STAT(10, 1); }
+        if (lane == 0) { L.far_list[atomicAdd(&L.counters->far_cells, 1)] = cell; PFT_STAT(10, 1); }
         continue;
       }
       // ---- (4) hand the cell's list to cand_octant_kernel (slots in superset order; the octant pass sorts them)
       {
-        unsigned short* dst = l1_slots + (size_t)cell * kL1Cap;
+        unsigned short* dst = L.l1_slots + (size_t)cell * kL1Cap;
         int w = 0;
 #pragma unroll
         for (int q = 0; q < kSuperCap / 32; ++q) {
@@ -1465,11 +1523,9 @@ __global__ void __launch_bounds__(256) cand_build_kernel(const IndexHeader* __re
         }
       }
       if (lane == sub) {
-        // item = cell | list length << 24 | (few queries: one list for the whole cell) << 31, and the cell's coordinates
-        my_item = cell | (n << 24) | (needed[cell] < kCoarseBelow ? (int)0x80000000 : 0);
-        my_xyz = (fx < 1024 && fy < 1024 && fz < 1024) ? (fx | (fy << 10) | (fz << 20) | (needed[cell] < kLightBelow ? (1 << 30) : 0)) : -1;
+        my_item = cell_item_pack(cell, n, fx, fy, fz, __ldg(&L.needed[cell]));
         my_valid = true;
-        if (indep) atomicOr(&built_bits[cell >> 5], 1u << (cell & 31));  // (the next weight() of the frame need not build it again)
+        if (indep) atomicOr(&L.built_bits[cell >> 5], 1u << (cell & 31));  // (the next weight() of the frame need not build it again)
       }
       PFT_STAT(15, lane == 0 ? 1 : 0);
     }
@@ -1478,9 +1534,9 @@ __global__ void __launch_bounds__(256) cand_build_kernel(const IndexHeader* __re
       const unsigned int bal = __ballot_sync(kFull, my_valid);
       if (bal) {
         int base = 0;
-        if (lane == 0) base = atomicAdd(&list_counters[4], __popc(bal));
+        if (lane == 0) base = atomicAdd(&L.counters->octant_cells, __popc(bal));
         base = __shfl_sync(kFull, base, 0);
-        if (my_valid) cell_items[base + __popc(bal & ((1u << lane) - 1u))] = make_int2(my_item, my_xyz);
+        if (my_valid) L.cell_items[base + __popc(bal & ((1u << lane) - 1u))] = my_item;
       }
     }
   }
@@ -1495,10 +1551,7 @@ __global__ void __launch_bounds__(256) cand_build_kernel(const IndexHeader* __re
 // that another kept entry beats everywhere in the octant never wins); ballot compaction keeps the order.  Entries
 // beyond the seventh go to groups of eight taken from a pool (the header carries the first group).  The eight records
 // are assembled in shared memory and written out together.
-__global__ void __launch_bounds__(256) cand_octant_kernel(const IndexHeader* __restrict__ hdr, const float4* __restrict__ pts, double max_d2,
-                                                          unsigned int* __restrict__ flists, unsigned int* __restrict__ pool,
-                                                          int* __restrict__ list_counters, const int2* __restrict__ cell_items,
-                                                          const unsigned short* __restrict__ l1_slots) {
+__global__ void __launch_bounds__(256) cand_octant_kernel(const IndexHeader* __restrict__ hdr, const float4* __restrict__ pts, double max_d2, const __grid_constant__ CandLists L) {
   __shared__ IndexHeader h;
   __shared__ float4 s_pt[8][kL1Cap];
   __shared__ unsigned int s_off[8][kL1Cap];
@@ -1506,10 +1559,10 @@ __global__ void __launch_bounds__(256) cand_octant_kernel(const IndexHeader* __r
   if (threadIdx.x == 0) h = *hdr;
   __syncthreads();
   if (!h.valid || !lists_on(h)) return;
-  const int n_items = list_counters[4];
+  const int n_items = L.counters->octant_cells;
   const float leaf = 1.0f / h.inv_leaf;
-  const float margin = 1.0e-5f + 4.0e-6f * leaf * (float)(abs(h.f_origin[0]) + abs(h.f_origin[1]) + abs(h.f_origin[2]) + h.f_dim[0] + h.f_dim[1] + h.f_dim[2]);
-  const float r_max = max_d2 >= 1.0e30 ? 1.0e15f : (float)sqrt(max_d2) * 1.00001f;
+  const float margin = list_margin(h);
+  const float r_max = list_reach(max_d2);
   const float rmax2 = r_max * r_max;
   const float quarter = 0.25f * leaf;
   // half extent of an octant box: the octant itself, the rounding of q * inv_leaf near its faces (margin) and of the
@@ -1524,39 +1577,28 @@ __global__ void __launch_bounds__(256) cand_octant_kernel(const IndexHeader* __r
   float4* spt = s_pt[wib];
   unsigned int* soff = s_off[wib];
   unsigned int* srec = s_rec[wib];
-  // can p (offset x, y, z from the octant centre) be at least as near as the competitor (offset cx, cy, cz) somewhere in
-  // the octant?  min over the cube of |q-p|^2 - |q-c|^2 = (|p|^2 - |c|^2) - 2 oh (|px-cx| + |py-cy| + |pz-cz|)
-  auto can_win_c = [&](float x, float y, float z, float cx, float cy, float cz) {
-    const float pn = (x * x + y * y) + z * z, cn = (cx * cx + cy * cy) + cz * cz;
-    const float fmin = (pn - cn) - 2.0f * (oh * ((fabsf(x - cx) + fabsf(y - cy)) + fabsf(z - cz)));
-    return fmin <= 1.0e-6f * (pn + cn) + 1.0e-9f;
-  };
+  auto can_win_c = [&](float x, float y, float z, float cx, float cy, float cz) { return cube_race(x, y, z, cx, cy, cz, oh).can_win(); };
   auto maxd2 = [&](float x, float y, float z) { const float u = fabsf(x) + oh, v = fabsf(y) + oh, w = fabsf(z) + oh; return (u * u + v * v) + w * w; };
   auto mind2 = [&](float x, float y, float z) {
     const float u = fmaxf(fabsf(x) - oh, 0.f), v = fmaxf(fabsf(y) - oh, 0.f), w = fmaxf(fabsf(z) - oh, 0.f);
     return (u * u + v * v) + w * w;
   };
   for (int it = warp; it < n_items; it += nwarps) {
-    const int2 item = cell_items[it];
-    const int cell = item.x & 0xffffff;
-    int n = (item.x >> 24) & 0x7f;
-    const bool coarse = item.x < 0;
-    int fx, fy, fz;
-    const bool light = item.y >= 0 && ((item.y >> 30) & 1);
-    if (item.y >= 0) { fx = item.y & 1023; fy = (item.y >> 10) & 1023; fz = (item.y >> 20) & 1023; }
-    else { fz = cell / (fdx * fdy); const int r2 = cell - fz * fdx * fdy; fy = r2 / fdx; fx = r2 - fy * fdx; }
+    const CellItem item = cell_item_unpack(__ldg(&L.cell_items[it]), fdx, fdy);
+    const int cell = item.cell, fx = item.fx, fy = item.fy, fz = item.fz;
+    int n = item.n;
     bool two = n > 32;
     // ---- the list in ascending order of the input index (rank = how many keys are smaller; keys are distinct)
     {
-      const unsigned short* src = l1_slots + (size_t)cell * kL1Cap;
-      const int s0 = lane < n ? (int)src[lane] : 0;
+      const unsigned short* src = L.l1_slots + (size_t)cell * kL1Cap;
+      const int s0 = lane < n ? (int)__ldg(&src[lane]) : 0;
       const float4 p0 = pts[s0];
       const int k0 = lane < n ? __float_as_int(p0.w) : 0x7fffffff;
       int r0 = 0;
       if (!two) {
         for (int c = 0; c < n; ++c) r0 += __shfl_sync(kFull, k0, c) < k0 ? 1 : 0;
       } else {
-        const int s1 = lane + 32 < n ? (int)src[lane + 32] : 0;
+        const int s1 = lane + 32 < n ? (int)__ldg(&src[lane + 32]) : 0;
         const float4 p1 = pts[s1];
         const int k1 = lane + 32 < n ? __float_as_int(p1.w) : 0x7fffffff;
         int r1 = 0;
@@ -1579,15 +1621,12 @@ __global__ void __launch_bounds__(256) cand_octant_kernel(const IndexHeader* __r
       const float4 ea = spt[ia ? lane : 0], eb = spt[ib ? lane + 32 : 0];
       const unsigned int oa = soff[ia ? lane : 0], ob = soff[ib ? lane + 32 : 0];
       const float ax = ea.x - ccx, ay = ea.y - ccy, az = ea.z - ccz, bx = eb.x - ccx, by = eb.y - ccy, bz = eb.z - ccz;
-      const float an = (ax * ax + ay * ay) + az * az, bn = (bx * bx + by * by) + bz * bz;
       bool la = ia, lb = ib;
       for (int c = 0; c < n; ++c) {
         const float4 pc = spt[c];
         const float cx = pc.x - ccx, cy = pc.y - ccy, cz = pc.z - ccz;
-        const float cn = (cx * cx + cy * cy) + cz * cz;
-        // min over the cube of |q-p|^2 - |q-c|^2: positive (beyond the rounding slack) = c is nearer everywhere
-        if ((an - cn) - 2.0f * (chh * ((fabsf(ax - cx) + fabsf(ay - cy)) + fabsf(az - cz))) > 1.0e-6f * (an + cn) + 1.0e-9f) la = false;
-        if (two && (bn - cn) - 2.0f * (chh * ((fabsf(bx - cx) + fabsf(by - cy)) + fabsf(bz - cz))) > 1.0e-6f * (bn + cn) + 1.0e-9f) lb = false;
+        if (cube_race(ax, ay, az, cx, cy, cz, chh).beaten()) la = false;  // c is nearer everywhere in the cell
+        if (two && cube_race(bx, by, bz, cx, cy, cz, chh).beaten()) lb = false;
       }
       const unsigned int ka = __ballot_sync(kFull, la), kb = __ballot_sync(kFull, lb);
       __syncwarp();
@@ -1597,9 +1636,9 @@ __global__ void __launch_bounds__(256) cand_octant_kernel(const IndexHeader* __r
       two = n > 32;
       __syncwarp();
     }
-    // records of octant o: word index of its first word (the octants form one dense lattice, x fastest)
-    auto rec_word = [&](int o) { return (((unsigned int)(2 * fz + (o >> 2)) * d2y + (unsigned int)(2 * fy + ((o >> 1) & 1))) * d2x + (unsigned int)(2 * fx + (o & 1))) * 8u; };
-    if (coarse || (light && n <= 7)) {
+    // word index of the first word of the record of octant o
+    auto rec_word = [&](int o) { return octant_record<unsigned int>(fx, fy, fz, o, d2x, d2y) * (unsigned int)kRecordWords; };
+    if (item.coarse || (item.light && n <= 7)) {
       // the cell's own list in every octant record: the cell has few queries (entries beyond the seventh in ONE run of pool
       // groups), or not many and the list fits one record anyway (a lookup evaluates seven slots whatever the length;
       // busy cells are still split: shorter lists mean fewer shared-memory wavefronts per lookup)
@@ -1607,19 +1646,19 @@ __global__ void __launch_bounds__(256) cand_octant_kernel(const IndexHeader* __r
       int pg = 0;
       if (n > 7) {
         const int need = (n - 7 + 7) >> 3;
-        if (lane == 0) pg = atomicAdd(&list_counters[3], need);
+        if (lane == 0) pg = atomicAdd(&L.counters->pool_groups, need);
         pg = __shfl_sync(kFull, pg, 0);
         if (pg + need > kPoolGroups) hw = kListOverflow;
         else {
           hw |= (unsigned int)pg << 8;
-          for (int t = 7 + lane; t < 7 + need * 8; t += 32) pool[(size_t)pg * 8 + (size_t)(t - 7)] = t < n ? soff[t] : dummy;
+          for (int t = 7 + lane; t < 7 + need * 8; t += 32) L.pool[(size_t)pg * 8 + (size_t)(t - 7)] = t < n ? soff[t] : dummy;
         }
       }
       // lane l: word (l & 7) of octants (l >> 3) and 4 + (l >> 3)
       const int w = lane & 7;
       const unsigned int val = w == 0 ? hw : ((hw != kListOverflow && w - 1 < n) ? soff[w - 1] : dummy);
-      flists[rec_word(lane >> 3) + (unsigned int)w] = val;
-      flists[rec_word(4 + (lane >> 3)) + (unsigned int)w] = val;
+      L.records[rec_word(lane >> 3) + (unsigned int)w] = val;
+      L.records[rec_word(4 + (lane >> 3)) + (unsigned int)w] = val;
       __syncwarp();
       continue;
     }
@@ -1678,26 +1717,26 @@ __global__ void __launch_bounds__(256) cand_octant_kernel(const IndexHeader* __r
       int pg = 0;
       if (cnt > 7) {  // (uniform within the group)
         const int need = (cnt - 7 + 7) >> 3;
-        if (e == 0) pg = atomicAdd(&list_counters[3], need);
+        if (e == 0) pg = atomicAdd(&L.counters->pool_groups, need);
         pg = __shfl_sync(gmask, pg, gbase);
         if (pg + need > kPoolGroups) hw = kListOverflow;
         else {
           hw |= (unsigned int)pg << 8;
           // pad the last group with the dummy slot (the lookup reads whole groups)
           const int tail = need * 8 - (cnt - 7);
-          if (e < tail) pool[(size_t)pg * 8 + (size_t)(cnt - 7 + e)] = dummy;
+          if (e < tail) L.pool[(size_t)pg * 8 + (size_t)(cnt - 7 + e)] = dummy;
         }
       }
       if (hw != kListOverflow) {
-        if (ka) { const int pos = __popc(ba & lt); if (pos < 7) srec[o * 8 + 1 + pos] = sa; else pool[(size_t)pg * 8 + (size_t)(pos - 7)] = sa; }
-        if (kb) { const int pos = __popc(ba) + __popc(bb & lt); if (pos < 7) srec[o * 8 + 1 + pos] = sb; else pool[(size_t)pg * 8 + (size_t)(pos - 7)] = sb; }
+        if (ka) { const int pos = __popc(ba & lt); if (pos < 7) srec[o * 8 + 1 + pos] = sa; else L.pool[(size_t)pg * 8 + (size_t)(pos - 7)] = sa; }
+        if (kb) { const int pos = __popc(ba) + __popc(bb & lt); if (pos < 7) srec[o * 8 + 1 + pos] = sb; else L.pool[(size_t)pg * 8 + (size_t)(pos - 7)] = sb; }
       }
       if (e == 0) srec[o * 8] = hw;
     }
     __syncwarp();
     // lane l: word (l & 7) of octant (l >> 3), then of octant 4 + (l >> 3)
-    flists[rec_word(lane >> 3) + (unsigned int)(lane & 7)] = srec[lane];
-    flists[rec_word(4 + (lane >> 3)) + (unsigned int)(lane & 7)] = srec[lane + 32];
+    L.records[rec_word(lane >> 3) + (unsigned int)(lane & 7)] = srec[lane];
+    L.records[rec_word(4 + (lane >> 3)) + (unsigned int)(lane & 7)] = srec[lane + 32];
     __syncwarp();
   }
   PFT_TRACE_MAX(1);
@@ -1705,11 +1744,7 @@ __global__ void __launch_bounds__(256) cand_octant_kernel(const IndexHeader* __r
 
 // second pass of the build: the cells queued by cand_build_kernel, one thread block each
 __global__ void __launch_bounds__(256) cand_build_far_kernel(const IndexHeader* __restrict__ hdr, const int* __restrict__ cs,
-                                                             const float4* __restrict__ pts, double max_d2,
-                                                             unsigned int* __restrict__ flists, unsigned int* __restrict__ xlists,
-                                                             int* __restrict__ list_counters, const int* __restrict__ far_list,
-                                                             const unsigned int* __restrict__ needed, int2* __restrict__ cell_items,
-                                                             unsigned short* __restrict__ l1_slots, unsigned int* __restrict__ built_bits) {
+                                                             const float4* __restrict__ pts, double max_d2, const __grid_constant__ CandLists L) {
   __shared__ IndexHeader h;
   __shared__ int s_cnt, s_xi;
   __shared__ int s_pref[34], s_start[32], s_ms[8];
@@ -1720,13 +1755,12 @@ __global__ void __launch_bounds__(256) cand_build_far_kernel(const IndexHeader* 
   if (threadIdx.x == 0) { h = *hdr; s_pref[32] = 0x7fffffff; }
   __syncthreads();
   if (!h.valid || !lists_on(h)) return;
-  const int n_far = list_counters[2];
+  const int n_far = L.counters->far_cells;
   const float leaf = 1.0f / h.inv_leaf;
-  const float margin = 1.0e-5f + 4.0e-6f * leaf * (float)(abs(h.f_origin[0]) + abs(h.f_origin[1]) + abs(h.f_origin[2]) + h.f_dim[0] + h.f_dim[1] + h.f_dim[2]);
-  const float r_max = max_d2 >= 1.0e30 ? 1.0e15f : (float)sqrt(max_d2) * 1.00001f;
+  const float margin = list_margin(h);
+  const float r_max = list_reach(max_d2);
   for (int idx = blockIdx.x; idx < n_far; idx += gridDim.x) {
-    build_cell_direct(h, cs, pts, far_list[idx], leaf, margin, r_max, flists, xlists, list_counters, s_pref, s_start, &s_cnt, s_m2, s_ms, &s_xi, s_list, s_pt4, s_key, s_key2,
-                      needed, cell_items, l1_slots, built_bits);
+    build_cell_direct(h, cs, pts, __ldg(&L.far_list[idx]), leaf, margin, r_max, L, s_pref, s_start, &s_cnt, s_m2, s_ms, &s_xi, s_list, s_pt4, s_key, s_key2);
     __syncthreads();
   }
   PFT_TRACE_MAX(2);
@@ -1740,9 +1774,9 @@ struct WeightArgs {
   const float4* pts2;         // {x, y, z, packed HSV} in cell order (what weight_lists_kernel stages)
   const unsigned int* hsv;    // packed HSV of every slot
   const RowEntry* table;      // kRows entries sorted by lb2
-  const unsigned int* flists;    // candidate lists (see cand_build_kernel): one record of 8 words per octant of the fine lattice
-  const unsigned int* pool;      // groups of eight entries for octant lists longer than seven
-  const unsigned int* xlists;    // extended lists (byte offsets, ascending input index, padded to a multiple of four)
+  const unsigned int* records;   // the three parts of the candidate lists the lookup reads (see CandLists)
+  const unsigned int* pool;
+  const unsigned int* xlists;
   const float4* model;        // {x,y,z,hsv} in tile order
   const int* model_perm;      // tile order -> order of the reference cloud as given
   int M;
@@ -1760,9 +1794,7 @@ template <bool USE_HSV, bool DYN, typename CS>
 __device__ __forceinline__ void weight_items(const WeightArgs& a, const IndexHeader& h, const CS* __restrict__ cs, const float4* __restrict__ pts,
                                              const unsigned int* __restrict__ hsv, const RowEntry* __restrict__ table, const float* __restrict__ lut_h,
                                              const float* __restrict__ lut_s) {
-  const int n = a.st->particle_num;
-  const int n_local = n > a.rank_id ? (n - a.rank_id + a.nranks - 1) / a.nranks : 0;
-  const int items = n_local * a.chunks;
+  const int items = rank_share(a.st->particle_num, a.rank_id, a.nranks) * a.chunks;
   const int lane = threadIdx.x & 31;
   // maximum_distance_^2 as the float just above it: every point with (double)d2 < max_d2 has d2 <= lim2
   const float lim2 = a.co.max_d2 >= 3.0e38 ? FLT_MAX : __double2float_ru(a.co.max_d2);
@@ -1957,9 +1989,7 @@ struct ListQuery { float x, y, z; unsigned int hsv; Rec8 r; };
 template <bool USE_HSV, bool DYN>
 __device__ __forceinline__ void weight_list_items(const WeightArgs& a, const IndexHeader& h, const unsigned char* __restrict__ sbase,
                                                   const float* __restrict__ lut_h, const float* __restrict__ lut_s) {
-  const int n = a.st->particle_num;
-  const int n_local = n > a.rank_id ? (n - a.rank_id + a.nranks - 1) / a.nranks : 0;
-  const int items = n_local * a.chunks;
+  const int items = rank_share(a.st->particle_num, a.rank_id, a.nranks) * a.chunks;
   const int lane = threadIdx.x & 31;
   // maximum_distance_^2 as the float just above it: (double)d2 < max_d2  <=>  d2 < lim2
   const float lim2 = a.co.max_d2 >= 3.0e38 ? FLT_MAX : __double2float_ru(a.co.max_d2);
@@ -2003,7 +2033,7 @@ __device__ __forceinline__ void weight_list_items(const WeightArgs& a, const Ind
       const int ix = __float2int_rd(q.x * inv2) - o2x, iy = __float2int_rd(q.y * inv2) - o2y, iz = __float2int_rd(q.z * inv2) - o2z;
       q.r.w[0] = kListOverflow;
       if ((unsigned int)ix < d2x && (unsigned int)iy < d2y && (unsigned int)iz < d2z)
-        q.r = load_rec8(a.flists + (size_t)(((unsigned int)iz * d2y + (unsigned int)iy) * d2x + (unsigned int)ix) * 8);
+        q.r = load_rec8(a.records + (size_t)octant_record<unsigned int>((unsigned int)ix, (unsigned int)iy, (unsigned int)iz, d2x, d2y) * kRecordWords);
       return q;
     };
     double val = 0.0;
@@ -2363,9 +2393,7 @@ __global__ void __launch_bounds__(256) weight_approx_kernel(const WeightApproxAr
   __shared__ OctHeaderD H;
   if (threadIdx.x == 0) H = *a.oct;
   __syncthreads();
-  const int n = a.st->particle_num;
-  const int n_local = n > a.rank_id ? (n - a.rank_id + a.nranks - 1) / a.nranks : 0;
-  const int items = n_local * a.chunks;
+  const int items = rank_share(a.st->particle_num, a.rank_id, a.nranks) * a.chunks;
   const int lane = threadIdx.x & 31;
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
   for (int item = warp; item < items; item += nwarps) {
